@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the driver-facing benchmark of the bmSparse hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--budget-s S]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--budget-s S] [--dump-outputs DIR]
 
 Headline (BASELINE.json configs[1]): bmSparse SpMV, fp16 values / fp32 x, y / fp32 accumulate, synthetic
 2-D Poisson 4096x4096 grid (16.7M rows, 83.9M nnz) -- metric "SpMV HBM GB/s" = algorithmic bytes of the
@@ -23,6 +23,13 @@ skipped and say so):
 
 --impl reference times the reference's own CPU path (cusp host CSR kernels compiled from the reference tree
 into oracle/_ref; the oracle port if that library is missing) on the same workload, on every host core.
+
+--dump-outputs DIR writes what the timed path computed in its last step (y of the last SpMV) as DIR/spmv_y.npy, float32
+(DIR/spmv_y_rank<r>.npy at N > 1), at most 64 MB in all: an output larger than that is written as a sample at fixed, seeded
+positions.  The inputs are the same in every run with the same arguments, so the files of two builds compare element for element.
+The JSON line counts the non-finite elements of each file.  At N = 1 every step is y = A x with the same x.  At N > 1 a step is
+x <- A x: the 5-point operator's largest eigenvalue is close to 8, so y overflows to inf / NaN after about 40 products, and the
+dumps only say something while warmup + steps stays below that.  .gitignore ignores *.npy outside tests/golden/.
 """
 from __future__ import annotations
 
@@ -44,6 +51,30 @@ GRID = 4096
 _OUT = sys.stdout
 SPGEMM_N, SPGEMM_K = 1_000_000, 16
 T_START = time.perf_counter()
+DUMP_BYTES = 64 * 10**6      # --dump-outputs writes at most this much in all (shared by the ranks)
+DUMP_SAMPLE = 1 << 22        # elements kept of an output too large to write whole
+
+
+def dump_outputs(d, outputs, rank, world):
+    """Write each output (a tensor or array) as d/<name>.npy in float32 / float64.  One that does not fit its share of DUMP_BYTES
+    is written as DUMP_SAMPLE elements at positions drawn with a fixed seed: the same positions in every run.  Returns what was
+    written, for the JSON line."""
+    os.makedirs(d, exist_ok=True)
+    share = DUMP_BYTES // (world * len(outputs))
+    written = {}
+    for name, t in outputs.items():
+        a = (t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)).ravel()
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)
+        total = a.size
+        if a.nbytes > share:
+            n = min(DUMP_SAMPLE, share // a.itemsize)
+            a = a[np.sort(np.random.default_rng(0).choice(total, n, replace=False))]
+        fname = f"{name}_rank{rank}.npy" if world > 1 else f"{name}.npy"
+        np.save(os.path.join(d, fname), a)
+        written[fname] = {"elements": int(a.size), "of": int(total), "sampled": a.size < total, "dtype": str(a.dtype),
+                          "nonfinite": int(a.size - np.count_nonzero(np.isfinite(a)))}
+    return written
 
 
 def peaks():
@@ -179,7 +210,7 @@ def reference_arm(args):
     nr, nc, rp, ci, v = G.poisson5pt(GRID, GRID)
     x = G.x_vector(nc)
     nblk_bytes = 444452864
-    steps = max(1, min(args.steps, 20 if world == 1 else 10))
+    steps = args.steps
     O.use_all_cores()
     for _ in range(max(args.warmup, 1)):
         O.ref_csr_spmv(nr, nc, rp, ci, v, x, omp=True) if O.ref_lib() is not None else O.csr_spmv(rp, ci, v, x, threads=O.max_threads())
@@ -354,7 +385,9 @@ def convert_section(B, torch, nr, nc, rp, ci, v, peak):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200,
+                    help="timed steps; --impl reference runs each of them once per CPU back-end (sequential, then OpenMP) and per slab, "
+                         "and --budget-s does not bound it")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--no-spgemm", action="store_true")
@@ -362,7 +395,13 @@ def main():
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--budget-s", type=float, default=float(os.environ.get("BMSP_BENCH_BUDGET_S", "300")),
                     help="wall-clock budget of the whole run; optional sections (spgemm comparisons, strong scaling) that would start after it are skipped")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write y of the last timed SpMV to DIR/spmv_y.npy (float32; a fixed, seeded sample when larger than 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path; --impl reference computes y on the host and does not dump it")
     args.warmup = max(args.warmup, 3)
     # native libraries (NCCL's version banner) print to fd 1: keep the real stdout for the one JSON line only
     global _OUT
@@ -446,6 +485,8 @@ def main():
         ms_total = float(t.item())
     ms_step = ms_total / K
     clocks = sampler.summary(t_start, t_end)
+    # ---- the last timed step's product, before anything below reuses its buffers
+    dumped = dump_outputs(args.dump_outputs, {"spmv_y": y if world == 1 else sharded.y_own()}, rank, world) if args.dump_outputs else None
 
     # ---- kernel-only duration of the dominant kernel (same stream, CUDA events, x resident): N = 1 uses the step itself
     kern_ms = ms_step
@@ -522,6 +563,8 @@ def main():
     }
     if not verified:
         line["verification_failed_on_rank"] = rank if not ok_local else "another rank"
+    if dumped is not None:
+        line["dump_outputs"] = {"dir": os.path.abspath(args.dump_outputs), "files": dumped}
 
     skipped = {}
     O = None

@@ -7,10 +7,17 @@
   * BC4M (full size) and R-MAT-16: conversion, SpMV and A*A against the oracle's OpenMP variants (oracle/bmsp_oracle.c;
     pinned to the scalar, reference-following functions in tests/test_oracle_golden.py): structure bit-exact, values within
     1e-3 * sum |a||b| (fp16 inputs, fp32 accumulation vs the oracle's double sums).
+  * U1M / BC4M / P4096 A*A without the reference's build: the same SHA-256 digests and values at 4096 fixed positions, stored
+    under tests/golden/ by tests/golden/make_fullsize_golden.py from the oracle's OpenMP product (whose C counts equal the
+    reference's on these inputs).
 """
+import os
+
 import numpy as np
 import pytest
 import torch
+
+from tests.util import GOLDEN, load_golden
 
 pytestmark = pytest.mark.gpu
 
@@ -84,6 +91,30 @@ def test_spgemm_full_size_vs_reference_cuda(B, oracle, refbin, tmp_path, name):
         ours = vals[v0:v0 + nv].astype(np.float64)
         bound = 1.5e-3 * mag[v0:v0 + nv].cpu().numpy().astype(np.float64) + 1e-6
         assert np.all(np.abs(ours - w["values"].astype(np.float64)) <= bound), f"{name}: values differ beyond the fp16-product tolerance"
+
+
+@pytest.mark.parametrize("name", ["p4096", "u1m", "bc4m"])
+def test_spgemm_full_size_vs_stored_digests(B, oracle, name):
+    """the products of test_spgemm_full_size_vs_reference_cuda against tests/golden/fullsize_spgemm.json and
+    fullsize_spgemm_samples.npz: C.keys / C.bmps / C.offsets bit for bit through the SHA-256 of the complete arrays, values at 4096
+    fixed positions within 1e-3 * sum |a||b| (fp16 inputs, fp32 accumulation vs the oracle's double sums)"""
+    O = oracle
+    rec = load_golden("fullsize_spgemm.json")["configs"][name]
+    smp = np.load(os.path.join(GOLDEN, "fullsize_spgemm_samples.npz"))
+    nr, nc, rp, ci, v = _gen(B, name)
+    A = B.bmSpMatrix.from_csr(nr, nc, rp, ci, v); Bt = B.bmSpMatrix.from_csr(nr, nc, rp, ci, v, transpose=True)
+    del rp, ci, v
+    C, info = B.bmSparse_mult(A, Bt)
+    assert (C.block_num, C.nnz) == (rec["c_blocks"], rec["c_nnz"])
+    k, b, o, vals = C.download()
+    assert o.size == rec["offsets_len"]
+    assert O.sha256_u64(k) == rec["sha256"]["keys"], "C.keys differ from the stored digest"
+    assert O.sha256_u64(b) == rec["sha256"]["bmps"], "C.bmps differ from the stored digest"
+    assert O.sha256_u64(o) == rec["sha256"]["offsets"], "C.offsets differ from the stored digest"
+    del k, b, o
+    pos = smp[f"{name}_pos"]
+    err = np.abs(vals[pos].astype(np.float64) - smp[f"{name}_values"])
+    assert np.all(err <= 1e-3 * smp[f"{name}_mag"] + 1e-30), f"{name}: max err/mag {float(np.max(err / np.maximum(smp[f'{name}_mag'], 1e-30)))}"
 
 
 @pytest.mark.parametrize("name", ["rmat16", "bc4m"])

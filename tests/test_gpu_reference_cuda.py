@@ -94,3 +94,44 @@ def test_b200_kernels_match_reference_cuda(oracle, refbin, tmp_path):
         k, b, o, vals = C.download()
         assert np.array_equal(k, ref.keys) and np.array_equal(b, ref.bmps[:k.size]) and np.array_equal(o, ref.offsets[:k.size + 1])
         assert np.array_equal(vals, ref.values)      # integer-valued stencil: exact on both sides
+
+
+def test_b200_kernels_match_stored_reference_outputs(oracle):
+    """our CUDA path without the reference's build, on both numeric paths:
+      * the reference's own outputs recorded in tests/golden/ref_cuda_golden.json: block and nonzero counts and the XOR of
+        keys and bitmaps exact, the value sum within the fp16-product tolerance; the fp32 SpMV sums exact;
+      * the 96 x 96 stencil of test_b200_kernels_match_reference_cuda: the SHA-256 of all four C arrays (integer values: exact),
+        stored in tests/golden/fullsize_spgemm.json by tests/golden/make_fullsize_golden.py from the oracle."""
+    import hashlib
+    import torch
+    import bmsparse_spgemm_spmv_b200 as B
+    O = oracle
+    rec = load_golden("ref_cuda_golden.json")["cases"]
+    g = load_golden("ragusa16.json")
+    rp, ci, v = random_csr(256, 256, 0.06, seed=77)
+    _, _, prp, pci, pv = B.generators.poisson5pt(64, 64)
+    mats = {"ragusa16_AxB": (B.bmSpMatrix.from_coo(24, 24, g["A"]["rows"], g["A"]["cols"], g["A"]["vals"]),
+                             B.bmSpMatrix.from_coo(24, 24, g["B"]["rows"], g["B"]["cols"], g["B"]["vals"], transpose=True)),
+            "poisson64_AxA": (B.bmSpMatrix.from_csr(4096, 4096, prp, pci, pv), B.bmSpMatrix.from_csr(4096, 4096, prp, pci, pv, transpose=True)),
+            "random256_AxA": (B.bmSpMatrix.from_csr(256, 256, rp, ci, v), B.bmSpMatrix.from_csr(256, 256, rp, ci, v, transpose=True))}
+    for name, (A, Bt) in mats.items():
+        r = rec[name]
+        for path in (0, 1):
+            C, _ = B.bmSparse_mult(A, Bt, numeric_path=path)
+            k, b, o, vals = C.download()
+            assert (C.block_num, C.nnz, int(o[-1])) == (r["C_blocks"], r["C_nnz"], r["offsets_last"]), (name, path)
+            assert int(np.bitwise_xor.reduce(k)) == r["keys_crc"] and int(np.bitwise_xor.reduce(b)) == r["bmps_crc"], (name, path)
+            vals = vals.astype(np.float64)
+            assert abs(float(vals.sum()) - r["values_sum"]) <= 2e-3 * float(np.abs(vals).sum()) + 1e-6, (name, path)
+    A32 = B.bmSpMatrix.from_csr(4096, 4096, prp, pci, pv, dtype=torch.float32)
+    y = B.bmSparse_SpMV(A32, torch.ones(4096, dtype=torch.float32, device="cuda")).cpu().numpy().astype(np.float64)
+    assert float(y.sum()) == rec["poisson64_spmv_ones"]["y_sum"] and float(np.abs(y).sum()) == rec["poisson64_spmv_ones"]["y_abs_sum"]
+    s96 = load_golden("fullsize_spgemm.json")["poisson96_AxA"]
+    nr, nc, rp, ci, v = B.generators.poisson5pt(96, 96)
+    A = B.bmSpMatrix.from_csr(nr, nc, rp, ci, v); Bt = B.bmSpMatrix.from_csr(nr, nc, rp, ci, v, transpose=True)
+    for path in (0, 1):
+        C, _ = B.bmSparse_mult(A, Bt, numeric_path=path)
+        k, b, o, vals = C.download()
+        assert (C.block_num, C.nnz) == (s96["c_blocks"], s96["c_nnz"]), path
+        assert (O.sha256_u64(k), O.sha256_u64(b), O.sha256_u64(o)) == (s96["sha256"]["keys"], s96["sha256"]["bmps"], s96["sha256"]["offsets"]), path
+        assert hashlib.sha256(np.ascontiguousarray(vals, np.float32).tobytes()).hexdigest() == s96["sha256"]["values_f32"], path
