@@ -47,6 +47,12 @@ struct bmsp_matrix_s {
     void* tile_desc = nullptr;  // [ntiles] TileDesc (spmv.cu): block / value / x-line ranges of every tile of 64 block rows
     uint32_t* tile_lines = nullptr;   // [nblk] distinct x lines (32 columns) of every tile, stored from the tile's first block index
     uint16_t* tile_xoff = nullptr;    // [nblk] per block: element offset of its 8-column x segment inside the tile's staged lines
+    // streaming kernel, matrices with at most PALETTE_MAX distinct bitmaps (stencils, bands): the bitmaps are replaced by a palette
+    // and tile_xoff / tile_rowpair by the two arrays below (spmv.cu, "bitmap palette").  spmv_npal == 0: today's arrays are used.
+    int32_t spmv_npal = 0;            // palette entries (distinct bitmaps), 0 = no palette
+    void* tile_palette = nullptr;     // [spmv_npal] 16-byte entries, sorted by bitmap
+    uint32_t* tile_word = nullptr;    // [nblk] per block: x offset (bits 0-15) | palette entry byte offset (bits 16-31)
+    uint32_t* tile_rowrel = nullptr;  // [nbr] per block row: (first block - tile's first block) | (first value - tile's first value) << 16
     int32_t* work = nullptr;    // block-parallel work items (int4 per item)
     int32_t n_work = 0, n_split = 0;
     float* split_partial = nullptr;

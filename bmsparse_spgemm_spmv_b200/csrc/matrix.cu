@@ -263,6 +263,7 @@ int bmsp_destroy(bmsp_matrix_t m) {
     dev_free(m->work, st); dev_free(m->split_partial, st); dev_free(m->split_rows, st); dev_free(m->split_list, st); dev_free(m->pmeta, st);
     dev_free(m->halo_tiles, st); dev_free(m->fine_ptr, st); dev_free(m->fine_bcol, st); dev_free(m->fine_kmask, st); dev_free(m->fine_rec, st);
     dev_free(m->tile_desc, st); dev_free(m->spmv_sched, st); dev_free(m->tile_rowpair, st); dev_free(m->tile_lines, st); dev_free(m->tile_xoff, st);
+    dev_free(m->tile_palette, st); dev_free(m->tile_word, st); dev_free(m->tile_rowrel, st);
     delete m;
     return BMSP_OK;
 }

@@ -114,17 +114,89 @@ constexpr int XL_MAX = 1900;       // distinct lines per tile (16-bit element of
 struct __align__(16) TileDesc { int32_t p0, nb; uint32_t v0; int32_t nv, nl, flags, lmin, lmax; int32_t nruns; uint32_t run_line[3], run_count[3]; int32_t pad; };
 static_assert(sizeof(TileDesc) == 64, "TileDesc is four 16-byte words");
 
+// ---- bitmap palette (streaming kernel) ----
+// A stencil or banded matrix has a handful of distinct bitmaps among millions of blocks (P4096: 4).  When a matrix has at most
+// PALETTE_MAX of them, the streaming kernel does not stream bitmaps (8 B per block), x offsets (2 B) and row pointers (8 B per block
+// row): it streams one 32-bit word per block -- the x offset and the byte offset of the block's palette entry -- and one u16 pair
+// per block row relative to its tile, and keeps the palette in shared memory.  An entry holds, per 32-bit bitmap half (rows 4h ..
+// 4h+3), the half itself and what the consumer would otherwise derive from it for every block: the value offsets and the shape.
+constexpr int PALETTE_MAX = 256;
+constexpr int PAL_SLOTS = 1024, PAL_GSLOTS = 2048;   // open-addressing tables: per CTA (shared) and per matrix (global)
+// entry = {half 0 bits, half 0 meta, half 1 bits, half 1 meta}; meta = value offset of the half * sizeof(T) (bits 0-7) | shape, one bit
+// each (bits 8-11, none: empty half) | PAL_SINGLE: 8 * row + column of the cell (bits 12-16) | values of the block * sizeof(T) (bits 20-31).
+// One-hot shapes are tested one bit at a time; a small integer would be compiled into an indirect jump.
+enum : uint32_t { PAL_DIAG = 1u << 8, PAL_TRI = 1u << 9, PAL_SINGLE = 1u << 10, PAL_GENERIC = 1u << 11 };
+struct PalScan { unsigned long long key[PAL_GSLOTS]; uint32_t count, has_zero, overflow, pad; };
+
+__device__ __forceinline__ uint32_t pal_hash(uint64_t b, int bits) { return (uint32_t)((b * 0x9E3779B97F4A7C15ull) >> (64 - bits)); }
+// insert the non-zero bitmap b: 1 = inserted, 0 = already present, -1 = table full
+__device__ __forceinline__ int pal_insert(unsigned long long* tab, int bits, uint64_t b) {
+    const uint32_t mask = (1u << bits) - 1u;
+    uint32_t i = pal_hash(b, bits);
+    for (uint32_t n = 0; n <= mask; n++, i = (i + 1u) & mask) {
+        unsigned long long cur = *reinterpret_cast<volatile unsigned long long*>(tab + i);
+        if (cur == b) return 0;
+        if (cur == 0ull) {
+            cur = atomicCAS(tab + i, 0ull, (unsigned long long)b);
+            if (cur == 0ull) return 1;
+            if (cur == b) return 0;
+        }
+    }
+    return -1;
+}
+
+// One pass over the bitmaps: every CTA collects its distinct bitmaps in shared memory, then merges them into the global table.  Gives up
+// (overflow) as soon as any table holds more than PALETTE_MAX; the order of the table is irrelevant (the host sorts the bitmaps).
+__global__ void __launch_bounds__(256) palette_scan_kernel(const uint64_t* __restrict__ bmps, int64_t nblk, PalScan* __restrict__ ps) {
+    __shared__ unsigned long long s_tab[PAL_SLOTS];
+    __shared__ uint32_t s_cnt, s_zero, s_over;
+    const int tid = threadIdx.x;
+    for (int i = tid; i < PAL_SLOTS; i += 256) s_tab[i] = 0ull;
+    if (tid == 0) { s_cnt = 0; s_zero = 0; s_over = 0; }
+    __syncthreads();
+    // a thread inserts at most one bitmap between two looks at the count: the table never holds more than PALETTE_MAX + 256 < PAL_SLOTS
+    uint32_t it = 0;
+    for (int64_t i = (int64_t)blockIdx.x * 256 + tid; i < nblk; i += (int64_t)gridDim.x * 256, it++) {
+        if (*reinterpret_cast<volatile uint32_t*>(&s_cnt) > (uint32_t)PALETTE_MAX) break;
+        if ((it & 15u) == 0 && *reinterpret_cast<volatile uint32_t*>(&ps->overflow)) break;
+        const uint64_t b = ld_stream_u64(bmps + i);
+        if (b == 0ull) { s_zero = 1; continue; }
+        const int r = pal_insert(s_tab, 10, b);
+        if (r > 0) atomicAdd(&s_cnt, 1u);
+        else if (r < 0) { s_over = 1; break; }
+    }
+    __syncthreads();
+    if (s_over || s_cnt > (uint32_t)PALETTE_MAX) { if (tid == 0) atomicExch(&ps->overflow, 1u); return; }
+    if (tid == 0 && s_zero) ps->has_zero = 1;
+    for (int j = tid; j < PAL_SLOTS; j += 256) {
+        const uint64_t b = s_tab[j];
+        if (b == 0ull) continue;
+        if (*reinterpret_cast<volatile uint32_t*>(&ps->overflow)) break;
+        const int r = pal_insert(ps->key, 11, b);
+        if (r < 0 || (r > 0 && atomicAdd(&ps->count, 1u) >= (uint32_t)PALETTE_MAX)) { atomicExch(&ps->overflow, 1u); break; }
+    }
+}
+
+// pal / npal: the sorted palette (streaming kernel with a palette: per block `word`, per block row `rowrel`; otherwise `xoff`)
 __global__ void __launch_bounds__(256) tile_plan_kernel(const int32_t* __restrict__ brp, const int32_t* __restrict__ bcol,
                                                         const uint32_t* __restrict__ rvb, int nbr, int ncols, int rt, int pitch, TileDesc* __restrict__ desc,
                                                         uint32_t* __restrict__ lines, uint16_t* __restrict__ xoff,
-                                                        unsigned long long* __restrict__ stats) {
+                                                        unsigned long long* __restrict__ stats, const uint64_t* __restrict__ bmps,
+                                                        const uint4* __restrict__ pal, int npal, uint32_t* __restrict__ word,
+                                                        uint32_t* __restrict__ rowrel) {
     __shared__ uint32_t s_key[PLAN_MAXB];
     __shared__ uint32_t s_uniq[PLAN_MAXB];
     __shared__ uint32_t s_w[9];
+    __shared__ uint64_t s_pal[PALETTE_MAX];
     const int t = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const int r0 = t * rt, r1 = min(r0 + rt, nbr);
     const int p0 = brp[r0], nb = brp[r1] - p0;
     const uint32_t v0 = rvb[r0], v1 = rvb[r1];
+    if (word) {
+        // tile-relative row pairs: read for staged tiles only, whose block and value counts are far below 65536 (shared memory)
+        for (int r = r0 + tid; r < r1; r += 256) rowrel[r] = (uint32_t)(brp[r] - p0) | ((rvb[r] - v0) << 16);
+        for (int i = tid; i < npal; i += 256) s_pal[i] = (uint64_t)pal[i].x << 32 | pal[i].z;
+    }
     TileDesc d;
     d.p0 = p0; d.nb = nb; d.v0 = v0; d.nv = (int32_t)(v1 - v0); d.nl = 0; d.flags = 0; d.lmin = 0; d.lmax = nb > 0 ? 0x7FFFFFFF : -1;
     d.nruns = 0; d.pad = 0;
@@ -182,7 +254,18 @@ __global__ void __launch_bounds__(256) tile_plan_kernel(const int32_t* __restric
                 const int mid = (lo + hi) >> 1;
                 if (s_uniq[mid] < line) lo = mid + 1; else hi = mid;
             }
-            xoff[p0 + i] = (uint16_t)(lo * pitch + (int)(c & 3u) * 8);
+            const uint32_t xo = (uint32_t)(lo * pitch + (int)(c & 3u) * 8);
+            if (word) {
+                const uint64_t b = bmps[p0 + i];
+                int pl = 0, ph = npal;
+                while (pl < ph) {
+                    const int mid = (pl + ph) >> 1;
+                    if (s_pal[mid] < b) pl = mid + 1; else ph = mid;
+                }
+                word[p0 + i] = xo | (uint32_t)pl << 20;              // entry byte offset (16 * code) in bits 16-31
+            } else {
+                xoff[p0 + i] = (uint16_t)xo;
+            }
         }
     if (tid == 0) {
         // flags: bit 0 = planned (x offsets valid), bit 1 = the last line reaches past the last column (guarded gather)
@@ -221,6 +304,8 @@ template <typename T>
 struct TileArgs {
     const uint64_t* bmps; const int32_t* bcol; const T* values; const int2* rowpair;   // rowpair[r] = (block_row_ptr[r], first value of row r)
     const TileDesc* desc; const uint32_t* lines; const uint16_t* xoff;
+    const uint32_t* word; const uint32_t* rowrel; const uint4* palette; int32_t npal;   // streaming kernel with a palette (tile_plan_kernel)
+    const int32_t* brp; const uint32_t* rvb;                                             // ... whose unstaged tiles read their row pointers here
     int32_t rows, nbr, cols, cap_blk, cap_val, cap_lines;
     int32_t tile0;       // first tile of this launch (row-range launches of the host-buffer pipeline)
     const int32_t* tile_list;   // streaming kernel: when set, the launch's q-th tile is tile_list[q] (boundary / interior launches of the multi-GPU product)
@@ -321,11 +406,78 @@ template <> __device__ __forceinline__ void lds_x4<__half>(uint32_t a, float (&o
     o[0] = f0.x; o[1] = f0.y; o[2] = f1.x; o[3] = f1.y;
 }
 
+// The four shapes of one bitmap half, each on its half's values from va0 on and its 8-column x segment at element offset xo of the
+// staged lines (xs31 = staged x + 31 elements).
 // XV: the staged x lines are dense (pitch 32) and 16-byte aligned, so the four x elements of a bitmap half are one vector load
+template <typename T, typename X, bool XV>
+__device__ __forceinline__ void half_diag(uint32_t va0, uint32_t xo, const int h, const uint32_t xs31, float (&acc)[4]) {
+    // diagonal block (the +-m neighbours of a stencil, any band at a multiple of 8): row i of the half holds exactly
+    // column 4h + i -- four straight multiply-adds, no bit walk (20 instructions instead of ~50)
+    constexpr uint32_t SV = sizeof(T), SX = sizeof(X);
+    const uint32_t xa = xs31 - 31u * SX + (xo + 4u * (uint32_t)h) * SX;
+    float x4[4];
+    if constexpr (XV) lds_x4<X>(xa, x4);
+    else {
+#pragma unroll
+        for (int i = 0; i < 4; i++) x4[i] = lds_as_f32<X>(xa + i * SX);
+    }
+#pragma unroll
+    for (int i = 0; i < 4; i++) acc[i] = fmaf(lds_as_f32<T>(va0 + i * SV), x4[i], acc[i]);
+}
+template <typename T, typename X, bool XV>
+__device__ __forceinline__ void half_tri(uint32_t va0, uint32_t xo, const int h, const uint32_t xs31, float (&acc)[4]) {
+    // tridiagonal block (the diagonal block of a stencil, any 3-wide band): row i of the half holds columns
+    // 4h+i-1 .. 4h+i+1, clipped to the block -- 11 values.  Written as 12 slots (3 per row) over the six x elements
+    // 4h-1 .. 4h+4 so that the code does not depend on h: slot 0 of the upper half (column -1) and slot 11 of the
+    // lower half (column 8) do not exist and are predicated off (their loads stay inside the staged tile).
+    constexpr uint32_t SV = sizeof(T), SX = sizeof(X);
+    const uint32_t vb = va0 + ((uint32_t)h - 1u) * SV;                       // slot s at vb + s * SV
+    const uint32_t xa = xs31 - 31u * SX + (xo + 4u * (uint32_t)h - 1u) * SX;   // x[4h-1+j] at xa + j * SX
+    float xl[6], v[12];
+    if constexpr (XV) {
+        float x4[4];
+        lds_x4<X>(xa + SX, x4);
+        xl[0] = lds_as_f32<X>(xa); xl[1] = x4[0]; xl[2] = x4[1]; xl[3] = x4[2]; xl[4] = x4[3]; xl[5] = lds_as_f32<X>(xa + 5 * SX);
+    } else {
+#pragma unroll
+        for (int j = 0; j < 6; j++) xl[j] = lds_as_f32<X>(xa + j * SX);
+    }
+#pragma unroll
+    for (int s = 0; s < 12; s++) v[s] = lds_as_f32<T>(vb + s * SV);
+    if (h) acc[0] = fmaf(v[0], xl[0], acc[0]);
+    acc[0] = fmaf(v[1], xl[1], acc[0]); acc[0] = fmaf(v[2], xl[2], acc[0]);
+    acc[1] = fmaf(v[3], xl[1], acc[1]); acc[1] = fmaf(v[4], xl[2], acc[1]); acc[1] = fmaf(v[5], xl[3], acc[1]);
+    acc[2] = fmaf(v[6], xl[2], acc[2]); acc[2] = fmaf(v[7], xl[3], acc[2]); acc[2] = fmaf(v[8], xl[4], acc[2]);
+    acc[3] = fmaf(v[9], xl[3], acc[3]); acc[3] = fmaf(v[10], xl[4], acc[3]);
+    if (!h) acc[3] = fmaf(v[11], xl[5], acc[3]);
+}
+template <typename T, typename X>
+__device__ __forceinline__ void half_single(uint32_t va0, uint32_t xo, const uint32_t t, const uint32_t xs31, float (&acc)[4]) {
+    // one value in this half, cell t = 8 * row + column (the +-1 neighbours of a stencil: a single cell in the whole block): one
+    // product, added to the row it belongs to
+    constexpr uint32_t SX = sizeof(X);
+    const float prod = lds_as_f32<T>(va0) * lds_as_f32<X>(xs31 - 31u * SX + (xo + (t & 7u)) * SX);
+    const uint32_t rr = t >> 3;
+    acc[0] += rr == 0u ? prod : 0.f; acc[1] += rr == 1u ? prod : 0.f;
+    acc[2] += rr == 2u ? prod : 0.f; acc[3] += rr == 3u ? prod : 0.f;
+}
+template <typename T, typename X>
+__device__ __forceinline__ void half_generic(uint32_t w, uint32_t va0, uint32_t xo, const uint32_t xs31, float (&acc)[4]) {
+    constexpr uint32_t SV = sizeof(T), SX = sizeof(X);
+    const uint32_t xb = xs31 + xo * SX;
+    const uint32_t b0 = w & 0xFF000000u, b1 = w & 0x00FF0000u, b2 = w & 0x0000FF00u, b3 = w & 0x000000FFu;
+    const uint32_t va1 = va0 + __popc(b0) * SV, va2 = va1 + __popc(b1) * SV, va3 = va2 + __popc(b2) * SV;
+    RowPair<T, X, 0>::run(acc[0], acc[1], b0, b1, va0, va1, xb);
+    RowPair<T, X, 1>::run(acc[2], acc[3], b2, b3, va2, va3, xb);
+}
+
+// The blocks of one block row seen by the thread that owns bitmap half h (rows 4h..4h+3).  Everything lives in
+// shared memory: bitmaps at a_bm, 16-bit x offsets at a_xo, the row's values from a_v on; xs31 = staged x + 31
+// elements.
 template <typename T, typename X, bool XV = false>
 __device__ __forceinline__ void tile_half_row(uint32_t a_bm, uint32_t a_xo, uint32_t a_v, int nb, const int h, const uint32_t xs31,
                                               float (&acc)[4]) {
-    constexpr uint32_t SV = sizeof(T), SX = sizeof(X);
+    constexpr uint32_t SV = sizeof(T);
     const uint32_t hm = 0u - (uint32_t)h;
 #pragma unroll 1
     for (int i = 0; i < nb; i++) {
@@ -336,57 +488,31 @@ __device__ __forceinline__ void tile_half_row(uint32_t a_bm, uint32_t a_xo, uint
         const uint32_t w = (w2.x & hm) | (w2.y & ~hm);
         const uint32_t va0 = a_v + (nhi & hm) * SV;
         a_v += (nhi + nlo) * SV;
-        if (w == (0x80402010u >> (4 * h))) {
-            // diagonal block (the +-m neighbours of a stencil, any band at a multiple of 8): row i of the half holds exactly
-            // column 4h + i -- four straight multiply-adds, no bit walk (20 instructions instead of ~50)
-            const uint32_t xa = xs31 - 31u * SX + (xo + 4u * (uint32_t)h) * SX;
-            float x4[4];
-            if constexpr (XV) lds_x4<X>(xa, x4);
-            else {
-#pragma unroll
-                for (int i = 0; i < 4; i++) x4[i] = lds_as_f32<X>(xa + i * SX);
-            }
-#pragma unroll
-            for (int i = 0; i < 4; i++) acc[i] = fmaf(lds_as_f32<T>(va0 + i * SV), x4[i], acc[i]);
-        } else if (w == (h ? 0x1C0E0703u : 0xC0E07038u)) {
-            // tridiagonal block (the diagonal block of a stencil, any 3-wide band): row i of the half holds columns
-            // 4h+i-1 .. 4h+i+1, clipped to the block -- 11 values.  Written as 12 slots (3 per row) over the six x elements
-            // 4h-1 .. 4h+4 so that the code does not depend on h: slot 0 of the upper half (column -1) and slot 11 of the
-            // lower half (column 8) do not exist and are predicated off (their loads stay inside the staged tile).
-            const uint32_t vb = va0 + ((uint32_t)h - 1u) * SV;                       // slot s at vb + s * SV
-            const uint32_t xa = xs31 - 31u * SX + (xo + 4u * (uint32_t)h - 1u) * SX;   // x[4h-1+j] at xa + j * SX
-            float xl[6], v[12];
-            if constexpr (XV) {
-                float x4[4];
-                lds_x4<X>(xa + SX, x4);
-                xl[0] = lds_as_f32<X>(xa); xl[1] = x4[0]; xl[2] = x4[1]; xl[3] = x4[2]; xl[4] = x4[3]; xl[5] = lds_as_f32<X>(xa + 5 * SX);
-            } else {
-#pragma unroll
-                for (int j = 0; j < 6; j++) xl[j] = lds_as_f32<X>(xa + j * SX);
-            }
-#pragma unroll
-            for (int s = 0; s < 12; s++) v[s] = lds_as_f32<T>(vb + s * SV);
-            if (h) acc[0] = fmaf(v[0], xl[0], acc[0]);
-            acc[0] = fmaf(v[1], xl[1], acc[0]); acc[0] = fmaf(v[2], xl[2], acc[0]);
-            acc[1] = fmaf(v[3], xl[1], acc[1]); acc[1] = fmaf(v[4], xl[2], acc[1]); acc[1] = fmaf(v[5], xl[3], acc[1]);
-            acc[2] = fmaf(v[6], xl[2], acc[2]); acc[2] = fmaf(v[7], xl[3], acc[2]); acc[2] = fmaf(v[8], xl[4], acc[2]);
-            acc[3] = fmaf(v[9], xl[3], acc[3]); acc[3] = fmaf(v[10], xl[4], acc[3]);
-            if (!h) acc[3] = fmaf(v[11], xl[5], acc[3]);
-        } else if (w && !(w & (w - 1u))) {
-            // one value in this half (the +-1 neighbours of a stencil: a single cell in the whole block): one product, added to
-            // the row it belongs to
-            const uint32_t t = 31u - (uint32_t)(31 - __clz((int)w));          // = 8 * row + column
-            const float prod = lds_as_f32<T>(va0) * lds_as_f32<X>(xs31 - 31u * SX + (xo + (t & 7u)) * SX);
-            const uint32_t rr = t >> 3;
-            acc[0] += rr == 0u ? prod : 0.f; acc[1] += rr == 1u ? prod : 0.f;
-            acc[2] += rr == 2u ? prod : 0.f; acc[3] += rr == 3u ? prod : 0.f;
-        } else if (w) {
-            const uint32_t xb = xs31 + xo * SX;
-            const uint32_t b0 = w & 0xFF000000u, b1 = w & 0x00FF0000u, b2 = w & 0x0000FF00u, b3 = w & 0x000000FFu;
-            const uint32_t va1 = va0 + __popc(b0) * SV, va2 = va1 + __popc(b1) * SV, va3 = va2 + __popc(b2) * SV;
-            RowPair<T, X, 0>::run(acc[0], acc[1], b0, b1, va0, va1, xb);
-            RowPair<T, X, 1>::run(acc[2], acc[3], b2, b3, va2, va3, xb);
-        }
+        if (w == (0x80402010u >> (4 * h))) half_diag<T, X, XV>(va0, xo, h, xs31, acc);
+        else if (w == (h ? 0x1C0E0703u : 0xC0E07038u)) half_tri<T, X, XV>(va0, xo, h, xs31, acc);
+        else if (w && !(w & (w - 1u))) half_single<T, X>(va0, xo, 31u - (uint32_t)(31 - __clz((int)w)), xs31, acc);
+        else if (w) half_generic<T, X>(w, va0, xo, xs31, acc);
+    }
+}
+
+// The same walk over a palette matrix: per block one 32-bit word (x offset | entry byte offset << 16) at a_w and the half's 8 bytes of
+// the palette entry at pal_h + entry offset {bits, meta}: no popc and no shape tests, the entry says it all.  The products and their
+// order per row are those of tile_half_row.
+template <typename T, typename X>
+__device__ __forceinline__ void tile_half_row_pal(uint32_t a_w, const uint32_t pal_h, uint32_t a_v, int nb, const int h, const uint32_t xs31,
+                                                  float (&acc)[4]) {
+#pragma unroll 1
+    for (int i = 0; i < nb; i++) {
+        const uint32_t wd = lds_u32(a_w);
+        a_w += 4;
+        const uint2 e = lds_v2(pal_h + (wd >> 16));
+        const uint32_t xo = wd & 0xFFFFu, m = e.y;
+        const uint32_t va0 = a_v + (m & 0xFFu);
+        a_v += m >> 20;
+        if (m & PAL_DIAG) half_diag<T, X, true>(va0, xo, h, xs31, acc);
+        else if (m & PAL_TRI) half_tri<T, X, true>(va0, xo, h, xs31, acc);
+        else if (m & PAL_SINGLE) half_single<T, X>(va0, xo, (m >> 12) & 31u, xs31, acc);
+        else if (m & PAL_GENERIC) half_generic<T, X>(e.x, va0, xo, xs31, acc);
     }
 }
 
@@ -709,15 +835,24 @@ __global__ void __launch_bounds__(RTT * TPR, MINB) spmv_tile_kernel(const TileAr
 //   consumers: wait for `full`, multiply out of shared memory, store y, arrive on the stage's `empty` mbarrier.
 // No CTA-wide barrier after start-up.  One producer warp serves one group: a warp issues its ~200 instructions per tile at one
 // every few cycles, so a single producer for a whole CTA of seven groups caps the SM at one tile per 0.7 us (measured).
+// pal: the palette variant -- a 32-byte header (the second 16 bytes: the tile's block and value counts as the last row's end), one
+// 32-bit word per block in place of bitmaps and x offsets (`bm`; `xo` unused), 4-byte relative row pairs
 struct StageLayout { uint32_t bm, xo, val, row, xs, stride; };
-inline StageLayout stage_layout(int rt, int cap_blk, int cap_val, int cap_lines, int vsize, int xsize) {
+inline StageLayout stage_layout(int rt, int cap_blk, int cap_val, int cap_lines, int vsize, int xsize, bool pal) {
     auto up16 = [](uint32_t v) { return (v + 15u) & ~15u; };
     StageLayout s;
-    s.bm = 16;                                                   // 16-byte header: {p0, v0, staged, -}
-    s.xo = up16(s.bm + (uint32_t)(cap_blk + 2) * 8);
-    s.val = up16(s.xo + (uint32_t)(cap_blk + 16) * 2);
-    s.row = up16(s.val + (uint32_t)(cap_val + 16) * vsize);
-    s.xs = up16(s.row + (uint32_t)(rt + 2) * 8);
+    if (pal) {
+        s.bm = 32;
+        s.xo = s.val = up16(s.bm + (uint32_t)(cap_blk + 4) * 4);
+        s.row = up16(s.val + (uint32_t)(cap_val + 16) * vsize);
+        s.xs = up16(s.row + (uint32_t)(rt + 4) * 4);
+    } else {
+        s.bm = 16;                                               // 16-byte header: {p0, v0, staged, -}
+        s.xo = up16(s.bm + (uint32_t)(cap_blk + 2) * 8);
+        s.val = up16(s.xo + (uint32_t)(cap_blk + 16) * 2);
+        s.row = up16(s.val + (uint32_t)(cap_val + 16) * vsize);
+        s.xs = up16(s.row + (uint32_t)(rt + 2) * 8);
+    }
     s.stride = (s.xs + (uint32_t)cap_lines * 32u * xsize + 16u + 127u) & ~127u;   // + 16: the tridiagonal path reads one element past
     return s;
 }
@@ -760,7 +895,8 @@ __device__ __noinline__ void halo_push_tile(const HaloDev* hd, int row, int rows
     if (gt == 0) { __threadfence_system(); halo_signal(*hd); }
 }
 
-template <typename T, typename X, int RTT, int NG, int MINB, typename H = NoHalo>
+// PAL: the matrix has a bitmap palette (see palette_scan_kernel); it is loaded once per CTA, behind the descriptor rings.
+template <typename T, typename X, int RTT, int NG, int MINB, typename H = NoHalo, bool PAL = false>
 __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(const __grid_constant__ StreamArgs<T> sa, const X* __restrict__ x,
                                                                                float* __restrict__ y, const __grid_constant__ H hd) {
     constexpr bool DIST = !std::is_same<H, NoHalo>::value;
@@ -775,11 +911,20 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
     const int spg = sa.spg, nstage = spg * NG;
     const uint32_t sbase = smem_u32(smem);
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)nstage * so.stride);      // full[nstage], empty[nstage]
+    const uint32_t pal_off = (uint32_t)nstage * (so.stride + 16u) + (uint32_t)NG * (DR * 64u) + 64u;   // PAL: barrier, then the entries
+    uint64_t* pal_bar = reinterpret_cast<uint64_t*>(smem + pal_off);
     if (tid == 0) {
         for (int s = 0; s < nstage; s++) { mbar_init(bars + s, 1); mbar_init(bars + nstage + s, GT / 32); }
+        if constexpr (PAL) mbar_init(pal_bar, 1);
         mbar_fence_init();
     }
     __syncthreads();
+    if constexpr (PAL) {
+        if (tid == 0) {
+            mbar_arrive_expect_tx(pal_bar, (uint32_t)a.npal * 16u);
+            bulk_g2s(smem + pal_off + 16, a.palette, (uint32_t)a.npal * 16u, pal_bar);
+        }
+    }
     const bool is_producer = warp < NG;
     const int g = NG == 1 ? 0 : (is_producer ? warp : (warp - NG) / (GT / 32));
     const int grid = (int)gridDim.x;
@@ -858,13 +1003,18 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
             const int r0 = t * RTT, nrow = min(RTT, a.nbr - r0);
             const uint32_t sp32 = gbase + (uint32_t)s * so.stride;
             unsigned char* sp = smem + (size_t)(g * spg + s) * so.stride;
-            const uint32_t nrb = (uint32_t)((nrow + 1 + 1) & ~1) * 8;
-            const int p0a = p0 & ~1, p0x = p0 & ~7;
+            // PAL: nrb = relative row pairs (4 B per block row), n8 = block words from p0a = p0 & ~3; otherwise int2 row pairs (one past
+            // the tile's last row), bitmaps from p0 & ~1 and x offsets from p0 & ~7
+            const uint32_t nrb = PAL ? (uint32_t)((nrow + 3) & ~3) * 4 : (uint32_t)((nrow + 1 + 1) & ~1) * 8;
+            const int p0a = PAL ? p0 & ~3 : p0 & ~1, p0x = p0 & ~7;
             uint32_t n8 = 0, n2 = 0, nvb = 0;
             int nlc = 0;                                                  // x lines that arrive by bulk copy
             if (staged && nb > 0) {
-                n8 = (uint32_t)((p0 + nb - p0a + 1) & ~1) * 8;
-                n2 = (uint32_t)((p0 + nb - p0x + 7) & ~7) * 2;
+                if constexpr (PAL) n8 = (uint32_t)((p0 + nb - p0a + 3) & ~3) * 4;
+                else {
+                    n8 = (uint32_t)((p0 + nb - p0a + 1) & ~1) * 8;
+                    n2 = (uint32_t)((p0 + nb - p0x + 7) & ~7) * 2;
+                }
                 nvb = ((v0 + (uint32_t)nv - v0a + (uint32_t)(VA - 1)) & ~(uint32_t)(VA - 1)) * (uint32_t)sizeof(T);
                 nlc = (d1.y & 2) ? nl - 1 : nl;                          // a last line that reaches past the last column is loaded by hand
             }
@@ -895,10 +1045,16 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
             const bool by_runs = d2.x > 0;
             if (lane == 0) {
                 *reinterpret_cast<int4*>(sp) = make_int4(p0, (int)v0, (staged ? 1 : 0) | (part ? 2 : 0), t);     // the consumers take the tile from here
+                if constexpr (PAL) *reinterpret_cast<uint32_t*>(sp + 16) = (uint32_t)nb | (uint32_t)nv << 16;
                 mbar_arrive_expect_tx(full + s, n8 + n2 + nvb + nrb + (uint32_t)nlc * 32u * SX);
-                bulk_g2s(sp + so.row, a.rowpair + r0, nrb, full + s);
-                if (n8) bulk_g2s(sp + so.bm, a.bmps + p0a, n8, full + s);
-                if (n2) bulk_g2s(sp + so.xo, a.xoff + p0x, n2, full + s);
+                if constexpr (PAL) {
+                    bulk_g2s(sp + so.row, a.rowrel + r0, nrb, full + s);
+                    if (n8) bulk_g2s(sp + so.bm, a.word + p0a, n8, full + s);
+                } else {
+                    bulk_g2s(sp + so.row, a.rowpair + r0, nrb, full + s);
+                    if (n8) bulk_g2s(sp + so.bm, a.bmps + p0a, n8, full + s);
+                    if (n2) bulk_g2s(sp + so.xo, a.xoff + p0x, n2, full + s);
+                }
                 if (nvb) bulk_g2s(sp + so.val, a.values + v0a, nvb, full + s);
                 if (nlc > 0 && by_runs) {                                 // up to three runs of consecutive lines
                     unsigned char* xs = sp + so.xs;
@@ -932,6 +1088,8 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
         // ------------------------------------------------------------------------------------------ consumers
         const int gt = tid - NG * 32 - g * GT;
         const int lbr = gt >> 1, h = gt & 1;
+        const uint32_t pal_h = sbase + pal_off + 16u + 8u * (uint32_t)h;    // PAL: this half's 8 bytes of entry 0
+        if constexpr (PAL) mbar_wait(pal_bar, 0);
         int s = 0; uint32_t par = 0;
         for (;;) {
             mbar_wait(full + s, par);
@@ -946,16 +1104,31 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
             const bool active = lbr < nrow && row < a.rows;
             float acc[4] = {0.f, 0.f, 0.f, 0.f};
             if (active) {
-                const uint2 rp = lds_v2(sb + so.row + 8u * lbr);          // (first block, first value) of this block row
-                const uint32_t pe = lds_u32(sb + so.row + 8u * lbr + 8u);
-                const uint32_t pb = rp.x, kv = rp.y;
-                if (staged) {
-                    const uint32_t rel = pb - (uint32_t)p0;
-                    const uint32_t a_bm = sb + so.bm + ((uint32_t)(p0 & 1) + rel) * 8u, a_xo = sb + so.xo + ((uint32_t)(p0 & 7) + rel) * 2u;
-                    const uint32_t a_v = sb + so.val + (kv - v0a) * (uint32_t)sizeof(T), xs31 = sb + so.xs + 31u * SX;
-                    tile_half_row<T, X, true>(a_bm, a_xo, a_v, (int)(pe - pb), h, xs31, acc);
+                if constexpr (PAL) {
+                    if (staged) {
+                        // (first block, first value) of this block row and of the next one, relative to the tile; the tile's counts end the last row
+                        const uint32_t rp = lds_u32(sb + so.row + 4u * lbr);
+                        const uint32_t re = lbr + 1 < nrow ? lds_u32(sb + so.row + 4u * lbr + 4u) : lds_u32(sb + 16u);
+                        const uint32_t rb = rp & 0xFFFFu;
+                        const uint32_t a_w = sb + so.bm + ((uint32_t)(p0 & 3) + rb) * 4u;
+                        const uint32_t a_v = sb + so.val + ((uint32_t)hdr.y - v0a + (rp >> 16)) * (uint32_t)sizeof(T), xs31 = sb + so.xs + 31u * SX;
+                        tile_half_row_pal<T, X>(a_w, pal_h, a_v, (int)((re & 0xFFFFu) - rb), h, xs31, acc);
+                    } else {
+                        const int br = r0 + lbr;
+                        half_block_row<T, X>(a.bmps, a.bcol, a.values, __ldg(a.brp + br), __ldg(a.brp + br + 1), __ldg(a.rvb + br), h, x, acc);
+                    }
                 } else {
-                    half_block_row<T, X>(a.bmps, a.bcol, a.values, (int)pb, (int)pe, kv, h, x, acc);
+                    const uint2 rp = lds_v2(sb + so.row + 8u * lbr);          // (first block, first value) of this block row
+                    const uint32_t pe = lds_u32(sb + so.row + 8u * lbr + 8u);
+                    const uint32_t pb = rp.x, kv = rp.y;
+                    if (staged) {
+                        const uint32_t rel = pb - (uint32_t)p0;
+                        const uint32_t a_bm = sb + so.bm + ((uint32_t)(p0 & 1) + rel) * 8u, a_xo = sb + so.xo + ((uint32_t)(p0 & 7) + rel) * 2u;
+                        const uint32_t a_v = sb + so.val + (kv - v0a) * (uint32_t)sizeof(T), xs31 = sb + so.xs + 31u * SX;
+                        tile_half_row<T, X, true>(a_bm, a_xo, a_v, (int)(pe - pb), h, xs31, acc);
+                    } else {
+                        half_block_row<T, X>(a.bmps, a.bcol, a.values, (int)pb, (int)pe, kv, h, x, acc);
+                    }
                 }
                 float* yr = y + row;
                 if (row + 4 <= a.rows) *reinterpret_cast<float4*>(yr) = make_float4(acc[0], acc[1], acc[2], acc[3]);
@@ -1164,6 +1337,48 @@ __global__ void work_fill_kernel(const int32_t* __restrict__ brp, int nbr, const
 
 static int env_int(const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; }
 
+// The streaming kernel's bitmap palette: collect the distinct bitmaps (palette_scan_kernel), sort them here and upload one 16-byte
+// entry per bitmap (layout at PalScan).  Leaves m->spmv_npal = 0 when the matrix has more than PALETTE_MAX distinct bitmaps.
+static int build_palette(bmsp_matrix_s* m, int vsize, cudaStream_t st, std::vector<uint4>& pal) {
+    m->spmv_npal = 0;
+    PalScan* ps = nullptr;
+    BMSP_TRY(dev_alloc((void**)&ps, sizeof(PalScan), st));
+    BMSP_CUDA(cudaMemsetAsync(ps, 0, sizeof(PalScan), st));
+    const int grid = (int)std::min<int64_t>(1024, std::max<int64_t>(1, ceil_div(m->nblk, 256 * 16)));
+    palette_scan_kernel<<<grid, 256, 0, st>>>(m->bmps, m->nblk, ps);
+    BMSP_KERNEL_CHECK();
+    std::vector<PalScan> h(1);
+    BMSP_CUDA(cudaMemcpyAsync(h.data(), ps, sizeof(PalScan), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));
+    dev_free(ps, st);
+    if (h[0].overflow) return BMSP_OK;
+    std::vector<uint64_t> keys;
+    for (int i = 0; i < PAL_GSLOTS; i++) if (h[0].key[i]) keys.push_back(h[0].key[i]);
+    if (h[0].has_zero) keys.push_back(0ull);
+    if (keys.empty() || keys.size() > (size_t)PALETTE_MAX) return BMSP_OK;
+    std::sort(keys.begin(), keys.end());
+    for (const uint64_t b : keys) {
+        const uint32_t hw[2] = {(uint32_t)(b >> 32), (uint32_t)b};      // half 0 = rows 0-3 (high word), half 1 = rows 4-7
+        const uint32_t nhi = (uint32_t)__builtin_popcount(hw[0]), ntot = nhi + (uint32_t)__builtin_popcount(hw[1]);
+        uint32_t meta[2];
+        for (int h2 = 0; h2 < 2; h2++) {
+            const uint32_t w = hw[h2];
+            // the tests of tile_half_row, in its order
+            uint32_t cls = 0, cell = 0;
+            if (w == (0x80402010u >> (4 * h2))) cls = PAL_DIAG;
+            else if (w == (h2 ? 0x1C0E0703u : 0xC0E07038u)) cls = PAL_TRI;
+            else if (w && !(w & (w - 1u))) { cls = PAL_SINGLE; cell = (uint32_t)__builtin_clz(w); }
+            else if (w) cls = PAL_GENERIC;
+            meta[h2] = (h2 ? nhi : 0u) * (uint32_t)vsize | cls | cell << 12 | ntot * (uint32_t)vsize << 20;
+        }
+        pal.push_back(make_uint4(hw[0], meta[0], hw[1], meta[1]));
+    }
+    BMSP_TRY(dev_alloc((void**)&m->tile_palette, sizeof(uint4) * pal.size(), st));
+    BMSP_CUDA(cudaMemcpyAsync(m->tile_palette, pal.data(), sizeof(uint4) * pal.size(), cudaMemcpyHostToDevice, st));
+    m->spmv_npal = (int32_t)pal.size();
+    return BMSP_OK;
+}
+
 // path 0 plan: tile descriptors, x lines and per-block x offsets; shared-memory capacities from the tile maxima
 // when they fit the per-CTA budget, else from the averages (larger tiles are then read from global memory).
 static int plan_tiles(bmsp_matrix_s* m, cudaStream_t st) {
@@ -1182,13 +1397,21 @@ static int plan_tiles(bmsp_matrix_s* m, cudaStream_t st) {
     m->spmv_kernel = force == 1 ? 1 : (force == 2 ? 0 : (rt == 64 ? 0 : 1));
     m->xl_pitch = m->spmv_kernel == 1 ? XL_STRIDE : 32;
     const int ntiles = (int)ceil_div(m->nbr, rt);
+    std::vector<uint4> pal;                    // kept until the synchronisation below (pageable source of the palette upload)
+    if (m->spmv_kernel == 0) BMSP_TRY(build_palette(m, vsize, st, pal));
+    const bool use_pal = m->spmv_npal > 0;
     unsigned long long* stats = nullptr;
     BMSP_TRY(dev_alloc((void**)&m->tile_desc, sizeof(TileDesc) * (size_t)ntiles, st));
     BMSP_TRY(dev_alloc_t(&m->tile_lines, (size_t)m->nblk + 8, st));
-    BMSP_TRY(dev_alloc_t(&m->tile_xoff, (size_t)m->nblk + 16, st));
-    BMSP_TRY(dev_alloc((void**)&m->tile_rowpair, sizeof(int2) * ((size_t)m->nbr + 1 + 8), st));
-    zip_rows_kernel<<<(unsigned)ceil_div(m->nbr + 1, 256), 256, 0, st>>>(m->brp, m->rvb, m->nbr + 1, (int2*)m->tile_rowpair);
-    BMSP_KERNEL_CHECK();
+    if (use_pal) {
+        BMSP_TRY(dev_alloc_t(&m->tile_word, (size_t)m->nblk + 8, st));
+        BMSP_TRY(dev_alloc_t(&m->tile_rowrel, (size_t)m->nbr + 8, st));
+    } else {
+        BMSP_TRY(dev_alloc_t(&m->tile_xoff, (size_t)m->nblk + 16, st));
+        BMSP_TRY(dev_alloc((void**)&m->tile_rowpair, sizeof(int2) * ((size_t)m->nbr + 1 + 8), st));
+        zip_rows_kernel<<<(unsigned)ceil_div(m->nbr + 1, 256), 256, 0, st>>>(m->brp, m->rvb, m->nbr + 1, (int2*)m->tile_rowpair);
+        BMSP_KERNEL_CHECK();
+    }
     BMSP_TRY(dev_alloc_t(&stats, 8, st));
     BMSP_CUDA(cudaMemsetAsync(stats, 0, 8 * sizeof(unsigned long long), st));
     if (m->spmv_kernel == 0 && !m->spmv_sched) {
@@ -1197,7 +1420,8 @@ static int plan_tiles(bmsp_matrix_s* m, cudaStream_t st) {
         BMSP_TRY(dev_alloc_t(&m->spmv_sched, (size_t)SCHED_SLOTS * 2, st));
         BMSP_CUDA(cudaMemsetAsync(m->spmv_sched, 0, sizeof(int32_t) * SCHED_SLOTS * 2, st));
     }
-    tile_plan_kernel<<<ntiles, 256, 0, st>>>(m->brp, m->bcol, m->rvb, m->nbr, m->cols, rt, m->xl_pitch, (TileDesc*)m->tile_desc, m->tile_lines, m->tile_xoff, stats);
+    tile_plan_kernel<<<ntiles, 256, 0, st>>>(m->brp, m->bcol, m->rvb, m->nbr, m->cols, rt, m->xl_pitch, (TileDesc*)m->tile_desc, m->tile_lines, m->tile_xoff,
+                                             stats, m->bmps, (const uint4*)m->tile_palette, m->spmv_npal, m->tile_word, m->tile_rowrel);
     BMSP_KERNEL_CHECK();
     unsigned long long h[8];
     BMSP_CUDA(cudaMemcpyAsync(h, stats, sizeof(h), cudaMemcpyDeviceToHost, st));
@@ -1217,6 +1441,9 @@ static int plan_tiles(bmsp_matrix_s* m, cudaStream_t st) {
         }
     }
     m->cap_blk = std::max(cb, 8); m->cap_val = std::max(cv, 8); m->cap_lines = std::max(cl, 1);
+    // the palette variant's relative row pairs are 16-bit: a staged tile has fewer than 65536 blocks and values (the 40 KB budget
+    // above keeps both far below that already)
+    if (use_pal) { m->cap_blk = std::min(m->cap_blk, 65528); m->cap_val = std::min(m->cap_val, 65528); }
     return BMSP_OK;
 }
 
@@ -1273,9 +1500,9 @@ static int launch_tile_kernel(const TileArgs<T>& a, const X* x, float* y, const 
 // Streaming kernel launch.  One group per CTA (NG = 1); MAXB bounds the CTAs per SM the registers allow.  Shared memory decides the
 // rest: as many CTAs per SM as fit with two stages each (a group needs a second stage to have its next tile arriving while it
 // multiplies the current one; P4096: 7 CTAs x 2 stages of 15.4 KB -- the measured optimum, see DESIGN.md section 7).
-template <typename T, typename X, int RTT, int NG, int MAXB, typename H>
-static int launch_stream_kernel(const TileArgs<T>& a, const X* x, float* y, const H& hd, int ntiles, cudaStream_t st, int32_t* sched = nullptr) {
-    auto kern = spmv_stream_kernel<T, X, RTT, NG, MAXB, H>;
+template <typename T, typename X, int RTT, int NG, int MAXB, typename H, bool PAL>
+static int launch_stream_kernel(const TileArgs<T>& a, const X* x, float* y, const H& hd, int ntiles, cudaStream_t st, int32_t* sched) {
+    auto kern = spmv_stream_kernel<T, X, RTT, NG, MAXB, H, PAL>;
     static int sms = 0;
     static size_t smem_max = 0;
     if (!sms) {
@@ -1288,9 +1515,9 @@ static int launch_stream_kernel(const TileArgs<T>& a, const X* x, float* y, cons
     }
     StreamArgs<T> sa;
     sa.t = a;
-    sa.so = stage_layout(RTT, a.cap_blk, a.cap_val, a.cap_lines, sizeof(T), sizeof(X));
+    sa.so = stage_layout(RTT, a.cap_blk, a.cap_val, a.cap_lines, sizeof(T), sizeof(X), PAL);
     sa.ntiles = ntiles;
-    const size_t fixed = (size_t)NG * STREAM_DR * 64 + 64;                               // descriptor rings
+    const size_t fixed = (size_t)NG * STREAM_DR * 64 + 64 + (PAL ? 16 + (size_t)a.npal * 16 : 0);   // descriptor rings (+ palette)
     const size_t per_stage = (size_t)NG * (sa.so.stride + 16);
     static const int want_ctas = env_int("BMSP_SPMV_CTAS", 0), want_spg = env_int("BMSP_SPMV_STAGES", 0);   // experiments
     int ctas = 0, spg = 0;
@@ -1331,6 +1558,8 @@ static int launch_spmv(bmsp_matrix_s* A, const X* x, float* y, cudaStream_t st, 
         a.tile0 = tile0; a.tile_list = nullptr;
         a.bmps = A->bmps; a.bcol = A->bcol; a.values = (const T*)A->values; a.rowpair = (const int2*)A->tile_rowpair;
         a.desc = (const TileDesc*)A->tile_desc; a.lines = A->tile_lines; a.xoff = A->tile_xoff;
+        a.word = A->tile_word; a.rowrel = A->tile_rowrel; a.palette = (const uint4*)A->tile_palette; a.npal = A->spmv_npal;
+        a.brp = A->brp; a.rvb = A->rvb;
         a.rows = A->rows; a.nbr = A->nbr; a.cols = A->cols; a.cap_blk = A->cap_blk; a.cap_val = A->cap_val; a.cap_lines = A->cap_lines;
         const int rt = A->tile_rows;
         a.so = tile_smem(rt, a.cap_blk, a.cap_val, a.cap_lines, sizeof(T), sizeof(X));
@@ -1346,10 +1575,16 @@ static int launch_spmv(bmsp_matrix_s* A, const X* x, float* y, cudaStream_t st, 
             if (ntiles < 0 && tile_list == nullptr) {
                 if (A->spmv_sched) sched = A->spmv_sched + 2 * (A->spmv_sched_next++ % SCHED_SLOTS);      // allocated and zeroed by the plan
             }
-            if (rt == 128) return launch_stream_kernel<T, X, 128, 1, 3, H>(a, x, y, hd, grid, st, sched);
-            if (rt == 32) return launch_stream_kernel<T, X, 32, 1, 8, H>(a, x, y, hd, grid, st, sched);
-            if (rt == 16) return launch_stream_kernel<T, X, 16, 1, 8, H>(a, x, y, hd, grid, st, sched);
-            return launch_stream_kernel<T, X, 64, 1, 7, H>(a, x, y, hd, grid, st, sched);
+            if (A->spmv_npal > 0) {
+                if (rt == 128) return launch_stream_kernel<T, X, 128, 1, 3, H, true>(a, x, y, hd, grid, st, sched);
+                if (rt == 32) return launch_stream_kernel<T, X, 32, 1, 8, H, true>(a, x, y, hd, grid, st, sched);
+                if (rt == 16) return launch_stream_kernel<T, X, 16, 1, 8, H, true>(a, x, y, hd, grid, st, sched);
+                return launch_stream_kernel<T, X, 64, 1, 7, H, true>(a, x, y, hd, grid, st, sched);
+            }
+            if (rt == 128) return launch_stream_kernel<T, X, 128, 1, 3, H, false>(a, x, y, hd, grid, st, sched);
+            if (rt == 32) return launch_stream_kernel<T, X, 32, 1, 8, H, false>(a, x, y, hd, grid, st, sched);
+            if (rt == 16) return launch_stream_kernel<T, X, 16, 1, 8, H, false>(a, x, y, hd, grid, st, sched);
+            return launch_stream_kernel<T, X, 64, 1, 7, H, false>(a, x, y, hd, grid, st, sched);
         }
         // default: one thread per bitmap half; BMSP_SPMV_VARIANT=1: one thread per block row (64-row tiles only).
         // Measured on P4096: 92.7 us vs 103.5 us (fewer instructions, but too few warps to hide the staging latency).

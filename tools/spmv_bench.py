@@ -34,5 +34,22 @@ for _ in range(reps):
 e1.record(); e1.synchronize()
 us = e0.elapsed_time(e1) / reps * 1e3
 nbytes = A.spmv_bytes()
+
+
+def stream_bytes():
+    """bytes the streaming kernel reads and writes per product, counted from the plan's rules (spmv.cu plan_spmv / plan_tiles);
+    None when another kernel runs.  Per block: a 4-byte word with a bitmap palette (<= 256 distinct bitmaps), else 8 B bitmap + 2 B x
+    offset; per block row 4 B (palette) or 8 B; fp16 values; x and y once; a 64-byte descriptor per tile of 64 block rows."""
+    nbr, nblk, nnz = (nr + 7) // 8, A.block_num, A.nnz
+    if nnz < 2.5 * nblk or (nblk * 26 + nnz * 2) / nbr + 8 > 320:
+        return None
+    npal = np.unique(A.download()[1]).size
+    meta = nblk * 4 + nbr * 4 if npal <= 256 else nblk * 10 + nbr * 8
+    return meta + nnz * 2 + nc * 4 + nr * 4 + (nbr + 63) // 64 * 64
+
+
+sb = stream_bytes()
+sb_txt = f"stream_MB={sb / 1e6:.1f} stream_GBps={sb / us / 1e3:.1f}" if sb else "stream_MB=n/a"
 print(f"SPMV {which} variant={os.environ.get('BMSP_SPMV_VARIANT', '0')} rows={nr} nnz={A.nnz} blocks={A.block_num} "
-      f"us={us:.2f} GBps={nbytes / us / 1e3:.1f} frac6468={nbytes / us / 1e3 / 6468.3:.3f} first_call_ms={plan_ms:.1f} ysum={float(y.double().sum()):.6e}")
+      f"us={us:.2f} GBps={nbytes / us / 1e3:.1f} {sb_txt} frac6468={nbytes / us / 1e3 / 6468.3:.3f} first_call_ms={plan_ms:.1f} "
+      f"ysum={float(y.double().sum()):.6e}")
