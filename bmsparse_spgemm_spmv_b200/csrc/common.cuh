@@ -39,9 +39,9 @@ struct bmsp_matrix_s {
     int32_t cap_blk = 0, cap_val = 0;   // per-tile smem capacities of the row-tiled kernels
     int32_t cap_lines = 0;      // staged x lines per tile (tile plan)
     int32_t tile_rows = 64;     // block rows per tile (64, 32 or 16)
-    int32_t spmv_kernel = 0;    // row-tiled path: 0 = streaming kernel (persistent CTAs, staged tiles in a shared-memory ring), 1 = one CTA per tile
+    int32_t spmv_kernel = 0;    // row-tiled path: 0 = streaming kernel (persistent CTAs, staged tiles in a shared-memory ring; 64-row tiles only), 1 = one CTA per tile
     int32_t xl_pitch = 32;      // elements between staged x lines (32 for the streaming kernel's bulk copies, 33 for the per-tile kernel)
-    int32_t* spmv_sched = nullptr;  // streaming kernel: SCHED_SLOTS x {next tile to claim, groups done}; a launch takes the next slot
+    int32_t* spmv_sched = nullptr;  // streaming kernel: SCHED_SLOTS x {next tile to claim, CTAs done}; a launch takes the next slot
     uint32_t spmv_sched_next = 0;
     void* tile_rowpair = nullptr;   // [nbr+1] int2 (block_row_ptr, first value) zipped for one bulk copy per tile
     void* tile_desc = nullptr;  // [ntiles] TileDesc (spmv.cu): block / value / x-line ranges of every tile of 64 block rows
@@ -61,13 +61,6 @@ struct bmsp_matrix_s {
     int32_t n_split_rows = 0;
     int32_t max_row_blocks = 0;
     void* host_pipe = nullptr;  // HostPipe (spmv.cu): streams, events and staging buffers of bmsp_spmv_host
-    // multi-GPU product (spmv.cu, bmsp_spmv_halo): the tiles that depend on the peers or push rows to them ("boundary"), and the rest
-    int32_t* halo_tiles = nullptr;      // [ntiles] boundary tiles first (ascending), then the interior tiles (ascending)
-    int32_t halo_n_boundary = -1;       // -1: not classified yet
-    int32_t halo_first = 0;             // the first boundary tile
-    cudaStream_t halo_side = nullptr;   // the boundary launch runs here, next to the interior launch on the caller's stream
-    cudaEvent_t halo_fork = nullptr, halo_join = nullptr;
-    int32_t halo_key[2 + 16] = {0};     // own column range + push ranges the lists were built for
     // Stream ordering of the handle's memory: every entry point that enqueues work on the arrays records its stream here
     // (bmsp::touch).  bmsp_destroy frees on that stream, so the frees are ordered behind the kernels that still read or write the
     // arrays; a handle that was used on more than one stream is drained with a device synchronisation first.  Streams passed to

@@ -255,13 +255,10 @@ int bmsp_destroy(bmsp_matrix_t m) {
     if (m->multi_stream) cudaDeviceSynchronize();
     cudaStream_t st = m->last_stream;
     spmv_host_release(m);
-    if (m->halo_side) { cudaStreamSynchronize(m->halo_side); cudaStreamDestroy(m->halo_side); }
-    if (m->halo_fork) cudaEventDestroy(m->halo_fork);
-    if (m->halo_join) cudaEventDestroy(m->halo_join);
     dev_free(m->keys, st); dev_free(m->bmps, st); dev_free(m->offsets, st); dev_free(m->values, st);
     dev_free(m->brp, st); dev_free(m->bcol, st); dev_free(m->rvb, st); dev_free(m->kmask, st);
     dev_free(m->work, st); dev_free(m->split_partial, st); dev_free(m->split_rows, st); dev_free(m->split_list, st); dev_free(m->pmeta, st);
-    dev_free(m->halo_tiles, st); dev_free(m->fine_ptr, st); dev_free(m->fine_bcol, st); dev_free(m->fine_kmask, st); dev_free(m->fine_rec, st);
+    dev_free(m->fine_ptr, st); dev_free(m->fine_bcol, st); dev_free(m->fine_kmask, st); dev_free(m->fine_rec, st);
     dev_free(m->tile_desc, st); dev_free(m->spmv_sched, st); dev_free(m->tile_rowpair, st); dev_free(m->tile_lines, st); dev_free(m->tile_xoff, st);
     dev_free(m->tile_palette, st); dev_free(m->tile_word, st); dev_free(m->tile_rowrel, st);
     delete m;

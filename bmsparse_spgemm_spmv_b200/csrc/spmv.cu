@@ -308,7 +308,6 @@ struct TileArgs {
     const int32_t* brp; const uint32_t* rvb;                                             // ... whose unstaged tiles read their row pointers here
     int32_t rows, nbr, cols, cap_blk, cap_val, cap_lines;
     int32_t tile0;       // first tile of this launch (row-range launches of the host-buffer pipeline)
-    const int32_t* tile_list;   // streaming kernel: when set, the launch's q-th tile is tile_list[q] (boundary / interior launches of the multi-GPU product)
     TileSmem so;
 };
 
@@ -516,34 +515,6 @@ __device__ __forceinline__ void tile_half_row_pal(uint32_t a_w, const uint32_t p
     }
 }
 
-// The blocks of one whole block row (all 8 matrix rows) walked by one thread: the per-block bookkeeping is paid
-// once per block instead of once per bitmap half.
-template <typename T, typename X>
-__device__ __forceinline__ void tile_block_row(uint32_t a_bm, uint32_t a_xo, uint32_t a_v, int nb, const uint32_t xs31, float (&acc)[8]) {
-    constexpr uint32_t SV = sizeof(T), SX = sizeof(X);
-#pragma unroll 1
-    for (int i = 0; i < nb; i++) {
-        const uint2 w2 = lds_v2(a_bm);                  // .y = rows 0-3, .x = rows 4-7
-        const uint32_t xo = lds_u16(a_xo);
-        a_bm += 8; a_xo += 2;
-        const uint32_t hi = w2.y, lo = w2.x;
-        const uint32_t xb = xs31 + xo * SX;
-        const uint32_t b0 = hi & 0xFF000000u, b1 = hi & 0x00FF0000u, b2 = hi & 0x0000FF00u, b3 = hi & 0x000000FFu;
-        const uint32_t b4 = lo & 0xFF000000u, b5 = lo & 0x00FF0000u, b6 = lo & 0x0000FF00u, b7 = lo & 0x000000FFu;
-        const uint32_t va0 = a_v, va1 = va0 + __popc(b0) * SV, va2 = va1 + __popc(b1) * SV, va3 = va2 + __popc(b2) * SV;
-        const uint32_t va4 = va3 + __popc(b3) * SV, va5 = va4 + __popc(b4) * SV, va6 = va5 + __popc(b5) * SV, va7 = va6 + __popc(b6) * SV;
-        a_v = va7 + __popc(b7) * SV;
-        if (hi) {
-            RowPair<T, X, 0>::run(acc[0], acc[1], b0, b1, va0, va1, xb);
-            RowPair<T, X, 1>::run(acc[2], acc[3], b2, b3, va2, va3, xb);
-        }
-        if (lo) {
-            RowPair<T, X, 0>::run(acc[4], acc[5], b4, b5, va4, va5, xb);
-            RowPair<T, X, 1>::run(acc[6], acc[7], b6, b7, va6, va7, xb);
-        }
-    }
-}
-
 template <typename X> __device__ __forceinline__ void sts_x(uint32_t a, X v);
 template <> __device__ __forceinline__ void sts_x<float>(uint32_t a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
 template <> __device__ __forceinline__ void sts_x<__half>(uint32_t a, __half v) {
@@ -627,33 +598,23 @@ __device__ __forceinline__ void halo_signal(const HaloDev& h) {
         for (int p = 0; p < h.n_peer; p++) st_release_sys(h.peer_flag[p], h.signal_epoch);
     }
 }
-// rows [row, row + NR) of y (NR a multiple of 4 or the ragged tail) to every peer range that contains them
-template <int NR>
-__device__ __forceinline__ void halo_store(const HaloDev& h, int row, int rows, const float (&acc)[NR]) {
+// rows [row, row + 4) of y (row a multiple of 4; the ragged tail stops at `rows`) to every peer range that contains them
+__device__ __forceinline__ void halo_store(const HaloDev& h, int row, int rows, const float (&acc)[4]) {
     for (int i = 0; i < h.n_push; i++) {
         const int lo = h.lo[i], hi = h.hi[i];
-        if (row >= hi || row + NR <= lo) continue;
+        if (row >= hi || row + 4 <= lo) continue;
         float* d = h.dst[i] + (row - lo);
-        if (row >= lo && row + NR <= hi && row + NR <= rows) {
-#pragma unroll
-            for (int q = 0; q < NR; q += 4) *reinterpret_cast<float4*>(d + q) = make_float4(acc[q], acc[q + 1], acc[q + 2], acc[q + 3]);
+        if (row >= lo && row + 4 <= hi && row + 4 <= rows) {
+            *reinterpret_cast<float4*>(d) = make_float4(acc[0], acc[1], acc[2], acc[3]);
         } else {
 #pragma unroll
-            for (int q = 0; q < NR; q++) if (row + q >= lo && row + q < hi && row + q < rows) d[q] = acc[q];
+            for (int q = 0; q < 4; q++) if (row + q >= lo && row + q < hi && row + q < rows) d[q] = acc[q];
         }
     }
 }
 
 __global__ void halo_wait_kernel(const HaloDev h) {
     if ((int)threadIdx.x < h.n_peer) halo_wait(h, threadIdx.x);
-}
-// publishes the epoch after a product whose kernels stored the peers' rows without fences of their own: the kernel boundary
-// orders those stores before this thread, its system fence and release stores carry them to the peers
-__global__ void halo_flag_kernel(const HaloDev h) {
-    if (threadIdx.x == 0) {
-        __threadfence_system();
-        for (int p = 0; p < h.n_peer; p++) st_release_sys(h.peer_flag[p], h.signal_epoch);
-    }
 }
 // stand-alone push (first exchange after set_x, and products that run the block-parallel kernel): every thread reads four rows of y
 // once and stores them to every peer range that contains them -- 16-byte stores, 512 contiguous bytes per warp and peer, all
@@ -678,21 +639,19 @@ __global__ void __launch_bounds__(256) halo_push_kernel(const float* __restrict_
     if (threadIdx.x == 0) halo_signal(h);
 }
 
-// One CTA per tile of RTT block rows, TPR threads per block row (1: a thread owns all 8 matrix rows of its block
-// row; 2: one thread per 32-bit bitmap half).  Every thread reads the 32-byte tile descriptor; thread 0 arms the
-// mbarrier and issues the bulk copies (row pointers, bitmaps, x offsets, values) while all threads gather the
-// tile's distinct x lines (coalesced 16-byte loads, stored at a 33-element pitch); latency is hidden by the CTAs
-// resident per SM, each in a different phase.
+// One CTA per tile of RTT block rows, two threads per block row (one per 32-bit bitmap half, 4 matrix rows each).  One thread
+// per block row (all 8 matrix rows) was measured slower on P4096: 103.5 us against 92.7 us -- fewer instructions, but too few
+// warps to hide the staging latency.  Every thread reads the 32-byte tile descriptor; thread 0 arms the mbarrier and issues the
+// bulk copies (row pointers, bitmaps, x offsets, values) while all threads gather the tile's distinct x lines (coalesced 16-byte
+// loads, stored at a 33-element pitch); latency is hidden by the CTAs resident per SM, each in a different phase.
 // H = HaloDev: the multi-GPU variant (waits for the peers' halo slices before gathering x, pushes its boundary rows).
-template <typename T, typename X, int RTT, int TPR, int MINB, typename H = NoHalo>
-__global__ void __launch_bounds__(RTT * TPR, MINB) spmv_tile_kernel(const TileArgs<T> a, const X* __restrict__ x, float* __restrict__ y, const H hd) {
+template <typename T, typename X, int RTT, int MINB, typename H = NoHalo>
+__global__ void __launch_bounds__(RTT * 2, MINB) spmv_tile_kernel(const TileArgs<T> a, const X* __restrict__ x, float* __restrict__ y, const H hd) {
     constexpr bool DIST = !std::is_same<H, NoHalo>::value;
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int VA = 16 / sizeof(T);   // values per 16 bytes
-    constexpr int NT = RTT * TPR;
-    constexpr int LPI = NT / 8;          // x lines per gather step (8 threads per line)
-    constexpr int GB = TPR == 1 ? 8 : 4; // gather steps in flight
-    static_assert(NT >= 8 && NT % 8 == 0, "8 threads per x line");
+    constexpr int LPI = RTT * 2 / 8;     // x lines per gather step (8 threads per line)
+    constexpr int GB = 4;                // gather steps in flight
     constexpr uint32_t SX = sizeof(X);
     const int tid = threadIdx.x;
     int t = blockIdx.x + a.tile0;
@@ -774,14 +733,11 @@ __global__ void __launch_bounds__(RTT * TPR, MINB) spmv_tile_kernel(const TileAr
     __syncthreads();                 // barrier initialised and armed, x lines visible
     mbar_wait(bar, 0);
 
-    const int lbr = tid / TPR, h = tid % TPR;
-    constexpr int NR = 8 / TPR;      // matrix rows per thread
-    const int row = (r0 + lbr) * 8 + h * NR;
+    const int lbr = tid >> 1, h = tid & 1;
+    const int row = (r0 + lbr) * 8 + h * 4;
     const bool active = lbr < nrow && row < a.rows;
     if (!DIST && !active) return;
-    float acc[NR];
-#pragma unroll
-    for (int q = 0; q < NR; q++) acc[q] = 0.f;
+    float acc[4] = {0.f, 0.f, 0.f, 0.f};
     if (active) {
         const uint2 rp = lds_v2(sbase + a.so.row + 8u * lbr);          // (first block, first value) of this block row
         const uint32_t pe = lds_u32(sbase + a.so.row + 8u * lbr + 8u);
@@ -790,29 +746,20 @@ __global__ void __launch_bounds__(RTT * TPR, MINB) spmv_tile_kernel(const TileAr
             const uint32_t rel = pb - (uint32_t)p0;
             const uint32_t a_bm = sbase + ((uint32_t)(p0 & 1) + rel) * 8u, a_xo = sbase + a.so.xo + ((uint32_t)(p0 & 7) + rel) * 2u;
             const uint32_t a_v = sbase + a.so.val + (kv - v0a) * (uint32_t)sizeof(T), xs31 = sbase + a.so.xs + 31u * SX;
-            if constexpr (TPR == 2) tile_half_row<T, X>(a_bm, a_xo, a_v, (int)(pe - pb), h, xs31, acc);
-            else tile_block_row<T, X>(a_bm, a_xo, a_v, (int)(pe - pb), xs31, acc);
-        } else if constexpr (TPR == 2) {
-            half_block_row<T, X>(a.bmps, a.bcol, a.values, (int)pb, (int)pe, kv, h, x, acc);
+            tile_half_row<T, X>(a_bm, a_xo, a_v, (int)(pe - pb), h, xs31, acc);
         } else {
-            float lo4[4] = {0.f, 0.f, 0.f, 0.f}, hi4[4] = {0.f, 0.f, 0.f, 0.f};
-            half_block_row<T, X>(a.bmps, a.bcol, a.values, (int)pb, (int)pe, kv, 0, x, lo4);
-            half_block_row<T, X>(a.bmps, a.bcol, a.values, (int)pb, (int)pe, kv, 1, x, hi4);
-#pragma unroll
-            for (int q = 0; q < 4; q++) { acc[q] = lo4[q]; acc[4 + q] = hi4[q]; }
+            half_block_row<T, X>(a.bmps, a.bcol, a.values, (int)pb, (int)pe, kv, h, x, acc);
         }
         float* yr = y + row;
-        if (row + NR <= a.rows) {
+        if (row + 4 <= a.rows) *reinterpret_cast<float4*>(yr) = make_float4(acc[0], acc[1], acc[2], acc[3]);
+        else {
 #pragma unroll
-            for (int q = 0; q < NR; q += 4) *reinterpret_cast<float4*>(yr + q) = make_float4(acc[q], acc[q + 1], acc[q + 2], acc[q + 3]);
-        } else {
-#pragma unroll
-            for (int q = 0; q < NR; q++) if (row + q < a.rows) yr[q] = acc[q];
+            for (int q = 0; q < 4; q++) if (row + q < a.rows) yr[q] = acc[q];
         }
     }
     if constexpr (DIST) {
         if (part) {
-            if (active) halo_store<NR>(hd, row, a.rows, acc);
+            if (active) halo_store(hd, row, a.rows, acc);
             __threadfence_system();
             __syncthreads();
             if (tid == 0) halo_signal(hd);
@@ -825,33 +772,38 @@ __global__ void __launch_bounds__(RTT * TPR, MINB) spmv_tile_kernel(const TileAr
 // Persistent CTAs, warp-specialised.  The one-CTA-per-tile kernel above holds a tile's shared memory through three dependent
 // global latencies (descriptor -> line list -> x lines) before it computes anything: with shared memory as the limiting
 // resource that idle time is what caps the bytes in flight (ncu, round 1: 58 % of the stall samples sit in that prologue).
-// Here a CTA is NG groups; a group is one producer warp plus 2*RTT consumer threads (two per block row, one per 32-bit bitmap
-// half) and owns `spg` tile-sized stages of shared memory.  Group g of CTA b takes the tiles b + (g + k NG) gridDim.x, k = 0, 1, ..
-// -- the SMs sweep the matrix together, so the x lines shared by neighbouring tiles are in L2 at the same time.
+// Here a CTA is one producer warp plus 2 * STREAM_RT consumer threads (two per block row, one per 32-bit bitmap half) and owns
+// `spg` tile-sized stages of shared memory.  CTA b takes the tiles b + k gridDim.x, k = 0, 1, .. -- the SMs sweep the matrix
+// together, so the x lines shared by neighbouring tiles are in L2 at the same time.  The kernel runs 64-row tiles only: on the
+// 16- and 32-row tiles of heavy rows it is slower than the per-tile kernel (plan_tiles).
 //   producer (one elected lane): keeps the 64-byte descriptors of its next tiles arriving by cp.async in a small ring, and as
 //     soon as a stage is released issues the tile's bulk copies -- row pointers, bitmaps, x offsets, values, and the tile's x
 //     lines as one copy per run of consecutive lines (three runs for a 5-point stencil; line by line, all lanes, for scattered
 //     tiles) -- all completing on the stage's `full` mbarrier.  A stage waits for ONE memory latency, not three.
 //   consumers: wait for `full`, multiply out of shared memory, store y, arrive on the stage's `empty` mbarrier.
-// No CTA-wide barrier after start-up.  One producer warp serves one group: a warp issues its ~200 instructions per tile at one
-// every few cycles, so a single producer for a whole CTA of seven groups caps the SM at one tile per 0.7 us (measured).
+// No CTA-wide barrier after start-up.  Every 128 consumers need a producer warp of their own: a warp issues its ~200 instructions
+// per tile at one every few cycles, so one producer for seven such consumer groups caps the SM at one tile per 0.7 us (measured).
+// Several groups with a producer each per CTA were slower than one group per CTA (P4096: 6 groups x 1 CTA 69.7 us, 1 x 7 67.8 us).
+constexpr int STREAM_RT = 64;      // block rows per tile
+constexpr int STREAM_CTAS = 7;     // CTAs per SM the kernel's registers must allow (P4096: 7 x 2 stages, the measured optimum)
 // pal: the palette variant -- a 32-byte header (the second 16 bytes: the tile's block and value counts as the last row's end), one
 // 32-bit word per block in place of bitmaps and x offsets (`bm`; `xo` unused), 4-byte relative row pairs
 struct StageLayout { uint32_t bm, xo, val, row, xs, stride; };
-inline StageLayout stage_layout(int rt, int cap_blk, int cap_val, int cap_lines, int vsize, int xsize, bool pal) {
+inline StageLayout stage_layout(int cap_blk, int cap_val, int cap_lines, int vsize, int xsize, bool pal) {
+    constexpr uint32_t rt = STREAM_RT;
     auto up16 = [](uint32_t v) { return (v + 15u) & ~15u; };
     StageLayout s;
     if (pal) {
         s.bm = 32;
         s.xo = s.val = up16(s.bm + (uint32_t)(cap_blk + 4) * 4);
         s.row = up16(s.val + (uint32_t)(cap_val + 16) * vsize);
-        s.xs = up16(s.row + (uint32_t)(rt + 4) * 4);
+        s.xs = up16(s.row + (rt + 4) * 4);
     } else {
         s.bm = 16;                                               // 16-byte header: {p0, v0, staged, -}
         s.xo = up16(s.bm + (uint32_t)(cap_blk + 2) * 8);
         s.val = up16(s.xo + (uint32_t)(cap_blk + 16) * 2);
         s.row = up16(s.val + (uint32_t)(cap_val + 16) * vsize);
-        s.xs = up16(s.row + (uint32_t)(rt + 2) * 8);
+        s.xs = up16(s.row + (rt + 2) * 8);
     }
     s.stride = (s.xs + (uint32_t)cap_lines * 32u * xsize + 16u + 127u) & ~127u;   // + 16: the tridiagonal path reads one element past
     return s;
@@ -861,9 +813,9 @@ template <typename T>
 struct StreamArgs {
     TileArgs<T> t;
     StageLayout so;
-    int32_t spg, ntiles;         // stages per group; tiles of this launch (tile0 .. tile0 + ntiles)
-    int32_t n_static;            // a group's first n_static tiles are its static share (tile slot q0 + k * qstep) ...
-    int32_t* sched;              // ... the rest it claims one at a time from sched[0]; sched[1] counts finished groups.  nullptr: all static
+    int32_t spg, ntiles;         // stages per CTA; tiles of this launch (tile0 .. tile0 + ntiles)
+    int32_t n_static;            // a CTA's first n_static tiles are its static share (tile slot blockIdx.x + k * gridDim.x) ...
+    int32_t* sched;              // ... the rest it claims one at a time from sched[0]; sched[1] counts finished CTAs.  nullptr: all static
 };
 
 __device__ __forceinline__ int4 lds_v4(uint32_t a) {
@@ -887,20 +839,20 @@ __device__ __noinline__ void halo_wait_all(const HaloDev* hd, int lane, bool ful
     if (lane < hd->n_peer) halo_wait(*hd, lane, full_fence);
 }
 __device__ __noinline__ void halo_push_tile(const HaloDev* hd, int row, int rows, bool active, float a0, float a1, float a2, float a3, int gt, int bar_id, int nthreads) {
-    if (active) { const float acc[4] = {a0, a1, a2, a3}; halo_store<4>(*hd, row, rows, acc); }
-    // the group's remote stores happen-before its barrier, the barrier before thread 0's system fence (cumulative), the fence
+    if (active) { const float acc[4] = {a0, a1, a2, a3}; halo_store(*hd, row, rows, acc); }
+    // the consumers' remote stores happen-before their barrier, the barrier before thread 0's system fence (cumulative), the fence
     // before the counter / flag: one fence per pushing tile instead of one per thread -- a system fence stalls its warp for
     // microseconds, and a CTA that stalls finishes its static share of the tiles that much later than everybody else
     asm volatile("bar.sync %0, %1;" ::"r"(bar_id), "r"(nthreads) : "memory");
     if (gt == 0) { __threadfence_system(); halo_signal(*hd); }
 }
 
-// PAL: the matrix has a bitmap palette (see palette_scan_kernel); it is loaded once per CTA, behind the descriptor rings.
-template <typename T, typename X, int RTT, int NG, int MINB, typename H = NoHalo, bool PAL = false>
-__global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(const __grid_constant__ StreamArgs<T> sa, const X* __restrict__ x,
-                                                                               float* __restrict__ y, const __grid_constant__ H hd) {
+// PAL: the matrix has a bitmap palette (see palette_scan_kernel); it is loaded once per CTA, behind the descriptor ring.
+template <typename T, typename X, typename H = NoHalo, bool PAL = false>
+__global__ void __launch_bounds__(32 + STREAM_RT * 2, STREAM_CTAS) spmv_stream_kernel(const __grid_constant__ StreamArgs<T> sa, const X* __restrict__ x,
+                                                                                    float* __restrict__ y, const __grid_constant__ H hd) {
     constexpr bool DIST = !std::is_same<H, NoHalo>::value;
-    constexpr int GT = RTT * 2;            // consumer threads of a group: two per block row
+    constexpr int GT = STREAM_RT * 2;      // consumer threads: two per block row
     constexpr int VA = 16 / sizeof(T);
     constexpr uint32_t SX = sizeof(X);
     constexpr int DR = STREAM_DR, PD = STREAM_PD;
@@ -908,13 +860,14 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
     const TileArgs<T>& a = sa.t;
     const StageLayout so = sa.so;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int spg = sa.spg, nstage = spg * NG;
+    const int spg = sa.spg;
     const uint32_t sbase = smem_u32(smem);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)nstage * so.stride);      // full[nstage], empty[nstage]
-    const uint32_t pal_off = (uint32_t)nstage * (so.stride + 16u) + (uint32_t)NG * (DR * 64u) + 64u;   // PAL: barrier, then the entries
+    uint64_t* full = reinterpret_cast<uint64_t*>(smem + (size_t)spg * so.stride);      // full[spg], empty[spg]
+    uint64_t* empty = full + spg;
+    const uint32_t pal_off = (uint32_t)spg * (so.stride + 16u) + DR * 64u + 64u;        // PAL: barrier, then the entries
     uint64_t* pal_bar = reinterpret_cast<uint64_t*>(smem + pal_off);
     if (tid == 0) {
-        for (int s = 0; s < nstage; s++) { mbar_init(bars + s, 1); mbar_init(bars + nstage + s, GT / 32); }
+        for (int s = 0; s < spg; s++) { mbar_init(full + s, 1); mbar_init(empty + s, GT / 32); }
         if constexpr (PAL) mbar_init(pal_bar, 1);
         mbar_fence_init();
     }
@@ -925,34 +878,27 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
             bulk_g2s(smem + pal_off + 16, a.palette, (uint32_t)a.npal * 16u, pal_bar);
         }
     }
-    const bool is_producer = warp < NG;
-    const int g = NG == 1 ? 0 : (is_producer ? warp : (warp - NG) / (GT / 32));
     const int grid = (int)gridDim.x;
-    // this group's tiles: q_k = blockIdx.x + (g + k NG) * grid, k = 0 .. n_k - 1
-    // Tile slots q = 0 .. ntiles - 1 in launch order.  A group's sequence of slots: q0 + k * qstep for its static share, then slots
-    // claimed from a counter (sa.sched).  Static shares alone leave the kernel as slow as its slowest CTA: a CTA that stalled -- a
-    // system fence after pushing rows to a peer costs microseconds, a tile of a clustered matrix can be several times the average --
-    // finishes its share that much later than the rest.  With the last part of the tiles handed out on demand the others absorb it.
-    const int q0 = (int)blockIdx.x + g * grid, qstep = NG * grid;
+    // Tile slots q = 0 .. ntiles - 1 in launch order.  A CTA's sequence of slots: blockIdx.x + k * grid for its static share, then
+    // slots claimed from a counter (sa.sched).  Static shares alone leave the kernel as slow as its slowest CTA: a CTA that stalled
+    // -- a system fence after pushing rows to a peer costs microseconds, a tile of a clustered matrix can be several times the
+    // average -- finishes its share that much later than the rest.  With the last part of the tiles handed out on demand the others
+    // absorb it.
+    const int q0 = (int)blockIdx.x;
     auto tile_at = [&](int q) {
-        if (a.tile_list) return a.tile_list[q];
         if constexpr (DIST) { q += hd.rot; if (q >= sa.ntiles) q -= sa.ntiles; }
         return a.tile0 + q;
     };
-    // the group's stages and their barriers
-    const uint32_t gbase = sbase + (uint32_t)(g * spg) * so.stride;
-    uint64_t* full = bars + g * spg;
-    uint64_t* empty = bars + nstage + g * spg;
 
-    if (is_producer) {
+    if (warp == 0) {
         // ------------------------------------------------------------------------------------------ producer
         // The descriptors of the next PD tiles travel global -> shared with cp.async (no register is waited on), one commit group
         // per tile; group k is complete once at most PD newer groups are pending.
-        const uint32_t ring = sbase + (uint32_t)nstage * (so.stride + 16u) + (uint32_t)g * (DR * 64u);
-        static_assert(NG * DR * 4 <= 64, "tile ids of the ring live in the 64 spare bytes behind it");
-        const uint32_t tq = sbase + (uint32_t)nstage * (so.stride + 16u) + (uint32_t)NG * (DR * 64u) + (uint32_t)g * (DR * 4u);
+        const uint32_t ring = sbase + (uint32_t)spg * (so.stride + 16u);
+        static_assert(DR * 4 <= 64, "tile ids of the ring live in the 64 spare bytes behind it");
+        const uint32_t tq = ring + DR * 64u;
         const int n_static = sa.sched ? sa.n_static : 0x7fffffff;
-        const int dyn_base = sa.sched ? sa.n_static * qstep : 0;
+        const int dyn_base = sa.sched ? sa.n_static * grid : 0;
         int pending = 0;                  // lane 0: the slot claimed for the next dynamic sequence number, asked for one iteration ahead
         bool ended = false;               // lane 0: a slot past the last tile has been seen (every later one is past it too)
         // descriptor of sequence number k (slot q) -> ring, its tile id -> tq; a slot past the end leaves the end marker (-1)
@@ -969,7 +915,7 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
             cp_async_commit();
         };
         if (lane == 0) {
-            for (int k = 0; k < PD; k++) issue(k, k < n_static ? q0 + k * qstep : (ended ? sa.ntiles : dyn_base + atomicAdd(sa.sched, 1)));
+            for (int k = 0; k < PD; k++) issue(k, k < n_static ? q0 + k * grid : (ended ? sa.ntiles : dyn_base + atomicAdd(sa.sched, 1)));
             if (PD >= n_static && !ended) pending = dyn_base + atomicAdd(sa.sched, 1);
         }
         int s = 0; uint32_t round = 0;
@@ -979,7 +925,7 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
                 // refill the ring, then make sure tile k's descriptor has landed.  The claim for the sequence number after this one
                 // goes out now and is looked at in the next iteration: the atomic's round trip never stalls the warp.
                 const int kk = k + PD;
-                const int q = kk < n_static ? q0 + kk * qstep : (ended ? sa.ntiles : pending);
+                const int q = kk < n_static ? q0 + kk * grid : (ended ? sa.ntiles : pending);
                 issue(kk, q);
                 if (kk + 1 >= n_static && !ended) pending = dyn_base + atomicAdd(sa.sched, 1);
                 cp_async_wait<PD>();
@@ -990,7 +936,7 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
                 // no more tiles: tell the consumers through the next stage's header
                 if (round) mbar_wait(empty + s, (round - 1u) & 1u);
                 if (lane == 0) {
-                    *reinterpret_cast<int4*>(smem + (size_t)(g * spg + s) * so.stride) = make_int4(0, 0, 0, -1);
+                    *reinterpret_cast<int4*>(smem + (size_t)s * so.stride) = make_int4(0, 0, 0, -1);
                     mbar_arrive(full + s);
                 }
                 break;
@@ -1000,9 +946,9 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
             const int p0 = d0.x, nb = d0.y, nv = d0.w, nl = d1.x;
             const uint32_t v0 = (uint32_t)d0.z, v0a = v0 & ~(uint32_t)(VA - 1);
             const bool staged = (d1.y & 1) && nb <= a.cap_blk && nv <= a.cap_val && nl <= a.cap_lines;
-            const int r0 = t * RTT, nrow = min(RTT, a.nbr - r0);
-            const uint32_t sp32 = gbase + (uint32_t)s * so.stride;
-            unsigned char* sp = smem + (size_t)(g * spg + s) * so.stride;
+            const int r0 = t * STREAM_RT, nrow = min(STREAM_RT, a.nbr - r0);
+            const uint32_t sp32 = sbase + (uint32_t)s * so.stride;
+            unsigned char* sp = smem + (size_t)s * so.stride;
             // PAL: nrb = relative row pairs (4 B per block row), n8 = block words from p0a = p0 & ~3; otherwise int2 row pairs (one past
             // the tile's last row), bitmaps from p0 & ~1 and x offsets from p0 & ~7
             const uint32_t nrb = PAL ? (uint32_t)((nrow + 3) & ~3) * 4 : (uint32_t)((nrow + 1 + 1) & ~1) * 8;
@@ -1034,7 +980,7 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
                     asm volatile("fence.proxy.async;" ::: "memory");
                 }
             }
-            // everything above is ready before the stage is: what follows the wait is the stage's critical path (a group has two
+            // everything above is ready before the stage is: what follows the wait is the stage's critical path (a CTA has two
             // stages; a microsecond between a stage's release and its next copies is a microsecond without loads in flight)
             if (round) mbar_wait(empty + s, (round - 1u) & 1u);          // the stage's previous tile has been consumed
             if (staged && nlc < nl) {
@@ -1080,24 +1026,24 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
             if (++s == spg) { s = 0; round++; }
         }
         if (sa.sched && lane == 0) {
-            // the last group to finish claiming re-arms the counters for the next launch that takes this slot
+            // the last CTA to finish claiming re-arms the counters for the next launch that takes this slot
             __threadfence();
-            if (atomicAdd(sa.sched + 1, 1) == NG * grid - 1) { sa.sched[0] = 0; sa.sched[1] = 0; }
+            if (atomicAdd(sa.sched + 1, 1) == grid - 1) { sa.sched[0] = 0; sa.sched[1] = 0; }
         }
     } else {
         // ------------------------------------------------------------------------------------------ consumers
-        const int gt = tid - NG * 32 - g * GT;
+        const int gt = tid - 32;
         const int lbr = gt >> 1, h = gt & 1;
         const uint32_t pal_h = sbase + pal_off + 16u + 8u * (uint32_t)h;    // PAL: this half's 8 bytes of entry 0
         if constexpr (PAL) mbar_wait(pal_bar, 0);
         int s = 0; uint32_t par = 0;
         for (;;) {
             mbar_wait(full + s, par);
-            const uint32_t sb = gbase + (uint32_t)s * so.stride;
+            const uint32_t sb = sbase + (uint32_t)s * so.stride;
             const int4 hdr = lds_v4(sb);                                  // {first block, first value, staged | pushes << 1, tile}
             const int t = hdr.w;
             if (t < 0) break;                                             // the producer ran out of tiles
-            const int r0 = t * RTT, nrow = min(RTT, a.nbr - r0);
+            const int r0 = t * STREAM_RT, nrow = min(STREAM_RT, a.nbr - r0);
             const int p0 = hdr.x; const uint32_t v0a = (uint32_t)hdr.y & ~(uint32_t)(VA - 1);
             const bool staged = (hdr.z & 1) != 0;
             const int row = (r0 + lbr) * 8 + h * 4;
@@ -1139,7 +1085,7 @@ __global__ void __launch_bounds__(NG * (32 + RTT * 2), MINB) spmv_stream_kernel(
             }
             if constexpr (DIST) {
                 if (hdr.z & 2)                                           // the producer found rows of this tile in a push range
-                    halo_push_tile(&hd, row, a.rows, active, acc[0], acc[1], acc[2], acc[3], gt, 1 + g, GT);
+                    halo_push_tile(&hd, row, a.rows, active, acc[0], acc[1], acc[2], acc[3], gt, 1, GT);
             }
             __syncwarp();
             if (lane == 0) mbar_arrive(empty + s);
@@ -1313,17 +1259,17 @@ __device__ __forceinline__ bool is_bundle(const int32_t* __restrict__ brp, int n
     for (int q = 0; q < BUNDLE_ROWS; q++) ok &= brp[g0 + q + 1] - brp[g0 + q] <= BUNDLE_MAXB;
     return ok;
 }
-__global__ void work_count_kernel(const int32_t* __restrict__ brp, int nbr, uint32_t* __restrict__ cnt, int bundles) {
+__global__ void work_count_kernel(const int32_t* __restrict__ brp, int nbr, uint32_t* __restrict__ cnt) {
     int br = blockIdx.x * blockDim.x + threadIdx.x;
     if (br >= nbr) return;
-    if (bundles && is_bundle(brp, nbr, br)) { cnt[br] = (br & (BUNDLE_ROWS - 1)) == 0 ? 1u : 0u; return; }
+    if (is_bundle(brp, nbr, br)) { cnt[br] = (br & (BUNDLE_ROWS - 1)) == 0 ? 1u : 0u; return; }
     int nb = brp[br + 1] - brp[br];
     cnt[br] = nb <= SLICE ? 1u : (uint32_t)((nb + SLICE - 1) / SLICE);
 }
-__global__ void work_fill_kernel(const int32_t* __restrict__ brp, int nbr, const uint32_t* __restrict__ ofs, int4* __restrict__ work, int bundles) {
+__global__ void work_fill_kernel(const int32_t* __restrict__ brp, int nbr, const uint32_t* __restrict__ ofs, int4* __restrict__ work) {
     int br = blockIdx.x * blockDim.x + threadIdx.x;
     if (br >= nbr) return;
-    if (bundles && is_bundle(brp, nbr, br)) {
+    if (is_bundle(brp, nbr, br)) {
         if ((br & (BUNDLE_ROWS - 1)) == 0) work[ofs[br]] = make_int4(br, brp[br], brp[br + BUNDLE_ROWS], 2);
         return;
     }
@@ -1387,14 +1333,13 @@ static int plan_tiles(bmsp_matrix_s* m, cudaStream_t st) {
     int rt = 64;
     const double row_bytes = ((double)m->nblk * (8 + 2 + 16) + (double)m->nnz * vsize) / m->nbr + 8;
     while (rt > 16 && row_bytes * rt > 20.0 * 1024) rt >>= 1;
-    if (const char* e = getenv("BMSP_SPMV_RT")) { const int v = atoi(e); if (v == 16 || v == 32 || v == 64 || v == 128) rt = v; }   // experiments
     m->tile_rows = rt;
-    // Light rows (64-block-row tiles: stencils, bands) stream through the persistent kernel.  Heavy rows (dense blocks: 16- or
-    // 32-row tiles of 17 KB) are bound by the bit walk, not by memory: a stage then feeds only one or two consumer warps and
-    // the one-CTA-per-tile kernel, which keeps 13 such tiles computing per SM, is faster (BC4M: 280 us vs 479 us).
-    // BMSP_SPMV_KERNEL = 1 / 2 forces the per-tile / the streaming kernel (A/B runs).
-    const int force = env_int("BMSP_SPMV_KERNEL", 0);
-    m->spmv_kernel = force == 1 ? 1 : (force == 2 ? 0 : (rt == 64 ? 0 : 1));
+    // Light rows (64-block-row tiles: stencils, bands) stream through the persistent kernel, which runs STREAM_RT-row tiles only.
+    // Heavy rows (dense blocks: 16- or 32-row tiles of 17 KB) are bound by the bit walk, not by memory: a stage then feeds only one
+    // or two consumer warps and the one-CTA-per-tile kernel, which keeps 13 such tiles computing per SM, is faster (BC4M: 280 us vs
+    // 479 us).  BMSP_SPMV_KERNEL=1 is a test hook: it puts the per-tile kernel behind a light matrix, the bit-exact reference of the
+    // streaming kernel.
+    m->spmv_kernel = (rt == STREAM_RT && env_int("BMSP_SPMV_KERNEL", 0) != 1) ? 0 : 1;
     m->xl_pitch = m->spmv_kernel == 1 ? XL_STRIDE : 32;
     const int ntiles = (int)ceil_div(m->nbr, rt);
     std::vector<uint4> pal;                    // kept until the synchronisation below (pageable source of the palette upload)
@@ -1454,8 +1399,7 @@ int plan_spmv(bmsp_matrix_s* m, cudaStream_t st) {
     if (m->spmv_path == 0) return plan_tiles(m, st);
     uint32_t* cnt = nullptr;
     BMSP_TRY(dev_alloc_t(&cnt, (size_t)m->nbr + 1, st));
-    static const int bundles = env_int("BMSP_SPMV_BUNDLES", 1);
-    work_count_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, cnt, bundles);
+    work_count_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, cnt);
     BMSP_KERNEL_CHECK();
     BMSP_TRY(exclusive_scan_u32(cnt, cnt, m->nbr, st));
     uint32_t total = 0;
@@ -1463,7 +1407,7 @@ int plan_spmv(bmsp_matrix_s* m, cudaStream_t st) {
     BMSP_CUDA(cudaStreamSynchronize(st));
     m->n_work = (int32_t)total;
     BMSP_TRY(dev_alloc((void**)&m->work, sizeof(int4) * (size_t)total, st));
-    work_fill_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, cnt, (int4*)m->work, bundles);
+    work_fill_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, cnt, (int4*)m->work);
     BMSP_KERNEL_CHECK();
     m->split_rows = (int32_t*)cnt;           // item offsets per block row, kept for the fix-up
     // sliced block rows (more than one item): listed on the device.  (Items minus block rows no longer says whether there are any:
@@ -1483,26 +1427,29 @@ int plan_spmv(bmsp_matrix_s* m, cudaStream_t st) {
     return BMSP_OK;
 }
 
-template <typename T, typename X, int RTT, int TPR, int MINB, typename H>
+template <typename T, typename X, int RTT, int MINB, typename H>
 static int launch_tile_kernel(const TileArgs<T>& a, const X* x, float* y, const H& hd, int grid, size_t smem, cudaStream_t st) {
-    auto kern = spmv_tile_kernel<T, X, RTT, TPR, MINB, H>;
+    auto kern = spmv_tile_kernel<T, X, RTT, MINB, H>;
     static size_t configured = 0;            // per instantiation
     if (configured < smem || configured == 0) {
         BMSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
         BMSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         configured = std::max<size_t>(smem, 1);
     }
-    kern<<<(unsigned)grid, RTT * TPR, smem, st>>>(a, x, y, hd);
+    kern<<<(unsigned)grid, RTT * 2, smem, st>>>(a, x, y, hd);
     BMSP_KERNEL_CHECK();
     return BMSP_OK;
 }
 
-// Streaming kernel launch.  One group per CTA (NG = 1); MAXB bounds the CTAs per SM the registers allow.  Shared memory decides the
-// rest: as many CTAs per SM as fit with two stages each (a group needs a second stage to have its next tile arriving while it
-// multiplies the current one; P4096: 7 CTAs x 2 stages of 15.4 KB -- the measured optimum, see DESIGN.md section 7).
-template <typename T, typename X, int RTT, int NG, int MAXB, typename H, bool PAL>
+// Streaming kernel launch.  STREAM_CTAS bounds the CTAs per SM the registers allow.  Shared memory decides the rest: as many CTAs
+// per SM as fit with two stages each (a CTA needs a second stage to have its next tile arriving while it multiplies the current
+// one; P4096: 7 CTAs x 2 stages of 15.4 KB -- the measured optimum, see DESIGN.md section 7).
+// The last STREAM_DYN_PCT per cent of every CTA's share are claimed at run time (P4096: 0 % 68.6 us, 12-25 % 66.5 us, 50 % 67.6 us,
+// 100 % 75.6 us -- 32 768 atomics on one address are too many).
+constexpr int STREAM_DYN_PCT = 25;
+template <typename T, typename X, typename H, bool PAL>
 static int launch_stream_kernel(const TileArgs<T>& a, const X* x, float* y, const H& hd, int ntiles, cudaStream_t st, int32_t* sched) {
-    auto kern = spmv_stream_kernel<T, X, RTT, NG, MAXB, H, PAL>;
+    auto kern = spmv_stream_kernel<T, X, H, PAL>;
     static int sms = 0;
     static size_t smem_max = 0;
     if (!sms) {
@@ -1515,19 +1462,17 @@ static int launch_stream_kernel(const TileArgs<T>& a, const X* x, float* y, cons
     }
     StreamArgs<T> sa;
     sa.t = a;
-    sa.so = stage_layout(RTT, a.cap_blk, a.cap_val, a.cap_lines, sizeof(T), sizeof(X), PAL);
+    sa.so = stage_layout(a.cap_blk, a.cap_val, a.cap_lines, sizeof(T), sizeof(X), PAL);
     sa.ntiles = ntiles;
-    const size_t fixed = (size_t)NG * STREAM_DR * 64 + 64 + (PAL ? 16 + (size_t)a.npal * 16 : 0);   // descriptor rings (+ palette)
-    const size_t per_stage = (size_t)NG * (sa.so.stride + 16);
-    static const int want_ctas = env_int("BMSP_SPMV_CTAS", 0), want_spg = env_int("BMSP_SPMV_STAGES", 0);   // experiments
+    const size_t fixed = (size_t)STREAM_DR * 64 + 64 + (PAL ? 16 + (size_t)a.npal * 16 : 0);   // descriptor ring (+ palette)
+    const size_t per_stage = (size_t)sa.so.stride + 16;
     int ctas = 0, spg = 0;
     size_t per_cta = 0;
-    for (int c = want_ctas > 0 ? std::min(want_ctas, MAXB) : MAXB; c >= 1; c--) {
+    for (int c = STREAM_CTAS; c >= 1; c--) {
         per_cta = std::min<size_t>(smem_max / c - 1024 - 256, 227 * 1024);               // 1 KB per resident CTA is the system's; 256 B allocation granule
         const int fit = per_cta > fixed ? (int)((per_cta - fixed) / per_stage) : 0;
         if (fit >= 2 || (c == 1 && fit >= 1)) { ctas = c; spg = std::min(fit, 8); break; }
     }
-    if (want_spg > 0) spg = std::min(spg, want_spg);
     if (ctas < 1 || spg < 1) { set_error("spmv: a tile stage of %u bytes does not fit shared memory", sa.so.stride); return BMSP_ERR_CUDA; }
     sa.spg = spg;
     const size_t smem = (size_t)spg * per_stage + fixed;
@@ -1537,13 +1482,11 @@ static int launch_stream_kernel(const TileArgs<T>& a, const X* x, float* y, cons
         BMSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         configured = std::max<size_t>(smem, 1);
     }
-    const int grid = std::max(1, std::min((int)ceil_div(ntiles, NG), sms * ctas));
-    // the last BMSP_SPMV_DYN percent of every group's share are claimed at run time (0: static shares, 100: every tile is claimed)
-    static const int dyn_pct = std::min(100, std::max(0, env_int("BMSP_SPMV_DYN", 25)));
-    const int share = ntiles / (grid * NG);
-    sa.sched = (sched && dyn_pct > 0 && share >= 2) ? sched : nullptr;
-    sa.n_static = sa.sched ? (int)((int64_t)share * (100 - dyn_pct) / 100) : 0;
-    kern<<<(unsigned)grid, NG * (32 + RTT * 2), smem, st>>>(sa, x, y, hd);
+    const int grid = std::max(1, std::min(ntiles, sms * ctas));
+    const int share = ntiles / grid;
+    sa.sched = (sched && share >= 2) ? sched : nullptr;
+    sa.n_static = sa.sched ? (int)((int64_t)share * (100 - STREAM_DYN_PCT) / 100) : 0;
+    kern<<<(unsigned)grid, 32 + STREAM_RT * 2, smem, st>>>(sa, x, y, hd);
     BMSP_KERNEL_CHECK();
     return BMSP_OK;
 }
@@ -1551,11 +1494,10 @@ static int launch_stream_kernel(const TileArgs<T>& a, const X* x, float* y, cons
 // tile0 / ntiles: path 0 only -- launch the tiles [tile0, tile0 + ntiles) (ntiles < 0: all of them).
 // hd: NoHalo, or HaloDev for the fused multi-GPU product (path 0, fp32 x, all tiles).
 template <typename T, typename X, typename H = NoHalo>
-static int launch_spmv(bmsp_matrix_s* A, const X* x, float* y, cudaStream_t st, int tile0 = 0, int ntiles = -1, const H& hd = H(),
-                       const int32_t* tile_list = nullptr) {
+static int launch_spmv(bmsp_matrix_s* A, const X* x, float* y, cudaStream_t st, int tile0 = 0, int ntiles = -1, const H& hd = H()) {
     if (A->spmv_path == 0) {
         TileArgs<T> a;
-        a.tile0 = tile0; a.tile_list = nullptr;
+        a.tile0 = tile0;
         a.bmps = A->bmps; a.bcol = A->bcol; a.values = (const T*)A->values; a.rowpair = (const int2*)A->tile_rowpair;
         a.desc = (const TileDesc*)A->tile_desc; a.lines = A->tile_lines; a.xoff = A->tile_xoff;
         a.word = A->tile_word; a.rowrel = A->tile_rowrel; a.palette = (const uint4*)A->tile_palette; a.npal = A->spmv_npal;
@@ -1566,32 +1508,18 @@ static int launch_spmv(bmsp_matrix_s* A, const X* x, float* y, cudaStream_t st, 
         const size_t smem = a.so.total;
         const int grid = ntiles < 0 ? (int)ceil_div(A->nbr, rt) : ntiles;
         if (grid <= 0) return BMSP_OK;
-        a.tile_list = tile_list;
         if (A->spmv_kernel == 0) {
-            // streaming kernel: one group (a producer warp + 2 * rt consumer threads) per CTA; CTAs per SM bounded by registers.
-            // A launch over all tiles takes one of the matrix's scheduler slots in turn (launches on different streams may overlap:
-            // they must not share a counter); launches over a tile range (the host-buffer pipeline's chunks) keep static shares.
+            // streaming kernel (tile_rows == STREAM_RT, plan_tiles).  A launch over all tiles takes one of the matrix's scheduler
+            // slots in turn (launches on different streams may overlap: they must not share a counter); launches over a tile range
+            // (the host-buffer pipeline's chunks) keep static shares.
             int32_t* sched = nullptr;
-            if (ntiles < 0 && tile_list == nullptr) {
-                if (A->spmv_sched) sched = A->spmv_sched + 2 * (A->spmv_sched_next++ % SCHED_SLOTS);      // allocated and zeroed by the plan
-            }
-            if (A->spmv_npal > 0) {
-                if (rt == 128) return launch_stream_kernel<T, X, 128, 1, 3, H, true>(a, x, y, hd, grid, st, sched);
-                if (rt == 32) return launch_stream_kernel<T, X, 32, 1, 8, H, true>(a, x, y, hd, grid, st, sched);
-                if (rt == 16) return launch_stream_kernel<T, X, 16, 1, 8, H, true>(a, x, y, hd, grid, st, sched);
-                return launch_stream_kernel<T, X, 64, 1, 7, H, true>(a, x, y, hd, grid, st, sched);
-            }
-            if (rt == 128) return launch_stream_kernel<T, X, 128, 1, 3, H, false>(a, x, y, hd, grid, st, sched);
-            if (rt == 32) return launch_stream_kernel<T, X, 32, 1, 8, H, false>(a, x, y, hd, grid, st, sched);
-            if (rt == 16) return launch_stream_kernel<T, X, 16, 1, 8, H, false>(a, x, y, hd, grid, st, sched);
-            return launch_stream_kernel<T, X, 64, 1, 7, H, false>(a, x, y, hd, grid, st, sched);
+            if (ntiles < 0 && A->spmv_sched) sched = A->spmv_sched + 2 * (A->spmv_sched_next++ % SCHED_SLOTS);      // allocated and zeroed by the plan
+            if (A->spmv_npal > 0) return launch_stream_kernel<T, X, H, true>(a, x, y, hd, grid, st, sched);
+            return launch_stream_kernel<T, X, H, false>(a, x, y, hd, grid, st, sched);
         }
-        // default: one thread per bitmap half; BMSP_SPMV_VARIANT=1: one thread per block row (64-row tiles only).
-        // Measured on P4096: 92.7 us vs 103.5 us (fewer instructions, but too few warps to hide the staging latency).
-        if (rt == 128) return launch_tile_kernel<T, X, 128, 2, 6, H>(a, x, y, hd, grid, smem, st);
-        if (rt == 32) return launch_tile_kernel<T, X, 32, 2, 24, H>(a, x, y, hd, grid, smem, st);
-        if (rt == 16) return launch_tile_kernel<T, X, 16, 2, 32, H>(a, x, y, hd, grid, smem, st);
-        return launch_tile_kernel<T, X, 64, 2, 12, H>(a, x, y, hd, grid, smem, st);
+        if (rt == 32) return launch_tile_kernel<T, X, 32, 24, H>(a, x, y, hd, grid, smem, st);
+        if (rt == 16) return launch_tile_kernel<T, X, 16, 32, H>(a, x, y, hd, grid, smem, st);
+        return launch_tile_kernel<T, X, 64, 12, H>(a, x, y, hd, grid, smem, st);
     }
     const unsigned grid1 = (unsigned)ceil_div(A->n_work, 8), grid2 = (unsigned)ceil_div((int64_t)A->n_split_rows * 32, 256);
     spmv_blockpar_kernel<T, X><<<grid1, 256, 0, st>>>(A->bmps, A->bcol, A->offsets, (const T*)A->values, (const int4*)A->work, A->n_work,
@@ -1843,55 +1771,6 @@ extern "C" int bmsp_halo_status(const bmsp_halo_desc* halo, void* stream, int32_
     return BMSP_OK;
 }
 
-// Multi-GPU product, row-tiled path: which tiles depend on the peers (their x lines leave the rank's own columns) or push rows
-// to them.  These "boundary" tiles run first, in a small launch of the halo variant of the streaming kernel (it waits for the
-// peers' epoch, multiplies, stores the peers' rows over NVLink and publishes the next epoch -- the peers get their rows a whole
-// kernel early); the interior tiles follow in a launch of the plain kernel.  One launch of the halo variant over all tiles cost
-// 75.7 us against 67.9 us for the plain kernel on P4096 (one GPU as its own peer) although 32 of 32768 tiles do anything special.
-__global__ void halo_classify_kernel(const TileDesc* __restrict__ desc, int ntiles, int rt, int rows, int own_c0, int own_c1, int n_push,
-                                     const int* __restrict__ lo, const int* __restrict__ hi, uint32_t* __restrict__ flag) {
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= ntiles) return;
-    const TileDesc d = desc[t];
-    bool b = d.nb > 0 && ((int64_t)d.lmin * 32 < own_c0 || ((int64_t)d.lmax + 1) * 32 > own_c1);
-    const int trow0 = t * rt * 8, trow1 = min(rows, (t + 1) * rt * 8);
-    for (int i = 0; i < n_push; i++) b |= lo[i] < trow1 && hi[i] > trow0;
-    flag[t] = b ? 1u : 0u;
-}
-__global__ void halo_lists_kernel(const uint32_t* __restrict__ flag, const uint32_t* __restrict__ pre, int ntiles, int32_t* __restrict__ list) {
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= ntiles) return;
-    const uint32_t nb = pre[ntiles];
-    list[flag[t] ? pre[t] : nb + ((uint32_t)t - pre[t])] = t;
-}
-static int halo_classify(bmsp_matrix_s* A, const HaloDev& h, cudaStream_t st) {
-    int32_t key[18] = {h.own_c0, h.own_c1};
-    for (int i = 0; i < h.n_push; i++) { key[2 + 2 * i] = h.lo[i]; key[3 + 2 * i] = h.hi[i]; }
-    if (A->halo_n_boundary >= 0 && !memcmp(key, A->halo_key, sizeof(key))) return BMSP_OK;
-    const int ntiles = (int)ceil_div(A->nbr, A->tile_rows);
-    if (!A->halo_tiles) BMSP_TRY(dev_alloc_t(&A->halo_tiles, (size_t)ntiles + 1, st));
-    uint32_t *flag = nullptr, *pre = nullptr; int* rng = nullptr;
-    BMSP_TRY(dev_alloc_t(&flag, (size_t)ntiles + 1, st));
-    BMSP_TRY(dev_alloc_t(&pre, (size_t)ntiles + 2, st));
-    BMSP_TRY(dev_alloc_t(&rng, 2 * HALO_MAX, st));
-    BMSP_CUDA(cudaMemcpyAsync(rng, h.lo, sizeof(int) * HALO_MAX, cudaMemcpyHostToDevice, st));
-    BMSP_CUDA(cudaMemcpyAsync(rng + HALO_MAX, h.hi, sizeof(int) * HALO_MAX, cudaMemcpyHostToDevice, st));
-    halo_classify_kernel<<<(unsigned)ceil_div(ntiles, 256), 256, 0, st>>>((const TileDesc*)A->tile_desc, ntiles, A->tile_rows, A->rows, h.own_c0, h.own_c1,
-                                                                        h.n_push, rng, rng + HALO_MAX, flag);
-    BMSP_KERNEL_CHECK();
-    BMSP_TRY(exclusive_scan_u32(flag, pre, ntiles, st));
-    halo_lists_kernel<<<(unsigned)ceil_div(ntiles, 256), 256, 0, st>>>(flag, pre, ntiles, A->halo_tiles);
-    BMSP_KERNEL_CHECK();
-    uint32_t nb = 0;
-    BMSP_CUDA(cudaMemcpyAsync(&nb, pre + ntiles, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    BMSP_CUDA(cudaMemcpyAsync(&A->halo_first, A->halo_tiles, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    BMSP_CUDA(cudaStreamSynchronize(st));          // also: the pageable h.lo / h.hi copies above are done
-    dev_free(flag, st); dev_free(pre, st); dev_free(rng, st);
-    A->halo_n_boundary = (int32_t)nb;
-    memcpy(A->halo_key, key, sizeof(key));
-    return BMSP_OK;
-}
-
 extern "C" int bmsp_spmv_halo(bmsp_matrix_t A, const float* x_ext, float* y_own, const bmsp_halo_desc* halo, uint32_t wait_epoch,
                               uint32_t signal_epoch, void* stream) {
     if (!A || !x_ext || !y_own) { set_error("bmsp_spmv_halo: null argument"); return BMSP_ERR_INVALID; }
@@ -1904,9 +1783,10 @@ extern "C" int bmsp_spmv_halo(bmsp_matrix_t A, const float* x_ext, float* y_own,
     h.wait_epoch = wait_epoch; h.signal_epoch = signal_epoch;
     if (A->rows == 0 || h.n_peer == 0) return A->rows == 0 ? BMSP_OK : bmsp_spmv(A, x_ext, BMSP_F32, y_own, stream);
     if (A->spmv_path < 0) BMSP_TRY(plan_spmv(A, st));
-    static int fused = -1;
-    if (fused < 0) { const char* e = getenv("BMSP_HALO_FUSED"); fused = e ? atoi(e) : 1; }
-    if (A->spmv_path == 0 && fused) {
+    if (A->spmv_path == 0) {
+        // One launch of the halo variant over all tiles.  Running the tiles that wait or push in a launch of their own ahead of the
+        // plain kernel over the rest was slower on P4096 (one GPU as its own peer): 85.7 us on the same stream (the small launch is
+        // all latency) and 79.5 us on a side stream, against 69.7 us.
         // tiles that own pushed rows (union of the ranges' tile intervals); they count down to the signal
         const int64_t rpt = (int64_t)A->tile_rows * 8;
         std::vector<std::pair<int64_t, int64_t>> iv;
@@ -1920,55 +1800,11 @@ extern "C" int bmsp_spmv_halo(bmsp_matrix_t A, const float* x_ext, float* y_own,
         }
         if (n == 0) { h.solo_tile = 0; n = 1; }
         h.n_sig = (uint32_t)n;
-        static int rotate = -1;
-        if (rotate < 0) { const char* e = getenv("BMSP_HALO_ROTATE"); rotate = e ? atoi(e) : 1; }
-        h.rot = rotate ? (int)(ceil_div(A->nbr, A->tile_rows) / 2) : 0;
-        static int split = -1;
-        // 0: one launch of the halo variant over all tiles (76 us on P4096, one GPU as its own peer; the plain kernel takes 68 us);
-        // 1: boundary launch, then interior launch on the same stream (85.7 us: the small launch is all latency);
-        // 2: the boundary launch on a side stream NEXT TO the interior launch
-        // (measured 79.5 us: the side-stream launch buys nothing either -- the default stays one launch)
-        if (split < 0) { const char* e = getenv("BMSP_HALO_SPLIT"); split = e ? atoi(e) : 0; }
-        const int ntiles = (int)ceil_div(A->nbr, A->tile_rows);
-        if (split && A->spmv_kernel == 0) {
-            BMSP_TRY(halo_classify(A, h, st));
-            const int nb = A->halo_n_boundary;
-            if (nb * 4 <= ntiles) {
-                // boundary tiles (the solo tile, if any, is tile 0: make sure it is among them) with the halo variant, the rest plain
-                if (h.solo_tile >= 0 && nb == 0) h.solo_tile = -2;           // nothing pushes and nothing waits: signal from a kernel of its own
-                cudaStream_t sb = st;
-                if (split == 2 && nb > 0 && ntiles > nb) {
-                    if (!A->halo_side) {
-                        BMSP_CUDA(cudaStreamCreateWithFlags(&A->halo_side, cudaStreamNonBlocking));
-                        BMSP_CUDA(cudaEventCreateWithFlags(&A->halo_fork, cudaEventDisableTiming));
-                        BMSP_CUDA(cudaEventCreateWithFlags(&A->halo_join, cudaEventDisableTiming));
-                    }
-                    sb = A->halo_side;
-                    BMSP_CUDA(cudaEventRecord(A->halo_fork, st));              // both launches read what the previous step wrote
-                    BMSP_CUDA(cudaStreamWaitEvent(sb, A->halo_fork, 0));
-                }
-                if (nb > 0) {
-                    if (h.solo_tile >= 0) h.solo_tile = A->halo_first;        // the first boundary tile signals on behalf of a rank that pushes nothing
-                    BMSP_TRY((A->dtype == BMSP_F16 ? launch_spmv<__half, float, HaloDev>(A, x_ext, y_own, sb, 0, nb, h, A->halo_tiles)
-                                                  : launch_spmv<float, float, HaloDev>(A, x_ext, y_own, sb, 0, nb, h, A->halo_tiles)));
-                    if (sb != st) BMSP_CUDA(cudaEventRecord(A->halo_join, sb));
-                } else {
-                    halo_wait_kernel<<<1, 32, 0, st>>>(h);
-                    BMSP_KERNEL_CHECK();
-                    halo_flag_kernel<<<1, 32, 0, st>>>(h);
-                    BMSP_KERNEL_CHECK();
-                }
-                if (ntiles > nb)
-                    BMSP_TRY((A->dtype == BMSP_F16 ? launch_spmv<__half, float, NoHalo>(A, x_ext, y_own, st, 0, ntiles - nb, NoHalo(), A->halo_tiles + nb)
-                                                  : launch_spmv<float, float, NoHalo>(A, x_ext, y_own, st, 0, ntiles - nb, NoHalo(), A->halo_tiles + nb)));
-                if (sb != st) BMSP_CUDA(cudaStreamWaitEvent(st, A->halo_join, 0));      // the step is complete on the caller's stream
-                return BMSP_OK;
-            }
-        }
+        h.rot = (int)(ceil_div(A->nbr, A->tile_rows) / 2);
         return A->dtype == BMSP_F16 ? launch_spmv<__half, float, HaloDev>(A, x_ext, y_own, st, 0, -1, h)
                                     : launch_spmv<float, float, HaloDev>(A, x_ext, y_own, st, 0, -1, h);
     }
-    // block-parallel path (and BMSP_HALO_FUSED=0): wait kernel, product, push kernel
+    // block-parallel path: wait kernel, product, push kernel
     halo_wait_kernel<<<1, 32, 0, st>>>(h);
     BMSP_KERNEL_CHECK();
     BMSP_TRY(bmsp_spmv(A, x_ext, BMSP_F32, y_own, stream));

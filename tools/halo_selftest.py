@@ -61,5 +61,5 @@ y_ref = y.clone()
 halo = timeit(halo_step)
 torch.cuda.synchronize()
 ok = torch.equal(y, y_ref) and torch.equal(sink[:GRID], y_ref[:GRID]) and torch.equal(sink[GRID:2 * GRID], y_ref[nr - GRID:])
-print(f"HALO_SELFTEST plain_us={plain:.2f} halo_variant_us={halo:.2f} rotate={os.environ.get('BMSP_HALO_ROTATE', '1')} fused={os.environ.get('BMSP_HALO_FUSED', '1')} "
+print(f"HALO_SELFTEST plain_us={plain:.2f} halo_variant_us={halo:.2f} "
       f"results_match={ok} signalled_epoch={int(out_flags[0])}")

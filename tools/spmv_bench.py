@@ -1,4 +1,4 @@
-"""Times bmsp_spmv on one generator config (CUDA events, inputs larger than L2).  BMSP_SPMV_VARIANT selects the kernel build.
+"""Times bmsp_spmv on one generator config (CUDA events, inputs larger than L2).  BMSP_LIB_PATH selects the library build.
 usage: python tools/spmv_bench.py [p4096|p2048|bc|u1m|rmat20] [reps]"""
 import os
 import sys
@@ -50,6 +50,6 @@ def stream_bytes():
 
 sb = stream_bytes()
 sb_txt = f"stream_MB={sb / 1e6:.1f} stream_GBps={sb / us / 1e3:.1f}" if sb else "stream_MB=n/a"
-print(f"SPMV {which} variant={os.environ.get('BMSP_SPMV_VARIANT', '0')} rows={nr} nnz={A.nnz} blocks={A.block_num} "
+print(f"SPMV {which} rows={nr} nnz={A.nnz} blocks={A.block_num} "
       f"us={us:.2f} GBps={nbytes / us / 1e3:.1f} {sb_txt} frac6468={nbytes / us / 1e3 / 6468.3:.3f} first_call_ms={plan_ms:.1f} "
       f"ysum={float(y.double().sum()):.6e}")
