@@ -25,9 +25,22 @@
 
 namespace bmsp {
 
+// the passes; as the template argument of apply_pair, drain and enumerate_row: what is done with a surviving pair
 enum { PASS_COUNT = 0, PASS_FILL = 1, PASS_NUMERIC = 2, PASS_NUMERIC_MMA = 3 };
-enum { MODE_SETBITS = 0, MODE_FILL = 1, MODE_NUMERIC = 2, MODE_MMA = 3 };
 constexpr int QSLOTS = 192;   // per-warp queue: 64 pairs (uint2) + 32 staged PairMeta (32 B each) for the MMA drain
+
+// Counters and maxima the kernels reduce into: one device allocation per product, zeroed first, read back by field.
+struct Counters {
+    int32_t max_words;              // rowinfo_kernel: the widest bit set of a block row, in 32-bit words
+    int32_t max_c_item;             // COUNT: the most C blocks of a work item (sizes FILL's shared C block stage)
+    int32_t max_nnz_item;           // FILL: the most C values of a work item
+    int32_t max_c_row;              // COUNT: the most C blocks of a block row (the MMA pass runs row by row)
+    int32_t queue[2];               // work-queue heads: the main launch, the heavy-row launch
+    unsigned long long surviving;   // COUNT: surviving pairs
+    unsigned long long sum_words;   // rowinfo_kernel: bit-set words over all block rows
+    unsigned long long max_cand;    // rowinfo_kernel: the most candidate pairs of a block row
+    unsigned long long sum_cand;    // rowinfo_kernel: candidate pairs
+};
 
 struct GemmArgs {
     const int32_t* a_brp; const int32_t* a_bcol; const uint64_t* a_bmps; const uint8_t* a_kmask; const uint64_t* a_off; const __half* a_val;
@@ -55,13 +68,12 @@ struct GemmArgs {
     uint32_t* row_count;       // COUNT out: C blocks per row (indexed row - row_begin)
     uint32_t* row_surv;        // COUNT out: surviving pairs per row; FILL/NUMERIC in: exclusive scan of it
     uint2* surv_list;          // FILL out / NUMERIC in: (A block, B block) of every surviving pair, row-segmented
-    int32_t* maxes;            // [0] max words, [1] max C blocks per row, [2] max C values per row
+    Counters* ctr;
     const int32_t* c_brp;      // FILL/NUMERIC in: C block-row pointers (indexed row - row_begin)
     uint64_t* c_keys; uint64_t* c_bmps; int32_t* c_bcol; uint8_t* c_kmask;
     uint64_t* c_off;           // FILL out: value offsets relative to the row; NUMERIC: rebased to absolute
     uint64_t* row_nnz;         // FILL out: values per row; NUMERIC in: exclusive scan of it (row value base)
     float* c_val;
-    unsigned long long* stats; // [0] candidate pairs, [1] surviving pairs (COUNT pass)
 };
 
 // boolean 8x8 product of an A bitmap (row-major) and a B bitmap in transposed-operand form:
@@ -129,9 +141,7 @@ __global__ void pack_meta_kernel(const uint64_t* __restrict__ bmps, const int32_
 __global__ void __launch_bounds__(256) rowinfo_kernel(const int32_t* __restrict__ a_brp, const int32_t* __restrict__ a_bcol,
                                                       const int32_t* __restrict__ b_brp, const int32_t* __restrict__ b_bcol,
                                                       int row_begin, int row_end, int2* __restrict__ rowinfo,
-                                                      unsigned long long* __restrict__ cand, int* __restrict__ maxes,
-                                                      unsigned long long* __restrict__ sum_words, unsigned long long* __restrict__ max_cand,
-                                                      unsigned long long* __restrict__ sum_cand) {
+                                                      unsigned long long* __restrict__ cand, Counters* __restrict__ ctr) {
     __shared__ unsigned long long s_words, s_maxc, s_cand;
     __shared__ int s_maxw;
     const int lane = threadIdx.x & 31;
@@ -167,20 +177,25 @@ __global__ void __launch_bounds__(256) rowinfo_kernel(const int32_t* __restrict_
     if (lane == 0) { atomicMax(&s_maxw, w_maxw); atomicAdd(&s_words, w_sum); atomicMax(&s_maxc, w_maxc); atomicAdd(&s_cand, w_cand); }
     __syncthreads();
     if (threadIdx.x == 0) {
-        if (s_maxw) atomicMax(maxes, s_maxw);
-        if (s_words) atomicAdd(sum_words, s_words);
-        if (s_maxc) atomicMax(max_cand, s_maxc);
-        if (s_cand) atomicAdd(sum_cand, s_cand);
+        if (s_maxw) atomicMax(&ctr->max_words, s_maxw);
+        if (s_words) atomicAdd(&ctr->sum_words, s_words);
+        if (s_maxc) atomicMax(&ctr->max_cand, s_maxc);
+        if (s_cand) atomicAdd(&ctr->sum_cand, s_cand);
     }
 }
 
-// CTA-wide exclusive scan over popc(bitset words) -> wrank (may be null); returns the total to every thread.
-__device__ __forceinline__ uint32_t rank_words(const uint32_t* bitset, uint32_t* wrank, int nwords, uint32_t* s_tmp) {
+__device__ __forceinline__ uint32_t popc(uint32_t w) { return __popc(w); }
+__device__ __forceinline__ uint32_t popc(uint64_t w) { return __popcll(w); }
+
+// CTA-wide exclusive scan of popc(words[i]), i < n: the prefix goes to out[i] (out may be null: the total only); returns the total
+// to every thread.  Ranks the bit set's words (32-bit) and scans the C blocks' value counts (64-bit bitmaps).
+template <typename W, typename O>
+__device__ __forceinline__ uint32_t scan_popc(const W* words, O* out, int n, uint32_t* s_tmp) {
     const int T = blockDim.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const int per = (nwords + T - 1) / T;
-    const int w0 = min(tid * per, nwords), w1 = min(w0 + per, nwords);
+    const int per = (n + T - 1) / T;
+    const int w0 = min(tid * per, n), w1 = min(w0 + per, n);
     uint32_t s = 0;
-    for (int w = w0; w < w1; w++) s += __popc(bitset[w]);
+    for (int w = w0; w < w1; w++) s += popc(words[w]);
     uint32_t inc = s;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -201,7 +216,7 @@ __device__ __forceinline__ uint32_t rank_words(const uint32_t* bitset, uint32_t*
     }
     __syncthreads();
     uint32_t run = s_tmp[wid] + inc - s;
-    if (wrank) for (int w = w0; w < w1; w++) { wrank[w] = run; run += __popc(bitset[w]); }
+    if (out) for (int w = w0; w < w1; w++) { out[w] = run; run += popc(words[w]); }
     const uint32_t total = s_tmp[32];
     __syncthreads();
     return total;
@@ -219,7 +234,7 @@ struct RowCtx {
     uint64_t* cbmp;      // FILL: staging (shared or global C.bmps+c0); NUMERIC: shared copy or null
     uint32_t* coff;      // NUMERIC: value offsets relative to the row, or null (global mode)
     float* acc;          // NUMERIC: shared accumulators or null (global atomics)
-    float* dense;        // NUMERIC_MMA: [ccount][64] fp32, lane-private slots (cell (r,c) at (c*4 + r/2) + 32*(r&1))
+    float* dense;        // NUMERIC_MMA: [ccount][64] fp32, two slots per lane (cell (r,c) at (c*4 + r/2) + 32*(r&1))
 };
 
 // index of the row of a work item that owns v, given the rows' ascending start offsets (A blocks, bit-set words or C blocks)
@@ -241,13 +256,13 @@ __device__ __forceinline__ int local_row(const int* bounds, int nr, int v) {
 // pairs' loads in flight per thread before it touches the first result (A/B on one box: U1M numeric 10.65 -> 9.55 ms, R-MAT-18
 // 146 -> 109 ms; the same batching in FILL and in the 8-lanes-per-pair walk cost more in registers than it hid in latency)
 struct PairIn { uint4 pm; uint4 bv8; uint64_t abmp; uint32_t aoff; };
-template <int MODE>
+template <int PASS>
 __device__ __forceinline__ PairIn load_pair(const GemmArgs& g, int a, int b) {
     PairIn in;
     in.pm = __ldg(g.b_pm + 2 * (int64_t)b);
-    in.bv8 = MODE == MODE_FILL ? make_uint4(0, 0, 0, 0) : __ldg(g.b_pm + 2 * (int64_t)b + 1);     // same sector
+    in.bv8 = PASS == PASS_FILL ? make_uint4(0, 0, 0, 0) : __ldg(g.b_pm + 2 * (int64_t)b + 1);     // same sector
     in.abmp = g.a_bmps[a];
-    in.aoff = MODE == MODE_FILL ? 0u : (uint32_t)g.a_off[a];
+    in.aoff = PASS == PASS_FILL ? 0u : (uint32_t)g.a_off[a];
     return in;
 }
 // value k (< 8) of a B block out of its record's inline copy
@@ -256,7 +271,7 @@ __device__ __forceinline__ float inline_val(const uint4& v, int k) {
     return __half2float(__ushort_as_half((unsigned short)((k & 1) ? (w >> 16) : (w & 0xFFFFu))));
 }
 
-template <int MODE>
+template <int PASS>
 __device__ __forceinline__ void apply_pair(const GemmArgs& g, const RowCtx& r, int a, const PairIn& in, int arow = -1) {
     const uint4 pm = in.pm;
     const uint64_t abmp = in.abmp, bbmp = ((uint64_t)pm.y << 32) | pm.x;
@@ -265,7 +280,7 @@ __device__ __forceinline__ void apply_pair(const GemmArgs& g, const RowCtx& r, i
     const int wi = r.wo[rl] + (j >> 5);
     const uint32_t word = r.bitset[wi];
     const int c = (int)r.wrank[wi] + __popc(word & ((1u << (j & 31)) - 1u));
-    if (MODE == MODE_FILL) {
+    if (PASS == PASS_FILL) {
         const uint64_t pb = pair_bitmap(abmp, bbmp);
         unsigned int* w = reinterpret_cast<unsigned int*>(&r.cbmp[c]);      // native 32-bit ATOMS.OR, not a 64-bit CAS loop
         if ((uint32_t)pb) atomicOr(w, (unsigned int)pb);
@@ -318,11 +333,6 @@ __device__ __forceinline__ int pair_class(uint64_t abmp, uint64_t bbmp) {
     return 8 - ((ca - 1) * 3 + (cb - 1));
 }
 
-template <int MODE>
-__device__ __forceinline__ void process_pair(const GemmArgs& g, const RowCtx& r, int a, int b, int arow = -1) {
-    apply_pair<MODE>(g, r, a, load_pair<MODE>(g, a, b), arow);
-}
-
 // ---- tensor-core path (dense blocks) -----------------------------------------------------------------
 // Two halves of an 8x8 fp16 operand row for mma.m16n8k8: the cells p0 = g*8 + 2t and p0+1 of a block, packed
 // as .f16x2 (absent cells are 0).  Works for the A block (cell = row*8 + k) and for the transposed-operand B
@@ -341,7 +351,7 @@ __device__ __forceinline__ uint32_t frag_pair(uint64_t bmp, const __half* __rest
 // shared staging area.  Stage 2: walk the batch; consecutive pairs that share the A block are multiplied two at a
 // time by one mma.sync.m16n8k8 (A-operand = the two B^t blocks stacked, B-operand = the A block, D = the two 8x8
 // fp32 products transposed); the fragments of the next step are loaded before the current MMA is issued.  Each
-// lane owns two fixed slots of every dense C block, so the accumulation needs neither atomics nor warp syncs.
+// lane owns two fixed slots of every dense C block, so the accumulation needs no warp syncs.
 struct PairMeta { uint64_t abmp, bbmp; uint32_t aoff, boff; int32_t cidx; uint32_t a; };   // 32 bytes
 
 __device__ __forceinline__ void drain_mma(const GemmArgs& g, const RowCtx& r, const uint2* q, int n, PairMeta* sm) {
@@ -380,37 +390,31 @@ __device__ __forceinline__ void drain_mma(const GemmArgs& g, const RowCtx& r, co
         asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5}, {%6}, {%0,%1,%2,%3};"
                      : "+f"(d0), "+f"(d1), "+f"(d2), "+f"(d3) : "r"(fa0), "r"(fa1), "r"(fb));
         // several warps of the CTA work on different A blocks of the row and may meet in a C block: shared-memory float atomics
-        // (one instruction each); a lone warp keeps its lane-private read-modify-write
+        // (one instruction each)
         float* a0 = r.dense + c0 * 64 + lane;
-        if (blockDim.x > 32) {
-            atomicAdd(a0, d0); atomicAdd(a0 + 32, d1);
-            if (two) { float* a1 = r.dense + c1 * 64 + lane; atomicAdd(a1, d2); atomicAdd(a1 + 32, d3); }
-        } else {
-            a0[0] += d0; a0[32] += d1;
-            if (two) { float* a1 = r.dense + c1 * 64 + lane; a1[0] += d2; a1[32] += d3; }
-        }
+        atomicAdd(a0, d0); atomicAdd(a0 + 32, d1);
+        if (two) { float* a1 = r.dense + c1 * 64 + lane; atomicAdd(a1, d2); atomicAdd(a1 + 32, d3); }
         i = nxt; fb = nfb; fa0 = nfa0; fa1 = nfa1; c0 = nc0; c1 = nc1; two = ntwo; cur_a = na;
     }
     __syncwarp();
 }
 
-template <int MODE>
+template <int PASS>
 __device__ __forceinline__ void drain(const GemmArgs& g, const RowCtx& r, const uint2* q, int n) {
-    if constexpr (MODE == MODE_MMA) {
+    if constexpr (PASS == PASS_NUMERIC_MMA) {
         drain_mma(g, r, q, n, reinterpret_cast<PairMeta*>(const_cast<uint2*>(q) + 64));
     } else {
         const int lane = threadIdx.x & 31;
-        if (lane < n) { const uint2 e = q[lane]; process_pair<MODE>(g, r, (int)e.x, (int)e.y); }
+        if (lane < n) { const uint2 e = q[lane]; apply_pair<PASS>(g, r, (int)e.x, load_pair<PASS>(g, (int)e.x, (int)e.y)); }
     }
 }
 
 // Candidate walk, four B blocks per lane and step: `slots` A blocks at a time, G lanes per A block, each lane
 // tests one aligned 32-bit word of B's inner-dimension masks (kmask) against the replicated mask of its A block.
-// Survivors set their C block column in the row's bit set; with LIST they are also appended to the row's segment
-// of the global pair list (one shared cursor bump per warp and step).
-template <bool LIST, bool STATS, bool BITS = true>
-__device__ __forceinline__ void enumerate_vec(const GemmArgs& g, const RowCtx& r, uint2* list, uint32_t* s_cursor,
-                                              unsigned long long& n_cand, uint32_t& n_surv) {
+// COUNT (!LIST): survivors set their C block column in the row's bit set and are counted per row.  FILL (LIST): they
+// are appended to the row's segment of the global pair list (one shared cursor bump per warp and step).
+template <bool LIST>
+__device__ __forceinline__ void enumerate_vec(const GemmArgs& g, const RowCtx& r, uint2* list, uint32_t* s_cursor, uint32_t& n_surv) {
     const int T = blockDim.x, tid = threadIdx.x, lane = tid & 31;
     const int Gs = g.G, slots = T / Gs, slot = tid / Gs, gl = tid % Gs;
     const int niter = (r.a1 - r.a0 + slots - 1) / slots;
@@ -438,11 +442,7 @@ __device__ __forceinline__ void enumerate_vec(const GemmArgs& g, const RowCtx& r
                 const int lo = max(b0 - bb, 0), hi = min(b1 - bb, 4);          // valid bytes [lo, hi)
                 const uint32_t vm = (0xFFFFFFFFu << (8 * lo)) & (hi >= 4 ? 0xFFFFFFFFu : ~(0xFFFFFFFFu << (8 * hi)));
                 nz = __vcmpne4(km4 & am4, 0u) & vm;                              // 0xFF in every surviving byte
-                if (STATS) { n_cand += (unsigned)(hi - lo); }
             }
-            const int cnt = __popc(nz) >> 3;
-            if (STATS) { n_surv += cnt; if (r.nr > 1 && cnt) atomicAdd(&r.rsurv[rl], (uint32_t)cnt); }   // single row: reduced by the caller
-            uint32_t rem = nz;
             if (LIST) {
                 // recompute per-byte positions without packing tricks (at most 4 survivors per lane)
                 uint32_t total = 0, base = 0;
@@ -461,12 +461,16 @@ __device__ __forceinline__ void enumerate_vec(const GemmArgs& g, const RowCtx& r
                     for (int i = 0; i < 4; i++)
                         if ((nz >> (8 * i)) & 1u) list[base + p4[i]] = make_uint2((uint32_t)a, (uint32_t)(bb + i));
                 }
-            }
-            while (BITS && rem) {
-                const int i = (__ffs(rem) - 1) >> 3;
-                rem &= ~(0xFFu << (8 * i));
-                const int j = g.b_bcol[bb + i] - jb;
-                atomicOr(&r.bitset[wb + (j >> 5)], 1u << (j & 31));
+            } else {
+                const int cnt = __popc(nz) >> 3;
+                n_surv += cnt;
+                if (r.nr > 1 && cnt) atomicAdd(&r.rsurv[rl], (uint32_t)cnt);      // single row: reduced by the caller
+                for (uint32_t rem = nz; rem;) {
+                    const int i = (__ffs(rem) - 1) >> 3;
+                    rem &= ~(0xFFu << (8 * i));
+                    const int j = g.b_bcol[bb + i] - jb;
+                    atomicOr(&r.bitset[wb + (j >> 5)], 1u << (j & 31));
+                }
             }
         }
     }
@@ -506,45 +510,10 @@ __global__ void fine_fill_kernel(const int32_t* __restrict__ brp, const uint8_t*
     }
 }
 
-// CTA-wide exclusive scan of popc(bmp[c]), c < n: writes the 64-bit prefix to off[c] and returns the total.
-__device__ __forceinline__ uint32_t scan_popc64(const uint64_t* bmp, uint64_t* off, int n, uint32_t* s_tmp) {
-    const int T = blockDim.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const int per = (n + T - 1) / T;
-    const int c0 = min(tid * per, n), c1 = min(c0 + per, n);
-    uint32_t s = 0;
-    for (int c = c0; c < c1; c++) s += __popcll(bmp[c]);
-    uint32_t inc = s;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        uint32_t t = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += t;
-    }
-    if (lane == 31) s_tmp[wid] = inc;
-    __syncthreads();
-    if (wid == 0) {
-        uint32_t v = lane < (T >> 5) ? s_tmp[lane] : 0, vi = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            uint32_t t = __shfl_up_sync(0xffffffffu, vi, o);
-            if (lane >= o) vi += t;
-        }
-        s_tmp[lane] = vi - v;
-        if (lane == 31) s_tmp[32] = vi;
-    }
-    __syncthreads();
-    uint32_t run = s_tmp[wid] + inc - s;
-    for (int c = c0; c < c1; c++) { off[c] = run; run += __popcll(bmp[c]); }
-    const uint32_t total = s_tmp[32];
-    __syncthreads();
-    return total;
-}
-
-// Walk the row's candidate pairs: `slots` A blocks at a time, G lanes per A block striding over the
-// B block row.  MODE_SETBITS marks C block columns; the other modes compact survivors through a
-// per-warp queue so that all 32 lanes work on surviving pairs.
-template <int MODE, bool STATS>
-__device__ __forceinline__ void enumerate_row(const GemmArgs& g, const RowCtx& r, uint2* q, unsigned long long& n_cand,
-                                              unsigned long long& n_surv) {
+// Walk the row's candidate pairs (MMA pass, one block row per work item): `slots` A blocks at a time, G lanes per A block striding
+// over the B block row; survivors are compacted through a per-warp queue so that all 32 lanes work on surviving pairs.
+template <int PASS>
+__device__ __forceinline__ void enumerate_row(const GemmArgs& g, const RowCtx& r, uint2* q) {
     const int T = blockDim.x, tid = threadIdx.x, lane = tid & 31;
     const int Gs = g.G, slots = T / Gs, slot = tid / Gs, gl = tid % Gs;
     int qn = 0;
@@ -564,32 +533,25 @@ __device__ __forceinline__ void enumerate_row(const GemmArgs& g, const RowCtx& r
             const int b = b0 + off + gl;
             const bool valid = b < b1;
             const bool surv = valid && (am & g.b_kmask[b]) != 0;
-            if (STATS) { n_cand += valid; n_surv += surv; }
-            if (MODE == MODE_SETBITS) {
-                if (surv) { const int j = g.b_bcol[b] - r.jbase; atomicOr(&r.bitset[j >> 5], 1u << (j & 31)); }
-            } else {
-                const uint32_t m = __ballot_sync(0xffffffffu, surv);
-                if (surv) q[qn + __popc(m & ((1u << lane) - 1u))] = make_uint2((uint32_t)a, (uint32_t)b);
-                qn += __popc(m);
+            const uint32_t m = __ballot_sync(0xffffffffu, surv);
+            if (surv) q[qn + __popc(m & ((1u << lane) - 1u))] = make_uint2((uint32_t)a, (uint32_t)b);
+            qn += __popc(m);
+            __syncwarp();
+            if (qn >= 32) {
+                drain<PASS>(g, r, q, 32);
                 __syncwarp();
-                if (qn >= 32) {
-                    drain<MODE>(g, r, q, 32);
-                    __syncwarp();
-                    uint2 t = make_uint2(0, 0);
-                    const bool mv = lane + 32 < qn;
-                    if (mv) t = q[32 + lane];
-                    __syncwarp();
-                    if (mv) q[lane] = t;
-                    qn -= 32;
-                    __syncwarp();
-                }
+                uint2 t = make_uint2(0, 0);
+                const bool mv = lane + 32 < qn;
+                if (mv) t = q[32 + lane];
+                __syncwarp();
+                if (mv) q[lane] = t;
+                qn -= 32;
+                __syncwarp();
             }
         }
     }
-    if (MODE != MODE_SETBITS) {
-        drain<MODE>(g, r, q, qn);
-        __syncwarp();
-    }
+    drain<PASS>(g, r, q, qn);
+    __syncwarp();
 }
 
 // Walk the surviving pairs of a work item through B's fine index: 8 lanes per A block, one bucket per bit of its kmask, the
@@ -614,7 +576,7 @@ __device__ __forceinline__ void fine_entry(const GemmArgs& g, const RowCtx& r, i
         in.pm = __ldg(g.f_rec + 2 * (int64_t)f);
         in.bv8 = FMODE == 2 ? __ldg(g.f_rec + 2 * (int64_t)f + 1) : make_uint4(0, 0, 0, 0);
         in.abmp = abmp; in.aoff = aoff;
-        apply_pair<FMODE == 1 ? MODE_FILL : MODE_NUMERIC>(g, r, a, in);
+        apply_pair<FMODE == 1 ? PASS_FILL : PASS_NUMERIC>(g, r, a, in);
     }
 }
 template <int FMODE, bool STATS>
@@ -636,8 +598,8 @@ __device__ __forceinline__ void fine_bucket(const GemmArgs& g, const RowCtx& r, 
         i0.pm = i1.pm = make_uint4(0, 0, 0, 0); i0.bv8 = i1.bv8 = make_uint4(0, 0, 0, 0);
         if (s0) { i0.pm = __ldg(g.f_rec + 2 * (int64_t)f); if (FMODE == 2) i0.bv8 = __ldg(g.f_rec + 2 * (int64_t)f + 1); }
         if (s1) { i1.pm = __ldg(g.f_rec + 2 * (int64_t)(f + step)); if (FMODE == 2) i1.bv8 = __ldg(g.f_rec + 2 * (int64_t)(f + step) + 1); }
-        if (s0) apply_pair<FMODE == 1 ? MODE_FILL : MODE_NUMERIC>(g, r, a, i0);
-        if (s1) apply_pair<FMODE == 1 ? MODE_FILL : MODE_NUMERIC>(g, r, a, i1);
+        if (s0) apply_pair<FMODE == 1 ? PASS_FILL : PASS_NUMERIC>(g, r, a, i0);
+        if (s1) apply_pair<FMODE == 1 ? PASS_FILL : PASS_NUMERIC>(g, r, a, i1);
     }
     if (f < f1 && !(below && (g.f_kmask[f] & below))) fine_entry<FMODE, STATS>(g, r, a, rl, jb, wb, abmp, aoff, f, cnt);
     }
@@ -719,7 +681,7 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
     __shared__ uint32_t s_cls[PAIR_CLASSES];           // FILL: pairs per class of the work item (zero between work items)
     if (tid < PAIR_CLASSES) s_cls[tid] = 0;
 
-    unsigned long long n_cand = 0, n_surv_total = 0;
+    unsigned long long n_surv_total = 0;
     int my_max1 = 0, my_max2 = 0, my_max3 = 0;         // per-thread maxima, published once when the CTA retires
     uint2* q = s_queue + wid * QSLOTS;
     const int R = g.row_list ? 1 : g.group;
@@ -787,22 +749,21 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
             __syncthreads();
             uint32_t ns = 0;
             if (g.f_ptr) enumerate_fine<0, true>(g, r, ns);
-            else enumerate_vec<false, true>(g, r, nullptr, nullptr, n_cand, ns);      // bits; survivors per row into s_rsurv
-            n_surv_total += ns;
+            else enumerate_vec<false>(g, r, nullptr, nullptr, ns);      // bits; survivors per row into s_rsurv
             if (nr == 1) {
 #pragma unroll
                 for (int o = 16; o; o >>= 1) ns += __shfl_xor_sync(0xffffffffu, ns, o);
                 if (lane == 0 && ns) atomicAdd(&s_rsurv[0], ns);
             }
             __syncthreads();
-            const uint32_t total = rank_words(r.bitset, nr > 1 ? r.wrank : nullptr, nwords, s_tmp);
+            const uint32_t total = scan_popc(r.bitset, nr > 1 ? r.wrank : nullptr, nwords, s_tmp);
             if (tid < nr) {
                 uint32_t cnt = total;
                 if (nr > 1) {
                     const int w0 = s_wo[tid], w1 = s_wo[tid + 1];
                     cnt = (w1 < nwords ? r.wrank[w1] : total) - (w0 < nwords ? r.wrank[w0] : total);
                 }
-                g.row_count[lrow + tid] = cnt; g.row_surv[lrow + tid] = s_rsurv[tid];
+                g.row_count[lrow + tid] = cnt; g.row_surv[lrow + tid] = s_rsurv[tid]; n_surv_total += s_rsurv[tid];
                 my_max3 = max(my_max3, (int)cnt);                                // largest single row (dense-block NUMERIC runs row by row)
             }
             if (tid == 0) my_max1 = max(my_max1, (int)total);
@@ -817,12 +778,12 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
                 // fine index: no pair list at all -- bits from the 5-byte bucket entries, then the records once
                 enumerate_fine<0, false>(g, r, ns);
                 __syncthreads();
-                rank_words(r.bitset, r.wrank, nwords, s_tmp);
+                scan_popc(r.bitset, r.wrank, nwords, s_tmp);
                 enumerate_fine<1, false>(g, r, ns);
             } else {
             // pair list only: a survivor's C block column comes with its packed B record (one sector, fetched here for the first time
             // and again -- from L2 -- by the pair pass below) instead of a separate random read of b_bcol per survivor
-            enumerate_vec<true, false, false>(g, r, list, s_cursor, n_cand, ns);
+            enumerate_vec<true>(g, r, list, s_cursor, ns);
             __syncthreads();
             for (uint32_t e = tid; e < nsurv; e += T) {
                 const uint2 pr = list[e];
@@ -831,7 +792,7 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
                 atomicOr(&r.bitset[r.wo[rl] + (j >> 5)], 1u << (j & 31));
             }
             __syncthreads();
-            rank_words(r.bitset, r.wrank, nwords, s_tmp);
+            scan_popc(r.bitset, r.wrank, nwords, s_tmp);
             if (nsurv <= (uint32_t)g.sort_max) {
                 // apply the pairs and leave the segment sorted by class for NUMERIC (counting sort through shared counters; a thread
                 // keeps its <= SORT_K pairs in registers between reading and rewriting the segment)
@@ -842,8 +803,8 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
                     slot[k] = 0xFFFFFFFFu;
                     if (e < nsurv) {
                         const uint2 pr = list[e];
-                        const PairIn in = load_pair<MODE_FILL>(g, (int)pr.x, (int)pr.y);
-                        apply_pair<MODE_FILL>(g, r, (int)pr.x, in);
+                        const PairIn in = load_pair<PASS_FILL>(g, (int)pr.x, (int)pr.y);
+                        apply_pair<PASS_FILL>(g, r, (int)pr.x, in);
                         const int cls = pair_class(in.abmp, ((uint64_t)in.pm.y << 32) | in.pm.x);
                         mine[k] = pr;
                         slot[k] = ((uint32_t)cls << 24) | atomicAdd(&s_cls[cls], 1u);
@@ -867,7 +828,7 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
                 __syncthreads();
                 if (tid < PAIR_CLASSES) s_cls[tid] = 0;
             } else {
-                for (uint32_t e = tid; e < nsurv; e += T) { const uint2 pr = list[e]; process_pair<MODE_FILL>(g, r, (int)pr.x, (int)pr.y); }
+                for (uint32_t e = tid; e < nsurv; e += T) { const uint2 pr = list[e]; apply_pair<PASS_FILL>(g, r, (int)pr.x, load_pair<PASS_FILL>(g, (int)pr.x, (int)pr.y)); }
             }
             }
             __syncthreads();
@@ -893,7 +854,7 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
             __syncthreads();
             // value offsets: scanned over the work item, then made relative to each block's own row (NUMERIC rebases them once the
             // row totals are scanned)
-            const uint32_t rn = scan_popc64(r.cbmp, g.c_off + c0, ccount, s_tmp);
+            const uint32_t rn = scan_popc(r.cbmp, g.c_off + c0, ccount, s_tmp);
             if (tid <= nr) { const int cs = s_cbr[tid] - c0; s_rowoff[tid] = cs < ccount ? (uint32_t)g.c_off[c0 + cs] : rn; }
             __syncthreads();
             if (nr > 1)
@@ -922,7 +883,7 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
                 for (int v = tid; v < ccount * 64; v += T) s_dense[v] = 0.f;
             }
             __syncthreads();
-            rank_words(r.bitset, r.wrank, nwords, s_tmp);
+            scan_popc(r.bitset, r.wrank, nwords, s_tmp);
             if (PASS == PASS_NUMERIC && g.f_ptr) {
                 uint32_t ns = 0;
                 enumerate_fine<2, false>(g, r, ns);
@@ -936,31 +897,35 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
                         h = 0;
                         for (uint32_t e0 = 0; e0 < nsurv; e0 += T) h += (uint32_t)__syncthreads_count(e0 + tid < nsurv && !(list[e0 + tid].x & PAIR_LIGHT_FLAG));
                     }
-                    for (uint64_t e = tid; e < (uint64_t)h * 8u; e += T) { const uint2 pr = list[e >> 3]; process_pair<MODE_NUMERIC>(g, r, (int)(pr.x & ~PAIR_LIGHT_FLAG), (int)pr.y, (int)(e & 7u)); }
-                    for (uint32_t e = h + tid; e < nsurv; e += T) { const uint2 pr = list[e]; process_pair<MODE_NUMERIC>(g, r, (int)(pr.x & ~PAIR_LIGHT_FLAG), (int)pr.y); }
+                    for (uint64_t e = tid; e < (uint64_t)h * 8u; e += T) {
+                        const uint2 pr = list[e >> 3]; const int a = (int)(pr.x & ~PAIR_LIGHT_FLAG);
+                        apply_pair<PASS_NUMERIC>(g, r, a, load_pair<PASS_NUMERIC>(g, a, (int)pr.y), (int)(e & 7u));
+                    }
+                    for (uint32_t e = h + tid; e < nsurv; e += T) {
+                        const uint2 pr = list[e]; const int a = (int)(pr.x & ~PAIR_LIGHT_FLAG);
+                        apply_pair<PASS_NUMERIC>(g, r, a, load_pair<PASS_NUMERIC>(g, a, (int)pr.y));
+                    }
                 } else if (MAXT == 1024) {            // 32 registers per thread: one pair at a time
-                    for (uint32_t e = tid; e < nsurv; e += T) { const uint2 pr = list[e]; process_pair<MODE_NUMERIC>(g, r, (int)pr.x, (int)pr.y); }
+                    for (uint32_t e = tid; e < nsurv; e += T) { const uint2 pr = list[e]; apply_pair<PASS_NUMERIC>(g, r, (int)pr.x, load_pair<PASS_NUMERIC>(g, (int)pr.x, (int)pr.y)); }
                 } else {
                     for (uint32_t e = tid; e < nsurv; e += 2 * T) {       // two pairs' loads in flight
                         const bool two = e + T < nsurv;
                         const uint2 p0 = list[e], p1 = two ? list[e + T] : make_uint2(0, 0);
-                        const PairIn i0 = load_pair<MODE_NUMERIC>(g, (int)p0.x, (int)p0.y);
+                        const PairIn i0 = load_pair<PASS_NUMERIC>(g, (int)p0.x, (int)p0.y);
                         PairIn i1 = i0;
-                        if (two) i1 = load_pair<MODE_NUMERIC>(g, (int)p1.x, (int)p1.y);
-                        apply_pair<MODE_NUMERIC>(g, r, (int)p0.x, i0);
-                        if (two) apply_pair<MODE_NUMERIC>(g, r, (int)p1.x, i1);
+                        if (two) i1 = load_pair<PASS_NUMERIC>(g, (int)p1.x, (int)p1.y);
+                        apply_pair<PASS_NUMERIC>(g, r, (int)p0.x, i0);
+                        if (two) apply_pair<PASS_NUMERIC>(g, r, (int)p1.x, i1);
                     }
                 }
             } else if (!fit) {
                 // too many C blocks for the dense accumulators: scalar products into global memory.  The row's pairs are enumerated
                 // again rather than read from the pair list: FILL may have written the list a group of rows at a time
-                unsigned long long dc = 0, ds = 0;
-                enumerate_row<MODE_NUMERIC, false>(g, r, q, dc, ds);
+                enumerate_row<PASS_NUMERIC>(g, r, q);
             } else {
-                unsigned long long dc = 0, ds = 0;
                 // every warp enumerates its own A blocks, so the pairs of an A block stay adjacent in its queue (two B blocks per MMA);
                 // walking FILL's pair list instead of enumerating a third time measured no faster (BC4M 19.2 vs 18.6 ms)
-                enumerate_row<MODE_MMA, false>(g, r, q, dc, ds);
+                enumerate_row<PASS_NUMERIC_MMA>(g, r, q);
             }
             __syncthreads();
             if (PASS == PASS_NUMERIC && fit) for (int v = tid; v < rownnz; v += T) g.c_val[vbase + v] = s_acc[v];
@@ -977,13 +942,13 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
         }
         __syncthreads();
     }
-    if (my_max1) atomicMax(g.maxes + 1, my_max1);
-    if (my_max2) atomicMax(g.maxes + 2, my_max2);
-    if (my_max3) atomicMax(g.maxes + 3, my_max3);
+    if (my_max1) atomicMax(&g.ctr->max_c_item, my_max1);
+    if (my_max2) atomicMax(&g.ctr->max_nnz_item, my_max2);
+    if (my_max3) atomicMax(&g.ctr->max_c_row, my_max3);
     if (PASS == PASS_COUNT) {
 #pragma unroll
-        for (int o = 16; o; o >>= 1) { n_cand += __shfl_xor_sync(0xffffffffu, n_cand, o); n_surv_total += __shfl_xor_sync(0xffffffffu, n_surv_total, o); }
-        if (lane == 0) { atomicAdd(g.stats, n_cand); atomicAdd(g.stats + 1, n_surv_total); }
+        for (int o = 16; o; o >>= 1) n_surv_total += __shfl_xor_sync(0xffffffffu, n_surv_total, o);
+        if (lane == 0) atomicAdd(&g.ctr->surviving, n_surv_total);
     }
 }
 
@@ -995,11 +960,6 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
 // B^t blocks are stacked as the 16x8 A-operand of mma.m16n8k8, the A block is the B-operand, D = the two 8x8 products transposed;
 // each lane owns two fixed slots of every dense C block in shared memory, so the accumulation needs no atomics.  The loads of the
 // next pair of B blocks are issued before the current MMA.  C block index of a pair: a per-row table over the row's column span.
-struct DenseArgs {
-    const int32_t* c_brp;      // [nrows+1] C block-row pointers (row - row_begin)
-    const uint64_t* row_nnz;   // [nrows+1] value base of every row
-    int32_t wcols;             // C block columns per window: a warp's accumulators cover wcols dense blocks (wcols * 256 bytes)
-};
 
 // values l and l + 32 of a block (cnt values from vals + off) in one register: low half = value l, high half = value l + 32
 __device__ __forceinline__ uint32_t load_block_vals(const __half* __restrict__ vals, uint32_t off, int cnt, int lane) {
@@ -1016,16 +976,16 @@ __device__ __forceinline__ uint32_t frag_shfl(uint64_t bmp, uint32_t packed, int
     return ((two & 2u) ? v0 : 0u) | (((two & 1u) ? v1 : 0u) << 16);
 }
 
-// One warp per block row; the row's C block columns are covered in windows of `wcols` columns so that a warp's dense accumulators
-// stay small (wcols = 16: 4 KB per warp, 48 warps per SM; with all of a 63-column row resident the SM held 12 warps and the pass
-// waited on its own loads: 23.7 ms).  Per A block the lanes test the B block row in parallel (block column inside the window,
-// inner-dimension masks overlap) and the survivors are taken two at a time off the ballot.
-template <int WARPS>
-__global__ void __launch_bounds__(WARPS * 32) spgemm_dense_kernel(GemmArgs g, DenseArgs da) {
-    extern __shared__ __align__(16) unsigned char smem[];
+// One warp per block row; the row's C block columns are covered in windows of DENSE_WCOLS columns so that a warp's dense
+// accumulators stay small (16 columns: 4 KB per warp, 48 warps per SM; BC4M NUMERIC 17.7 -> 10.1 ms against the generic MMA pass;
+// with all of a 63-column row resident the SM held 12 warps and the pass waited on its own loads: 23.7 ms).  Per A block the lanes
+// test the B block row in parallel (block column inside the window, inner-dimension masks overlap) and the survivors are taken two
+// at a time off the ballot.
+constexpr int DENSE_WARPS = 4, DENSE_WCOLS = 16;
+__global__ void __launch_bounds__(DENSE_WARPS * 32) spgemm_dense_kernel(GemmArgs g) {
+    __shared__ float s_dense_all[DENSE_WARPS * DENSE_WCOLS * 64];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int wcols = da.wcols;
-    float* s_dense = reinterpret_cast<float*>(smem) + (size_t)wid * wcols * 64;
+    float* s_dense = s_dense_all + wid * DENSE_WCOLS * 64;
     const int p0 = (lane >> 2) * 8 + (lane & 3) * 2;
     const int P0 = (lane & 3) * 16 + (lane >> 2);          // slot L <-> cell (r = 2t, c = g), slot L + 32 <-> (2t + 1, g)
     const int nrows = g.row_end - g.row_begin;
@@ -1035,15 +995,15 @@ __global__ void __launch_bounds__(WARPS * 32) spgemm_dense_kernel(GemmArgs g, De
         lrow = __shfl_sync(0xffffffffu, lrow, 0);
         if (lrow >= nrows) break;
         const int row = g.row_begin + lrow;
-        const int c0 = da.c_brp[lrow], ccount = da.c_brp[lrow + 1] - c0;
+        const int c0 = g.c_brp[lrow], ccount = g.c_brp[lrow + 1] - c0;
         if (ccount == 0) continue;
-        const uint64_t vbase = da.row_nnz[lrow];
+        const uint64_t vbase = g.row_nnz[lrow];
         for (int c = lane; c < ccount; c += 32) g.c_off[c0 + c] += vbase;       // FILL left row-relative offsets: absolute from here on
         const int jfirst = g.c_bcol[c0], jlast = g.c_bcol[c0 + ccount - 1];
         const int a0 = g.a_brp[row], a1 = g.a_brp[row + 1];
         int cdone = 0;                                                           // C blocks of the windows already stored
-        for (int jw = jfirst; jw <= jlast; jw += wcols) {
-            for (int v = lane; v < wcols * 64; v += 32) s_dense[v] = 0.f;
+        for (int jw = jfirst; jw <= jlast; jw += DENSE_WCOLS) {
+            for (int v = lane; v < DENSE_WCOLS * 64; v += 32) s_dense[v] = 0.f;
             __syncwarp();
             for (int a = a0; a < a1; a++) {
                 const int k = g.a_bcol[a];
@@ -1053,7 +1013,7 @@ __global__ void __launch_bounds__(WARPS * 32) spgemm_dense_kernel(GemmArgs g, De
                 for (int bb = b0; bb < b1; bb += 32) {
                     const int b = bb + lane;
                     bool in = false;
-                    if (b < b1) { const int j = g.b_bcol[b] - jw; in = j >= 0 && j < wcols && (am & g.b_kmask[b]) != 0; }
+                    if (b < b1) { const int j = g.b_bcol[b] - jw; in = j >= 0 && j < DENSE_WCOLS && (am & g.b_kmask[b]) != 0; }
                     uint32_t mask = __ballot_sync(0xffffffffu, in);
                     if (!mask) continue;
                     if (!have_fb) {
@@ -1092,7 +1052,7 @@ __global__ void __launch_bounds__(WARPS * 32) spgemm_dense_kernel(GemmArgs g, De
             // the window's C blocks out: compact the dense accumulators through C's bitmaps
             while (cdone < ccount) {
                 const int j = g.c_bcol[c0 + cdone] - jw;
-                if (j >= wcols) break;
+                if (j >= DENSE_WCOLS) break;
                 const uint64_t bmp = g.c_bmps[c0 + cdone];
                 float* dst = g.c_val + g.c_off[c0 + cdone];
                 if ((bmp >> (63 - P0)) & 1ull) dst[rank64(bmp, P0)] = s_dense[j * 64 + lane];
@@ -1195,6 +1155,178 @@ static int launch_pass(GemmArgs& g, int T, int sms, cudaStream_t st, const RowSp
     return BMSP_OK;
 }
 
+static double block_density(const bmsp_matrix_s* m) { return m->nblk ? (double)m->nnz / m->nblk : 0.0; }
+static int clampi(double v, int lo, int hi) { return (int)std::min<double>(hi, std::max<double>(lo, v)); }
+
+// Row statistics and the heavy-row split.  rowinfo_kernel writes every block row's bit-set span and candidate pairs and reduces
+// the maxima and sums into ctr; they are read back into h.  Rows with at least BMSP_SPGEMM_HEAVY candidate pairs (default 2^20;
+// 0 disables the split) are heavy when the heaviest row has four times that.  The variable is a test hook:
+// tests/test_gpu_spgemm.py::test_heavy_row_split lowers it so that small inputs run the split.
+static int plan_rows(const bmsp_matrix_s* A, const bmsp_matrix_s* Bt, int rb, int re, int sms, int2* rowinfo, unsigned long long* cand,
+                     Counters* ctr, Counters& h, RowSplit& sp, cudaStream_t st) {
+    const int nrows = re - rb;
+    if (nrows > 0) {
+        rowinfo_kernel<<<(unsigned)std::min<int64_t>(ceil_div(nrows, 8), (int64_t)sms * 8), 256, 0, st>>>(A->brp, A->bcol, Bt->brp, Bt->bcol, rb, re,
+                                                                                                        rowinfo, cand, ctr);
+        BMSP_KERNEL_CHECK();
+    }
+    BMSP_CUDA(cudaMemcpyAsync(&h, ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));
+    const char* e = getenv("BMSP_SPGEMM_HEAVY");
+    const long long heavy_min = e ? atoll(e) : (1ll << 20);
+    if (heavy_min <= 0 || nrows <= 1 || h.max_cand < 4ull * (unsigned long long)heavy_min) return BMSP_OK;
+    std::vector<unsigned long long> hc((size_t)nrows);
+    BMSP_CUDA(cudaMemcpyAsync(hc.data(), cand, sizeof(unsigned long long) * (size_t)nrows, cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));
+    std::vector<int32_t> heavy, order;
+    for (int i = 0; i < nrows; i++) if (hc[i] >= (unsigned long long)heavy_min) heavy.push_back(rb + i);
+    std::sort(heavy.begin(), heavy.end(), [&](int32_t x, int32_t y) { return hc[x - rb] != hc[y - rb] ? hc[x - rb] > hc[y - rb] : x < y; });
+    order = heavy;
+    for (int i = 0; i < nrows; i++) if (hc[i] < (unsigned long long)heavy_min) order.push_back(rb + i);
+    sp.n_heavy = (int)heavy.size(); sp.n_light = nrows - sp.n_heavy;
+    BMSP_TRY(dev_alloc_t(&sp.list, (size_t)nrows + 1, st));
+    BMSP_CUDA(cudaMemcpyAsync(sp.list, order.data(), sizeof(int32_t) * (size_t)nrows, cudaMemcpyHostToDevice, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));       // `order` dies with this scope
+    BMSP_CUDA(cudaStreamCreateWithFlags(&sp.side, cudaStreamNonBlocking));
+    BMSP_CUDA(cudaEventCreateWithFlags(&sp.fork, cudaEventDisableTiming));
+    BMSP_CUDA(cudaEventCreateWithFlags(&sp.join, cudaEventDisableTiming));
+    sp.active = sp.n_heavy > 0;
+    return BMSP_OK;
+}
+
+// B's packed block records: built once per B operand, reused by later products
+static int ensure_pmeta(bmsp_matrix_s* Bt, cudaStream_t st) {
+    if (Bt->pmeta || Bt->nblk == 0) return BMSP_OK;
+    BMSP_TRY(dev_alloc(&Bt->pmeta, 2 * sizeof(uint4) * (size_t)Bt->nblk, st));
+    pack_meta_kernel<<<(unsigned)ceil_div(Bt->nblk, 256), 256, 0, st>>>(Bt->bmps, Bt->bcol, Bt->offsets, (const __half*)Bt->values, Bt->nnz,
+                                                                      (uint4*)Bt->pmeta, Bt->nblk);
+    BMSP_KERNEL_CHECK();
+    return BMSP_OK;
+}
+
+// Fine index of B for sparse-block operands (about one value per block: uniform random, R-MAT): examined once per B operand, by
+// the rule below only (U1M A*A: 30.8 ms by the candidate scan, 18.9 ms through the buckets).
+static int ensure_fine_index(bmsp_matrix_s* Bt, const bmsp_matrix_s* A, cudaStream_t st) {
+    if (Bt->fine_state != 0 || Bt->nblk == 0 || (int64_t)Bt->nbr * 8 + 1 >= 0x7FFFFFFFll) return BMSP_OK;
+    if (!(block_density(Bt) <= 2.0 && block_density(A) <= 4.0)) return BMSP_OK;
+    const size_t nb = (size_t)Bt->nbr * 8;
+    uint32_t* fp = nullptr;
+    BMSP_TRY(dev_alloc_t(&fp, nb + 2, st));
+    uint32_t longest = 0, total = 0;
+    const int status = [&]() -> int {
+        BMSP_CUDA(cudaMemsetAsync(fp, 0, sizeof(uint32_t) * (nb + 2), st));
+        fine_count_kernel<<<(unsigned)ceil_div(Bt->nblk, 256), 256, 0, st>>>(Bt->keys, Bt->kmask, Bt->nblk, fp);
+        BMSP_KERNEL_CHECK();
+        // the longest bucket: slot nb + 1 of the zeroed array
+        fine_max_kernel<<<(unsigned)ceil_div((int64_t)nb, 256), 256, 0, st>>>(fp, (int64_t)nb, fp + nb + 1);
+        BMSP_KERNEL_CHECK();
+        BMSP_CUDA(cudaMemcpyAsync(&longest, fp + nb + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        BMSP_TRY(exclusive_scan_u32(fp, fp, (int64_t)nb, st));
+        BMSP_CUDA(cudaMemcpyAsync(&total, fp + nb, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        BMSP_CUDA(cudaStreamSynchronize(st));
+        return BMSP_OK;
+    }();
+    if (status != BMSP_OK) { dev_free(fp, st); return status; }
+    // worth it while the buckets replicate little (a block with m inner indices sits in m buckets) and are of similar length:
+    // a power-law B (R-MAT) has hub buckets of 10^4 entries next to a mean of 2, and the candidate scan, which spreads a B block
+    // row over up to 32 lanes, handles those better (R-MAT-18 A*A: 164 ms by scan, 181 ms through the buckets)
+    const double mean_bucket = (double)total / std::max<double>(1.0, (double)nb);
+    const bool even = (double)longest <= 32.0 * std::max(mean_bucket, 1.0) || longest <= 512;
+    if (!((double)total <= 1.5 * (double)Bt->nblk && even)) { dev_free(fp, st); Bt->fine_state = -1; return BMSP_OK; }
+    Bt->fine_ptr = fp; Bt->fine_n = total;
+    BMSP_TRY(dev_alloc_t(&Bt->fine_bcol, (size_t)total + 4, st));
+    BMSP_TRY(dev_alloc_t(&Bt->fine_kmask, (size_t)total + 16, st));
+    BMSP_TRY(dev_alloc(&Bt->fine_rec, 2 * sizeof(uint4) * ((size_t)total + 1), st));
+    fine_fill_kernel<<<(unsigned)ceil_div((int64_t)nb, 128), 128, 0, st>>>(Bt->brp, Bt->kmask, (const uint4*)Bt->pmeta, Bt->nbr, fp, Bt->fine_bcol,
+                                                                         Bt->fine_kmask, (uint4*)Bt->fine_rec);
+    BMSP_KERNEL_CHECK();
+    Bt->fine_state = 1;
+    return BMSP_OK;
+}
+
+// The numeric path: the requested one, else by about dA * dB / 8 products per surviving pair (dA, dB: values per block) -- scalar
+// lanes for sparse blocks, mma.sync from 40 on
+static int numeric_path(const bmsp_matrix_s* A, const bmsp_matrix_s* Bt, const bmsp_spgemm_opts* opts) {
+    const int path = opts ? opts->numeric_path : -1;
+    return path >= 0 ? path : (block_density(A) * block_density(Bt) / 8.0 >= 40.0 ? 1 : 0);
+}
+
+struct Plan {
+    int T;           // threads per CTA of COUNT, FILL and the scalar NUMERIC pass
+    int mma_batch;   // work items per queue atomic of the generic MMA pass
+};
+
+// Launch shape of the passes from the operands' averages and the row statistics: fills g's shape fields.
+static Plan plan_launch(GemmArgs& g, const bmsp_matrix_s* A, const bmsp_matrix_s* Bt, int nrows, const Counters& h, bool split,
+                        bool fine, int path) {
+    const double avgB = Bt->nbr ? (double)Bt->nblk / Bt->nbr : 0.0;
+    const double avgA = A->nbr ? (double)A->nblk / A->nbr : 0.0;
+    const double avg_cand = avgA * avgB;
+    // G lanes share one A block, each lane tests 4 B blocks per step
+    int G = 1;
+    while (G < 32 && G * 4 < avgB) G <<= 1;
+    // Tiny rows (stencils: 25 candidate pairs per block row) are processed 16 rows at a time by 128-thread CTAs: one warp per row
+    // leaves the SM at 32 one-warp CTAs, each waiting on its own chain of dependent loads (P4096 A*A: 21.7 ms, cuSPARSE 13.0 ms;
+    // 8 rows per work item: 12.7 ms, 16: 12.3 ms).  P4096 has 2.1 M block rows: one atomic on the queue head per row and pass cost
+    // more than the rows
+    const int group = (avg_cand <= 96 && !split && (int64_t)16 * h.max_words <= 8192) ? 16 : 1;
+    int T = group > 1 ? 128 : (avg_cand <= 96 ? 32 : (avg_cand <= 2048 ? 128 : 256));
+    // Walking B's fine index a row's passes wait on record loads and are held to 3-4 CTAs per SM by the row's bit set in shared
+    // memory: more threads per CTA are more loads in flight for the same shared memory (512 threads; no measurement of 256 / 512 /
+    // 1024 is recorded)
+    if (fine && T == 256 && !split) T = 512;
+    g.G = G;
+    g.group = group;
+    // (four / two lanes per pair with two / four rows each were measured on P4096: NUMERIC 8.35 / 8.97 ms against 7.45 ms with eight)
+    g.split8 = block_density(A) >= 4.0;
+    // FILL sorts its pair-list segments by class only for the pass that reads them, the scalar NUMERIC pass with 8 lanes per pair
+    // (P4096 A*A: 11.5 ms unsorted, 8.0 ms sorted)
+    g.sort_max = (g.split8 && path == 0) ? SORT_K * T : 0;
+    g.batch = group > 1 ? 2 : (avg_cand <= 96 ? 32 : (avg_cand <= 2048 ? 4 : 1));
+    // Shared-memory capacities decide how many CTAs an SM holds, and these passes are latency-bound: size them for the rows
+    // that can use them.  When every row fits, take the maxima; when the typical row would not fit anyway (R-MAT: C rows of
+    // 10^4..10^5 blocks spanning every block column), keep the CTAs small -- those rows run from global scratch / global
+    // atomics either way and need the occupancy (R-MAT-17 NUMERIC: 102 KB per CTA = 2 CTAs per SM, 14 % issue utilisation).
+    const double avg_words = nrows ? (double)h.sum_words / nrows : 0.0;
+    g.cap_words = (int64_t)group * h.max_words <= 8192 ? std::max(1, group * h.max_words) : (avg_words > 4096.0 ? 256 : 8192);
+    g.max_words = group * h.max_words;
+    return Plan{T, avg_cand <= 96 ? 32 : 1};
+}
+
+// NUMERIC: the dense-block kernel for narrow rows of dense blocks, the generic mma.sync pass for the other dense-block products,
+// the scalar pass for sparse blocks
+static int run_numeric(GemmArgs& g, const bmsp_matrix_s* C, const Counters& h, const Plan& plan, int path, const RowSplit& sp, int nrows,
+                       int sms, cudaStream_t st) {
+    if (path == 1 && !sp.active && (int64_t)h.max_words * 32 <= 1024) {
+        // narrow rows: one warp per block row, dense accumulators for a window of C columns in shared memory
+        int occ = 0;
+        BMSP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, spgemm_dense_kernel, DENSE_WARPS * 32, 0));
+        if (occ < 1) { set_error("spgemm dense pass does not fit"); return BMSP_ERR_CUDA; }
+        BMSP_CUDA(cudaMemsetAsync(g.work_counter, 0, sizeof(int32_t), st));
+        const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((int64_t)sms * occ, ceil_div(nrows, DENSE_WARPS)));
+        spgemm_dense_kernel<<<grid, DENSE_WARPS * 32, 0, st>>>(g);
+        BMSP_KERNEL_CHECK();
+        return BMSP_OK;
+    }
+    if (path == 1) {
+        const int max_c_row = std::max(1, h.max_c_row);
+        GemmArgs gm = g;
+        gm.cap_c = std::min(max_c_row, 192);
+        if (max_c_row > gm.cap_c) BMSP_CUDA(cudaMemsetAsync(C->values, 0, (size_t)C->nnz * 4, st));
+        gm.group = 1; gm.batch = plan.mma_batch;          // one block row per work item: pairs of an A block stay adjacent
+        // two warps per block row, sharing the row's accumulators (BC4M numeric, one box: 32 threads 19.5 ms, 64: 17.7 ms, 128:
+        // 20.2 ms -- a row has ~10 A blocks x 4 lanes to hand out)
+        return launch_pass_t<PASS_NUMERIC_MMA, 256>(gm, 64, sms, nrows, st);
+    }
+    const int max_c = h.max_c_item, max_rownnz = h.max_nnz_item;
+    const double avg_c = nrows ? (double)C->nblk / nrows : 0.0, avg_nnz = nrows ? (double)C->nnz / nrows : 0.0;
+    if (max_c <= 4096 && max_rownnz <= 12288) { g.cap_c = std::max(1, max_c); g.cap_nnz = std::max(1, max_rownnz); }
+    else if (avg_c <= 512.0 && avg_nnz <= 1536.0) { g.cap_c = clampi(4.0 * avg_c, 256, 2048); g.cap_nnz = clampi(4.0 * avg_nnz, 1024, 8192); }
+    else { g.cap_c = 64; g.cap_nnz = 256; }
+    if (max_c > g.cap_c || max_rownnz > g.cap_nnz) BMSP_CUDA(cudaMemsetAsync(C->values, 0, (size_t)C->nnz * 4, st));
+    return launch_pass<PASS_NUMERIC>(g, plan.T, sms, st, sp);
+}
+
 extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts* opts, void* stream, bmsp_matrix_t* Cout,
                            bmsp_spgemm_info* info) {
     if (!A || !Bt || !Cout) { set_error("bmsp_spgemm: null argument"); return BMSP_ERR_INVALID; }
@@ -1220,7 +1352,7 @@ extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_
     if (verbose) BMSP_CUDA(cudaEventRecord(ev[0], st));
 
     // ---- scratch
-    int2* rowinfo = nullptr; unsigned long long* cand = nullptr; int32_t* small = nullptr;   // small: maxes[3], counter, pad, stats[2]
+    int2* rowinfo = nullptr; unsigned long long* cand = nullptr; Counters* ctr = nullptr;
     uint32_t *row_count = nullptr, *row_surv = nullptr; uint64_t* row_nnz = nullptr; uint2* surv_list = nullptr;
     bmsp_matrix_s* C = new bmsp_matrix_s();
     touch(C, st);
@@ -1234,7 +1366,7 @@ extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_
         if (sp.side) { cudaStreamSynchronize(sp.side); cudaStreamDestroy(sp.side); }
         if (sp.fork) cudaEventDestroy(sp.fork);
         if (sp.join) cudaEventDestroy(sp.join);
-        dev_free(rowinfo, st); dev_free(cand, st); dev_free(small, st); dev_free(row_count, st); dev_free(row_surv, st);
+        dev_free(rowinfo, st); dev_free(cand, st); dev_free(ctr, st); dev_free(row_count, st); dev_free(row_surv, st);
         dev_free(row_nnz, st); dev_free(surv_list, st); dev_free(g_bitset, st); dev_free(g_wrank, st);
         for (auto& e : ev) if (e) cudaEventDestroy(e);
     };
@@ -1244,145 +1376,28 @@ extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_
 
     SG_TRY(dev_alloc_t(&rowinfo, (size_t)nrows + 1, st));
     SG_TRY(dev_alloc_t(&cand, (size_t)nrows + 1, st));
-    SG_TRY(dev_alloc_t(&small, 24, st));
+    SG_TRY(dev_alloc_t(&ctr, 1, st));
     SG_TRY(dev_alloc_t(&row_count, (size_t)nrows + 2, st));
     SG_TRY(dev_alloc_t(&row_surv, (size_t)nrows + 2, st));
     SG_TRY(dev_alloc_t(&row_nnz, (size_t)nrows + 2, st));
-    SG_CUDA(cudaMemsetAsync(small, 0, 24 * sizeof(int32_t), st));
-    int32_t* maxes = small; int32_t* counter = small + 4; unsigned long long* stats = (unsigned long long*)(small + 8);
-    unsigned long long* sum_words = (unsigned long long*)(small + 12);
-    unsigned long long* max_cand = (unsigned long long*)(small + 14);
-    unsigned long long* sum_cand = (unsigned long long*)(small + 16);
+    SG_CUDA(cudaMemsetAsync(ctr, 0, sizeof(Counters), st));
 
-    int32_t h_small[24] = {0};
-    if (nrows > 0) {
-        rowinfo_kernel<<<(unsigned)std::min<int64_t>(ceil_div(nrows, 8), (int64_t)sms * 8), 256, 0, st>>>(A->brp, A->bcol, Bt->brp, Bt->bcol, rb, re, rowinfo, cand, maxes, sum_words, max_cand, sum_cand);
-        SG_CUDA(cudaGetLastError());
-    }
-    SG_CUDA(cudaMemcpyAsync(h_small, small, sizeof(h_small), cudaMemcpyDeviceToHost, st));
-    SG_CUDA(cudaStreamSynchronize(st));
-    const int max_words = h_small[0];
-    unsigned long long h_sum_words = 0;
-    memcpy(&h_sum_words, h_small + 12, sizeof(h_sum_words));
-    // Shared-memory capacities decide how many CTAs an SM holds, and these passes are latency-bound: size them for the rows
-    // that can use them.  When every row fits, take the maxima; when the typical row would not fit anyway (R-MAT: C rows of
-    // 10^4..10^5 blocks spanning every block column), keep the CTAs small -- those rows run from global scratch / global
-    // atomics either way and need the occupancy (R-MAT-17 NUMERIC: 102 KB per CTA = 2 CTAs per SM, 14 % issue utilisation).
-    const double avg_words = nrows ? (double)h_sum_words / nrows : 0.0;
-    unsigned long long h_max_cand = 0;
-    memcpy(&h_max_cand, h_small + 14, sizeof(h_max_cand));
-    {
-        const char* e = getenv("BMSP_SPGEMM_HEAVY");      // candidate pairs that make a row heavy (0 disables the split; tests lower it)
-        const long long heavy_min = e ? atoll(e) : (1ll << 20);
-        if (heavy_min > 0 && nrows > 1 && h_max_cand >= 4ull * (unsigned long long)heavy_min) {
-            std::vector<unsigned long long> hc((size_t)nrows);
-            SG_CUDA(cudaMemcpyAsync(hc.data(), cand, sizeof(unsigned long long) * (size_t)nrows, cudaMemcpyDeviceToHost, st));
-            SG_CUDA(cudaStreamSynchronize(st));
-            std::vector<int32_t> heavy, order;
-            for (int i = 0; i < nrows; i++) if (hc[i] >= (unsigned long long)heavy_min) heavy.push_back(rb + i);
-            std::sort(heavy.begin(), heavy.end(), [&](int32_t x, int32_t y) { return hc[x - rb] != hc[y - rb] ? hc[x - rb] > hc[y - rb] : x < y; });
-            order = heavy;
-            for (int i = 0; i < nrows; i++) if (hc[i] < (unsigned long long)heavy_min) order.push_back(rb + i);
-            sp.n_heavy = (int)heavy.size(); sp.n_light = nrows - sp.n_heavy;
-            SG_TRY(dev_alloc_t(&sp.list, (size_t)nrows + 1, st));
-            SG_CUDA(cudaMemcpyAsync(sp.list, order.data(), sizeof(int32_t) * (size_t)nrows, cudaMemcpyHostToDevice, st));
-            SG_CUDA(cudaStreamSynchronize(st));       // `order` dies with this scope
-            SG_CUDA(cudaStreamCreateWithFlags(&sp.side, cudaStreamNonBlocking));
-            SG_CUDA(cudaEventCreateWithFlags(&sp.fork, cudaEventDisableTiming));
-            SG_CUDA(cudaEventCreateWithFlags(&sp.join, cudaEventDisableTiming));
-            sp.active = sp.n_heavy > 0;
-        }
-    }
+    Counters h{};
+    SG_TRY(plan_rows(A, Bt, rb, re, sms, rowinfo, cand, ctr, h, sp, st));
+    SG_TRY(ensure_pmeta(Bt, st));
+    SG_TRY(ensure_fine_index(Bt, A, st));
+    const bool use_fine = Bt->fine_state == 1;
+    const int path = numeric_path(A, Bt, opts);
 
-    // ---- launch shape from averages: G lanes share one A block, each lane tests 4 B blocks per step
-    const double avgB = Bt->nbr ? (double)Bt->nblk / Bt->nbr : 0.0;
-    const double avgA = A->nbr ? (double)A->nblk / A->nbr : 0.0;
-    int G = 1;
-    while (G < 32 && G * 4 < avgB) G <<= 1;
-    const double avg_cand = avgA * avgB;
-    // Tiny rows (stencils: 25 candidate pairs per block row) are processed 16 rows at a time by 128-thread CTAs: one warp per row
-    // leaves the SM at 32 one-warp CTAs, each waiting on its own chain of dependent loads (P4096 A*A: 21.7 ms, cuSPARSE 13.0 ms)
-    int group = 1;
-    if (avg_cand <= 96 && !sp.active && (int64_t)16 * max_words <= 8192) group = 16;
-    if (const char* e = getenv("BMSP_SPGEMM_GROUP")) { const int v = atoi(e); if (v >= 1 && v <= 16 && !sp.active && (int64_t)v * max_words <= 8192) group = v; }
-    int T = group > 1 ? 128 : (avg_cand <= 96 ? 32 : (avg_cand <= 2048 ? 128 : 256));
-    if (G > T) G = T;
-
-    if (!Bt->pmeta && Bt->nblk > 0) {      // built once per B operand, reused by later products
-        SG_TRY(dev_alloc((void**)&Bt->pmeta, 2 * sizeof(uint4) * (size_t)Bt->nblk, st));
-        pack_meta_kernel<<<(unsigned)ceil_div(Bt->nblk, 256), 256, 0, st>>>(Bt->bmps, Bt->bcol, Bt->offsets, (const __half*)Bt->values, Bt->nnz,
-                                                                          (uint4*)Bt->pmeta, Bt->nblk);
-        SG_CUDA(cudaGetLastError());
-    }
-    // Fine index of B for sparse-block operands (about one value per block: uniform random, R-MAT): built once per B operand.
-    {
-        static const int fine_env = [] { const char* e = getenv("BMSP_SPGEMM_FINE"); return e ? atoi(e) : -1; }();      // 0 / 1 force it off / on
-        const double dAq = A->nblk ? (double)A->nnz / A->nblk : 0.0, dBq = Bt->nblk ? (double)Bt->nnz / Bt->nblk : 0.0;
-        const bool want = fine_env >= 0 ? fine_env == 1 : (dBq <= 2.0 && dAq <= 4.0);
-        if (want && Bt->fine_state == 0 && Bt->nblk > 0 && (int64_t)Bt->nbr * 8 + 1 < 0x7FFFFFFFll) {
-            uint32_t* fp = nullptr;
-            SG_TRY(dev_alloc_t(&fp, (size_t)Bt->nbr * 8 + 2, st));
-            SG_CUDA(cudaMemsetAsync(fp, 0, sizeof(uint32_t) * ((size_t)Bt->nbr * 8 + 2), st));
-            fine_count_kernel<<<(unsigned)ceil_div(Bt->nblk, 256), 256, 0, st>>>(Bt->keys, Bt->kmask, Bt->nblk, fp);
-            SG_CUDA(cudaGetLastError());
-            // the longest bucket (read back with the total below): slot nbr * 8 + 1 of the zeroed array
-            fine_max_kernel<<<(unsigned)ceil_div((int64_t)Bt->nbr * 8, 256), 256, 0, st>>>(fp, (int64_t)Bt->nbr * 8, fp + (size_t)Bt->nbr * 8 + 1);
-            SG_CUDA(cudaGetLastError());
-            uint32_t longest = 0;
-            if (cudaMemcpyAsync(&longest, fp + (size_t)Bt->nbr * 8 + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess) status = BMSP_ERR_CUDA;
-            status = exclusive_scan_u32(fp, fp, (int64_t)Bt->nbr * 8, st);
-            uint32_t total = 0;
-            if (status == BMSP_OK && cudaMemcpyAsync(&total, fp + (size_t)Bt->nbr * 8, sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess) status = BMSP_ERR_CUDA;
-            if (status == BMSP_OK && cudaStreamSynchronize(st) != cudaSuccess) status = BMSP_ERR_CUDA;
-            if (status != BMSP_OK) { dev_free(fp, st); return fail(status); }
-            // worth it while the buckets replicate little (a block with m inner indices sits in m buckets) and are of similar length:
-            // a power-law B (R-MAT) has hub buckets of 10^4 entries next to a mean of 2, and the candidate scan, which spreads a B block
-            // row over up to 32 lanes, handles those better (R-MAT-18 A*A: 164 ms by scan, 181 ms through the buckets)
-            const double mean_bucket = (double)total / std::max<double>(1.0, (double)Bt->nbr * 8);
-            const bool even = (double)longest <= 32.0 * std::max(mean_bucket, 1.0) || longest <= 512;
-            if (((double)total <= 1.5 * (double)Bt->nblk && even) || fine_env == 1) {
-                Bt->fine_ptr = fp; Bt->fine_n = total;
-                SG_TRY(dev_alloc_t(&Bt->fine_bcol, (size_t)total + 4, st));
-                SG_TRY(dev_alloc_t(&Bt->fine_kmask, (size_t)total + 16, st));
-                SG_TRY(dev_alloc((void**)&Bt->fine_rec, 2 * sizeof(uint4) * ((size_t)total + 1), st));
-                fine_fill_kernel<<<(unsigned)ceil_div((int64_t)Bt->nbr * 8, 128), 128, 0, st>>>(Bt->brp, Bt->kmask, (const uint4*)Bt->pmeta, Bt->nbr, fp, Bt->fine_bcol,
-                                                                                             Bt->fine_kmask, (uint4*)Bt->fine_rec);
-                SG_CUDA(cudaGetLastError());
-                Bt->fine_state = 1;
-            } else { dev_free(fp, st); Bt->fine_state = -1; }
-        }
-        if (!want && fine_env == 0) {}
-    }
-    const bool use_fine = Bt->fine_state == 1 && [] { const char* e = getenv("BMSP_SPGEMM_FINE"); return !e || atoi(e) != 0; }();
-    // Walking B's fine index a row's passes wait on record loads and are held to 3-4 CTAs per SM by the row's bit set in shared
-    // memory: more threads per CTA are more loads in flight for the same shared memory
-    if (use_fine && T == 256 && !sp.active) {
-        static const int t_env = [] { const char* e = getenv("BMSP_SPGEMM_T"); return e ? atoi(e) : 512; }();
-        if (t_env == 256 || t_env == 512 || t_env == 1024) T = t_env;
-    }
     GemmArgs g;
     memset(&g, 0, sizeof(g));
     if (use_fine) { g.f_ptr = Bt->fine_ptr; g.f_bcol = Bt->fine_bcol; g.f_kmask = Bt->fine_kmask; g.f_rec = (const uint4*)Bt->fine_rec; }
     g.b_pm = (const uint4*)Bt->pmeta;
     g.a_brp = A->brp; g.a_bcol = A->bcol; g.a_bmps = A->bmps; g.a_kmask = A->kmask; g.a_off = A->offsets; g.a_val = (const __half*)A->values;
     g.b_brp = Bt->brp; g.b_bcol = Bt->bcol; g.b_bmps = Bt->bmps; g.b_kmask = Bt->kmask; g.b_off = Bt->offsets; g.b_val = (const __half*)Bt->values;
-    g.rowinfo = rowinfo; g.row_begin = rb; g.row_end = re; g.G = G;
-    // P4096 A*A: 2.1 M block rows of 25 candidate pairs -- one atomic on the queue head per row and pass cost more than the rows
-    g.group = group;
-    // (four / two lanes per pair with two / four rows each were measured on P4096: NUMERIC 8.35 / 8.97 ms against 7.45 ms with eight)
-    g.split8 = A->nblk > 0 && (double)A->nnz / (double)A->nblk >= 4.0;
-    {   // FILL sorts its pair-list segments by class only for the pass that reads them: the scalar NUMERIC pass with 8 lanes per pair
-        const double dA0 = A->nblk ? (double)A->nnz / A->nblk : 0.0, dB0 = Bt->nblk ? (double)Bt->nnz / Bt->nblk : 0.0;
-        int path0 = opts ? opts->numeric_path : -1;
-        if (path0 < 0) path0 = (dA0 * dB0 / 8.0 >= 40.0) ? 1 : 0;
-        static const int sort_env = [] { const char* e = getenv("BMSP_SPGEMM_SORT"); return e ? atoi(e) : 1; }();
-        g.sort_max = (g.split8 && path0 == 0 && sort_env) ? SORT_K * T : 0;
-    }
-    g.batch = group > 1 ? 2 : (avg_cand <= 96 ? 32 : (avg_cand <= 2048 ? 4 : 1));
-    g.cap_words = (int64_t)group * max_words <= 8192 ? std::max(1, group * max_words) : (avg_words > 4096.0 ? 256 : 8192);
-    g.cap_c = 0; g.cap_nnz = 0;
-    g.max_words = group * max_words;
-    g.work_counter = counter; g.row_count = row_count; g.row_surv = row_surv; g.row_nnz = row_nnz; g.maxes = maxes; g.stats = stats;
+    g.rowinfo = rowinfo; g.row_begin = rb; g.row_end = re;
+    g.work_counter = &ctr->queue[0]; g.ctr = ctr; g.row_count = row_count; g.row_surv = row_surv; g.row_nnz = row_nnz;
+    const Plan plan = plan_launch(g, A, Bt, nrows, h, sp.active, use_fine, path);
 
     if (g.max_words > g.cap_words) {
         // over-cap rows use per-CTA global scratch; size it for the largest persistent grid (32 CTAs/SM)
@@ -1396,26 +1411,23 @@ extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_
     // ---- COUNT: C blocks and surviving pairs per block row
     int64_t c_size = 0, n_surv = 0;
     if (nrows > 0) {
-        SG_TRY(launch_pass<PASS_COUNT>(g, T, sms, st, sp));
+        SG_TRY(launch_pass<PASS_COUNT>(g, plan.T, sms, st, sp));
         SG_TRY(exclusive_scan_u32(row_count, row_count, nrows, st));
         SG_TRY(exclusive_scan_u32(row_surv, row_surv, nrows, st));
         uint32_t tot[2] = {0, 0};
         SG_CUDA(cudaMemcpyAsync(&tot[0], row_count + nrows, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
         SG_CUDA(cudaMemcpyAsync(&tot[1], row_surv + nrows, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        SG_CUDA(cudaMemcpyAsync(h_small, small, sizeof(h_small), cudaMemcpyDeviceToHost, st));
+        SG_CUDA(cudaMemcpyAsync(&h, ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
         SG_CUDA(cudaStreamSynchronize(st));
         c_size = tot[0]; n_surv = tot[1];
     }
     if (verbose) SG_CUDA(cudaEventRecord(ev[3], st));
-    unsigned long long h_stats[2];
-    memcpy(h_stats, h_small + 8, sizeof(h_stats));
-    if (use_fine) memcpy(&h_stats[0], h_small + 16, sizeof(unsigned long long));     // the fine walk never sees the pairs it skips: candidates from P0
-    if (c_size > 0x7FFFFFFFll || h_stats[1] > 0xFFFFFFFFull) {
+    if (c_size > 0x7FFFFFFFll || h.surviving > 0xFFFFFFFFull) {
         set_error("product too large for one call: %lld C blocks, %llu surviving pairs (shard A's block rows with brow_begin/brow_end)",
-                  (long long)c_size, h_stats[1]);
+                  (long long)c_size, h.surviving);
         return fail(BMSP_ERR_TOO_LARGE);
     }
-    const int max_c = h_small[1];
+    const int max_c = h.max_c_item;
 
     C->nblk = c_size; C->offsets_len = c_size + 1;
     SG_TRY(dev_alloc_t(&C->keys, (size_t)c_size + 2, st));
@@ -1431,75 +1443,32 @@ extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_
 
     // ---- FILL: pair list, keys, bitmaps, row-relative value offsets
     const double avg_c = nrows ? (double)c_size / nrows : 0.0;
-    auto clampi = [](double v, int lo, int hi) { return (int)std::min<double>(hi, std::max<double>(lo, v)); };
     g.cap_c = max_c <= 4096 ? std::max(1, max_c) : (avg_c <= 512.0 ? clampi(4.0 * avg_c, 256, 2048) : 64);
     if (c_size > 0) {
         if (max_c > g.cap_c) SG_CUDA(cudaMemsetAsync(C->bmps, 0, sizeof(uint64_t) * c_size, st));
-        SG_TRY(launch_pass<PASS_FILL>(g, T, sms, st, sp));
+        SG_TRY(launch_pass<PASS_FILL>(g, plan.T, sms, st, sp));
     } else if (nrows > 0) {
         SG_CUDA(cudaMemsetAsync(row_nnz, 0, sizeof(uint64_t) * ((size_t)nrows + 1), st));
     }
     SG_TRY(exclusive_scan_u64(row_nnz, row_nnz, nrows, st));
     uint64_t c_nnz = 0;
     SG_CUDA(cudaMemcpyAsync(&c_nnz, row_nnz + nrows, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    SG_CUDA(cudaMemcpyAsync(h_small, small, sizeof(h_small), cudaMemcpyDeviceToHost, st));
+    SG_CUDA(cudaMemcpyAsync(&h, ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
     SG_CUDA(cudaStreamSynchronize(st));
     if (c_nnz > 0xFFFFFFFFull) { set_error("C has %llu values (> 2^32-1)", (unsigned long long)c_nnz); return fail(BMSP_ERR_TOO_LARGE); }
-    const int max_rownnz = h_small[2];
     C->nnz = (int64_t)c_nnz;
     SG_TRY(dev_alloc(&C->values, (size_t)c_nnz * 4 + 16, st));
     if (verbose) SG_CUDA(cudaEventRecord(ev[1], st));
 
-    // ---- NUMERIC: scalar lanes for sparse blocks, mma.sync for dense ones (about dA*dB/8 products per pair)
     g.c_val = (float*)C->values;
-    const double dA = A->nblk ? (double)A->nnz / A->nblk : 0.0, dB = Bt->nblk ? (double)Bt->nnz / Bt->nblk : 0.0;
-    int path = opts ? opts->numeric_path : -1;
-    if (path < 0) path = (dA * dB / 8.0 >= 40.0) ? 1 : 0;
-    if (c_nnz > 0) {
-        static const int dense_env = [] { const char* e = getenv("BMSP_SPGEMM_DENSE"); return e ? atoi(e) : 1; }();
-        const int max_c_row0 = std::max(1, h_small[3]);
-        if (path == 1 && dense_env && !sp.active && (int64_t)max_words * 32 <= 1024) {
-            // narrow rows of dense blocks: one warp per block row, dense accumulators for a window of C columns in shared memory
-            constexpr int WARPS = 4;
-            DenseArgs da;
-            static const int wc_env = [] { const char* e = getenv("BMSP_SPGEMM_WCOLS"); return e ? atoi(e) : 16; }();
-            da.c_brp = (const int32_t*)row_count; da.row_nnz = row_nnz; da.wcols = std::max(8, std::min(wc_env, 64));
-            const size_t smem = (size_t)WARPS * (size_t)da.wcols * 256;
-            auto kern = spgemm_dense_kernel<WARPS>;
-            SG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
-            int occ = 0;
-            SG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, WARPS * 32, smem));
-            if (occ < 1) { set_error("spgemm dense pass does not fit: smem %zu", smem); return fail(BMSP_ERR_CUDA); }
-            SG_CUDA(cudaMemsetAsync(g.work_counter, 0, sizeof(int32_t), st));
-            const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((int64_t)sms * occ, ceil_div(nrows, WARPS)));
-            kern<<<grid, WARPS * 32, smem, st>>>(g, da);
-            SG_CUDA(cudaGetLastError());
-        } else if (path == 1) {
-            const int max_c_row = std::max(1, h_small[3]);                         // recorded by COUNT
-            g.cap_c = std::min(max_c_row, 192);
-            if (max_c_row > g.cap_c) SG_CUDA(cudaMemsetAsync(C->values, 0, (size_t)c_nnz * 4, st));
-            GemmArgs gm = g;
-            gm.group = 1; gm.batch = avg_cand <= 96 ? 32 : 1;          // one warp per block row: pairs of an A block stay adjacent
-            int Tm = 64;             // two warps per block row in the dense-block pass, sharing the row's accumulators (BC4M numeric, one box:
-                                     // 32 threads 19.5 ms, 64: 17.7 ms, 128: 20.2 ms -- a row has ~10 A blocks x 4 lanes to hand out)
-            if (const char* e = getenv("BMSP_SPGEMM_MMA_T")) { const int v = atoi(e); if (v == 32 || v == 64 || v == 128 || v == 256) Tm = v; }
-            SG_TRY((launch_pass_t<PASS_NUMERIC_MMA, 256>(gm, Tm, sms, nrows, st)));
-        } else {
-            const double avg_nnz = nrows ? (double)c_nnz / nrows : 0.0;
-            if (max_c <= 4096 && max_rownnz <= 12288) { g.cap_c = std::max(1, max_c); g.cap_nnz = std::max(1, max_rownnz); }
-            else if (avg_c <= 512.0 && avg_nnz <= 1536.0) { g.cap_c = clampi(4.0 * avg_c, 256, 2048); g.cap_nnz = clampi(4.0 * avg_nnz, 1024, 8192); }
-            else { g.cap_c = 64; g.cap_nnz = 256; }
-            if (max_c > g.cap_c || max_rownnz > g.cap_nnz) SG_CUDA(cudaMemsetAsync(C->values, 0, (size_t)c_nnz * 4, st));
-            SG_TRY(launch_pass<PASS_NUMERIC>(g, T, sms, st, sp));
-        }
-    }
+    if (c_nnz > 0) SG_TRY(run_numeric(g, C, h, plan, path, sp, nrows, sms, st));
     finish_rows_kernel<<<(unsigned)ceil_div(C->nbr + 1, 256), 256, 0, st>>>(row_count, row_nnz, rb, re, C->nbr, C->brp, C->rvb, C->offsets, c_size, c_nnz);
     SG_CUDA(cudaGetLastError());
     if (verbose) SG_CUDA(cudaEventRecord(ev[2], st));
 
     if (info) {
         memset(info, 0, sizeof(*info));
-        info->candidate_pairs = (int64_t)h_stats[0]; info->surviving_pairs = (int64_t)h_stats[1];
+        info->candidate_pairs = (int64_t)h.sum_cand; info->surviving_pairs = (int64_t)h.surviving;
         info->c_blocks = c_size; info->c_nnz = (int64_t)c_nnz; info->numeric_path = path;
         if (verbose) {
             SG_CUDA(cudaEventSynchronize(ev[2]));

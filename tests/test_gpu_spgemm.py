@@ -83,13 +83,6 @@ def test_random(B, oracle, n, m, p, density, path):
     assert info.numeric_path == path
 
 
-def test_mma_path_wide_rows_fall_back(B, oracle):
-    """a block row of C with more blocks than the dense-accumulator cap (192) must take the global fallback"""
-    a = random_csr(16, 64, 0.9, seed=3)
-    b = random_csr(64, 8 * 400, 0.5, seed=4)
-    _mult_check(B, oracle, (16, 64), a, (64, 8 * 400), b, numeric_path=1)
-
-
 def test_generators_square(B, oracle):
     G = B.generators
     for gen in (lambda: G.poisson5pt(40, 36), lambda: G.block_clustered(96), lambda: G.uniform_random(2048, 16),
