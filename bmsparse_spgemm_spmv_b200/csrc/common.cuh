@@ -109,6 +109,9 @@ int exclusive_scan_u64(const uint64_t* in, uint64_t* out, int64_t n, cudaStream_
 int derive_compact(bmsp_matrix_s* m, cudaStream_t st);
 int plan_spmv(bmsp_matrix_s* m, cudaStream_t st);
 void spmv_host_release(bmsp_matrix_s* m);
+// rebuild every copy of m's values that the library derived from them (SpGEMM's packed B records and fine index; spgemm.cu), on
+// st: after m's values changed.  The SpMV plan holds no values and is kept.
+int refresh_value_copies(bmsp_matrix_s* m, cudaStream_t st);
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
@@ -122,6 +125,23 @@ __device__ __forceinline__ uint32_t kmask_of(uint64_t bmp) {
 
 __device__ __forceinline__ float val_to_f32(const __half v) { return __half2float(v); }
 __device__ __forceinline__ float val_to_f32(const float v) { return v; }
+
+// value conversion on ingest (round to nearest)
+template <typename Tin, typename Tout> __device__ __forceinline__ Tout conv(Tin v);
+template <> __device__ __forceinline__ __half conv<float, __half>(float v) { return __float2half_rn(v); }
+template <> __device__ __forceinline__ __half conv<__half, __half>(__half v) { return v; }
+template <> __device__ __forceinline__ float conv<float, float>(float v) { return v; }
+template <> __device__ __forceinline__ float conv<__half, float>(__half v) { return __half2float(v); }
+
+// 8x8 bit-matrix transpose (three masked swaps); with MSB-first cell numbering the main diagonal is
+// bits 63,54,...,0, so the classic delta-swap constants apply unchanged.
+__device__ __forceinline__ uint64_t transpose8x8(uint64_t x) {
+    uint64_t t;
+    t = (x ^ (x >> 7)) & 0x00AA00AA00AA00AAull;  x = x ^ t ^ (t << 7);
+    t = (x ^ (x >> 14)) & 0x0000CCCC0000CCCCull; x = x ^ t ^ (t << 14);
+    t = (x ^ (x >> 28)) & 0x00000000F0F0F0F0ull; x = x ^ t ^ (t << 28);
+    return x;
+}
 
 // streaming (read-once) loads: keep them out of L1 and mark evict-first in L2 so that x stays resident
 __device__ __forceinline__ uint64_t ld_stream_u64(const uint64_t* p) {

@@ -182,13 +182,7 @@ __global__ void __launch_bounds__(1024) emit_kernel(const uint64_t* __restrict__
         atomicOr((unsigned long long*)(bmps + blk), ((unsigned long long)hi << 32) | lo);
 }
 
-// K4: values in sorted order, 8 per thread, 16-byte stores.
-template <typename Tin, typename Tout> __device__ __forceinline__ Tout conv(Tin v);
-template <> __device__ __forceinline__ __half conv<float, __half>(float v) { return __float2half_rn(v); }
-template <> __device__ __forceinline__ __half conv<__half, __half>(__half v) { return v; }
-template <> __device__ __forceinline__ float conv<float, float>(float v) { return v; }
-template <> __device__ __forceinline__ float conv<__half, float>(__half v) { return __half2float(v); }
-
+// K4: values in sorted order, 8 per thread, 16-byte stores (conv: common.cuh).
 template <typename Tin, typename Tout>
 __global__ void __launch_bounds__(256) values_kernel(const Tin* __restrict__ vals, const int32_t* __restrict__ s_src, int64_t nnz,
                                                      Tout* __restrict__ out) {
@@ -289,16 +283,7 @@ static int convert_device_csr(int32_t rows, int32_t cols, int64_t nnz, const int
 }
 
 // ---------------------------------------------------------------------------- block transpose
-// 8x8 bit-matrix transpose (three masked swaps); with MSB-first cell numbering the main diagonal is
-// bits 63,54,...,0, so the classic delta-swap constants apply unchanged.
-__device__ __forceinline__ uint64_t transpose8x8(uint64_t x) {
-    uint64_t t;
-    t = (x ^ (x >> 7)) & 0x00AA00AA00AA00AAull;  x = x ^ t ^ (t << 7);
-    t = (x ^ (x >> 14)) & 0x0000CCCC0000CCCCull; x = x ^ t ^ (t << 14);
-    t = (x ^ (x >> 28)) & 0x00000000F0F0F0F0ull; x = x ^ t ^ (t << 28);
-    return x;
-}
-
+// (transpose8x8: common.cuh)
 // One thread per block: new bitmap = transpose; value of cell p=(hi,lo) moves to the rank of cell (lo,hi).
 template <typename Tin, typename Tout>
 __global__ void block_transpose_kernel(const uint64_t* __restrict__ bmps, const uint64_t* __restrict__ offsets,

@@ -332,12 +332,13 @@ extern "C" int bmsp_to_coo(bmsp_matrix_t m, int32_t* rows, int32_t* cols, float*
     return BMSP_OK;
 }
 
-// ------------------------------------------------------------------------------------ bmSparse -> CSR on the device
+// ------------------------------------------------------------------------------------ bmSparse <-> CSR on the device
 // The blocks of a block row are already in ascending block column and a bitmap is row-major inside a block, so CSR order is an
 // 8-way merge in reverse: entry (r, c) of block b goes to row_ptr[r] + (cells of row r in the earlier blocks of the block row) +
 // (cells of row r left of c in this block).  Pass 1 counts the cells per matrix row (one thread per block), a scan gives row_ptr,
 // pass 2 runs one warp per block row: lanes <-> blocks, 32 at a time; the eight per-row counts of a block travel as two 64-bit
-// words of four 16-bit fields through one warp scan each.
+// words of four 16-bit fields through one warp scan each.  The same walk run backwards scatters CSR values into the compact order
+// (bmsp_set_values_csr).
 __global__ void csr_count_kernel(const uint64_t* __restrict__ keys, const uint64_t* __restrict__ bmps, int64_t nblk, int32_t rows,
                                  uint32_t* __restrict__ row_cnt) {
     const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -351,20 +352,19 @@ __global__ void csr_count_kernel(const uint64_t* __restrict__ keys, const uint64
     }
 }
 
-template <typename T>
-__global__ void __launch_bounds__(256) csr_fill_kernel(const int32_t* __restrict__ brp, const int32_t* __restrict__ bcol, const uint64_t* __restrict__ bmps,
-                                                       const uint64_t* __restrict__ offsets, const T* __restrict__ values, int32_t nbr, int32_t rows,
-                                                       const uint32_t* __restrict__ row_ptr, int32_t* __restrict__ col_idx, float* __restrict__ vals) {
+// The cells of block row br in CSR order, one warp: cell(slot, r, col, k) for every cell -- slot its CSR position, r its row inside
+// the block row, k its index in the compact values.  base[r]: the first slot of row r of the block row (warp-uniform); on return it
+// is advanced past the row's cells.  TRANSPOSED: a transposed-operand matrix holds cell (r, c) at bit 63-(c*8+r); the CSR slot still
+// comes from the row-major counts, the compact index is the cell's rank in the stored (column-major) bitmap.
+template <bool TRANSPOSED, typename F>
+__device__ __forceinline__ void csr_walk_block_row(const int32_t* __restrict__ brp, const int32_t* __restrict__ bcol, const uint64_t* __restrict__ bmps,
+                                                   const uint64_t* __restrict__ offsets, int br, uint32_t (&base)[8], F&& cell) {
     const int lane = threadIdx.x & 31;
-    const int br = blockIdx.x * 8 + (threadIdx.x >> 5);
-    if (br >= nbr) return;
-    uint32_t base[8];                     // next free slot of each of the block row's eight matrix rows (warp-uniform)
-#pragma unroll
-    for (int r = 0; r < 8; r++) base[r] = (int64_t)br * 8 + r < rows ? row_ptr[(int64_t)br * 8 + r] : 0u;
     for (int b0 = brp[br]; b0 < brp[br + 1]; b0 += 32) {
         const int b = b0 + lane;
         const bool valid = b < brp[br + 1];
-        const uint64_t bmp = valid ? bmps[b] : 0ull;
+        const uint64_t stored = valid ? bmps[b] : 0ull;
+        const uint64_t bmp = TRANSPOSED ? transpose8x8(stored) : stored;     // row-major
         uint64_t lo = 0, hi = 0;          // per-row counts, 16-bit fields: rows 0-3 in lo, 4-7 in hi
 #pragma unroll
         for (int r = 0; r < 4; r++) {
@@ -391,13 +391,72 @@ __global__ void __launch_bounds__(256) csr_fill_kernel(const int32_t* __restrict
                 uint32_t slot = 0;
 #pragma unroll
                 for (int q = 0; q < 8; q++) if (q == r) slot = base[q] + ex + in_row[q]++;
-                col_idx[slot] = c0 + (p & 7);
-                vals[slot] = val_to_f32(values[k++]);
+                if (TRANSPOSED) {
+                    const int t = (p & 7) * 8 + r;                      // the cell's bit in the stored bitmap
+                    cell(slot, r, c0 + (p & 7), k + (t ? __popcll(stored >> (64 - t)) : 0));
+                } else {
+                    cell(slot, r, c0 + (p & 7), k++);
+                }
             }
         }
         const uint64_t tlo = __shfl_sync(0xffffffffu, ilo, 31), thi = __shfl_sync(0xffffffffu, ihi, 31);
 #pragma unroll
         for (int r = 0; r < 4; r++) { base[r] += (uint32_t)((tlo >> (16 * r)) & 0xFFFFu); base[4 + r] += (uint32_t)((thi >> (16 * r)) & 0xFFFFu); }
+    }
+}
+
+template <typename T>
+__global__ void __launch_bounds__(256) csr_fill_kernel(const int32_t* __restrict__ brp, const int32_t* __restrict__ bcol, const uint64_t* __restrict__ bmps,
+                                                       const uint64_t* __restrict__ offsets, const T* __restrict__ values, int32_t nbr, int32_t rows,
+                                                       const uint32_t* __restrict__ row_ptr, int32_t* __restrict__ col_idx, float* __restrict__ vals) {
+    const int br = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (br >= nbr) return;
+    uint32_t base[8];                     // next free slot of each of the block row's eight matrix rows (warp-uniform)
+#pragma unroll
+    for (int r = 0; r < 8; r++) base[r] = (int64_t)br * 8 + r < rows ? row_ptr[(int64_t)br * 8 + r] : 0u;
+    csr_walk_block_row<false>(brp, bcol, bmps, offsets, br, base, [&](uint32_t slot, int, int32_t col, uint64_t k) {
+        col_idx[slot] = col;
+        vals[slot] = val_to_f32(values[k]);
+    });
+}
+
+// CSR values -> the compact values of a matrix with the same pattern.  CHECK: writes nothing and raises *flag on any difference of
+// pattern -- a row_ptr entry outside [0, nnz] or decreasing, a row whose length is not its cell count, an entry whose column is not
+// its cell's.  col_idx is read inside the row's own [row_ptr[r], row_ptr[r+1]) only, so a malformed CSR is never read out of
+// bounds.  !CHECK: the scatter, launched once the check has passed.
+template <bool TRANSPOSED, bool CHECK, typename Tin, typename Tout>
+__global__ void __launch_bounds__(256) csr_scatter_kernel(const int32_t* __restrict__ brp, const int32_t* __restrict__ bcol, const uint64_t* __restrict__ bmps,
+                                                          const uint64_t* __restrict__ offsets, int32_t nbr, int32_t rows, int64_t nnz,
+                                                          const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ col_idx,
+                                                          const Tin* __restrict__ vals, Tout* __restrict__ out, int32_t* __restrict__ flag) {
+    const int lane = threadIdx.x & 31;
+    const int br = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (br >= nbr) return;
+    uint32_t base[8], end[8];
+    bool bad = false;                     // warp-uniform until the walk
+#pragma unroll
+    for (int r = 0; r < 8; r++) {
+        const int64_t R = (int64_t)br * 8 + r;
+        int32_t lo = 0, hi = 0;
+        if (R < rows) { lo = row_ptr[R]; hi = row_ptr[R + 1]; }
+        bad |= lo < 0 || hi < lo || (int64_t)hi > nnz;
+        base[r] = (uint32_t)lo; end[r] = (uint32_t)hi;
+    }
+    if (CHECK && bad) { if (lane == 0) atomicOr(flag, 1); return; }
+    csr_walk_block_row<TRANSPOSED>(brp, bcol, bmps, offsets, br, base, [&](uint32_t slot, int r, int32_t col, uint64_t k) {
+        if (CHECK) {
+            uint32_t e = 0;
+#pragma unroll
+            for (int q = 0; q < 8; q++) if (q == r) e = end[q];
+            if (slot >= e || col_idx[slot] != col) bad = true;
+        } else {
+            out[k] = conv<Tin, Tout>(vals[slot]);
+        }
+    });
+    if (CHECK) {
+#pragma unroll
+        for (int r = 0; r < 8; r++) bad |= base[r] != end[r];          // base: the row's start + its cells
+        if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(flag, 1);
     }
 }
 
@@ -435,6 +494,116 @@ extern "C" int bmsp_to_csr(bmsp_matrix_t m, int32_t* row_ptr, int32_t* col_idx, 
         if (e == cudaSuccess && m->nnz) e = cudaMemcpyAsync(vals, d_v, sizeof(float) * (size_t)m->nnz, cudaMemcpyDeviceToHost, st);
         if (e == cudaSuccess) e = cudaStreamSynchronize(st);
         if (e != cudaSuccess) s = cuda_fail(e, "bmsp_to_csr: copy out", __FILE__, __LINE__);
+    }
+    dev_free(d_rp, st); dev_free(d_ci, st); dev_free(d_v, st);
+    return s;
+}
+
+// ------------------------------------------------------------------------------------ new values, same structure
+template <typename Tin, typename Tout>
+__global__ void convert_values_kernel(const Tin* __restrict__ in, Tout* __restrict__ out, int64_t n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = conv<Tin, Tout>(in[i]);
+}
+
+// device values in m's compact order -> m->values, converted to m's dtype
+static int values_from_device(bmsp_matrix_s* m, const void* v, int32_t dtype, cudaStream_t st) {
+    if (m->nnz == 0) return BMSP_OK;
+    if (dtype == m->dtype) {
+        BMSP_CUDA(cudaMemcpyAsync(m->values, v, (size_t)m->nnz * dtype_size(dtype), cudaMemcpyDeviceToDevice, st));
+        return BMSP_OK;
+    }
+    const unsigned grid = (unsigned)ceil_div(m->nnz, 256);
+    if (dtype == BMSP_F32) convert_values_kernel<float, __half><<<grid, 256, 0, st>>>((const float*)v, (__half*)m->values, m->nnz);
+    else convert_values_kernel<__half, float><<<grid, 256, 0, st>>>((const __half*)v, (float*)m->values, m->nnz);
+    BMSP_KERNEL_CHECK();
+    return BMSP_OK;
+}
+
+template <bool TRANSPOSED, bool CHECK, typename Tin, typename Tout>
+static int launch_scatter(bmsp_matrix_s* m, const int32_t* rp, const int32_t* ci, const void* vals, int32_t* flag, cudaStream_t st) {
+    csr_scatter_kernel<TRANSPOSED, CHECK, Tin, Tout><<<(unsigned)ceil_div(m->nbr, 8), 256, 0, st>>>(m->brp, m->bcol, m->bmps, m->offsets, m->nbr, m->rows,
+                                                                                                  m->nnz, rp, ci, (const Tin*)vals, (Tout*)m->values, flag);
+    BMSP_KERNEL_CHECK();
+    return BMSP_OK;
+}
+template <bool TRANSPOSED>
+static int scatter_values(bmsp_matrix_s* m, const int32_t* rp, const void* vals, int32_t vals_dtype, cudaStream_t st) {
+    if (vals_dtype == BMSP_F32 && m->dtype == BMSP_F16) return launch_scatter<TRANSPOSED, false, float, __half>(m, rp, nullptr, vals, nullptr, st);
+    if (vals_dtype == BMSP_F16 && m->dtype == BMSP_F16) return launch_scatter<TRANSPOSED, false, __half, __half>(m, rp, nullptr, vals, nullptr, st);
+    if (vals_dtype == BMSP_F32) return launch_scatter<TRANSPOSED, false, float, float>(m, rp, nullptr, vals, nullptr, st);
+    return launch_scatter<TRANSPOSED, false, __half, float>(m, rp, nullptr, vals, nullptr, st);
+}
+
+// device CSR with m's pattern -> m->values: the check pass, one read-back of its flag, then the scatter
+static int set_values_csr_device(bmsp_matrix_s* m, const int32_t* rp, const int32_t* ci, const void* vals, int32_t vals_dtype, cudaStream_t st) {
+    if (m->nbr == 0) return BMSP_OK;
+    int32_t* flag = nullptr;
+    BMSP_TRY(dev_alloc_t(&flag, 1, st));
+    int32_t h = 0;
+    const int s = [&]() -> int {
+        BMSP_CUDA(cudaMemsetAsync(flag, 0, sizeof(int32_t), st));
+        if (m->transposed) BMSP_TRY((launch_scatter<true, true, __half, __half>(m, rp, ci, nullptr, flag, st)));
+        else BMSP_TRY((launch_scatter<false, true, __half, __half>(m, rp, ci, nullptr, flag, st)));
+        BMSP_CUDA(cudaMemcpyAsync(&h, flag, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        BMSP_CUDA(cudaStreamSynchronize(st));
+        return BMSP_OK;
+    }();
+    dev_free(flag, st);
+    if (s != BMSP_OK) return s;
+    if (h) { set_error("bmsp_set_values_csr: the CSR's pattern differs from the matrix's"); return BMSP_ERR_INVALID; }
+    return m->transposed ? scatter_values<true>(m, rp, vals, vals_dtype, st) : scatter_values<false>(m, rp, vals, vals_dtype, st);
+}
+
+extern "C" int bmsp_set_values(bmsp_matrix_t m, const void* values, int32_t dtype, int32_t mem, void* stream) {
+    if (!m || (values && dtype != BMSP_F16 && dtype != BMSP_F32)) { set_error("bmsp_set_values: invalid argument"); return BMSP_ERR_INVALID; }
+    cudaStream_t st = (cudaStream_t)stream;
+    touch(m, st);
+    if (values && mem == BMSP_DEVICE) BMSP_TRY(values_from_device(m, values, dtype, st));
+    else if (values && m->nnz > 0) {
+        if (dtype == m->dtype) {
+            BMSP_CUDA(cudaMemcpyAsync(m->values, values, (size_t)m->nnz * dtype_size(dtype), cudaMemcpyHostToDevice, st));
+        } else {
+            void* d = nullptr;
+            BMSP_TRY(dev_alloc(&d, (size_t)m->nnz * dtype_size(dtype), st));
+            cudaError_t e = cudaMemcpyAsync(d, values, (size_t)m->nnz * dtype_size(dtype), cudaMemcpyHostToDevice, st);
+            const int s = e == cudaSuccess ? values_from_device(m, d, dtype, st) : cuda_fail(e, "bmsp_set_values: copy in", __FILE__, __LINE__);
+            dev_free(d, st);
+            if (s != BMSP_OK) return s;
+        }
+    }
+    BMSP_TRY(refresh_value_copies(m, st));
+    if (values && mem == BMSP_HOST) BMSP_CUDA(cudaStreamSynchronize(st));      // host buffers may be freed by the caller
+    return BMSP_OK;
+}
+
+extern "C" int bmsp_set_values_csr(bmsp_matrix_t m, const int32_t* row_ptr, const int32_t* col_idx, const void* vals, int32_t vals_dtype,
+                                   int32_t mem, void* stream) {
+    if (!m || !row_ptr || (m->nnz > 0 && (!col_idx || !vals)) || (vals_dtype != BMSP_F16 && vals_dtype != BMSP_F32)) {
+        set_error("bmsp_set_values_csr: invalid argument");
+        return BMSP_ERR_INVALID;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    touch(m, st);
+    if (mem == BMSP_DEVICE) {
+        BMSP_TRY(set_values_csr_device(m, row_ptr, col_idx, vals, vals_dtype, st));
+        return refresh_value_copies(m, st);
+    }
+    if (row_ptr[0] != 0 || (int64_t)row_ptr[m->rows] != m->nnz) {
+        set_error("bmsp_set_values_csr: row_ptr spans %lld entries, the matrix has %lld values", (long long)row_ptr[m->rows] - row_ptr[0], (long long)m->nnz);
+        return BMSP_ERR_INVALID;
+    }
+    const size_t vs = vals_dtype == BMSP_F16 ? 2 : 4;
+    int32_t *d_rp = nullptr, *d_ci = nullptr; void* d_v = nullptr;
+    int s = BMSP_OK;
+    if ((s = dev_alloc_t(&d_rp, (size_t)m->rows + 1, st)) == BMSP_OK && (s = dev_alloc_t(&d_ci, (size_t)m->nnz, st)) == BMSP_OK &&
+        (s = dev_alloc(&d_v, (size_t)m->nnz * vs, st)) == BMSP_OK) {
+        cudaError_t e = cudaMemcpyAsync(d_rp, row_ptr, sizeof(int32_t) * ((size_t)m->rows + 1), cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess && m->nnz) e = cudaMemcpyAsync(d_ci, col_idx, sizeof(int32_t) * (size_t)m->nnz, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess && m->nnz) e = cudaMemcpyAsync(d_v, vals, (size_t)m->nnz * vs, cudaMemcpyHostToDevice, st);
+        s = e == cudaSuccess ? set_values_csr_device(m, d_rp, d_ci, d_v, vals_dtype, st) : cuda_fail(e, "bmsp_set_values_csr: copy in", __FILE__, __LINE__);
+        if (s == BMSP_OK) s = refresh_value_copies(m, st);
+        if (s == BMSP_OK && (e = cudaStreamSynchronize(st)) != cudaSuccess) s = cuda_fail(e, "bmsp_set_values_csr: sync", __FILE__, __LINE__);
     }
     dev_free(d_rp, st); dev_free(d_ci, st); dev_free(d_v, st);
     return s;

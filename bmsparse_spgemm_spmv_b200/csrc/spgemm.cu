@@ -651,7 +651,9 @@ __device__ __forceinline__ void enumerate_fine(const GemmArgs& g, const RowCtx& 
     }
 }
 
-template <int PASS, int MAXT>
+// REUSE (NUMERIC passes of a kept plan, bmsp_spgemm_numeric): C's value offsets are absolute already -- the first NUMERIC pass made
+// them so in place -- and are read, never written.
+template <int PASS, int MAXT, bool REUSE = false>
 __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int T = blockDim.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, nwarps = T >> 5;
@@ -868,9 +870,10 @@ __global__ void __launch_bounds__(MAXT) spgemm_pass_kernel(GemmArgs g) {
             const bool fit = PASS == PASS_NUMERIC ? (ccount <= g.cap_c && rownnz <= g.cap_nnz) : (ccount <= g.cap_c);
             for (int c = tid; c < ccount; c += T) {
                 const int rl = local_row(s_cbr, nr, c0 + c);
-                const uint64_t local = s_rowoff[rl] + g.c_off[c0 + c];      // relative to the work item's first value
+                // relative to the work item's first value
+                const uint64_t local = REUSE ? g.c_off[c0 + c] - vbase : s_rowoff[rl] + g.c_off[c0 + c];
                 if (PASS == PASS_NUMERIC && fit) { s_cbmp[c] = g.c_bmps[c0 + c]; s_coff[c] = (uint32_t)local; }
-                g.c_off[c0 + c] = vbase + local;                             // absolute from here on
+                if (!REUSE) g.c_off[c0 + c] = vbase + local;                 // absolute from here on
                 const int j = g.c_bcol[c0 + c] - s_jb[rl];                   // bit set from C's own block columns
                 atomicOr(&r.bitset[s_wo[rl] + (j >> 5)], 1u << (j & 31));
             }
@@ -982,6 +985,7 @@ __device__ __forceinline__ uint32_t frag_shfl(uint64_t bmp, uint32_t packed, int
 // test the B block row in parallel (block column inside the window, inner-dimension masks overlap) and the survivors are taken two
 // at a time off the ballot.
 constexpr int DENSE_WARPS = 4, DENSE_WCOLS = 16;
+template <bool REUSE = false>      // as spgemm_pass_kernel's
 __global__ void __launch_bounds__(DENSE_WARPS * 32) spgemm_dense_kernel(GemmArgs g) {
     __shared__ float s_dense_all[DENSE_WARPS * DENSE_WCOLS * 64];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -997,8 +1001,10 @@ __global__ void __launch_bounds__(DENSE_WARPS * 32) spgemm_dense_kernel(GemmArgs
         const int row = g.row_begin + lrow;
         const int c0 = g.c_brp[lrow], ccount = g.c_brp[lrow + 1] - c0;
         if (ccount == 0) continue;
-        const uint64_t vbase = g.row_nnz[lrow];
-        for (int c = lane; c < ccount; c += 32) g.c_off[c0 + c] += vbase;       // FILL left row-relative offsets: absolute from here on
+        if (!REUSE) {
+            const uint64_t vbase = g.row_nnz[lrow];
+            for (int c = lane; c < ccount; c += 32) g.c_off[c0 + c] += vbase;   // FILL left row-relative offsets: absolute from here on
+        }
         const int jfirst = g.c_bcol[c0], jlast = g.c_bcol[c0 + ccount - 1];
         const int a0 = g.a_brp[row], a1 = g.a_brp[row + 1];
         int cdone = 0;                                                           // C blocks of the windows already stored
@@ -1106,10 +1112,10 @@ extern "C" int bmsp_debug_pair_bitmap(int64_t n, const uint64_t* a_host, const u
     return BMSP_OK;
 }
 
-template <int PASS, int MAXT>
+template <int PASS, int MAXT, bool REUSE = false>
 static int launch_pass_t(const GemmArgs& g, int T, int sms, int nrows, cudaStream_t st) {
     const size_t smem = pass_smem_bytes(PASS, T, g.cap_words, g.cap_c, g.cap_nnz, g.row_list ? 1 : g.group);
-    auto kern = spgemm_pass_kernel<PASS, MAXT>;
+    auto kern = spgemm_pass_kernel<PASS, MAXT, REUSE>;
     BMSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
     int occ = 0;
     BMSP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, T, smem));
@@ -1135,11 +1141,11 @@ struct RowSplit {
     size_t heavy_scratch_off = 0;  // words: the heavy launch's slice of g_bitset / g_wrank
 };
 
-template <int PASS>
+template <int PASS, bool REUSE = false>
 static int launch_pass(GemmArgs& g, int T, int sms, cudaStream_t st, const RowSplit& sp) {
     if (!sp.active) {
-        if (T > 256) return launch_pass_t<PASS, 1024>(g, T, sms, (int)ceil_div(g.row_end - g.row_begin, g.group), st);
-        return launch_pass_t<PASS, 256>(g, T, sms, (int)ceil_div(g.row_end - g.row_begin, g.group), st);
+        if (T > 256) return launch_pass_t<PASS, 1024, REUSE>(g, T, sms, (int)ceil_div(g.row_end - g.row_begin, g.group), st);
+        return launch_pass_t<PASS, 256, REUSE>(g, T, sms, (int)ceil_div(g.row_end - g.row_begin, g.group), st);
     }
     GemmArgs gh = g, gl = g;
     gh.group = gl.group = 1;
@@ -1148,8 +1154,8 @@ static int launch_pass(GemmArgs& g, int T, int sms, cudaStream_t st, const RowSp
     gl.row_list = sp.list + sp.n_heavy; gl.n_list = sp.n_light;
     BMSP_CUDA(cudaEventRecord(sp.fork, st));
     BMSP_CUDA(cudaStreamWaitEvent(sp.side, sp.fork, 0));
-    BMSP_TRY((launch_pass_t<PASS, 1024>(gh, 1024, sms, sp.n_heavy, sp.side)));
-    if (sp.n_light > 0) BMSP_TRY((launch_pass_t<PASS, 256>(gl, T, sms, sp.n_light, st)));
+    BMSP_TRY((launch_pass_t<PASS, 1024, REUSE>(gh, 1024, sms, sp.n_heavy, sp.side)));
+    if (sp.n_light > 0) BMSP_TRY((launch_pass_t<PASS, 256, REUSE>(gl, T, sms, sp.n_light, st)));
     BMSP_CUDA(cudaEventRecord(sp.join, sp.side));
     BMSP_CUDA(cudaStreamWaitEvent(st, sp.join, 0));
     return BMSP_OK;
@@ -1194,14 +1200,31 @@ static int plan_rows(const bmsp_matrix_s* A, const bmsp_matrix_s* Bt, int rb, in
     return BMSP_OK;
 }
 
-// B's packed block records: built once per B operand, reused by later products
-static int ensure_pmeta(bmsp_matrix_s* Bt, cudaStream_t st) {
-    if (Bt->pmeta || Bt->nblk == 0) return BMSP_OK;
-    BMSP_TRY(dev_alloc(&Bt->pmeta, 2 * sizeof(uint4) * (size_t)Bt->nblk, st));
+// the two copies of a B operand's values that products keep, (re)written in place: the packed block records and the fine index's
+static int pack_meta(bmsp_matrix_s* Bt, cudaStream_t st) {
     pack_meta_kernel<<<(unsigned)ceil_div(Bt->nblk, 256), 256, 0, st>>>(Bt->bmps, Bt->bcol, Bt->offsets, (const __half*)Bt->values, Bt->nnz,
                                                                       (uint4*)Bt->pmeta, Bt->nblk);
     BMSP_KERNEL_CHECK();
     return BMSP_OK;
+}
+static int fine_fill(bmsp_matrix_s* Bt, cudaStream_t st) {
+    fine_fill_kernel<<<(unsigned)ceil_div((int64_t)Bt->nbr * 8, 128), 128, 0, st>>>(Bt->brp, Bt->kmask, (const uint4*)Bt->pmeta, Bt->nbr, Bt->fine_ptr,
+                                                                                   Bt->fine_bcol, Bt->fine_kmask, (uint4*)Bt->fine_rec);
+    BMSP_KERNEL_CHECK();
+    return BMSP_OK;
+}
+
+int bmsp::refresh_value_copies(bmsp_matrix_s* m, cudaStream_t st) {
+    if (m->pmeta && m->nblk > 0) BMSP_TRY(pack_meta(m, st));
+    if (m->fine_state == 1) BMSP_TRY(fine_fill(m, st));
+    return BMSP_OK;
+}
+
+// B's packed block records: built once per B operand, reused by later products
+static int ensure_pmeta(bmsp_matrix_s* Bt, cudaStream_t st) {
+    if (Bt->pmeta || Bt->nblk == 0) return BMSP_OK;
+    BMSP_TRY(dev_alloc(&Bt->pmeta, 2 * sizeof(uint4) * (size_t)Bt->nblk, st));
+    return pack_meta(Bt, st);
 }
 
 // Fine index of B for sparse-block operands (about one value per block: uniform random, R-MAT): examined once per B operand, by
@@ -1237,9 +1260,7 @@ static int ensure_fine_index(bmsp_matrix_s* Bt, const bmsp_matrix_s* A, cudaStre
     BMSP_TRY(dev_alloc_t(&Bt->fine_bcol, (size_t)total + 4, st));
     BMSP_TRY(dev_alloc_t(&Bt->fine_kmask, (size_t)total + 16, st));
     BMSP_TRY(dev_alloc(&Bt->fine_rec, 2 * sizeof(uint4) * ((size_t)total + 1), st));
-    fine_fill_kernel<<<(unsigned)ceil_div((int64_t)nb, 128), 128, 0, st>>>(Bt->brp, Bt->kmask, (const uint4*)Bt->pmeta, Bt->nbr, fp, Bt->fine_bcol,
-                                                                         Bt->fine_kmask, (uint4*)Bt->fine_rec);
-    BMSP_KERNEL_CHECK();
+    BMSP_TRY(fine_fill(Bt, st));
     Bt->fine_state = 1;
     return BMSP_OK;
 }
@@ -1294,17 +1315,19 @@ static Plan plan_launch(GemmArgs& g, const bmsp_matrix_s* A, const bmsp_matrix_s
 }
 
 // NUMERIC: the dense-block kernel for narrow rows of dense blocks, the generic mma.sync pass for the other dense-block products,
-// the scalar pass for sparse blocks
+// the scalar pass for sparse blocks.  REUSE: a kept plan's rerun (C's offsets are absolute).  Every launch zeroes its own queue heads,
+// and C's values are zeroed here whenever rows accumulate with global atomics, so a rerun needs nothing else reset.
+template <bool REUSE = false>
 static int run_numeric(GemmArgs& g, const bmsp_matrix_s* C, const Counters& h, const Plan& plan, int path, const RowSplit& sp, int nrows,
                        int sms, cudaStream_t st) {
     if (path == 1 && !sp.active && (int64_t)h.max_words * 32 <= 1024) {
         // narrow rows: one warp per block row, dense accumulators for a window of C columns in shared memory
         int occ = 0;
-        BMSP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, spgemm_dense_kernel, DENSE_WARPS * 32, 0));
+        BMSP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, spgemm_dense_kernel<REUSE>, DENSE_WARPS * 32, 0));
         if (occ < 1) { set_error("spgemm dense pass does not fit"); return BMSP_ERR_CUDA; }
         BMSP_CUDA(cudaMemsetAsync(g.work_counter, 0, sizeof(int32_t), st));
         const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((int64_t)sms * occ, ceil_div(nrows, DENSE_WARPS)));
-        spgemm_dense_kernel<<<grid, DENSE_WARPS * 32, 0, st>>>(g);
+        spgemm_dense_kernel<REUSE><<<grid, DENSE_WARPS * 32, 0, st>>>(g);
         BMSP_KERNEL_CHECK();
         return BMSP_OK;
     }
@@ -1316,7 +1339,7 @@ static int run_numeric(GemmArgs& g, const bmsp_matrix_s* C, const Counters& h, c
         gm.group = 1; gm.batch = plan.mma_batch;          // one block row per work item: pairs of an A block stay adjacent
         // two warps per block row, sharing the row's accumulators (BC4M numeric, one box: 32 threads 19.5 ms, 64: 17.7 ms, 128:
         // 20.2 ms -- a row has ~10 A blocks x 4 lanes to hand out)
-        return launch_pass_t<PASS_NUMERIC_MMA, 256>(gm, 64, sms, nrows, st);
+        return launch_pass_t<PASS_NUMERIC_MMA, 256, REUSE>(gm, 64, sms, nrows, st);
     }
     const int max_c = h.max_c_item, max_rownnz = h.max_nnz_item;
     const double avg_c = nrows ? (double)C->nblk / nrows : 0.0, avg_nnz = nrows ? (double)C->nnz / nrows : 0.0;
@@ -1324,16 +1347,40 @@ static int run_numeric(GemmArgs& g, const bmsp_matrix_s* C, const Counters& h, c
     else if (avg_c <= 512.0 && avg_nnz <= 1536.0) { g.cap_c = clampi(4.0 * avg_c, 256, 2048); g.cap_nnz = clampi(4.0 * avg_nnz, 1024, 8192); }
     else { g.cap_c = 64; g.cap_nnz = 256; }
     if (max_c > g.cap_c || max_rownnz > g.cap_nnz) BMSP_CUDA(cudaMemsetAsync(C->values, 0, (size_t)C->nnz * 4, st));
-    return launch_pass<PASS_NUMERIC>(g, plan.T, sms, st, sp);
+    return launch_pass<PASS_NUMERIC, REUSE>(g, plan.T, sms, st, sp);
 }
 
-extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts* opts, void* stream, bmsp_matrix_t* Cout,
-                           bmsp_spgemm_info* info) {
+// What a product allocates besides C, and the launch state of its NUMERIC pass.  bmsp_spgemm frees all of it after the product; a
+// plan keeps what its NUMERIC launch reads (bmsp_spgemm_plan_create).
+struct ProductState {
+    int2* rowinfo = nullptr; unsigned long long* cand = nullptr; Counters* ctr = nullptr;
+    uint32_t *row_count = nullptr, *row_surv = nullptr; uint64_t* row_nnz = nullptr; uint2* surv_list = nullptr;
+    uint32_t *g_bitset = nullptr, *g_wrank = nullptr;
+    size_t surv_n = 0, scratch_n = 0;   // entries of surv_list and of each of g_bitset / g_wrank
+    RowSplit sp;
+    GemmArgs g;
+    Counters h{};
+    Plan plan{};
+    int path = 0, nrows = 0, sms = 0;
+    bool use_fine = false;
+    void release(cudaStream_t st) {
+        dev_free(sp.list, st);
+        if (sp.side) { cudaStreamSynchronize(sp.side); cudaStreamDestroy(sp.side); }
+        if (sp.fork) cudaEventDestroy(sp.fork);
+        if (sp.join) cudaEventDestroy(sp.join);
+        dev_free(rowinfo, st); dev_free(cand, st); dev_free(ctr, st); dev_free(row_count, st); dev_free(row_surv, st);
+        dev_free(row_nnz, st); dev_free(surv_list, st); dev_free(g_bitset, st); dev_free(g_wrank, st);
+    }
+};
+
+// C = A * Bt: COUNT, FILL, NUMERIC.  On success the scratch stays in `s` (the caller frees or keeps it); on failure it is freed and
+// C destroyed.
+static int spgemm_run(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts* opts, cudaStream_t st, ProductState& s, bmsp_matrix_t* Cout,
+                      bmsp_spgemm_info* info) {
     if (!A || !Bt || !Cout) { set_error("bmsp_spgemm: null argument"); return BMSP_ERR_INVALID; }
     if (A->transposed || !Bt->transposed) { set_error("bmsp_spgemm: A must be plain and B in transposed-operand form (SPGEMM.cu:1261-1262)"); return BMSP_ERR_INVALID; }
     if (A->dtype != BMSP_F16 || Bt->dtype != BMSP_F16) { set_error("bmsp_spgemm: operands must be fp16 (bmSparse_mult<half,float>)"); return BMSP_ERR_UNSUPPORTED; }
     if (A->cols != Bt->rows) { set_error("bmsp_spgemm: inner dimensions differ (%d vs %d)", A->cols, Bt->rows); return BMSP_ERR_INVALID; }
-    cudaStream_t st = (cudaStream_t)stream;
     touch(A, st); touch(Bt, st);
     int rb = 0, re = A->nbr;
     // brow_range_set: the range is taken literally ([r, r) multiplies nothing: a shard that owns no rows); without it the legacy
@@ -1343,7 +1390,8 @@ extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_
     const int nrows = re - rb;
     const bool verbose = opts && opts->verbose;
 
-    int dev = 0, sms = 0;
+    int dev = 0;
+    int& sms = s.sms;
     BMSP_CUDA(cudaGetDevice(&dev));
     BMSP_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
 
@@ -1352,25 +1400,18 @@ extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_
     if (verbose) BMSP_CUDA(cudaEventRecord(ev[0], st));
 
     // ---- scratch
-    int2* rowinfo = nullptr; unsigned long long* cand = nullptr; Counters* ctr = nullptr;
-    uint32_t *row_count = nullptr, *row_surv = nullptr; uint64_t* row_nnz = nullptr; uint2* surv_list = nullptr;
+    s.nrows = nrows;
+    int2*& rowinfo = s.rowinfo; unsigned long long*& cand = s.cand; Counters*& ctr = s.ctr;
+    uint32_t*& row_count = s.row_count; uint32_t*& row_surv = s.row_surv; uint64_t*& row_nnz = s.row_nnz; uint2*& surv_list = s.surv_list;
     bmsp_matrix_s* C = new bmsp_matrix_s();
     touch(C, st);
     C->rows = A->rows; C->cols = Bt->cols; C->dtype = BMSP_F32; C->transposed = 0;
     C->nbr = (int32_t)ceil_div(C->rows, 8);
-    uint32_t *g_bitset = nullptr, *g_wrank = nullptr;
-    RowSplit sp;
+    uint32_t*& g_bitset = s.g_bitset; uint32_t*& g_wrank = s.g_wrank;
+    RowSplit& sp = s.sp;
     int status = BMSP_OK;
-    auto cleanup = [&]() {
-        dev_free(sp.list, st);
-        if (sp.side) { cudaStreamSynchronize(sp.side); cudaStreamDestroy(sp.side); }
-        if (sp.fork) cudaEventDestroy(sp.fork);
-        if (sp.join) cudaEventDestroy(sp.join);
-        dev_free(rowinfo, st); dev_free(cand, st); dev_free(ctr, st); dev_free(row_count, st); dev_free(row_surv, st);
-        dev_free(row_nnz, st); dev_free(surv_list, st); dev_free(g_bitset, st); dev_free(g_wrank, st);
-        for (auto& e : ev) if (e) cudaEventDestroy(e);
-    };
-    auto fail = [&](int code) { cleanup(); bmsp_destroy(C); return code; };
+    auto drop_events = [&]() { for (auto& e : ev) if (e) cudaEventDestroy(e); };
+    auto fail = [&](int code) { s.release(st); s = ProductState(); drop_events(); bmsp_destroy(C); return code; };
 #define SG_TRY(x) do { status = (x); if (status != BMSP_OK) return fail(status); } while (0)
 #define SG_CUDA(x) do { cudaError_t e__ = (x); if (e__ != cudaSuccess) return fail(cuda_fail(e__, #x, __FILE__, __LINE__)); } while (0)
 
@@ -1382,14 +1423,14 @@ extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_
     SG_TRY(dev_alloc_t(&row_nnz, (size_t)nrows + 2, st));
     SG_CUDA(cudaMemsetAsync(ctr, 0, sizeof(Counters), st));
 
-    Counters h{};
+    Counters& h = s.h;
     SG_TRY(plan_rows(A, Bt, rb, re, sms, rowinfo, cand, ctr, h, sp, st));
     SG_TRY(ensure_pmeta(Bt, st));
     SG_TRY(ensure_fine_index(Bt, A, st));
-    const bool use_fine = Bt->fine_state == 1;
-    const int path = numeric_path(A, Bt, opts);
+    const bool use_fine = s.use_fine = Bt->fine_state == 1;
+    const int path = s.path = numeric_path(A, Bt, opts);
 
-    GemmArgs g;
+    GemmArgs& g = s.g;
     memset(&g, 0, sizeof(g));
     if (use_fine) { g.f_ptr = Bt->fine_ptr; g.f_bcol = Bt->fine_bcol; g.f_kmask = Bt->fine_kmask; g.f_rec = (const uint4*)Bt->fine_rec; }
     g.b_pm = (const uint4*)Bt->pmeta;
@@ -1397,12 +1438,12 @@ extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_
     g.b_brp = Bt->brp; g.b_bcol = Bt->bcol; g.b_bmps = Bt->bmps; g.b_kmask = Bt->kmask; g.b_off = Bt->offsets; g.b_val = (const __half*)Bt->values;
     g.rowinfo = rowinfo; g.row_begin = rb; g.row_end = re;
     g.work_counter = &ctr->queue[0]; g.ctr = ctr; g.row_count = row_count; g.row_surv = row_surv; g.row_nnz = row_nnz;
-    const Plan plan = plan_launch(g, A, Bt, nrows, h, sp.active, use_fine, path);
+    const Plan plan = s.plan = plan_launch(g, A, Bt, nrows, h, sp.active, use_fine, path);
 
     if (g.max_words > g.cap_words) {
         // over-cap rows use per-CTA global scratch; size it for the largest persistent grid (32 CTAs/SM)
         sp.heavy_scratch_off = (size_t)sms * 32 * g.max_words;                // + 2 heavy CTAs per SM
-        const size_t n = sp.heavy_scratch_off + (size_t)sms * 2 * g.max_words;
+        const size_t n = s.scratch_n = sp.heavy_scratch_off + (size_t)sms * 2 * g.max_words;
         SG_TRY(dev_alloc_t(&g_bitset, n, st));
         SG_TRY(dev_alloc_t(&g_wrank, n, st));
         g.g_bitset = g_bitset; g.g_wrank = g_wrank;
@@ -1437,7 +1478,8 @@ extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_
     SG_TRY(dev_alloc_t(&C->kmask, (size_t)c_size + 16, st));
     SG_TRY(dev_alloc_t(&C->brp, (size_t)C->nbr + 1 + 8, st));
     SG_TRY(dev_alloc_t(&C->rvb, (size_t)C->nbr + 1 + 8, st));
-    SG_TRY(dev_alloc_t(&surv_list, use_fine ? (size_t)1 : (size_t)n_surv + 1, st));
+    s.surv_n = use_fine ? (size_t)1 : (size_t)n_surv + 1;
+    SG_TRY(dev_alloc_t(&surv_list, s.surv_n, st));
     g.c_brp = (const int32_t*)row_count; g.c_keys = C->keys; g.c_bmps = C->bmps; g.c_bcol = C->bcol; g.c_kmask = C->kmask;
     g.c_off = C->offsets; g.surv_list = surv_list;
 
@@ -1479,9 +1521,76 @@ extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_
             info->total_ms = info->symbolic_ms + info->numeric_ms;
         }
     }
-    cleanup();
+    drop_events();
     *Cout = C;
     return BMSP_OK;
 #undef SG_TRY
 #undef SG_CUDA
+}
+
+extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts* opts, void* stream, bmsp_matrix_t* Cout,
+                           bmsp_spgemm_info* info) {
+    cudaStream_t st = (cudaStream_t)stream;
+    ProductState s;
+    BMSP_TRY(spgemm_run(A, Bt, opts, st, s, Cout, info));
+    s.release(st);
+    return BMSP_OK;
+}
+
+// ---- plans: C's structure kept, its values recomputed from the operands' current values ---------------------------------------
+// A plan keeps what the chosen NUMERIC launch reads: the row tables (bit-set spans, C's block-row pointers, surviving-pair bases,
+// value bases), the counters block (queue heads), the over-cap bit-set scratch, the heavy-row split (row list, side stream, events)
+// and, for the scalar pass over the candidate scan only, FILL's pair list -- left sorted by pair class, which depends on bitmaps
+// alone.  The fine-index walk, the dense-block kernel and the generic MMA pass enumerate their pairs and keep no list.
+struct bmsp_spgemm_plan_s {
+    bmsp_matrix_s *A = nullptr, *Bt = nullptr, *C = nullptr;
+    ProductState s;
+    int64_t bytes = 0;
+    cudaStream_t last_stream = nullptr;   // stream ordering of the plan's scratch, as bmsp_matrix_s::last_stream
+    bool multi_stream = false;
+};
+
+static int64_t alloc_bytes(size_t n) { return n ? (int64_t)(n + BMSP_PAD_BYTES) : 0; }
+
+extern "C" int bmsp_spgemm_plan_create(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts* opts, void* stream,
+                                       bmsp_spgemm_plan_t* plan, bmsp_matrix_t* Cout, bmsp_spgemm_info* info) {
+    if (!plan) { set_error("bmsp_spgemm_plan_create: null argument"); return BMSP_ERR_INVALID; }
+    *plan = nullptr;
+    cudaStream_t st = (cudaStream_t)stream;
+    ProductState s;
+    BMSP_TRY(spgemm_run(A, Bt, opts, st, s, Cout, info));
+    dev_free(s.cand, st); s.cand = nullptr;
+    if (s.path == 1 || s.use_fine) { dev_free(s.surv_list, st); s.surv_list = nullptr; s.g.surv_list = nullptr; s.surv_n = 0; }
+    bmsp_spgemm_plan_s* p = new bmsp_spgemm_plan_s();
+    p->A = A; p->Bt = Bt; p->C = *Cout; p->s = s; p->last_stream = st;
+    const size_t nr = (size_t)s.nrows;
+    p->bytes = alloc_bytes((nr + 1) * sizeof(int2)) + alloc_bytes(sizeof(Counters)) + 2 * alloc_bytes((nr + 2) * sizeof(uint32_t)) +
+               alloc_bytes((nr + 2) * sizeof(uint64_t)) + alloc_bytes(s.surv_n * sizeof(uint2)) + 2 * alloc_bytes(s.scratch_n * sizeof(uint32_t)) +
+               (s.sp.list ? alloc_bytes((nr + 1) * sizeof(int32_t)) : 0);
+    *plan = p;
+    return BMSP_OK;
+}
+
+extern "C" int bmsp_spgemm_numeric(bmsp_spgemm_plan_t p, void* stream) {
+    if (!p) { set_error("bmsp_spgemm_numeric: null plan"); return BMSP_ERR_INVALID; }
+    cudaStream_t st = (cudaStream_t)stream;
+    touch(p->A, st); touch(p->Bt, st); touch(p->C, st);
+    if (p->last_stream != st) p->multi_stream = true;
+    p->last_stream = st;
+    if (p->C->nnz > 0) BMSP_TRY(run_numeric<true>(p->s.g, p->C, p->s.h, p->s.plan, p->s.path, p->s.sp, p->s.nrows, p->s.sms, st));
+    return refresh_value_copies(p->C, st);
+}
+
+extern "C" int bmsp_spgemm_plan_bytes(bmsp_spgemm_plan_t p, int64_t* bytes) {
+    if (!p || !bytes) { set_error("bmsp_spgemm_plan_bytes: null argument"); return BMSP_ERR_INVALID; }
+    *bytes = p->bytes;
+    return BMSP_OK;
+}
+
+extern "C" int bmsp_spgemm_plan_destroy(bmsp_spgemm_plan_t p) {
+    if (!p) return BMSP_OK;
+    if (p->multi_stream) cudaDeviceSynchronize();
+    p->s.release(p->last_stream);
+    delete p;
+    return BMSP_OK;
 }

@@ -132,8 +132,65 @@ class bmSpMatrix:
 
     @property
     def values(self):
+        """The values in compact order, aliasing the handle's memory.  After writing through this alias, call set_values(None): the
+        library keeps copies of a SpGEMM B operand's values, and only set_values refreshes them."""
         v = self._view()
         return _alias(v.values, v.nnz, "<f2" if v.dtype == L.F16 else "<f4", self.dtype, self)
+
+    # ---- new values, same structure -----------------------------------------------------------
+    def set_values(self, values, stream=None):
+        """Overwrite the values in compact order (the order of .values): a torch tensor (CUDA: asynchronous on the stream; CPU:
+        synchronous) or a numpy array, fp16 or fp32 (anything else is taken as fp32), converted to the matrix's dtype.  None: the
+        values were written in place through .values; refresh the library's copies of them."""
+        lib = L.lib()
+        if values is None:
+            L.check(lib.bmsp_set_values(self._h, None, L.F32, L.DEVICE, _stream_ptr(stream)))
+            return
+        if isinstance(values, torch.Tensor) and values.is_cuda:
+            v = values.contiguous()
+            if v.dtype not in (torch.float16, torch.float32):
+                v = v.to(torch.float32)
+            if v.numel() != self.nnz:
+                raise ValueError(f"set_values: {v.numel()} values for a matrix with {self.nnz}")
+            L.check(lib.bmsp_set_values(self._h, C.c_void_p(v.data_ptr()), _dt(v.dtype), L.DEVICE, _stream_ptr(stream)))
+            if v is not values and stream is not None:
+                v.record_stream(stream)        # the temporary outlives this call on `stream`
+            return
+        v = values.numpy() if isinstance(values, torch.Tensor) else np.asarray(values)
+        v = np.ascontiguousarray(v.reshape(-1))
+        if v.dtype not in (np.float16, np.float32):
+            v = v.astype(np.float32)
+        if v.size != self.nnz:
+            raise ValueError(f"set_values: {v.size} values for a matrix with {self.nnz}")
+        L.check(lib.bmsp_set_values(self._h, v.ctypes.data_as(C.c_void_p), L.F16 if v.dtype == np.float16 else L.F32, L.HOST,
+                                    _stream_ptr(stream)))
+
+    def set_values_csr(self, row_ptr, col_idx, vals, stream=None):
+        """New values as a CSR with exactly this matrix's pattern (the arrays from_csr took, for either orientation): CUDA tensors
+        or host arrays, as from_csr takes them.  A different pattern raises BmspError (INVALID) and leaves the values unchanged."""
+        lib = L.lib()
+        v = self._view()
+        if isinstance(row_ptr, torch.Tensor) and row_ptr.is_cuda:
+            rp = row_ptr.to(torch.int32).contiguous(); ci = col_idx.to(torch.int32).contiguous(); x = vals.contiguous()
+            if x.dtype not in (torch.float16, torch.float32):
+                x = x.to(torch.float32)
+            n_rp, n_ci, n_v = rp.numel(), ci.numel(), x.numel()
+            ptrs = (C.c_void_p(rp.data_ptr()), C.c_void_p(ci.data_ptr()), C.c_void_p(x.data_ptr()))
+            dt, mem = _dt(x.dtype), L.DEVICE
+        else:
+            rp = np.ascontiguousarray(row_ptr, np.int32); ci = np.ascontiguousarray(col_idx, np.int32); x = np.ascontiguousarray(vals)
+            if x.dtype not in (np.float16, np.float32):
+                x = x.astype(np.float32)
+            n_rp, n_ci, n_v = rp.size, ci.size, x.size
+            ptrs = tuple(a.ctypes.data_as(C.c_void_p) for a in (rp, ci, x))
+            dt, mem = (L.F16 if x.dtype == np.float16 else L.F32), L.HOST
+        if n_rp != v.num_rows + 1 or n_ci != n_v:
+            raise ValueError("set_values_csr: row_ptr needs num_rows + 1 entries, col_idx and vals one per value")
+        if n_ci != v.nnz:      # the library reads nnz entries of col_idx and vals
+            raise L.BmspError(1, f"set_values_csr: the CSR has {n_ci} entries, the matrix {v.nnz} values")
+        L.check(lib.bmsp_set_values_csr(self._h, *ptrs, dt, mem, _stream_ptr(stream)))
+        if mem == L.DEVICE:
+            (stream if stream is not None else torch.cuda.current_stream()).synchronize()      # rp / ci / x temporaries die here
 
     @property
     def block_row_ptr(self):

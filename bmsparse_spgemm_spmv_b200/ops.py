@@ -2,6 +2,9 @@
 
   bmSparse_SpMV(A, v, u, batched)                    src/bmSparse_SPMV.cu:191-230
   bmSparse_mult(A, B, C, mode, VERBOSE, tc_version)  src/bmSparse_SPGEMM.cu:827-1223
+
+and bmSparse_mult_plan, which the reference does not have: the same product, kept so that C's values can be recomputed after the
+operands' values change.
 """
 from __future__ import annotations
 
@@ -43,13 +46,17 @@ def bmSparse_SpMV_host(A: bmSpMatrix, v: torch.Tensor, u: torch.Tensor | None = 
     return u
 
 
+def _spgemm_opts(mode, tc_version, VERBOSE, numeric_path, brow_range):
+    return L.SpgemmOpts(int(mode), int(tc_version), int(bool(VERBOSE)), int(numeric_path),
+                        brow_range[0] if brow_range is not None else 0, brow_range[1] if brow_range is not None else 0,
+                        int(brow_range is not None))
+
+
 def bmSparse_mult(A: bmSpMatrix, B: bmSpMatrix, C_out: bmSpMatrix | None = None, mode=0, VERBOSE: bool = False,
                   tc_version: int = 5, numeric_path: int = -1, brow_range=None, stream=None):
     """C = A * B with B in transposed-operand form (built with transpose=True, SPGEMM.cu:1262).
     Returns (C, info).  `mode` / `tc_version` are accepted for drop-in compatibility and ignored."""
-    opts = L.SpgemmOpts(int(mode), int(tc_version), int(bool(VERBOSE)), int(numeric_path),
-                        brow_range[0] if brow_range is not None else 0, brow_range[1] if brow_range is not None else 0,
-                        int(brow_range is not None))
+    opts = _spgemm_opts(mode, tc_version, VERBOSE, numeric_path, brow_range)
     info = L.SpgemmInfo()
     out = C_out if C_out is not None else bmSpMatrix()
     if out._h:
@@ -57,3 +64,48 @@ def bmSparse_mult(A: bmSpMatrix, B: bmSpMatrix, C_out: bmSpMatrix | None = None,
         out._h = C.c_void_p()
     L.check(L.lib().bmsp_spgemm(A._h, B._h, C.byref(opts), _stream_ptr(stream), C.byref(out._h), C.byref(info)))
     return out, info
+
+
+class SpGEMMPlan:
+    """C = A * B kept for reuse: C's structure and what its numeric pass reads.  After A's or B's values change
+    (bmSpMatrix.set_values / set_values_csr), numeric() recomputes C's values alone.  Holds A, B and C, so the plan is always
+    released before them.  Its calls must be ordered on one stream at a time."""
+
+    def __init__(self, h, A, B, C, info):
+        self._h, self.A, self.B, self.C, self.info = h, A, B, C, info
+
+    def numeric(self, stream=None):
+        """Recompute C's values from A's and B's current values: enqueued on the stream, no host synchronisation and no
+        allocation, so it can be captured into a CUDA graph."""
+        if not self._h:
+            raise ValueError("SpGEMMPlan is closed")
+        L.check(L.lib().bmsp_spgemm_numeric(self._h, _stream_ptr(stream)))
+        return self.C
+
+    @property
+    def nbytes(self) -> int:
+        """device memory the plan retains besides C and the operands"""
+        n = C.c_int64()
+        L.check(L.lib().bmsp_spgemm_plan_bytes(self._h, C.byref(n)))
+        return n.value
+
+    def close(self):
+        if self._h:
+            L.lib().bmsp_spgemm_plan_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def bmSparse_mult_plan(A: bmSpMatrix, B: bmSpMatrix, VERBOSE: bool = False, numeric_path: int = -1, brow_range=None, stream=None):
+    """bmSparse_mult(A, B, ...) that keeps its plan: returns a SpGEMMPlan whose .C and .info are what bmSparse_mult returns."""
+    opts = _spgemm_opts(0, 5, VERBOSE, numeric_path, brow_range)
+    info = L.SpgemmInfo()
+    out = bmSpMatrix()
+    h = C.c_void_p()
+    L.check(L.lib().bmsp_spgemm_plan_create(A._h, B._h, C.byref(opts), _stream_ptr(stream), C.byref(h), C.byref(out._h), C.byref(info)))
+    return SpGEMMPlan(h, A, B, out, info)

@@ -132,6 +132,21 @@ int bmsp_create_from_arrays(int32_t rows, int32_t cols, int64_t block_num, int64
 
 int bmsp_destroy(bmsp_matrix_t m);
 
+/* New values, same structure.  Overwrite m's values; keys, bitmaps and offsets stay.  values: m's nnz entries in m's own compact
+ * order (the order of bmsp_view.values), fp32 or fp16 (dtype), host or device memory (mem); converted to m's dtype with round to
+ * nearest, as the constructors convert.  values == NULL: the caller has written m's values in place through bmsp_view.values, and
+ * only the library's own copies of them are refreshed.  Every copy a product keeps (a B operand's packed records and fine index)
+ * is rewritten; the SpMV plan holds no values and is kept.  A device source is asynchronous on `stream`; a host source is
+ * synchronous.  No counterpart in the reference. */
+int bmsp_set_values(bmsp_matrix_t m, const void* values, int32_t dtype, int32_t mem, void* stream);
+/* The same, with the values given as a CSR that has exactly m's pattern: row_ptr int32[num_rows+1], col_idx int32 ascending in
+ * each row, vals fp32 or fp16.  Works for both orientations: a plain A and a transposed-operand Bt built from the same CSR take
+ * the same arrays.  A different pattern (an extra, missing or moved entry, a row_ptr that does not span nnz) fails with
+ * BMSP_ERR_INVALID and leaves m's values as they were.  The pattern is checked on the device before anything is written, and the
+ * check's result is read back once: the call synchronises `stream`. */
+int bmsp_set_values_csr(bmsp_matrix_t m, const int32_t* row_ptr, const int32_t* col_idx, const void* vals, int32_t vals_dtype,
+                        int32_t mem, void* stream);
+
 /* ---- access -------------------------------------------------------------------------------- */
 int bmsp_get(bmsp_matrix_t m, bmsp_view* view);
 /* Copy the four interchange arrays to host buffers (any may be NULL).  offsets gets offsets_len. */
@@ -176,6 +191,23 @@ int bmsp_spmv_bytes(bmsp_matrix_t A, int32_t x_dtype, int64_t* bytes);
  * opts and info may be NULL.  Synchronises the stream twice (C sizes must reach the host). */
 int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts* opts, void* stream,
                 bmsp_matrix_t* C, bmsp_spgemm_info* info);
+
+/* SpGEMM plans: the same A * B formed again and again with new values on an unchanged pattern (AMG set-up, Jacobian products,
+ * iterations over a fixed graph).  C's structure depends on the operands' structure only, so a plan keeps C and what its NUMERIC
+ * pass reads, and bmsp_spgemm_numeric recomputes C's values alone.  No counterpart in the reference. */
+typedef struct bmsp_spgemm_plan_s* bmsp_spgemm_plan_t;
+/* Runs C = A * Bt exactly as bmsp_spgemm does (same opts, errors, C and info; synchronises twice) and keeps what the numeric
+ * pass needs.  The plan holds A, Bt and C by pointer: destroy it before any of them. */
+int bmsp_spgemm_plan_create(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts* opts, void* stream,
+                            bmsp_spgemm_plan_t* plan, bmsp_matrix_t* C, bmsp_spgemm_info* info);
+/* Recomputes C's values from A's and Bt's current values (bmsp_set_values / bmsp_set_values_csr).  Only enqueues work on
+ * `stream`: no host synchronisation, no allocation, no read-back, so it can be captured into a CUDA graph.  A plan owns its
+ * queue counters and scratch: its calls must be ordered on one stream at a time; different plans may run concurrently. */
+int bmsp_spgemm_numeric(bmsp_spgemm_plan_t plan, void* stream);
+/* Device memory the plan retains (bytes, allocation padding included; C and the operands not counted). */
+int bmsp_spgemm_plan_bytes(bmsp_spgemm_plan_t plan, int64_t* bytes);
+/* Frees the plan's memory, ordered behind its last bmsp_spgemm_numeric.  Call before A, Bt or C are destroyed. */
+int bmsp_spgemm_plan_destroy(bmsp_spgemm_plan_t plan);
 
 /* Plain form <-> transposed-operand form of the same matrix (bitmap 8x8 transpose + value
  * permutation inside each block; keys unchanged).  The reference can only get the B operand by
