@@ -6,6 +6,8 @@
 #include <string>
 #include <cstdio>
 #include <cstdarg>
+#include <memory>
+#include <utility>
 #include "../../include/bmsparse_b200.h"
 
 #define BMSP_PAD_BYTES 256   // every array is over-allocated so 16-byte bulk copies may overrun the tail
@@ -88,8 +90,9 @@ int cuda_fail(cudaError_t e, const char* what, const char* file, int line);
 
 #define BMSP_KERNEL_CHECK() BMSP_CUDA(cudaGetLastError())
 
-// record that work on m's arrays was enqueued on st (see bmsp_matrix_s::last_stream)
-inline void touch(bmsp_matrix_s* m, cudaStream_t st) {
+// record that work on m's memory was enqueued on st (see bmsp_matrix_s::last_stream; SpGEMM plans follow the same rule)
+template <typename M>
+inline void touch(M* m, cudaStream_t st) {
     if (m->touched && m->last_stream != st) m->multi_stream = true;
     m->last_stream = st; m->touched = true;
 }
@@ -99,6 +102,31 @@ int dev_alloc(void** p, size_t bytes, cudaStream_t st);
 void dev_free(void* p, cudaStream_t st);
 template <typename T>
 inline int dev_alloc_t(T** p, size_t n, cudaStream_t st) { return dev_alloc((void**)p, n * sizeof(T), st); }
+
+// One device allocation of n T, freed on the stream it was allocated on when the buffer goes out of scope, unless release() handed
+// it to an owner.
+template <typename T>
+class DevBuf {
+public:
+    DevBuf() = default;
+    DevBuf(DevBuf&& o) noexcept : p_(o.p_), st_(o.st_) { o.p_ = nullptr; }
+    DevBuf& operator=(DevBuf&& o) noexcept { std::swap(p_, o.p_); std::swap(st_, o.st_); return *this; }
+    ~DevBuf() { reset(); }
+    int alloc(size_t n, cudaStream_t st) { reset(); st_ = st; return dev_alloc_t(&p_, n, st); }
+    T* get() const { return p_; }
+    void reset() { dev_free(p_, st_); p_ = nullptr; }
+    T* release() { T* p = p_; p_ = nullptr; return p; }
+private:
+    T* p_ = nullptr;
+    cudaStream_t st_ = nullptr;
+};
+
+// A handle under construction: bmsp_destroy frees whatever it holds unless release() handed it to the caller.
+struct HandleDeleter { void operator()(bmsp_matrix_s* m) const { bmsp_destroy(m); } };
+using HandlePtr = std::unique_ptr<bmsp_matrix_s, HandleDeleter>;
+// A new handle used on st, with its shape and the interchange arrays: keys / bmps / offsets for nblk blocks (+2 entries) and values
+// for nnz values (+16 bytes).  nnz < 0 leaves the values to the caller (a product's C: FILL finds its value count).
+int new_handle(int32_t rows, int32_t cols, int64_t nblk, int64_t nnz, int32_t dtype, int32_t transposed, cudaStream_t st, HandlePtr& out);
 
 // out[0..n] = exclusive scan of in[0..n-1] (out has n+1 entries, out[n] = total).  in may be nullptr
 // when a transform kernel filled out[0..n-1] in place (in == out allowed).

@@ -211,75 +211,61 @@ static size_t dsize(int dtype) { return dtype == BMSP_F16 ? 2 : 4; }
 static int convert_device_csr(int32_t rows, int32_t cols, int64_t nnz, const int32_t* rp, const int32_t* ci, const void* vals,
                               int vals_dtype, int transposed, int out_dtype, cudaStream_t st, bmsp_matrix_t* out) {
     if (nnz > 0xFFFFFFFFll) { set_error("nnz %lld exceeds 2^32-1", (long long)nnz); return BMSP_ERR_TOO_LARGE; }
-    bmsp_matrix_s* m = new bmsp_matrix_s();
-    touch(m, st);
-    m->rows = rows; m->cols = cols; m->nnz = nnz; m->dtype = out_dtype; m->transposed = transposed;
-    uint64_t* s_key = nullptr; uint8_t* s_p = nullptr; int32_t* s_src = nullptr; int32_t* flags = nullptr;
-    uint32_t* counts = nullptr; int32_t* chunk_row = nullptr;
-    int status = BMSP_OK;
-    auto cleanup = [&]() { dev_free(s_key, st); dev_free(s_p, st); dev_free(s_src, st); dev_free(flags, st); dev_free(counts, st); dev_free(chunk_row, st); };
-    auto fail = [&](int code) { cleanup(); bmsp_destroy(m); return code; };
-#define CV_TRY(x) do { status = (x); if (status != BMSP_OK) return fail(status); } while (0)
-#define CV_CUDA(x) do { cudaError_t e__ = (x); if (e__ != cudaSuccess) return fail(cuda_fail(e__, #x, __FILE__, __LINE__)); } while (0)
+    DevBuf<uint64_t> s_key; DevBuf<uint8_t> s_p; DevBuf<int32_t> s_src, flags, chunk_row; DevBuf<uint32_t> counts;
     int64_t tiles = ceil_div(nnz, 1024);
     uint32_t nblk32 = 0;
-    CV_TRY(dev_alloc_t(&flags, 1, st));
-    CV_CUDA(cudaMemsetAsync(flags, 0, sizeof(int32_t), st));
+    BMSP_TRY(flags.alloc(1, st));
+    BMSP_CUDA(cudaMemsetAsync(flags.get(), 0, sizeof(int32_t), st));
     {
-        check_rowptr_kernel<<<(unsigned)ceil_div((int64_t)rows + 1, 256), 256, 0, st>>>(rp, rows, nnz, flags);
-        CV_CUDA(cudaGetLastError());
+        check_rowptr_kernel<<<(unsigned)ceil_div((int64_t)rows + 1, 256), 256, 0, st>>>(rp, rows, nnz, flags.get());
+        BMSP_KERNEL_CHECK();
         int32_t hflags = 0;
-        CV_CUDA(cudaMemcpyAsync(&hflags, flags, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        CV_CUDA(cudaStreamSynchronize(st));
-        if (hflags & FLAG_ROWPTR) { set_error("row_ptr must start at 0, end at nnz and never decrease"); return fail(BMSP_ERR_INVALID); }
+        BMSP_CUDA(cudaMemcpyAsync(&hflags, flags.get(), sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        BMSP_CUDA(cudaStreamSynchronize(st));
+        if (hflags & FLAG_ROWPTR) { set_error("row_ptr must start at 0, end at nnz and never decrease"); return BMSP_ERR_INVALID; }
     }
     if (nnz > 0) {
-        CV_TRY(dev_alloc_t(&s_key, (size_t)nnz, st));
-        CV_TRY(dev_alloc_t(&s_p, (size_t)nnz, st));
-        CV_TRY(dev_alloc_t(&s_src, (size_t)nnz + 8, st));
-        CV_TRY(dev_alloc_t(&counts, (size_t)tiles + 1, st));
+        BMSP_TRY(s_key.alloc((size_t)nnz, st));
+        BMSP_TRY(s_p.alloc((size_t)nnz, st));
+        BMSP_TRY(s_src.alloc((size_t)nnz + 8, st));
+        BMSP_TRY(counts.alloc((size_t)tiles + 1, st));
         const int64_t nchunks = ceil_div(nnz, RANK_T);
-        CV_TRY(dev_alloc_t(&chunk_row, (size_t)nchunks + 1, st));
-        chunk_row_kernel<<<(unsigned)ceil_div(nchunks + 1, 256), 256, 0, st>>>(rp, rows, nnz, chunk_row, nchunks);
-        CV_CUDA(cudaGetLastError());
+        BMSP_TRY(chunk_row.alloc((size_t)nchunks + 1, st));
+        chunk_row_kernel<<<(unsigned)ceil_div(nchunks + 1, 256), 256, 0, st>>>(rp, rows, nnz, chunk_row.get(), nchunks);
+        BMSP_KERNEL_CHECK();
         unsigned grid = (unsigned)nchunks;
-        if (transposed) rank_kernel<true><<<grid, RANK_T, 0, st>>>(rp, ci, rows, cols, nnz, chunk_row, s_key, s_p, s_src, flags);
-        else            rank_kernel<false><<<grid, RANK_T, 0, st>>>(rp, ci, rows, cols, nnz, chunk_row, s_key, s_p, s_src, flags);
-        CV_CUDA(cudaGetLastError());
+        if (transposed) rank_kernel<true><<<grid, RANK_T, 0, st>>>(rp, ci, rows, cols, nnz, chunk_row.get(), s_key.get(), s_p.get(), s_src.get(), flags.get());
+        else            rank_kernel<false><<<grid, RANK_T, 0, st>>>(rp, ci, rows, cols, nnz, chunk_row.get(), s_key.get(), s_p.get(), s_src.get(), flags.get());
+        BMSP_KERNEL_CHECK();
         int32_t hflags = 0;
-        CV_CUDA(cudaMemcpyAsync(&hflags, flags, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        CV_CUDA(cudaStreamSynchronize(st));
-        if (hflags & FLAG_RANGE) { set_error("column index outside [0, %d)", cols); return fail(BMSP_ERR_RANGE); }
-        if (hflags & FLAG_UNSORTED) { set_error("CSR column indices must ascend inside each row"); return fail(BMSP_ERR_UNSORTED); }
-        if (hflags & FLAG_DUP) { set_error("duplicate (row, col) entries are not supported"); return fail(BMSP_ERR_DUPLICATE); }
-        head_count_kernel<<<(unsigned)tiles, 1024, 0, st>>>(s_key, nnz, counts);
-        CV_CUDA(cudaGetLastError());
-        CV_TRY(exclusive_scan_u32(counts, counts, tiles, st));
-        CV_CUDA(cudaMemcpyAsync(&nblk32, counts + tiles, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        CV_CUDA(cudaStreamSynchronize(st));
+        BMSP_CUDA(cudaMemcpyAsync(&hflags, flags.get(), sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        BMSP_CUDA(cudaStreamSynchronize(st));
+        if (hflags & FLAG_RANGE) { set_error("column index outside [0, %d)", cols); return BMSP_ERR_RANGE; }
+        if (hflags & FLAG_UNSORTED) { set_error("CSR column indices must ascend inside each row"); return BMSP_ERR_UNSORTED; }
+        if (hflags & FLAG_DUP) { set_error("duplicate (row, col) entries are not supported"); return BMSP_ERR_DUPLICATE; }
+        head_count_kernel<<<(unsigned)tiles, 1024, 0, st>>>(s_key.get(), nnz, counts.get());
+        BMSP_KERNEL_CHECK();
+        BMSP_TRY(exclusive_scan_u32(counts.get(), counts.get(), tiles, st));
+        BMSP_CUDA(cudaMemcpyAsync(&nblk32, counts.get() + tiles, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        BMSP_CUDA(cudaStreamSynchronize(st));
     }
-    m->nblk = nblk32; m->offsets_len = m->nblk;
-    CV_TRY(dev_alloc_t(&m->keys, (size_t)m->nblk + 2, st));
-    CV_TRY(dev_alloc_t(&m->bmps, (size_t)m->nblk + 2, st));
-    CV_TRY(dev_alloc_t(&m->offsets, (size_t)m->nblk + 2, st));
-    CV_TRY(dev_alloc(&m->values, (size_t)nnz * dsize(out_dtype) + 16, st));
+    HandlePtr m;
+    BMSP_TRY(new_handle(rows, cols, nblk32, nnz, out_dtype, transposed, st, m));
     if (nnz > 0) {
-        CV_CUDA(cudaMemsetAsync(m->bmps, 0, sizeof(uint64_t) * m->nblk, st));
-        emit_kernel<<<(unsigned)tiles, 1024, 0, st>>>(s_key, s_p, nnz, counts, m->keys, m->bmps, m->offsets);
-        CV_CUDA(cudaGetLastError());
+        BMSP_CUDA(cudaMemsetAsync(m->bmps, 0, sizeof(uint64_t) * m->nblk, st));
+        emit_kernel<<<(unsigned)tiles, 1024, 0, st>>>(s_key.get(), s_p.get(), nnz, counts.get(), m->keys, m->bmps, m->offsets);
+        BMSP_KERNEL_CHECK();
+        const int32_t* src = s_src.get();
         unsigned grid = (unsigned)ceil_div(ceil_div(nnz, 8), 256);
-        if (vals_dtype == BMSP_F32 && out_dtype == BMSP_F16) values_kernel<float, __half><<<grid, 256, 0, st>>>((const float*)vals, s_src, nnz, (__half*)m->values);
-        else if (vals_dtype == BMSP_F16 && out_dtype == BMSP_F16) values_kernel<__half, __half><<<grid, 256, 0, st>>>((const __half*)vals, s_src, nnz, (__half*)m->values);
-        else if (vals_dtype == BMSP_F32 && out_dtype == BMSP_F32) values_kernel<float, float><<<grid, 256, 0, st>>>((const float*)vals, s_src, nnz, (float*)m->values);
-        else values_kernel<__half, float><<<grid, 256, 0, st>>>((const __half*)vals, s_src, nnz, (float*)m->values);
-        CV_CUDA(cudaGetLastError());
+        if (vals_dtype == BMSP_F32 && out_dtype == BMSP_F16) values_kernel<float, __half><<<grid, 256, 0, st>>>((const float*)vals, src, nnz, (__half*)m->values);
+        else if (vals_dtype == BMSP_F16 && out_dtype == BMSP_F16) values_kernel<__half, __half><<<grid, 256, 0, st>>>((const __half*)vals, src, nnz, (__half*)m->values);
+        else if (vals_dtype == BMSP_F32 && out_dtype == BMSP_F32) values_kernel<float, float><<<grid, 256, 0, st>>>((const float*)vals, src, nnz, (float*)m->values);
+        else values_kernel<__half, float><<<grid, 256, 0, st>>>((const __half*)vals, src, nnz, (float*)m->values);
+        BMSP_KERNEL_CHECK();
     }
-    CV_TRY(derive_compact(m, st));
-    cleanup();
-    *out = m;
+    BMSP_TRY(derive_compact(m.get(), st));
+    *out = m.release();
     return BMSP_OK;
-#undef CV_TRY
-#undef CV_CUDA
 }
 
 // ---------------------------------------------------------------------------- block transpose
@@ -323,19 +309,18 @@ int bmsp_create_from_csr(int32_t rows, int32_t cols, int64_t nnz, const int32_t*
     if (mem == BMSP_DEVICE)
         return convert_device_csr(rows, cols, nnz, row_ptr, col_idx, vals, vals_dtype, transposed, out_dtype, st, out);
     if (row_ptr[0] != 0 || (int64_t)row_ptr[rows] != nnz) { set_error("row_ptr[0] must be 0 and row_ptr[rows] == nnz"); return BMSP_ERR_INVALID; }
-    int32_t *d_rp = nullptr, *d_ci = nullptr; void* d_v = nullptr;
-    BMSP_TRY(dev_alloc_t(&d_rp, (size_t)rows + 1, st));
-    BMSP_TRY(dev_alloc_t(&d_ci, (size_t)nnz, st));
-    BMSP_TRY(dev_alloc(&d_v, (size_t)nnz * dsize(vals_dtype), st));
-    BMSP_CUDA(cudaMemcpyAsync(d_rp, row_ptr, sizeof(int32_t) * ((size_t)rows + 1), cudaMemcpyHostToDevice, st));
+    DevBuf<int32_t> d_rp, d_ci; DevBuf<char> d_v;
+    BMSP_TRY(d_rp.alloc((size_t)rows + 1, st));
+    BMSP_TRY(d_ci.alloc((size_t)nnz, st));
+    BMSP_TRY(d_v.alloc((size_t)nnz * dsize(vals_dtype), st));
+    BMSP_CUDA(cudaMemcpyAsync(d_rp.get(), row_ptr, sizeof(int32_t) * ((size_t)rows + 1), cudaMemcpyHostToDevice, st));
     if (nnz) {
-        BMSP_CUDA(cudaMemcpyAsync(d_ci, col_idx, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, st));
-        BMSP_CUDA(cudaMemcpyAsync(d_v, vals, (size_t)nnz * dsize(vals_dtype), cudaMemcpyHostToDevice, st));
+        BMSP_CUDA(cudaMemcpyAsync(d_ci.get(), col_idx, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, st));
+        BMSP_CUDA(cudaMemcpyAsync(d_v.get(), vals, (size_t)nnz * dsize(vals_dtype), cudaMemcpyHostToDevice, st));
     }
-    int s = convert_device_csr(rows, cols, nnz, d_rp, d_ci, d_v, vals_dtype, transposed, out_dtype, st, out);
-    cudaStreamSynchronize(st);
-    dev_free(d_rp, st); dev_free(d_ci, st); dev_free(d_v, st);
-    return s;
+    BMSP_TRY(convert_device_csr(rows, cols, nnz, d_rp.get(), d_ci.get(), d_v.get(), vals_dtype, transposed, out_dtype, st, out));
+    BMSP_CUDA(cudaStreamSynchronize(st));      // host buffers may be freed by the caller
+    return BMSP_OK;
 }
 
 // host COO -> CSR (counting sort by row, columns sorted inside each row); duplicates summed when `merge`
@@ -512,30 +497,21 @@ int bmsp_block_transpose(bmsp_matrix_t A, int32_t out_dtype, void* stream, bmsp_
     if (!A || !At || (out_dtype != BMSP_F16 && out_dtype != BMSP_F32)) { set_error("bmsp_block_transpose: invalid argument"); return BMSP_ERR_INVALID; }
     cudaStream_t st = (cudaStream_t)stream;
     touch(A, st);
-    bmsp_matrix_s* m = new bmsp_matrix_s();
-    touch(m, st);
-    m->rows = A->rows; m->cols = A->cols; m->nnz = A->nnz; m->nblk = A->nblk; m->offsets_len = A->offsets_len;
-    m->dtype = out_dtype; m->transposed = !A->transposed;
-    int s;
-    auto fail = [&](int code) { bmsp_destroy(m); return code; };
-    if ((s = dev_alloc_t(&m->keys, (size_t)m->nblk + 2, st))) return fail(s);
-    if ((s = dev_alloc_t(&m->bmps, (size_t)m->nblk + 2, st))) return fail(s);
-    if ((s = dev_alloc_t(&m->offsets, (size_t)m->nblk + 2, st))) return fail(s);
-    if ((s = dev_alloc(&m->values, (size_t)m->nnz * dsize(out_dtype) + 16, st))) return fail(s);
+    HandlePtr m;
+    BMSP_TRY(new_handle(A->rows, A->cols, A->nblk, A->nnz, out_dtype, !A->transposed, st, m));
+    m->offsets_len = A->offsets_len;
     if (m->nblk) {
-        cudaError_t ce = cudaMemcpyAsync(m->keys, A->keys, sizeof(uint64_t) * m->nblk, cudaMemcpyDeviceToDevice, st);
-        if (ce == cudaSuccess) ce = cudaMemcpyAsync(m->offsets, A->offsets, sizeof(uint64_t) * m->offsets_len, cudaMemcpyDeviceToDevice, st);
-        if (ce != cudaSuccess) return fail(cuda_fail(ce, "block_transpose: copy keys/offsets", __FILE__, __LINE__));
+        BMSP_CUDA(cudaMemcpyAsync(m->keys, A->keys, sizeof(uint64_t) * m->nblk, cudaMemcpyDeviceToDevice, st));
+        BMSP_CUDA(cudaMemcpyAsync(m->offsets, A->offsets, sizeof(uint64_t) * m->offsets_len, cudaMemcpyDeviceToDevice, st));
         unsigned grid = (unsigned)ceil_div(m->nblk, 128);
         if (A->dtype == BMSP_F16 && out_dtype == BMSP_F16) block_transpose_kernel<__half, __half><<<grid, 128, 0, st>>>(A->bmps, A->offsets, (const __half*)A->values, m->bmps, (__half*)m->values, m->nblk);
         else if (A->dtype == BMSP_F32 && out_dtype == BMSP_F16) block_transpose_kernel<float, __half><<<grid, 128, 0, st>>>(A->bmps, A->offsets, (const float*)A->values, m->bmps, (__half*)m->values, m->nblk);
         else if (A->dtype == BMSP_F32 && out_dtype == BMSP_F32) block_transpose_kernel<float, float><<<grid, 128, 0, st>>>(A->bmps, A->offsets, (const float*)A->values, m->bmps, (float*)m->values, m->nblk);
         else block_transpose_kernel<__half, float><<<grid, 128, 0, st>>>(A->bmps, A->offsets, (const __half*)A->values, m->bmps, (float*)m->values, m->nblk);
-        ce = cudaGetLastError();
-        if (ce != cudaSuccess) return fail(cuda_fail(ce, "block_transpose", __FILE__, __LINE__));
+        BMSP_KERNEL_CHECK();
     }
-    if ((s = derive_compact(m, st))) return fail(s);
-    *At = m;
+    BMSP_TRY(derive_compact(m.get(), st));
+    *At = m.release();
     return BMSP_OK;
 }
 

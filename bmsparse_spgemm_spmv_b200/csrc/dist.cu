@@ -61,19 +61,18 @@ extern "C" int bmsp_partition_block_rows(bmsp_matrix_t A, bmsp_matrix_t Bt, int3
     const int nbr = A->nbr;
     bounds[0] = 0; bounds[nparts] = nbr;
     if (nbr == 0) { for (int p = 1; p < nparts; p++) bounds[p] = 0; return BMSP_OK; }
-    uint64_t* w = nullptr;
-    BMSP_TRY(dev_alloc_t(&w, (size_t)nbr + 2, st));
-    if (weight_spgemm) cand_weight_kernel<<<(unsigned)ceil_div(nbr, 8), 256, 0, st>>>(A->brp, A->bcol, Bt->brp, nbr, w);
+    DevBuf<uint64_t> w;
+    BMSP_TRY(w.alloc((size_t)nbr + 2, st));
+    if (weight_spgemm) cand_weight_kernel<<<(unsigned)ceil_div(nbr, 8), 256, 0, st>>>(A->brp, A->bcol, Bt->brp, nbr, w.get());
     else {
         const bool blockpar = A->nblk > 0 && (double)A->nnz / (double)A->nblk < 2.5;      // same rule as plan_spmv
-        spmv_weight_kernel<<<(unsigned)ceil_div(nbr, 256), 256, 0, st>>>(A->brp, A->rvb, nbr, A->dtype == BMSP_F16 ? 2 : 4, blockpar ? 330 + 76 * (uint64_t)(nparts - 1) : 40, w);
+        spmv_weight_kernel<<<(unsigned)ceil_div(nbr, 256), 256, 0, st>>>(A->brp, A->rvb, nbr, A->dtype == BMSP_F16 ? 2 : 4, blockpar ? 330 + 76 * (uint64_t)(nparts - 1) : 40, w.get());
     }
     BMSP_KERNEL_CHECK();
-    BMSP_TRY(exclusive_scan_u64(w, w, nbr, st));
+    BMSP_TRY(exclusive_scan_u64(w.get(), w.get(), nbr, st));
     std::vector<uint64_t> h((size_t)nbr + 1);
-    BMSP_CUDA(cudaMemcpyAsync(h.data(), w, sizeof(uint64_t) * ((size_t)nbr + 1), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(h.data(), w.get(), sizeof(uint64_t) * ((size_t)nbr + 1), cudaMemcpyDeviceToHost, st));
     BMSP_CUDA(cudaStreamSynchronize(st));
-    dev_free(w, st);
     const uint64_t total = h[nbr];
     for (int p = 1; p < nparts; p++) {
         const uint64_t target = (uint64_t)((long double)total * p / nparts);
@@ -95,29 +94,18 @@ extern "C" int bmsp_slice_block_rows(bmsp_matrix_t A, int32_t r0, int32_t r1, in
     BMSP_CUDA(cudaStreamSynchronize(st));
     const int64_t nblk = hb[1] - hb[0], nnz = (int64_t)hv[1] - hv[0];
     const size_t vs = A->dtype == BMSP_F16 ? 2 : 4;
-    bmsp_matrix_s* m = new bmsp_matrix_s();
-    touch(m, st);
-    m->cols = A->cols; m->dtype = A->dtype; m->transposed = A->transposed;
-    m->rows = rebase_rows ? std::min<int64_t>((int64_t)(r1 - r0) * 8, (int64_t)A->rows - (int64_t)r0 * 8) : A->rows;
-    if (m->rows < 0) m->rows = 0;
-    m->nblk = nblk; m->nnz = nnz; m->offsets_len = nblk;
-    int s;
-    auto fail = [&](int code) { bmsp_destroy(m); return code; };
-    if ((s = dev_alloc_t(&m->keys, (size_t)nblk + 2, st))) return fail(s);
-    if ((s = dev_alloc_t(&m->bmps, (size_t)nblk + 2, st))) return fail(s);
-    if ((s = dev_alloc_t(&m->offsets, (size_t)nblk + 2, st))) return fail(s);
-    if ((s = dev_alloc(&m->values, (size_t)nnz * vs + 16, st))) return fail(s);
+    const int64_t rows = rebase_rows ? std::min<int64_t>((int64_t)(r1 - r0) * 8, (int64_t)A->rows - (int64_t)r0 * 8) : A->rows;
+    HandlePtr m;
+    BMSP_TRY(new_handle((int32_t)std::max<int64_t>(rows, 0), A->cols, nblk, nnz, A->dtype, A->transposed, st, m));
     if (nblk) {
-        cudaError_t ce = cudaMemcpyAsync(m->keys, A->keys + hb[0], 8 * nblk, cudaMemcpyDeviceToDevice, st);
-        if (ce == cudaSuccess) ce = cudaMemcpyAsync(m->bmps, A->bmps + hb[0], 8 * nblk, cudaMemcpyDeviceToDevice, st);
-        if (ce == cudaSuccess) ce = cudaMemcpyAsync(m->offsets, A->offsets + hb[0], 8 * nblk, cudaMemcpyDeviceToDevice, st);
-        if (ce == cudaSuccess && nnz) ce = cudaMemcpyAsync(m->values, (const char*)A->values + (size_t)hv[0] * vs, (size_t)nnz * vs, cudaMemcpyDeviceToDevice, st);
-        if (ce != cudaSuccess) return fail(cuda_fail(ce, "slice: copy arrays", __FILE__, __LINE__));
+        BMSP_CUDA(cudaMemcpyAsync(m->keys, A->keys + hb[0], 8 * nblk, cudaMemcpyDeviceToDevice, st));
+        BMSP_CUDA(cudaMemcpyAsync(m->bmps, A->bmps + hb[0], 8 * nblk, cudaMemcpyDeviceToDevice, st));
+        BMSP_CUDA(cudaMemcpyAsync(m->offsets, A->offsets + hb[0], 8 * nblk, cudaMemcpyDeviceToDevice, st));
+        if (nnz) BMSP_CUDA(cudaMemcpyAsync(m->values, (const char*)A->values + (size_t)hv[0] * vs, (size_t)nnz * vs, cudaMemcpyDeviceToDevice, st));
         slice_rebase_kernel<<<(unsigned)ceil_div(nblk, 256), 256, 0, st>>>(m->keys, m->offsets, nblk, nblk, rebase_rows ? (uint64_t)r0 : 0, hv[0]);
-        ce = cudaGetLastError();
-        if (ce != cudaSuccess) return fail(cuda_fail(ce, "slice", __FILE__, __LINE__));
+        BMSP_KERNEL_CHECK();
     }
-    if ((s = derive_compact(m, st))) return fail(s);
-    *out = m;
+    BMSP_TRY(derive_compact(m.get(), st));
+    *out = m.release();
     return BMSP_OK;
 }

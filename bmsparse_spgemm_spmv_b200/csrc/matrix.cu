@@ -124,15 +124,13 @@ static int exclusive_scan_impl(const T* in, T* out, int64_t n, cudaStream_t st, 
         BMSP_KERNEL_CHECK();
         return BMSP_OK;
     }
-    T* sums = nullptr;
-    BMSP_TRY(dev_alloc_t(&sums, (size_t)tiles + 1, st));
-    scan_tile_sums<T><<<(unsigned)tiles, THREADS, 0, st>>>(in, sums, n);
+    DevBuf<T> sums;
+    BMSP_TRY(sums.alloc((size_t)tiles + 1, st));
+    scan_tile_sums<T><<<(unsigned)tiles, THREADS, 0, st>>>(in, sums.get(), n);
     BMSP_KERNEL_CHECK();
-    int s = exclusive_scan_impl<T>(sums, sums, tiles, st, 0);
-    if (s != BMSP_OK) { dev_free(sums, st); return s; }
-    scan_tiles<T><<<(unsigned)tiles, THREADS, 0, st>>>(in, out, sums, n, write_total);
+    BMSP_TRY(exclusive_scan_impl<T>(sums.get(), sums.get(), tiles, st, 0));
+    scan_tiles<T><<<(unsigned)tiles, THREADS, 0, st>>>(in, out, sums.get(), n, write_total);
     BMSP_KERNEL_CHECK();
-    dev_free(sums, st);
     return BMSP_OK;
 }
 
@@ -189,11 +187,24 @@ int derive_compact(bmsp_matrix_s* m, cudaStream_t st) {
     return BMSP_OK;
 }
 
+static size_t dtype_size(int dtype) { return dtype == BMSP_F16 ? 2 : 4; }
+
+int new_handle(int32_t rows, int32_t cols, int64_t nblk, int64_t nnz, int32_t dtype, int32_t transposed, cudaStream_t st, HandlePtr& out) {
+    out.reset(new bmsp_matrix_s());
+    bmsp_matrix_s* m = out.get();
+    touch(m, st);
+    m->rows = rows; m->cols = cols; m->nblk = nblk; m->nnz = std::max<int64_t>(nnz, 0); m->offsets_len = nblk;
+    m->dtype = dtype; m->transposed = transposed;
+    BMSP_TRY(dev_alloc_t(&m->keys, (size_t)nblk + 2, st));
+    BMSP_TRY(dev_alloc_t(&m->bmps, (size_t)nblk + 2, st));
+    BMSP_TRY(dev_alloc_t(&m->offsets, (size_t)nblk + 2, st));
+    if (nnz >= 0) BMSP_TRY(dev_alloc(&m->values, (size_t)nnz * dtype_size(dtype) + 16, st));
+    return BMSP_OK;
+}
+
 }  // namespace bmsp
 
 using namespace bmsp;
-
-static size_t dtype_size(int dtype) { return dtype == BMSP_F16 ? 2 : 4; }
 
 extern "C" {
 
@@ -223,29 +234,19 @@ int bmsp_create_from_arrays(int32_t rows, int32_t cols, int64_t block_num, int64
         return BMSP_ERR_INVALID;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    bmsp_matrix_s* m = new bmsp_matrix_s();
-    touch(m, st);
-    m->rows = rows; m->cols = cols; m->nblk = block_num; m->nnz = nnz; m->offsets_len = offsets_len;
-    m->dtype = dtype; m->transposed = transposed;
+    HandlePtr m;
+    BMSP_TRY(new_handle(rows, cols, block_num, nnz, dtype, transposed, st, m));
+    m->offsets_len = offsets_len;
     cudaMemcpyKind kind = mem == BMSP_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
-    int s = BMSP_OK;
-    auto fail = [&](int code) { bmsp_destroy(m); return code; };
-    if ((s = dev_alloc_t(&m->keys, (size_t)block_num + 2, st))) return fail(s);
-    if ((s = dev_alloc_t(&m->bmps, (size_t)block_num + 2, st))) return fail(s);
-    if ((s = dev_alloc_t(&m->offsets, (size_t)block_num + 2, st))) return fail(s);
-    if ((s = dev_alloc(&m->values, (size_t)nnz * dtype_size(dtype) + 16, st))) return fail(s);
     if (block_num > 0) {
-        if (cudaMemcpyAsync(m->keys, keys, sizeof(uint64_t) * block_num, kind, st) != cudaSuccess ||
-            cudaMemcpyAsync(m->bmps, bmps, sizeof(uint64_t) * block_num, kind, st) != cudaSuccess ||
-            cudaMemcpyAsync(m->offsets, offsets, sizeof(uint64_t) * offsets_len, kind, st) != cudaSuccess)
-            return fail(cuda_fail(cudaGetLastError(), "copy structure", __FILE__, __LINE__));
+        BMSP_CUDA(cudaMemcpyAsync(m->keys, keys, sizeof(uint64_t) * block_num, kind, st));
+        BMSP_CUDA(cudaMemcpyAsync(m->bmps, bmps, sizeof(uint64_t) * block_num, kind, st));
+        BMSP_CUDA(cudaMemcpyAsync(m->offsets, offsets, sizeof(uint64_t) * offsets_len, kind, st));
     }
-    if (nnz > 0 && cudaMemcpyAsync(m->values, values, (size_t)nnz * dtype_size(dtype), kind, st) != cudaSuccess)
-        return fail(cuda_fail(cudaGetLastError(), "copy values", __FILE__, __LINE__));
-    if ((s = derive_compact(m, st))) return fail(s);
-    if (mem == BMSP_HOST && cudaStreamSynchronize(st) != cudaSuccess)   // host buffers may be freed by the caller
-        return fail(cuda_fail(cudaGetLastError(), "sync", __FILE__, __LINE__));
-    *out = m;
+    if (nnz > 0) BMSP_CUDA(cudaMemcpyAsync(m->values, values, (size_t)nnz * dtype_size(dtype), kind, st));
+    BMSP_TRY(derive_compact(m.get(), st));
+    if (mem == BMSP_HOST) BMSP_CUDA(cudaStreamSynchronize(st));   // host buffers may be freed by the caller
+    *out = m.release();
     return BMSP_OK;
 }
 
@@ -314,21 +315,20 @@ extern "C" int bmsp_to_coo(bmsp_matrix_t m, int32_t* rows, int32_t* cols, float*
     if (m->nnz == 0) return BMSP_OK;
     if (m->multi_stream) BMSP_CUDA(cudaDeviceSynchronize());
     cudaStream_t st = m->last_stream;          // ordered behind whatever produced the arrays
-    int32_t *dr = nullptr, *dc = nullptr; float* dv = nullptr;
-    BMSP_TRY(dev_alloc_t(&dr, (size_t)m->nnz, st));
-    BMSP_TRY(dev_alloc_t(&dc, (size_t)m->nnz, st));
-    BMSP_TRY(dev_alloc_t(&dv, (size_t)m->nnz, st));
+    DevBuf<int32_t> dr, dc; DevBuf<float> dv;
+    BMSP_TRY(dr.alloc((size_t)m->nnz, st));
+    BMSP_TRY(dc.alloc((size_t)m->nnz, st));
+    BMSP_TRY(dv.alloc((size_t)m->nnz, st));
     unsigned grid = (unsigned)ceil_div(m->nblk, 128);
     if (m->dtype == BMSP_F16)
-        to_coo_kernel<__half><<<grid, 128, 0, st>>>(m->keys, m->bmps, m->offsets, (const __half*)m->values, m->transposed, dr, dc, dv, m->nblk);
+        to_coo_kernel<__half><<<grid, 128, 0, st>>>(m->keys, m->bmps, m->offsets, (const __half*)m->values, m->transposed, dr.get(), dc.get(), dv.get(), m->nblk);
     else
-        to_coo_kernel<float><<<grid, 128, 0, st>>>(m->keys, m->bmps, m->offsets, (const float*)m->values, m->transposed, dr, dc, dv, m->nblk);
+        to_coo_kernel<float><<<grid, 128, 0, st>>>(m->keys, m->bmps, m->offsets, (const float*)m->values, m->transposed, dr.get(), dc.get(), dv.get(), m->nblk);
     BMSP_KERNEL_CHECK();
-    BMSP_CUDA(cudaMemcpyAsync(rows, dr, sizeof(int32_t) * m->nnz, cudaMemcpyDeviceToHost, st));
-    BMSP_CUDA(cudaMemcpyAsync(cols, dc, sizeof(int32_t) * m->nnz, cudaMemcpyDeviceToHost, st));
-    BMSP_CUDA(cudaMemcpyAsync(vals, dv, sizeof(float) * m->nnz, cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(rows, dr.get(), sizeof(int32_t) * m->nnz, cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(cols, dc.get(), sizeof(int32_t) * m->nnz, cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(vals, dv.get(), sizeof(float) * m->nnz, cudaMemcpyDeviceToHost, st));
     BMSP_CUDA(cudaStreamSynchronize(st));
-    dev_free(dr, st); dev_free(dc, st); dev_free(dv, st);
     return BMSP_OK;
 }
 
@@ -483,20 +483,18 @@ extern "C" int bmsp_to_csr(bmsp_matrix_t m, int32_t* row_ptr, int32_t* col_idx, 
     cudaStream_t st = (cudaStream_t)stream;
     touch(m, st);
     if (mem == BMSP_DEVICE) return to_csr_device(m, row_ptr, col_idx, vals, st);
-    int32_t *d_rp = nullptr, *d_ci = nullptr; float* d_v = nullptr;
-    BMSP_TRY(dev_alloc_t(&d_rp, (size_t)m->rows + 2, st));
-    BMSP_TRY(dev_alloc_t(&d_ci, (size_t)m->nnz + 1, st));
-    BMSP_TRY(dev_alloc_t(&d_v, (size_t)m->nnz + 1, st));
-    int s = to_csr_device(m, d_rp, d_ci, d_v, st);
-    if (s == BMSP_OK) {
-        cudaError_t e = cudaMemcpyAsync(row_ptr, d_rp, sizeof(int32_t) * ((size_t)m->rows + 1), cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess && m->nnz) e = cudaMemcpyAsync(col_idx, d_ci, sizeof(int32_t) * (size_t)m->nnz, cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess && m->nnz) e = cudaMemcpyAsync(vals, d_v, sizeof(float) * (size_t)m->nnz, cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-        if (e != cudaSuccess) s = cuda_fail(e, "bmsp_to_csr: copy out", __FILE__, __LINE__);
+    DevBuf<int32_t> d_rp, d_ci; DevBuf<float> d_v;
+    BMSP_TRY(d_rp.alloc((size_t)m->rows + 2, st));
+    BMSP_TRY(d_ci.alloc((size_t)m->nnz + 1, st));
+    BMSP_TRY(d_v.alloc((size_t)m->nnz + 1, st));
+    BMSP_TRY(to_csr_device(m, d_rp.get(), d_ci.get(), d_v.get(), st));
+    BMSP_CUDA(cudaMemcpyAsync(row_ptr, d_rp.get(), sizeof(int32_t) * ((size_t)m->rows + 1), cudaMemcpyDeviceToHost, st));
+    if (m->nnz) {
+        BMSP_CUDA(cudaMemcpyAsync(col_idx, d_ci.get(), sizeof(int32_t) * (size_t)m->nnz, cudaMemcpyDeviceToHost, st));
+        BMSP_CUDA(cudaMemcpyAsync(vals, d_v.get(), sizeof(float) * (size_t)m->nnz, cudaMemcpyDeviceToHost, st));
     }
-    dev_free(d_rp, st); dev_free(d_ci, st); dev_free(d_v, st);
-    return s;
+    BMSP_CUDA(cudaStreamSynchronize(st));
+    return BMSP_OK;
 }
 
 // ------------------------------------------------------------------------------------ new values, same structure
@@ -538,19 +536,14 @@ static int scatter_values(bmsp_matrix_s* m, const int32_t* rp, const void* vals,
 // device CSR with m's pattern -> m->values: the check pass, one read-back of its flag, then the scatter
 static int set_values_csr_device(bmsp_matrix_s* m, const int32_t* rp, const int32_t* ci, const void* vals, int32_t vals_dtype, cudaStream_t st) {
     if (m->nbr == 0) return BMSP_OK;
-    int32_t* flag = nullptr;
-    BMSP_TRY(dev_alloc_t(&flag, 1, st));
+    DevBuf<int32_t> flag;
+    BMSP_TRY(flag.alloc(1, st));
+    BMSP_CUDA(cudaMemsetAsync(flag.get(), 0, sizeof(int32_t), st));
+    if (m->transposed) BMSP_TRY((launch_scatter<true, true, __half, __half>(m, rp, ci, nullptr, flag.get(), st)));
+    else BMSP_TRY((launch_scatter<false, true, __half, __half>(m, rp, ci, nullptr, flag.get(), st)));
     int32_t h = 0;
-    const int s = [&]() -> int {
-        BMSP_CUDA(cudaMemsetAsync(flag, 0, sizeof(int32_t), st));
-        if (m->transposed) BMSP_TRY((launch_scatter<true, true, __half, __half>(m, rp, ci, nullptr, flag, st)));
-        else BMSP_TRY((launch_scatter<false, true, __half, __half>(m, rp, ci, nullptr, flag, st)));
-        BMSP_CUDA(cudaMemcpyAsync(&h, flag, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        BMSP_CUDA(cudaStreamSynchronize(st));
-        return BMSP_OK;
-    }();
-    dev_free(flag, st);
-    if (s != BMSP_OK) return s;
+    BMSP_CUDA(cudaMemcpyAsync(&h, flag.get(), sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));
     if (h) { set_error("bmsp_set_values_csr: the CSR's pattern differs from the matrix's"); return BMSP_ERR_INVALID; }
     return m->transposed ? scatter_values<true>(m, rp, vals, vals_dtype, st) : scatter_values<false>(m, rp, vals, vals_dtype, st);
 }
@@ -564,12 +557,10 @@ extern "C" int bmsp_set_values(bmsp_matrix_t m, const void* values, int32_t dtyp
         if (dtype == m->dtype) {
             BMSP_CUDA(cudaMemcpyAsync(m->values, values, (size_t)m->nnz * dtype_size(dtype), cudaMemcpyHostToDevice, st));
         } else {
-            void* d = nullptr;
-            BMSP_TRY(dev_alloc(&d, (size_t)m->nnz * dtype_size(dtype), st));
-            cudaError_t e = cudaMemcpyAsync(d, values, (size_t)m->nnz * dtype_size(dtype), cudaMemcpyHostToDevice, st);
-            const int s = e == cudaSuccess ? values_from_device(m, d, dtype, st) : cuda_fail(e, "bmsp_set_values: copy in", __FILE__, __LINE__);
-            dev_free(d, st);
-            if (s != BMSP_OK) return s;
+            DevBuf<char> d;
+            BMSP_TRY(d.alloc((size_t)m->nnz * dtype_size(dtype), st));
+            BMSP_CUDA(cudaMemcpyAsync(d.get(), values, (size_t)m->nnz * dtype_size(dtype), cudaMemcpyHostToDevice, st));
+            BMSP_TRY(values_from_device(m, d.get(), dtype, st));
         }
     }
     BMSP_TRY(refresh_value_copies(m, st));
@@ -594,19 +585,19 @@ extern "C" int bmsp_set_values_csr(bmsp_matrix_t m, const int32_t* row_ptr, cons
         return BMSP_ERR_INVALID;
     }
     const size_t vs = vals_dtype == BMSP_F16 ? 2 : 4;
-    int32_t *d_rp = nullptr, *d_ci = nullptr; void* d_v = nullptr;
-    int s = BMSP_OK;
-    if ((s = dev_alloc_t(&d_rp, (size_t)m->rows + 1, st)) == BMSP_OK && (s = dev_alloc_t(&d_ci, (size_t)m->nnz, st)) == BMSP_OK &&
-        (s = dev_alloc(&d_v, (size_t)m->nnz * vs, st)) == BMSP_OK) {
-        cudaError_t e = cudaMemcpyAsync(d_rp, row_ptr, sizeof(int32_t) * ((size_t)m->rows + 1), cudaMemcpyHostToDevice, st);
-        if (e == cudaSuccess && m->nnz) e = cudaMemcpyAsync(d_ci, col_idx, sizeof(int32_t) * (size_t)m->nnz, cudaMemcpyHostToDevice, st);
-        if (e == cudaSuccess && m->nnz) e = cudaMemcpyAsync(d_v, vals, (size_t)m->nnz * vs, cudaMemcpyHostToDevice, st);
-        s = e == cudaSuccess ? set_values_csr_device(m, d_rp, d_ci, d_v, vals_dtype, st) : cuda_fail(e, "bmsp_set_values_csr: copy in", __FILE__, __LINE__);
-        if (s == BMSP_OK) s = refresh_value_copies(m, st);
-        if (s == BMSP_OK && (e = cudaStreamSynchronize(st)) != cudaSuccess) s = cuda_fail(e, "bmsp_set_values_csr: sync", __FILE__, __LINE__);
+    DevBuf<int32_t> d_rp, d_ci; DevBuf<char> d_v;
+    BMSP_TRY(d_rp.alloc((size_t)m->rows + 1, st));
+    BMSP_TRY(d_ci.alloc((size_t)m->nnz, st));
+    BMSP_TRY(d_v.alloc((size_t)m->nnz * vs, st));
+    BMSP_CUDA(cudaMemcpyAsync(d_rp.get(), row_ptr, sizeof(int32_t) * ((size_t)m->rows + 1), cudaMemcpyHostToDevice, st));
+    if (m->nnz) {
+        BMSP_CUDA(cudaMemcpyAsync(d_ci.get(), col_idx, sizeof(int32_t) * (size_t)m->nnz, cudaMemcpyHostToDevice, st));
+        BMSP_CUDA(cudaMemcpyAsync(d_v.get(), vals, (size_t)m->nnz * vs, cudaMemcpyHostToDevice, st));
     }
-    dev_free(d_rp, st); dev_free(d_ci, st); dev_free(d_v, st);
-    return s;
+    BMSP_TRY(set_values_csr_device(m, d_rp.get(), d_ci.get(), d_v.get(), vals_dtype, st));
+    BMSP_TRY(refresh_value_copies(m, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));
+    return BMSP_OK;
 }
 
 // ------------------------------------------------------------------------------------ compare on the device
@@ -663,47 +654,41 @@ extern "C" int bmsp_compare_csr(bmsp_matrix_t m, const int32_t* row_ptr, const i
     if (!m || !row_ptr) { set_error("bmsp_compare_csr: null argument"); return BMSP_ERR_INVALID; }
     cudaStream_t st = (cudaStream_t)stream;
     touch(m, st);
-    int32_t *a_rp = nullptr, *a_ci = nullptr, *b_rp = nullptr, *b_ci = nullptr; float *a_v = nullptr, *b_v = nullptr;
-    unsigned long long* acc = nullptr;
-    int s = BMSP_OK;
-    auto cleanup = [&]() { dev_free(a_rp, st); dev_free(a_ci, st); dev_free(a_v, st); dev_free(acc, st); if (mem != BMSP_DEVICE) { dev_free(b_rp, st); dev_free(b_ci, st); dev_free(b_v, st); } };
-#define CMP_TRY(x) do { s = (x); if (s != BMSP_OK) { cleanup(); return s; } } while (0)
-#define CMP_CUDA(x) do { cudaError_t e__ = (x); if (e__ != cudaSuccess) { cleanup(); return cuda_fail(e__, #x, __FILE__, __LINE__); } } while (0)
-    CMP_TRY(dev_alloc_t(&a_rp, (size_t)m->rows + 2, st));
-    CMP_TRY(dev_alloc_t(&a_ci, (size_t)m->nnz + 1, st));
-    CMP_TRY(dev_alloc_t(&a_v, (size_t)m->nnz + 1, st));
-    CMP_TRY(dev_alloc_t(&acc, 8, st));
-    CMP_CUDA(cudaMemsetAsync(acc, 0, 8 * sizeof(unsigned long long), st));
-    CMP_TRY(to_csr_device(m, a_rp, a_ci, a_v, st));
-    if (mem == BMSP_DEVICE) { b_rp = const_cast<int32_t*>(row_ptr); b_ci = const_cast<int32_t*>(col_idx); b_v = const_cast<float*>(vals); }
-    else {
+    DevBuf<int32_t> a_rp, a_ci, b_rp_d, b_ci_d; DevBuf<float> a_v, b_v_d; DevBuf<unsigned long long> acc;
+    BMSP_TRY(a_rp.alloc((size_t)m->rows + 2, st));
+    BMSP_TRY(a_ci.alloc((size_t)m->nnz + 1, st));
+    BMSP_TRY(a_v.alloc((size_t)m->nnz + 1, st));
+    BMSP_TRY(acc.alloc(8, st));
+    BMSP_CUDA(cudaMemsetAsync(acc.get(), 0, 8 * sizeof(unsigned long long), st));
+    BMSP_TRY(to_csr_device(m, a_rp.get(), a_ci.get(), a_v.get(), st));
+    const int32_t *b_rp = row_ptr, *b_ci = col_idx; const float* b_v = vals;
+    if (mem != BMSP_DEVICE) {
         const int64_t n = row_ptr[m->rows];
-        CMP_TRY(dev_alloc_t(&b_rp, (size_t)m->rows + 2, st));
-        CMP_TRY(dev_alloc_t(&b_ci, (size_t)n + 1, st));
-        CMP_TRY(dev_alloc_t(&b_v, (size_t)n + 1, st));
-        CMP_CUDA(cudaMemcpyAsync(b_rp, row_ptr, sizeof(int32_t) * ((size_t)m->rows + 1), cudaMemcpyHostToDevice, st));
+        BMSP_TRY(b_rp_d.alloc((size_t)m->rows + 2, st));
+        BMSP_TRY(b_ci_d.alloc((size_t)n + 1, st));
+        BMSP_TRY(b_v_d.alloc((size_t)n + 1, st));
+        BMSP_CUDA(cudaMemcpyAsync(b_rp_d.get(), row_ptr, sizeof(int32_t) * ((size_t)m->rows + 1), cudaMemcpyHostToDevice, st));
         if (n) {
-            CMP_CUDA(cudaMemcpyAsync(b_ci, col_idx, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
-            CMP_CUDA(cudaMemcpyAsync(b_v, vals, sizeof(float) * (size_t)n, cudaMemcpyHostToDevice, st));
+            BMSP_CUDA(cudaMemcpyAsync(b_ci_d.get(), col_idx, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
+            BMSP_CUDA(cudaMemcpyAsync(b_v_d.get(), vals, sizeof(float) * (size_t)n, cudaMemcpyHostToDevice, st));
         }
+        b_rp = b_rp_d.get(); b_ci = b_ci_d.get(); b_v = b_v_d.get();
     }
     if (m->rows > 0) {
-        compare_rows_kernel<<<(unsigned)ceil_div(m->rows, 256), 256, 0, st>>>(m->rows, a_rp, a_ci, a_v, b_rp, b_ci, b_v, acc, reinterpret_cast<double*>(acc + 4));
-        CMP_CUDA(cudaGetLastError());
+        compare_rows_kernel<<<(unsigned)ceil_div(m->rows, 256), 256, 0, st>>>(m->rows, a_rp.get(), a_ci.get(), a_v.get(), b_rp, b_ci, b_v, acc.get(),
+                                                                              reinterpret_cast<double*>(acc.get() + 4));
+        BMSP_KERNEL_CHECK();
     }
     unsigned long long h[8];
-    CMP_CUDA(cudaMemcpyAsync(h, acc, sizeof(h), cudaMemcpyDeviceToHost, st));
-    CMP_CUDA(cudaStreamSynchronize(st));
+    BMSP_CUDA(cudaMemcpyAsync(h, acc.get(), sizeof(h), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));
     double sum, mx;
     memcpy(&sum, &h[4], 8); memcpy(&mx, &h[3], 8);
     if (only_in_m) *only_in_m = (int64_t)h[0];
     if (only_in_csr) *only_in_csr = (int64_t)h[1];
     if (mean_rel_err) *mean_rel_err = h[2] ? sum / (double)h[2] : 0.0;
     if (max_rel_err) *max_rel_err = mx;
-    cleanup();
     return BMSP_OK;
-#undef CMP_TRY
-#undef CMP_CUDA
 }
 
 extern "C" int bmsp_compare(bmsp_matrix_t m, int64_t nnz, const int32_t* rows, const int32_t* cols, const float* vals,

@@ -1099,16 +1099,15 @@ __global__ void finish_rows_kernel(const uint32_t* __restrict__ c_brp_local, con
 using namespace bmsp;
 
 extern "C" int bmsp_debug_pair_bitmap(int64_t n, const uint64_t* a_host, const uint64_t* bt_host, uint64_t* out_host) {
-    uint64_t *a = nullptr, *b = nullptr, *o = nullptr;
+    DevBuf<uint64_t> a, b, o;
     cudaStream_t st = 0;
-    BMSP_TRY(dev_alloc_t(&a, (size_t)n, st)); BMSP_TRY(dev_alloc_t(&b, (size_t)n, st)); BMSP_TRY(dev_alloc_t(&o, (size_t)n, st));
-    BMSP_CUDA(cudaMemcpyAsync(a, a_host, 8 * n, cudaMemcpyHostToDevice, st));
-    BMSP_CUDA(cudaMemcpyAsync(b, bt_host, 8 * n, cudaMemcpyHostToDevice, st));
-    pair_bitmap_test_kernel<<<(unsigned)ceil_div(n, 256), 256, 0, st>>>(a, b, o, n);
+    BMSP_TRY(a.alloc((size_t)n, st)); BMSP_TRY(b.alloc((size_t)n, st)); BMSP_TRY(o.alloc((size_t)n, st));
+    BMSP_CUDA(cudaMemcpyAsync(a.get(), a_host, 8 * n, cudaMemcpyHostToDevice, st));
+    BMSP_CUDA(cudaMemcpyAsync(b.get(), bt_host, 8 * n, cudaMemcpyHostToDevice, st));
+    pair_bitmap_test_kernel<<<(unsigned)ceil_div(n, 256), 256, 0, st>>>(a.get(), b.get(), o.get(), n);
     BMSP_KERNEL_CHECK();
-    BMSP_CUDA(cudaMemcpyAsync(out_host, o, 8 * n, cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(out_host, o.get(), 8 * n, cudaMemcpyDeviceToHost, st));
     BMSP_CUDA(cudaStreamSynchronize(st));
-    dev_free(a, st); dev_free(b, st); dev_free(o, st);
     return BMSP_OK;
 }
 
@@ -1134,11 +1133,16 @@ static int launch_pass_t(const GemmArgs& g, int T, int sms, int nrows, cudaStrea
 // tail of the launch.
 struct RowSplit {
     bool active = false;
-    int32_t* list = nullptr;       // device: heavy rows (descending weight) then light rows (ascending index)
+    DevBuf<int32_t> list;          // heavy rows (descending weight) then light rows (ascending index)
     int n_heavy = 0, n_light = 0;
     cudaStream_t side = nullptr;
     cudaEvent_t fork = nullptr, join = nullptr;
     size_t heavy_scratch_off = 0;  // words: the heavy launch's slice of g_bitset / g_wrank
+    ~RowSplit() {                  // the body runs before `list` is freed
+        if (side) { cudaStreamSynchronize(side); cudaStreamDestroy(side); }
+        if (fork) cudaEventDestroy(fork);
+        if (join) cudaEventDestroy(join);
+    }
 };
 
 template <int PASS, bool REUSE = false>
@@ -1149,9 +1153,9 @@ static int launch_pass(GemmArgs& g, int T, int sms, cudaStream_t st, const RowSp
     }
     GemmArgs gh = g, gl = g;
     gh.group = gl.group = 1;
-    gh.row_list = sp.list; gh.n_list = sp.n_heavy; gh.work_counter = g.work_counter + 1; gh.G = 32; gh.batch = 1;
+    gh.row_list = sp.list.get(); gh.n_list = sp.n_heavy; gh.work_counter = g.work_counter + 1; gh.G = 32; gh.batch = 1;
     if (g.g_bitset) { gh.g_bitset = g.g_bitset + sp.heavy_scratch_off; gh.g_wrank = g.g_wrank + sp.heavy_scratch_off; }
-    gl.row_list = sp.list + sp.n_heavy; gl.n_list = sp.n_light;
+    gl.row_list = sp.list.get() + sp.n_heavy; gl.n_list = sp.n_light;
     BMSP_CUDA(cudaEventRecord(sp.fork, st));
     BMSP_CUDA(cudaStreamWaitEvent(sp.side, sp.fork, 0));
     BMSP_TRY((launch_pass_t<PASS, 1024, REUSE>(gh, 1024, sms, sp.n_heavy, sp.side)));
@@ -1190,8 +1194,8 @@ static int plan_rows(const bmsp_matrix_s* A, const bmsp_matrix_s* Bt, int rb, in
     order = heavy;
     for (int i = 0; i < nrows; i++) if (hc[i] < (unsigned long long)heavy_min) order.push_back(rb + i);
     sp.n_heavy = (int)heavy.size(); sp.n_light = nrows - sp.n_heavy;
-    BMSP_TRY(dev_alloc_t(&sp.list, (size_t)nrows + 1, st));
-    BMSP_CUDA(cudaMemcpyAsync(sp.list, order.data(), sizeof(int32_t) * (size_t)nrows, cudaMemcpyHostToDevice, st));
+    BMSP_TRY(sp.list.alloc((size_t)nrows + 1, st));
+    BMSP_CUDA(cudaMemcpyAsync(sp.list.get(), order.data(), sizeof(int32_t) * (size_t)nrows, cudaMemcpyHostToDevice, st));
     BMSP_CUDA(cudaStreamSynchronize(st));       // `order` dies with this scope
     BMSP_CUDA(cudaStreamCreateWithFlags(&sp.side, cudaStreamNonBlocking));
     BMSP_CUDA(cudaEventCreateWithFlags(&sp.fork, cudaEventDisableTiming));
@@ -1201,30 +1205,34 @@ static int plan_rows(const bmsp_matrix_s* A, const bmsp_matrix_s* Bt, int rb, in
 }
 
 // the two copies of a B operand's values that products keep, (re)written in place: the packed block records and the fine index's
-static int pack_meta(bmsp_matrix_s* Bt, cudaStream_t st) {
+// (the destinations are arguments: a first build writes them before they are published in Bt)
+static int pack_meta(const bmsp_matrix_s* Bt, void* pmeta, cudaStream_t st) {
     pack_meta_kernel<<<(unsigned)ceil_div(Bt->nblk, 256), 256, 0, st>>>(Bt->bmps, Bt->bcol, Bt->offsets, (const __half*)Bt->values, Bt->nnz,
-                                                                      (uint4*)Bt->pmeta, Bt->nblk);
+                                                                      (uint4*)pmeta, Bt->nblk);
     BMSP_KERNEL_CHECK();
     return BMSP_OK;
 }
-static int fine_fill(bmsp_matrix_s* Bt, cudaStream_t st) {
-    fine_fill_kernel<<<(unsigned)ceil_div((int64_t)Bt->nbr * 8, 128), 128, 0, st>>>(Bt->brp, Bt->kmask, (const uint4*)Bt->pmeta, Bt->nbr, Bt->fine_ptr,
-                                                                                   Bt->fine_bcol, Bt->fine_kmask, (uint4*)Bt->fine_rec);
+static int fine_fill(const bmsp_matrix_s* Bt, const uint32_t* fptr, uint32_t* fbcol, uint8_t* fkmask, void* frec, cudaStream_t st) {
+    fine_fill_kernel<<<(unsigned)ceil_div((int64_t)Bt->nbr * 8, 128), 128, 0, st>>>(Bt->brp, Bt->kmask, (const uint4*)Bt->pmeta, Bt->nbr, fptr,
+                                                                                   fbcol, fkmask, (uint4*)frec);
     BMSP_KERNEL_CHECK();
     return BMSP_OK;
 }
 
 int bmsp::refresh_value_copies(bmsp_matrix_s* m, cudaStream_t st) {
-    if (m->pmeta && m->nblk > 0) BMSP_TRY(pack_meta(m, st));
-    if (m->fine_state == 1) BMSP_TRY(fine_fill(m, st));
+    if (m->pmeta && m->nblk > 0) BMSP_TRY(pack_meta(m, m->pmeta, st));
+    if (m->fine_state == 1) BMSP_TRY(fine_fill(m, m->fine_ptr, m->fine_bcol, m->fine_kmask, m->fine_rec, st));
     return BMSP_OK;
 }
 
 // B's packed block records: built once per B operand, reused by later products
 static int ensure_pmeta(bmsp_matrix_s* Bt, cudaStream_t st) {
     if (Bt->pmeta || Bt->nblk == 0) return BMSP_OK;
-    BMSP_TRY(dev_alloc(&Bt->pmeta, 2 * sizeof(uint4) * (size_t)Bt->nblk, st));
-    return pack_meta(Bt, st);
+    DevBuf<uint4> pm;
+    BMSP_TRY(pm.alloc(2 * (size_t)Bt->nblk, st));
+    BMSP_TRY(pack_meta(Bt, pm.get(), st));
+    Bt->pmeta = pm.release();
+    return BMSP_OK;
 }
 
 // Fine index of B for sparse-block operands (about one value per block: uniform random, R-MAT): examined once per B operand, by
@@ -1233,34 +1241,32 @@ static int ensure_fine_index(bmsp_matrix_s* Bt, const bmsp_matrix_s* A, cudaStre
     if (Bt->fine_state != 0 || Bt->nblk == 0 || (int64_t)Bt->nbr * 8 + 1 >= 0x7FFFFFFFll) return BMSP_OK;
     if (!(block_density(Bt) <= 2.0 && block_density(A) <= 4.0)) return BMSP_OK;
     const size_t nb = (size_t)Bt->nbr * 8;
-    uint32_t* fp = nullptr;
-    BMSP_TRY(dev_alloc_t(&fp, nb + 2, st));
+    DevBuf<uint32_t> fp;
+    BMSP_TRY(fp.alloc(nb + 2, st));
+    BMSP_CUDA(cudaMemsetAsync(fp.get(), 0, sizeof(uint32_t) * (nb + 2), st));
+    fine_count_kernel<<<(unsigned)ceil_div(Bt->nblk, 256), 256, 0, st>>>(Bt->keys, Bt->kmask, Bt->nblk, fp.get());
+    BMSP_KERNEL_CHECK();
+    // the longest bucket: slot nb + 1 of the zeroed array
+    fine_max_kernel<<<(unsigned)ceil_div((int64_t)nb, 256), 256, 0, st>>>(fp.get(), (int64_t)nb, fp.get() + nb + 1);
+    BMSP_KERNEL_CHECK();
     uint32_t longest = 0, total = 0;
-    const int status = [&]() -> int {
-        BMSP_CUDA(cudaMemsetAsync(fp, 0, sizeof(uint32_t) * (nb + 2), st));
-        fine_count_kernel<<<(unsigned)ceil_div(Bt->nblk, 256), 256, 0, st>>>(Bt->keys, Bt->kmask, Bt->nblk, fp);
-        BMSP_KERNEL_CHECK();
-        // the longest bucket: slot nb + 1 of the zeroed array
-        fine_max_kernel<<<(unsigned)ceil_div((int64_t)nb, 256), 256, 0, st>>>(fp, (int64_t)nb, fp + nb + 1);
-        BMSP_KERNEL_CHECK();
-        BMSP_CUDA(cudaMemcpyAsync(&longest, fp + nb + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        BMSP_TRY(exclusive_scan_u32(fp, fp, (int64_t)nb, st));
-        BMSP_CUDA(cudaMemcpyAsync(&total, fp + nb, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        BMSP_CUDA(cudaStreamSynchronize(st));
-        return BMSP_OK;
-    }();
-    if (status != BMSP_OK) { dev_free(fp, st); return status; }
+    BMSP_CUDA(cudaMemcpyAsync(&longest, fp.get() + nb + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    BMSP_TRY(exclusive_scan_u32(fp.get(), fp.get(), (int64_t)nb, st));
+    BMSP_CUDA(cudaMemcpyAsync(&total, fp.get() + nb, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));
     // worth it while the buckets replicate little (a block with m inner indices sits in m buckets) and are of similar length:
     // a power-law B (R-MAT) has hub buckets of 10^4 entries next to a mean of 2, and the candidate scan, which spreads a B block
     // row over up to 32 lanes, handles those better (R-MAT-18 A*A: 164 ms by scan, 181 ms through the buckets)
     const double mean_bucket = (double)total / std::max<double>(1.0, (double)nb);
     const bool even = (double)longest <= 32.0 * std::max(mean_bucket, 1.0) || longest <= 512;
-    if (!((double)total <= 1.5 * (double)Bt->nblk && even)) { dev_free(fp, st); Bt->fine_state = -1; return BMSP_OK; }
-    Bt->fine_ptr = fp; Bt->fine_n = total;
-    BMSP_TRY(dev_alloc_t(&Bt->fine_bcol, (size_t)total + 4, st));
-    BMSP_TRY(dev_alloc_t(&Bt->fine_kmask, (size_t)total + 16, st));
-    BMSP_TRY(dev_alloc(&Bt->fine_rec, 2 * sizeof(uint4) * ((size_t)total + 1), st));
-    BMSP_TRY(fine_fill(Bt, st));
+    if (!((double)total <= 1.5 * (double)Bt->nblk && even)) { Bt->fine_state = -1; return BMSP_OK; }
+    DevBuf<uint32_t> fbcol; DevBuf<uint8_t> fkmask; DevBuf<uint4> frec;
+    BMSP_TRY(fbcol.alloc((size_t)total + 4, st));
+    BMSP_TRY(fkmask.alloc((size_t)total + 16, st));
+    BMSP_TRY(frec.alloc(2 * ((size_t)total + 1), st));
+    BMSP_TRY(fine_fill(Bt, fp.get(), fbcol.get(), fkmask.get(), frec.get(), st));
+    Bt->fine_ptr = fp.release(); Bt->fine_bcol = fbcol.release(); Bt->fine_kmask = fkmask.release(); Bt->fine_rec = frec.release();
+    Bt->fine_n = total;
     Bt->fine_state = 1;
     return BMSP_OK;
 }
@@ -1350,12 +1356,14 @@ static int run_numeric(GemmArgs& g, const bmsp_matrix_s* C, const Counters& h, c
     return launch_pass<PASS_NUMERIC, REUSE>(g, plan.T, sms, st, sp);
 }
 
-// What a product allocates besides C, and the launch state of its NUMERIC pass.  bmsp_spgemm frees all of it after the product; a
-// plan keeps what its NUMERIC launch reads (bmsp_spgemm_plan_create).
+// What a product allocates, and the launch state of its NUMERIC pass.  bmsp_spgemm frees all of it after the product; a plan keeps
+// what its NUMERIC launch reads (bmsp_spgemm_plan_create).  Members are destroyed in reverse order: `sp` drains its side stream
+// before the scratch and C, which the side stream's launches use, are freed.
 struct ProductState {
-    int2* rowinfo = nullptr; unsigned long long* cand = nullptr; Counters* ctr = nullptr;
-    uint32_t *row_count = nullptr, *row_surv = nullptr; uint64_t* row_nnz = nullptr; uint2* surv_list = nullptr;
-    uint32_t *g_bitset = nullptr, *g_wrank = nullptr;
+    HandlePtr C;                        // until spgemm_run hands it out
+    DevBuf<int2> rowinfo; DevBuf<unsigned long long> cand; DevBuf<Counters> ctr;
+    DevBuf<uint32_t> row_count, row_surv; DevBuf<uint64_t> row_nnz; DevBuf<uint2> surv_list;
+    DevBuf<uint32_t> g_bitset, g_wrank;
     size_t surv_n = 0, scratch_n = 0;   // entries of surv_list and of each of g_bitset / g_wrank
     RowSplit sp;
     GemmArgs g;
@@ -1363,18 +1371,10 @@ struct ProductState {
     Plan plan{};
     int path = 0, nrows = 0, sms = 0;
     bool use_fine = false;
-    void release(cudaStream_t st) {
-        dev_free(sp.list, st);
-        if (sp.side) { cudaStreamSynchronize(sp.side); cudaStreamDestroy(sp.side); }
-        if (sp.fork) cudaEventDestroy(sp.fork);
-        if (sp.join) cudaEventDestroy(sp.join);
-        dev_free(rowinfo, st); dev_free(cand, st); dev_free(ctr, st); dev_free(row_count, st); dev_free(row_surv, st);
-        dev_free(row_nnz, st); dev_free(surv_list, st); dev_free(g_bitset, st); dev_free(g_wrank, st);
-    }
 };
 
-// C = A * Bt: COUNT, FILL, NUMERIC.  On success the scratch stays in `s` (the caller frees or keeps it); on failure it is freed and
-// C destroyed.
+// C = A * Bt: COUNT, FILL, NUMERIC.  On success the scratch stays in `s` (the caller frees or keeps it with s); on failure C is
+// destroyed with s.
 static int spgemm_run(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts* opts, cudaStream_t st, ProductState& s, bmsp_matrix_t* Cout,
                       bmsp_spgemm_info* info) {
     if (!A || !Bt || !Cout) { set_error("bmsp_spgemm: null argument"); return BMSP_ERR_INVALID; }
@@ -1395,38 +1395,32 @@ static int spgemm_run(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts*
     BMSP_CUDA(cudaGetDevice(&dev));
     BMSP_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
 
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};       // start, after FILL, end, after COUNT
-    if (verbose) for (auto& e : ev) BMSP_CUDA(cudaEventCreate(&e));
+    struct Timing {
+        cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};   // start, after FILL, end, after COUNT
+        ~Timing() { for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e); }
+    } t;
+    cudaEvent_t* ev = t.ev;
+    if (verbose) for (int i = 0; i < 4; i++) BMSP_CUDA(cudaEventCreate(&ev[i]));
     if (verbose) BMSP_CUDA(cudaEventRecord(ev[0], st));
 
     // ---- scratch
     s.nrows = nrows;
-    int2*& rowinfo = s.rowinfo; unsigned long long*& cand = s.cand; Counters*& ctr = s.ctr;
-    uint32_t*& row_count = s.row_count; uint32_t*& row_surv = s.row_surv; uint64_t*& row_nnz = s.row_nnz; uint2*& surv_list = s.surv_list;
-    bmsp_matrix_s* C = new bmsp_matrix_s();
-    touch(C, st);
-    C->rows = A->rows; C->cols = Bt->cols; C->dtype = BMSP_F32; C->transposed = 0;
-    C->nbr = (int32_t)ceil_div(C->rows, 8);
-    uint32_t*& g_bitset = s.g_bitset; uint32_t*& g_wrank = s.g_wrank;
-    RowSplit& sp = s.sp;
-    int status = BMSP_OK;
-    auto drop_events = [&]() { for (auto& e : ev) if (e) cudaEventDestroy(e); };
-    auto fail = [&](int code) { s.release(st); s = ProductState(); drop_events(); bmsp_destroy(C); return code; };
-#define SG_TRY(x) do { status = (x); if (status != BMSP_OK) return fail(status); } while (0)
-#define SG_CUDA(x) do { cudaError_t e__ = (x); if (e__ != cudaSuccess) return fail(cuda_fail(e__, #x, __FILE__, __LINE__)); } while (0)
-
-    SG_TRY(dev_alloc_t(&rowinfo, (size_t)nrows + 1, st));
-    SG_TRY(dev_alloc_t(&cand, (size_t)nrows + 1, st));
-    SG_TRY(dev_alloc_t(&ctr, 1, st));
-    SG_TRY(dev_alloc_t(&row_count, (size_t)nrows + 2, st));
-    SG_TRY(dev_alloc_t(&row_surv, (size_t)nrows + 2, st));
-    SG_TRY(dev_alloc_t(&row_nnz, (size_t)nrows + 2, st));
-    SG_CUDA(cudaMemsetAsync(ctr, 0, sizeof(Counters), st));
+    BMSP_TRY(s.rowinfo.alloc((size_t)nrows + 1, st));
+    BMSP_TRY(s.cand.alloc((size_t)nrows + 1, st));
+    BMSP_TRY(s.ctr.alloc(1, st));
+    BMSP_TRY(s.row_count.alloc((size_t)nrows + 2, st));
+    BMSP_TRY(s.row_surv.alloc((size_t)nrows + 2, st));
+    BMSP_TRY(s.row_nnz.alloc((size_t)nrows + 2, st));
+    Counters* ctr = s.ctr.get();
+    uint32_t *row_count = s.row_count.get(), *row_surv = s.row_surv.get();
+    uint64_t* row_nnz = s.row_nnz.get();
+    BMSP_CUDA(cudaMemsetAsync(ctr, 0, sizeof(Counters), st));
 
     Counters& h = s.h;
-    SG_TRY(plan_rows(A, Bt, rb, re, sms, rowinfo, cand, ctr, h, sp, st));
-    SG_TRY(ensure_pmeta(Bt, st));
-    SG_TRY(ensure_fine_index(Bt, A, st));
+    RowSplit& sp = s.sp;
+    BMSP_TRY(plan_rows(A, Bt, rb, re, sms, s.rowinfo.get(), s.cand.get(), ctr, h, sp, st));
+    BMSP_TRY(ensure_pmeta(Bt, st));
+    BMSP_TRY(ensure_fine_index(Bt, A, st));
     const bool use_fine = s.use_fine = Bt->fine_state == 1;
     const int path = s.path = numeric_path(A, Bt, opts);
 
@@ -1436,7 +1430,7 @@ static int spgemm_run(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts*
     g.b_pm = (const uint4*)Bt->pmeta;
     g.a_brp = A->brp; g.a_bcol = A->bcol; g.a_bmps = A->bmps; g.a_kmask = A->kmask; g.a_off = A->offsets; g.a_val = (const __half*)A->values;
     g.b_brp = Bt->brp; g.b_bcol = Bt->bcol; g.b_bmps = Bt->bmps; g.b_kmask = Bt->kmask; g.b_off = Bt->offsets; g.b_val = (const __half*)Bt->values;
-    g.rowinfo = rowinfo; g.row_begin = rb; g.row_end = re;
+    g.rowinfo = s.rowinfo.get(); g.row_begin = rb; g.row_end = re;
     g.work_counter = &ctr->queue[0]; g.ctr = ctr; g.row_count = row_count; g.row_surv = row_surv; g.row_nnz = row_nnz;
     const Plan plan = s.plan = plan_launch(g, A, Bt, nrows, h, sp.active, use_fine, path);
 
@@ -1444,76 +1438,76 @@ static int spgemm_run(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts*
         // over-cap rows use per-CTA global scratch; size it for the largest persistent grid (32 CTAs/SM)
         sp.heavy_scratch_off = (size_t)sms * 32 * g.max_words;                // + 2 heavy CTAs per SM
         const size_t n = s.scratch_n = sp.heavy_scratch_off + (size_t)sms * 2 * g.max_words;
-        SG_TRY(dev_alloc_t(&g_bitset, n, st));
-        SG_TRY(dev_alloc_t(&g_wrank, n, st));
-        g.g_bitset = g_bitset; g.g_wrank = g_wrank;
+        BMSP_TRY(s.g_bitset.alloc(n, st));
+        BMSP_TRY(s.g_wrank.alloc(n, st));
+        g.g_bitset = s.g_bitset.get(); g.g_wrank = s.g_wrank.get();
     }
 
     // ---- COUNT: C blocks and surviving pairs per block row
     int64_t c_size = 0, n_surv = 0;
     if (nrows > 0) {
-        SG_TRY(launch_pass<PASS_COUNT>(g, plan.T, sms, st, sp));
-        SG_TRY(exclusive_scan_u32(row_count, row_count, nrows, st));
-        SG_TRY(exclusive_scan_u32(row_surv, row_surv, nrows, st));
+        BMSP_TRY(launch_pass<PASS_COUNT>(g, plan.T, sms, st, sp));
+        BMSP_TRY(exclusive_scan_u32(row_count, row_count, nrows, st));
+        BMSP_TRY(exclusive_scan_u32(row_surv, row_surv, nrows, st));
         uint32_t tot[2] = {0, 0};
-        SG_CUDA(cudaMemcpyAsync(&tot[0], row_count + nrows, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        SG_CUDA(cudaMemcpyAsync(&tot[1], row_surv + nrows, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        SG_CUDA(cudaMemcpyAsync(&h, ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
-        SG_CUDA(cudaStreamSynchronize(st));
+        BMSP_CUDA(cudaMemcpyAsync(&tot[0], row_count + nrows, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        BMSP_CUDA(cudaMemcpyAsync(&tot[1], row_surv + nrows, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        BMSP_CUDA(cudaMemcpyAsync(&h, ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
+        BMSP_CUDA(cudaStreamSynchronize(st));
         c_size = tot[0]; n_surv = tot[1];
     }
-    if (verbose) SG_CUDA(cudaEventRecord(ev[3], st));
+    if (verbose) BMSP_CUDA(cudaEventRecord(ev[3], st));
     if (c_size > 0x7FFFFFFFll || h.surviving > 0xFFFFFFFFull) {
         set_error("product too large for one call: %lld C blocks, %llu surviving pairs (shard A's block rows with brow_begin/brow_end)",
                   (long long)c_size, h.surviving);
-        return fail(BMSP_ERR_TOO_LARGE);
+        return BMSP_ERR_TOO_LARGE;
     }
     const int max_c = h.max_c_item;
 
-    C->nblk = c_size; C->offsets_len = c_size + 1;
-    SG_TRY(dev_alloc_t(&C->keys, (size_t)c_size + 2, st));
-    SG_TRY(dev_alloc_t(&C->bmps, (size_t)c_size + 2, st));
-    SG_TRY(dev_alloc_t(&C->offsets, (size_t)c_size + 2, st));
-    SG_TRY(dev_alloc_t(&C->bcol, (size_t)c_size + 8, st));
-    SG_TRY(dev_alloc_t(&C->kmask, (size_t)c_size + 16, st));
-    SG_TRY(dev_alloc_t(&C->brp, (size_t)C->nbr + 1 + 8, st));
-    SG_TRY(dev_alloc_t(&C->rvb, (size_t)C->nbr + 1 + 8, st));
+    BMSP_TRY(new_handle(A->rows, Bt->cols, c_size, -1, BMSP_F32, 0, st, s.C));      // values: once FILL has counted them
+    bmsp_matrix_s* C = s.C.get();
+    C->offsets_len = c_size + 1;
+    C->nbr = (int32_t)ceil_div(C->rows, 8);
+    BMSP_TRY(dev_alloc_t(&C->bcol, (size_t)c_size + 8, st));
+    BMSP_TRY(dev_alloc_t(&C->kmask, (size_t)c_size + 16, st));
+    BMSP_TRY(dev_alloc_t(&C->brp, (size_t)C->nbr + 1 + 8, st));
+    BMSP_TRY(dev_alloc_t(&C->rvb, (size_t)C->nbr + 1 + 8, st));
     s.surv_n = use_fine ? (size_t)1 : (size_t)n_surv + 1;
-    SG_TRY(dev_alloc_t(&surv_list, s.surv_n, st));
+    BMSP_TRY(s.surv_list.alloc(s.surv_n, st));
     g.c_brp = (const int32_t*)row_count; g.c_keys = C->keys; g.c_bmps = C->bmps; g.c_bcol = C->bcol; g.c_kmask = C->kmask;
-    g.c_off = C->offsets; g.surv_list = surv_list;
+    g.c_off = C->offsets; g.surv_list = s.surv_list.get();
 
     // ---- FILL: pair list, keys, bitmaps, row-relative value offsets
     const double avg_c = nrows ? (double)c_size / nrows : 0.0;
     g.cap_c = max_c <= 4096 ? std::max(1, max_c) : (avg_c <= 512.0 ? clampi(4.0 * avg_c, 256, 2048) : 64);
     if (c_size > 0) {
-        if (max_c > g.cap_c) SG_CUDA(cudaMemsetAsync(C->bmps, 0, sizeof(uint64_t) * c_size, st));
-        SG_TRY(launch_pass<PASS_FILL>(g, plan.T, sms, st, sp));
+        if (max_c > g.cap_c) BMSP_CUDA(cudaMemsetAsync(C->bmps, 0, sizeof(uint64_t) * c_size, st));
+        BMSP_TRY(launch_pass<PASS_FILL>(g, plan.T, sms, st, sp));
     } else if (nrows > 0) {
-        SG_CUDA(cudaMemsetAsync(row_nnz, 0, sizeof(uint64_t) * ((size_t)nrows + 1), st));
+        BMSP_CUDA(cudaMemsetAsync(row_nnz, 0, sizeof(uint64_t) * ((size_t)nrows + 1), st));
     }
-    SG_TRY(exclusive_scan_u64(row_nnz, row_nnz, nrows, st));
+    BMSP_TRY(exclusive_scan_u64(row_nnz, row_nnz, nrows, st));
     uint64_t c_nnz = 0;
-    SG_CUDA(cudaMemcpyAsync(&c_nnz, row_nnz + nrows, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    SG_CUDA(cudaMemcpyAsync(&h, ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
-    SG_CUDA(cudaStreamSynchronize(st));
-    if (c_nnz > 0xFFFFFFFFull) { set_error("C has %llu values (> 2^32-1)", (unsigned long long)c_nnz); return fail(BMSP_ERR_TOO_LARGE); }
+    BMSP_CUDA(cudaMemcpyAsync(&c_nnz, row_nnz + nrows, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(&h, ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));
+    if (c_nnz > 0xFFFFFFFFull) { set_error("C has %llu values (> 2^32-1)", (unsigned long long)c_nnz); return BMSP_ERR_TOO_LARGE; }
     C->nnz = (int64_t)c_nnz;
-    SG_TRY(dev_alloc(&C->values, (size_t)c_nnz * 4 + 16, st));
-    if (verbose) SG_CUDA(cudaEventRecord(ev[1], st));
+    BMSP_TRY(dev_alloc(&C->values, (size_t)c_nnz * 4 + 16, st));
+    if (verbose) BMSP_CUDA(cudaEventRecord(ev[1], st));
 
     g.c_val = (float*)C->values;
-    if (c_nnz > 0) SG_TRY(run_numeric(g, C, h, plan, path, sp, nrows, sms, st));
+    if (c_nnz > 0) BMSP_TRY(run_numeric(g, C, h, plan, path, sp, nrows, sms, st));
     finish_rows_kernel<<<(unsigned)ceil_div(C->nbr + 1, 256), 256, 0, st>>>(row_count, row_nnz, rb, re, C->nbr, C->brp, C->rvb, C->offsets, c_size, c_nnz);
-    SG_CUDA(cudaGetLastError());
-    if (verbose) SG_CUDA(cudaEventRecord(ev[2], st));
+    BMSP_KERNEL_CHECK();
+    if (verbose) BMSP_CUDA(cudaEventRecord(ev[2], st));
 
     if (info) {
         memset(info, 0, sizeof(*info));
         info->candidate_pairs = (int64_t)h.sum_cand; info->surviving_pairs = (int64_t)h.surviving;
         info->c_blocks = c_size; info->c_nnz = (int64_t)c_nnz; info->numeric_path = path;
         if (verbose) {
-            SG_CUDA(cudaEventSynchronize(ev[2]));
+            BMSP_CUDA(cudaEventSynchronize(ev[2]));
             cudaEventElapsedTime(&info->symbolic_ms, ev[0], ev[1]);
             cudaEventElapsedTime(&info->numeric_ms, ev[1], ev[2]);
             cudaEventElapsedTime(&info->count_ms, ev[0], ev[3]);
@@ -1521,20 +1515,14 @@ static int spgemm_run(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts*
             info->total_ms = info->symbolic_ms + info->numeric_ms;
         }
     }
-    drop_events();
-    *Cout = C;
+    *Cout = s.C.release();
     return BMSP_OK;
-#undef SG_TRY
-#undef SG_CUDA
 }
 
 extern "C" int bmsp_spgemm(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts* opts, void* stream, bmsp_matrix_t* Cout,
                            bmsp_spgemm_info* info) {
-    cudaStream_t st = (cudaStream_t)stream;
     ProductState s;
-    BMSP_TRY(spgemm_run(A, Bt, opts, st, s, Cout, info));
-    s.release(st);
-    return BMSP_OK;
+    return spgemm_run(A, Bt, opts, (cudaStream_t)stream, s, Cout, info);
 }
 
 // ---- plans: C's structure kept, its values recomputed from the operands' current values ---------------------------------------
@@ -1546,8 +1534,8 @@ struct bmsp_spgemm_plan_s {
     bmsp_matrix_s *A = nullptr, *Bt = nullptr, *C = nullptr;
     ProductState s;
     int64_t bytes = 0;
-    cudaStream_t last_stream = nullptr;   // stream ordering of the plan's scratch, as bmsp_matrix_s::last_stream
-    bool multi_stream = false;
+    cudaStream_t last_stream = nullptr;   // stream ordering of the plan's scratch, as bmsp_matrix_s::last_stream (touch)
+    bool multi_stream = false, touched = false;
 };
 
 static int64_t alloc_bytes(size_t n) { return n ? (int64_t)(n + BMSP_PAD_BYTES) : 0; }
@@ -1557,26 +1545,25 @@ extern "C" int bmsp_spgemm_plan_create(bmsp_matrix_t A, bmsp_matrix_t Bt, const 
     if (!plan) { set_error("bmsp_spgemm_plan_create: null argument"); return BMSP_ERR_INVALID; }
     *plan = nullptr;
     cudaStream_t st = (cudaStream_t)stream;
-    ProductState s;
+    std::unique_ptr<bmsp_spgemm_plan_s> p(new bmsp_spgemm_plan_s());
+    ProductState& s = p->s;
     BMSP_TRY(spgemm_run(A, Bt, opts, st, s, Cout, info));
-    dev_free(s.cand, st); s.cand = nullptr;
-    if (s.path == 1 || s.use_fine) { dev_free(s.surv_list, st); s.surv_list = nullptr; s.g.surv_list = nullptr; s.surv_n = 0; }
-    bmsp_spgemm_plan_s* p = new bmsp_spgemm_plan_s();
-    p->A = A; p->Bt = Bt; p->C = *Cout; p->s = s; p->last_stream = st;
+    s.cand.reset();
+    if (s.path == 1 || s.use_fine) { s.surv_list.reset(); s.g.surv_list = nullptr; s.surv_n = 0; }
+    p->A = A; p->Bt = Bt; p->C = *Cout;
+    touch(p.get(), st);
     const size_t nr = (size_t)s.nrows;
     p->bytes = alloc_bytes((nr + 1) * sizeof(int2)) + alloc_bytes(sizeof(Counters)) + 2 * alloc_bytes((nr + 2) * sizeof(uint32_t)) +
                alloc_bytes((nr + 2) * sizeof(uint64_t)) + alloc_bytes(s.surv_n * sizeof(uint2)) + 2 * alloc_bytes(s.scratch_n * sizeof(uint32_t)) +
-               (s.sp.list ? alloc_bytes((nr + 1) * sizeof(int32_t)) : 0);
-    *plan = p;
+               (s.sp.list.get() ? alloc_bytes((nr + 1) * sizeof(int32_t)) : 0);
+    *plan = p.release();
     return BMSP_OK;
 }
 
 extern "C" int bmsp_spgemm_numeric(bmsp_spgemm_plan_t p, void* stream) {
     if (!p) { set_error("bmsp_spgemm_numeric: null plan"); return BMSP_ERR_INVALID; }
     cudaStream_t st = (cudaStream_t)stream;
-    touch(p->A, st); touch(p->Bt, st); touch(p->C, st);
-    if (p->last_stream != st) p->multi_stream = true;
-    p->last_stream = st;
+    touch(p->A, st); touch(p->Bt, st); touch(p->C, st); touch(p, st);
     if (p->C->nnz > 0) BMSP_TRY(run_numeric<true>(p->s.g, p->C, p->s.h, p->s.plan, p->s.path, p->s.sp, p->s.nrows, p->s.sms, st));
     return refresh_value_copies(p->C, st);
 }
@@ -1589,8 +1576,7 @@ extern "C" int bmsp_spgemm_plan_bytes(bmsp_spgemm_plan_t p, int64_t* bytes) {
 
 extern "C" int bmsp_spgemm_plan_destroy(bmsp_spgemm_plan_t p) {
     if (!p) return BMSP_OK;
-    if (p->multi_stream) cudaDeviceSynchronize();
-    p->s.release(p->last_stream);
+    if (p->multi_stream) cudaDeviceSynchronize();     // else the scratch is freed on the one stream the plan used
     delete p;
     return BMSP_OK;
 }

@@ -1284,19 +1284,18 @@ __global__ void work_fill_kernel(const int32_t* __restrict__ brp, int nbr, const
 static int env_int(const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; }
 
 // The streaming kernel's bitmap palette: collect the distinct bitmaps (palette_scan_kernel), sort them here and upload one 16-byte
-// entry per bitmap (layout at PalScan).  Leaves m->spmv_npal = 0 when the matrix has more than PALETTE_MAX distinct bitmaps.
-static int build_palette(bmsp_matrix_s* m, int vsize, cudaStream_t st, std::vector<uint4>& pal) {
-    m->spmv_npal = 0;
-    PalScan* ps = nullptr;
-    BMSP_TRY(dev_alloc((void**)&ps, sizeof(PalScan), st));
-    BMSP_CUDA(cudaMemsetAsync(ps, 0, sizeof(PalScan), st));
+// entry per bitmap (layout at PalScan) into `palette`.  Leaves pal empty when the matrix has more than PALETTE_MAX distinct bitmaps.
+static int build_palette(const bmsp_matrix_s* m, int vsize, cudaStream_t st, std::vector<uint4>& pal, DevBuf<uint4>& palette) {
+    DevBuf<PalScan> ps;
+    BMSP_TRY(ps.alloc(1, st));
+    BMSP_CUDA(cudaMemsetAsync(ps.get(), 0, sizeof(PalScan), st));
     const int grid = (int)std::min<int64_t>(1024, std::max<int64_t>(1, ceil_div(m->nblk, 256 * 16)));
-    palette_scan_kernel<<<grid, 256, 0, st>>>(m->bmps, m->nblk, ps);
+    palette_scan_kernel<<<grid, 256, 0, st>>>(m->bmps, m->nblk, ps.get());
     BMSP_KERNEL_CHECK();
     std::vector<PalScan> h(1);
-    BMSP_CUDA(cudaMemcpyAsync(h.data(), ps, sizeof(PalScan), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(h.data(), ps.get(), sizeof(PalScan), cudaMemcpyDeviceToHost, st));
     BMSP_CUDA(cudaStreamSynchronize(st));
-    dev_free(ps, st);
+    ps.reset();
     if (h[0].overflow) return BMSP_OK;
     std::vector<uint64_t> keys;
     for (int i = 0; i < PAL_GSLOTS; i++) if (h[0].key[i]) keys.push_back(h[0].key[i]);
@@ -1319,59 +1318,61 @@ static int build_palette(bmsp_matrix_s* m, int vsize, cudaStream_t st, std::vect
         }
         pal.push_back(make_uint4(hw[0], meta[0], hw[1], meta[1]));
     }
-    BMSP_TRY(dev_alloc((void**)&m->tile_palette, sizeof(uint4) * pal.size(), st));
-    BMSP_CUDA(cudaMemcpyAsync(m->tile_palette, pal.data(), sizeof(uint4) * pal.size(), cudaMemcpyHostToDevice, st));
-    m->spmv_npal = (int32_t)pal.size();
+    BMSP_TRY(palette.alloc(pal.size(), st));
+    BMSP_CUDA(cudaMemcpyAsync(palette.get(), pal.data(), sizeof(uint4) * pal.size(), cudaMemcpyHostToDevice, st));
     return BMSP_OK;
 }
 
 // path 0 plan: tile descriptors, x lines and per-block x offsets; shared-memory capacities from the tile maxima
-// when they fit the per-CTA budget, else from the averages (larger tiles are then read from global memory).
+// when they fit the per-CTA budget, else from the averages (larger tiles are then read from global memory).  Built in locals and
+// published in m, then spmv_path = 0, once all of it exists.
 static int plan_tiles(bmsp_matrix_s* m, cudaStream_t st) {
     const int vsize = m->dtype == BMSP_F16 ? 2 : 4;
     // tile height: 64 block rows unless an average tile (bitmaps, x offsets, values, ~x lines) would not fit ~20 KB
     int rt = 64;
     const double row_bytes = ((double)m->nblk * (8 + 2 + 16) + (double)m->nnz * vsize) / m->nbr + 8;
     while (rt > 16 && row_bytes * rt > 20.0 * 1024) rt >>= 1;
-    m->tile_rows = rt;
     // Light rows (64-block-row tiles: stencils, bands) stream through the persistent kernel, which runs STREAM_RT-row tiles only.
     // Heavy rows (dense blocks: 16- or 32-row tiles of 17 KB) are bound by the bit walk, not by memory: a stage then feeds only one
     // or two consumer warps and the one-CTA-per-tile kernel, which keeps 13 such tiles computing per SM, is faster (BC4M: 280 us vs
     // 479 us).  BMSP_SPMV_KERNEL=1 is a test hook: it puts the per-tile kernel behind a light matrix, the bit-exact reference of the
     // streaming kernel.
-    m->spmv_kernel = (rt == STREAM_RT && env_int("BMSP_SPMV_KERNEL", 0) != 1) ? 0 : 1;
-    m->xl_pitch = m->spmv_kernel == 1 ? XL_STRIDE : 32;
+    const int kernel = (rt == STREAM_RT && env_int("BMSP_SPMV_KERNEL", 0) != 1) ? 0 : 1;
+    const int xl_pitch = kernel == 1 ? XL_STRIDE : 32;
     const int ntiles = (int)ceil_div(m->nbr, rt);
     std::vector<uint4> pal;                    // kept until the synchronisation below (pageable source of the palette upload)
-    if (m->spmv_kernel == 0) BMSP_TRY(build_palette(m, vsize, st, pal));
-    const bool use_pal = m->spmv_npal > 0;
-    unsigned long long* stats = nullptr;
-    BMSP_TRY(dev_alloc((void**)&m->tile_desc, sizeof(TileDesc) * (size_t)ntiles, st));
-    BMSP_TRY(dev_alloc_t(&m->tile_lines, (size_t)m->nblk + 8, st));
+    DevBuf<uint4> palette;
+    if (kernel == 0) BMSP_TRY(build_palette(m, vsize, st, pal, palette));
+    const int npal = (int)pal.size();
+    const bool use_pal = npal > 0;
+    DevBuf<TileDesc> desc; DevBuf<uint32_t> lines, word, rowrel; DevBuf<uint16_t> xoff; DevBuf<int2> rowpair;
+    DevBuf<unsigned long long> stats; DevBuf<int32_t> sched;
+    BMSP_TRY(desc.alloc((size_t)ntiles, st));
+    BMSP_TRY(lines.alloc((size_t)m->nblk + 8, st));
     if (use_pal) {
-        BMSP_TRY(dev_alloc_t(&m->tile_word, (size_t)m->nblk + 8, st));
-        BMSP_TRY(dev_alloc_t(&m->tile_rowrel, (size_t)m->nbr + 8, st));
+        BMSP_TRY(word.alloc((size_t)m->nblk + 8, st));
+        BMSP_TRY(rowrel.alloc((size_t)m->nbr + 8, st));
     } else {
-        BMSP_TRY(dev_alloc_t(&m->tile_xoff, (size_t)m->nblk + 16, st));
-        BMSP_TRY(dev_alloc((void**)&m->tile_rowpair, sizeof(int2) * ((size_t)m->nbr + 1 + 8), st));
-        zip_rows_kernel<<<(unsigned)ceil_div(m->nbr + 1, 256), 256, 0, st>>>(m->brp, m->rvb, m->nbr + 1, (int2*)m->tile_rowpair);
+        BMSP_TRY(xoff.alloc((size_t)m->nblk + 16, st));
+        BMSP_TRY(rowpair.alloc((size_t)m->nbr + 1 + 8, st));
+        zip_rows_kernel<<<(unsigned)ceil_div(m->nbr + 1, 256), 256, 0, st>>>(m->brp, m->rvb, m->nbr + 1, rowpair.get());
         BMSP_KERNEL_CHECK();
     }
-    BMSP_TRY(dev_alloc_t(&stats, 8, st));
-    BMSP_CUDA(cudaMemsetAsync(stats, 0, 8 * sizeof(unsigned long long), st));
-    if (m->spmv_kernel == 0 && !m->spmv_sched) {
+    BMSP_TRY(stats.alloc(8, st));
+    BMSP_CUDA(cudaMemsetAsync(stats.get(), 0, 8 * sizeof(unsigned long long), st));
+    if (kernel == 0 && !m->spmv_sched) {
         // tile-claim counters of the streaming kernel (zero before the plan's synchronisation below, so that no later launch -- on
         // whatever stream, captured in a graph or not -- has to wait for them)
-        BMSP_TRY(dev_alloc_t(&m->spmv_sched, (size_t)SCHED_SLOTS * 2, st));
-        BMSP_CUDA(cudaMemsetAsync(m->spmv_sched, 0, sizeof(int32_t) * SCHED_SLOTS * 2, st));
+        BMSP_TRY(sched.alloc((size_t)SCHED_SLOTS * 2, st));
+        BMSP_CUDA(cudaMemsetAsync(sched.get(), 0, sizeof(int32_t) * SCHED_SLOTS * 2, st));
     }
-    tile_plan_kernel<<<ntiles, 256, 0, st>>>(m->brp, m->bcol, m->rvb, m->nbr, m->cols, rt, m->xl_pitch, (TileDesc*)m->tile_desc, m->tile_lines, m->tile_xoff,
-                                             stats, m->bmps, (const uint4*)m->tile_palette, m->spmv_npal, m->tile_word, m->tile_rowrel);
+    tile_plan_kernel<<<ntiles, 256, 0, st>>>(m->brp, m->bcol, m->rvb, m->nbr, m->cols, rt, xl_pitch, desc.get(), lines.get(), xoff.get(),
+                                             stats.get(), m->bmps, palette.get(), npal, word.get(), rowrel.get());
     BMSP_KERNEL_CHECK();
     unsigned long long h[8];
-    BMSP_CUDA(cudaMemcpyAsync(h, stats, sizeof(h), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(h, stats.get(), sizeof(h), cudaMemcpyDeviceToHost, st));
     BMSP_CUDA(cudaStreamSynchronize(st));
-    dev_free(stats, st);
+    stats.reset();
     // capacities: the tile maxima when they fit the per-CTA budget, else 1.25 x the averages (larger tiles are then
     // read from global memory by the kernel)
     auto up8 = [](long long v) { return (int)((v + 7) & ~7ll); };
@@ -1385,45 +1386,53 @@ static int plan_tiles(bmsp_matrix_s* m, cudaStream_t st) {
             cb = std::max(64, up8(cb * 3 / 4)); cv = std::max(256, up8(cv * 3 / 4)); cl = std::max(16, cl * 3 / 4);
         }
     }
-    m->cap_blk = std::max(cb, 8); m->cap_val = std::max(cv, 8); m->cap_lines = std::max(cl, 1);
+    cb = std::max(cb, 8); cv = std::max(cv, 8);
     // the palette variant's relative row pairs are 16-bit: a staged tile has fewer than 65536 blocks and values (the 40 KB budget
     // above keeps both far below that already)
-    if (use_pal) { m->cap_blk = std::min(m->cap_blk, 65528); m->cap_val = std::min(m->cap_val, 65528); }
+    if (use_pal) { cb = std::min(cb, 65528); cv = std::min(cv, 65528); }
+    m->cap_blk = cb; m->cap_val = cv; m->cap_lines = std::max(cl, 1);
+    m->tile_rows = rt; m->spmv_kernel = kernel; m->xl_pitch = xl_pitch; m->spmv_npal = npal;
+    m->tile_palette = palette.release(); m->tile_desc = desc.release(); m->tile_lines = lines.release(); m->tile_word = word.release();
+    m->tile_rowrel = rowrel.release(); m->tile_xoff = xoff.release(); m->tile_rowpair = rowpair.release();
+    if (sched.get()) m->spmv_sched = sched.release();
+    m->spmv_path = 0;
     return BMSP_OK;
 }
 
+// The plan of the first product on m; path 1 is built in locals like path 0 and published, then spmv_path = 1.
 int plan_spmv(bmsp_matrix_s* m, cudaStream_t st) {
     if (m->transposed || m->nbr == 0) { m->spmv_path = -1; return BMSP_OK; }
     const double per_blk = m->nblk ? (double)m->nnz / (double)m->nblk : 0.0;
-    m->spmv_path = per_blk >= 2.5 ? 0 : 1;
-    if (m->spmv_path == 0) return plan_tiles(m, st);
-    uint32_t* cnt = nullptr;
-    BMSP_TRY(dev_alloc_t(&cnt, (size_t)m->nbr + 1, st));
-    work_count_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, cnt);
+    if (per_blk >= 2.5) return plan_tiles(m, st);
+    DevBuf<uint32_t> cnt;                    // item offsets per block row, kept for the fix-up
+    BMSP_TRY(cnt.alloc((size_t)m->nbr + 1, st));
+    work_count_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, cnt.get());
     BMSP_KERNEL_CHECK();
-    BMSP_TRY(exclusive_scan_u32(cnt, cnt, m->nbr, st));
+    BMSP_TRY(exclusive_scan_u32(cnt.get(), cnt.get(), m->nbr, st));
     uint32_t total = 0;
-    BMSP_CUDA(cudaMemcpyAsync(&total, cnt + m->nbr, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(&total, cnt.get() + m->nbr, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     BMSP_CUDA(cudaStreamSynchronize(st));
-    m->n_work = (int32_t)total;
-    BMSP_TRY(dev_alloc((void**)&m->work, sizeof(int4) * (size_t)total, st));
-    work_fill_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, cnt, (int4*)m->work);
+    DevBuf<int4> work;
+    BMSP_TRY(work.alloc((size_t)total, st));
+    work_fill_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, cnt.get(), work.get());
     BMSP_KERNEL_CHECK();
-    m->split_rows = (int32_t*)cnt;           // item offsets per block row, kept for the fix-up
     // sliced block rows (more than one item): listed on the device.  (Items minus block rows no longer says whether there are any:
     // a bundle is one item for four block rows.)  A sliced row has at least two items, so there are at most total / 2 of them.
-    {
-        const size_t cap = (size_t)total / 2 + 1;
-        BMSP_TRY(dev_alloc_t(&m->split_list, cap + 1, st));
-        int32_t* cntr = m->split_list + cap;
-        BMSP_CUDA(cudaMemsetAsync(cntr, 0, sizeof(int32_t), st));
-        split_list_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->split_rows, m->nbr, m->split_list, cntr);
-        BMSP_KERNEL_CHECK();
-        BMSP_CUDA(cudaMemcpyAsync(&m->n_split_rows, cntr, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        BMSP_CUDA(cudaStreamSynchronize(st));
-        m->n_split = m->n_split_rows;         // > 0 iff some block row is sliced
-        if (m->n_split > 0) BMSP_TRY(dev_alloc_t(&m->split_partial, (size_t)total * 8, st));
-    }
+    const size_t cap = (size_t)total / 2 + 1;
+    DevBuf<int32_t> list; DevBuf<float> partial;
+    BMSP_TRY(list.alloc(cap + 1, st));
+    int32_t* cntr = list.get() + cap;
+    BMSP_CUDA(cudaMemsetAsync(cntr, 0, sizeof(int32_t), st));
+    split_list_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>((const int32_t*)cnt.get(), m->nbr, list.get(), cntr);
+    BMSP_KERNEL_CHECK();
+    int32_t n_split_rows = 0;
+    BMSP_CUDA(cudaMemcpyAsync(&n_split_rows, cntr, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));
+    if (n_split_rows > 0) BMSP_TRY(partial.alloc((size_t)total * 8, st));
+    m->n_work = (int32_t)total; m->work = (int32_t*)work.release();
+    m->split_rows = (int32_t*)cnt.release(); m->split_list = list.release(); m->split_partial = partial.release();
+    m->n_split_rows = m->n_split = n_split_rows;       // > 0 iff some block row is sliced
+    m->spmv_path = 1;
     return BMSP_OK;
 }
 
@@ -1542,8 +1551,8 @@ struct HostPipe {
     cudaStream_t s_in = nullptr, s_out = nullptr;
     cudaEvent_t ev_start = nullptr, ev_done = nullptr;
     std::vector<cudaEvent_t> ev_x, ev_k;
-    void* x_dev = nullptr;
-    float* y_dev = nullptr;
+    DevBuf<char> x_dev;
+    DevBuf<float> y_dev;
     // the whole pipeline of one (x_host, y_host) pair captured as a CUDA graph: one launch instead of ~7 API calls per chunk
     cudaStream_t s_cap = nullptr;
     cudaGraphExec_t gexec = nullptr;
@@ -1552,18 +1561,28 @@ struct HostPipe {
     int nchunks = 0;
     std::vector<int> tile_lo;        // [nchunks+1] first tile of every chunk (path 0); {0, 0} for path 1
     std::vector<int64_t> x_need;     // [nchunks]  columns that must be resident before the chunk runs
+    ~HostPipe() {                    // the body runs before x_dev / y_dev are freed
+        if (s_in) { cudaStreamSynchronize(s_in); cudaStreamDestroy(s_in); }
+        if (s_out) { cudaStreamSynchronize(s_out); cudaStreamDestroy(s_out); }
+        if (s_cap) { cudaStreamSynchronize(s_cap); cudaStreamDestroy(s_cap); }
+        if (gexec) cudaGraphExecDestroy(gexec);
+        if (ev_start) cudaEventDestroy(ev_start);
+        if (ev_done) cudaEventDestroy(ev_done);
+        for (auto e : ev_x) if (e) cudaEventDestroy(e);
+        for (auto e : ev_k) if (e) cudaEventDestroy(e);
+    }
 };
 
+// A's pipeline, built on the first call and published in A only when complete
 static int host_pipe_get(bmsp_matrix_s* A, cudaStream_t st, HostPipe** out) {
     if (A->host_pipe) { *out = (HostPipe*)A->host_pipe; return BMSP_OK; }
-    HostPipe* hp = new HostPipe();
-    A->host_pipe = hp;        // released by spmv_host_release (bmsp_destroy) whatever happens below
+    std::unique_ptr<HostPipe> hp(new HostPipe());
     BMSP_CUDA(cudaStreamCreateWithFlags(&hp->s_in, cudaStreamNonBlocking));
     BMSP_CUDA(cudaStreamCreateWithFlags(&hp->s_out, cudaStreamNonBlocking));
     BMSP_CUDA(cudaEventCreateWithFlags(&hp->ev_start, cudaEventDisableTiming));
     BMSP_CUDA(cudaEventCreateWithFlags(&hp->ev_done, cudaEventDisableTiming));
-    BMSP_TRY(dev_alloc(&hp->x_dev, (size_t)A->cols * 4 + 256, st));
-    BMSP_TRY(dev_alloc_t(&hp->y_dev, (size_t)A->rows + 64, st));
+    BMSP_TRY(hp->x_dev.alloc((size_t)A->cols * 4 + 256, st));
+    BMSP_TRY(hp->y_dev.alloc((size_t)A->rows + 64, st));
     BMSP_CUDA(cudaStreamCreateWithFlags(&hp->s_cap, cudaStreamNonBlocking));
     int want = 8;      // P4096 on PCIe 5 x16: 8 chunks 1.67 ms, 16: 1.68, 32: 1.84 (per-chunk dependencies cost more than the shorter fill saves)
     if (const char* e = getenv("BMSP_HOST_CHUNKS")) want = std::max(1, atoi(e));
@@ -1592,23 +1611,12 @@ static int host_pipe_get(bmsp_matrix_s* A, cudaStream_t st, HostPipe** out) {
     hp->ev_x.resize(hp->nchunks); hp->ev_k.resize(hp->nchunks);
     for (auto& e : hp->ev_x) BMSP_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     for (auto& e : hp->ev_k) BMSP_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    *out = hp;
+    A->host_pipe = *out = hp.release();
     return BMSP_OK;
 }
 
 void spmv_host_release(bmsp_matrix_s* m) {
-    HostPipe* hp = (HostPipe*)m->host_pipe;
-    if (!hp) return;
-    if (hp->s_in) { cudaStreamSynchronize(hp->s_in); cudaStreamDestroy(hp->s_in); }
-    if (hp->s_out) { cudaStreamSynchronize(hp->s_out); cudaStreamDestroy(hp->s_out); }
-    if (hp->s_cap) { cudaStreamSynchronize(hp->s_cap); cudaStreamDestroy(hp->s_cap); }
-    if (hp->gexec) cudaGraphExecDestroy(hp->gexec);
-    if (hp->ev_start) cudaEventDestroy(hp->ev_start);
-    if (hp->ev_done) cudaEventDestroy(hp->ev_done);
-    for (auto e : hp->ev_x) if (e) cudaEventDestroy(e);
-    for (auto e : hp->ev_k) if (e) cudaEventDestroy(e);
-    dev_free(hp->x_dev, m->last_stream); dev_free(hp->y_dev, m->last_stream);     // the product kernels ran on the caller's stream
-    delete hp;
+    delete (HostPipe*)m->host_pipe;
     m->host_pipe = nullptr;
 }
 
@@ -1629,7 +1637,7 @@ template <typename T>
 static int spmv_host_run(bmsp_matrix_s* A, HostPipe* hp, const void* x_host, int32_t x_dtype, float* y_host, cudaStream_t st) {
     const size_t xs = x_dtype == BMSP_F16 ? 2 : 4;
     float* y_map = A->spmv_path == 0 ? mapped_host_ptr(y_host) : nullptr;     // row-tiled kernel only: it stores 512 contiguous bytes per warp
-    float* y_out = y_map ? y_map : hp->y_dev;
+    float* y_out = y_map ? y_map : hp->y_dev.get();
     BMSP_CUDA(cudaEventRecord(hp->ev_start, st));         // earlier work on st (and the previous call) is done with x_dev / y_dev
     BMSP_CUDA(cudaStreamWaitEvent(hp->s_in, hp->ev_start, 0));
     BMSP_CUDA(cudaStreamWaitEvent(hp->s_out, hp->ev_start, 0));
@@ -1639,7 +1647,7 @@ static int spmv_host_run(bmsp_matrix_s* A, HostPipe* hp, const void* x_host, int
     for (int c = 0; c < hp->nchunks; c++) {
         const int64_t need = hp->x_need[c];
         if (need > sent) {
-            BMSP_CUDA(cudaMemcpyAsync((char*)hp->x_dev + sent * xs, (const char*)x_host + sent * xs, (size_t)(need - sent) * xs,
+            BMSP_CUDA(cudaMemcpyAsync(hp->x_dev.get() + sent * xs, (const char*)x_host + sent * xs, (size_t)(need - sent) * xs,
                                       cudaMemcpyHostToDevice, hp->s_in));
             BMSP_CUDA(cudaEventRecord(hp->ev_x[c], hp->s_in));
             BMSP_CUDA(cudaStreamWaitEvent(st, hp->ev_x[c], 0));
@@ -1649,16 +1657,16 @@ static int spmv_host_run(bmsp_matrix_s* A, HostPipe* hp, const void* x_host, int
         if (A->spmv_path == 0) {
             const int t0 = hp->tile_lo[c], t1 = hp->tile_lo[c + 1];
             row0 = std::min<int64_t>(A->rows, t0 * rows_per_tile); row1 = std::min<int64_t>(A->rows, t1 * rows_per_tile);
-            if (x_dtype == BMSP_F32) BMSP_TRY((launch_spmv<T, float>(A, (const float*)hp->x_dev, y_out, st, t0, t1 - t0)));
-            else BMSP_TRY((launch_spmv<T, __half>(A, (const __half*)hp->x_dev, y_out, st, t0, t1 - t0)));
+            if (x_dtype == BMSP_F32) BMSP_TRY((launch_spmv<T, float>(A, (const float*)hp->x_dev.get(), y_out, st, t0, t1 - t0)));
+            else BMSP_TRY((launch_spmv<T, __half>(A, (const __half*)hp->x_dev.get(), y_out, st, t0, t1 - t0)));
         } else {
-            if (x_dtype == BMSP_F32) BMSP_TRY((launch_spmv<T, float>(A, (const float*)hp->x_dev, y_out, st)));
-            else BMSP_TRY((launch_spmv<T, __half>(A, (const __half*)hp->x_dev, y_out, st)));
+            if (x_dtype == BMSP_F32) BMSP_TRY((launch_spmv<T, float>(A, (const float*)hp->x_dev.get(), y_out, st)));
+            else BMSP_TRY((launch_spmv<T, __half>(A, (const __half*)hp->x_dev.get(), y_out, st)));
         }
         if (row1 > row0 && !y_map) {
             BMSP_CUDA(cudaEventRecord(hp->ev_k[c], st));
             BMSP_CUDA(cudaStreamWaitEvent(hp->s_out, hp->ev_k[c], 0));
-            BMSP_CUDA(cudaMemcpyAsync(y_host + row0, hp->y_dev + row0, (size_t)(row1 - row0) * 4, cudaMemcpyDeviceToHost, hp->s_out));
+            BMSP_CUDA(cudaMemcpyAsync(y_host + row0, hp->y_dev.get() + row0, (size_t)(row1 - row0) * 4, cudaMemcpyDeviceToHost, hp->s_out));
         }
     }
     BMSP_CUDA(cudaEventRecord(hp->ev_done, hp->s_out));
