@@ -8,6 +8,8 @@
 #include <cstdarg>
 #include <memory>
 #include <utility>
+#include <vector>
+#include <algorithm>
 #include "../../include/bmsparse_b200.h"
 
 #define BMSP_PAD_BYTES 256   // every array is over-allocated so 16-byte bulk copies may overrun the tail
@@ -142,6 +144,54 @@ void spmv_host_release(bmsp_matrix_s* m);
 int refresh_value_copies(bmsp_matrix_s* m, cudaStream_t st);
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
+
+// ---------------------------------------------------------------------------- interchange (data in and out of a matrix)
+static inline size_t dtype_bytes(int32_t dtype) { return dtype == BMSP_F16 ? 2 : 4; }
+
+// f(__half{}) for BMSP_F16, f(float{}) for BMSP_F32: the value type of a dtype code, for a generic lambda that launches the
+// instantiation of that type.  Two nested calls dispatch an (input, output) pair.
+template <typename F>
+inline auto with_value_type(int32_t dtype, F&& f) { return dtype == BMSP_F16 ? f(__half{}) : f(float{}); }
+
+// An array argument of an entry point that takes host or device input (mem): BMSP_DEVICE input is used where it is; any other input
+// is copied into buf on st, and p is pointed at the copy.  buf is freed on st when it goes out of scope.  An entry point that staged
+// host input synchronises st before it returns: its caller may free the host array then.
+template <typename T>
+int stage(DevBuf<char>& buf, const T*& p, size_t bytes, int32_t mem, cudaStream_t st) {
+    if (mem == BMSP_DEVICE) return BMSP_OK;
+    BMSP_TRY(buf.alloc(bytes, st));
+    if (bytes) BMSP_CUDA(cudaMemcpyAsync(buf.get(), p, bytes, cudaMemcpyHostToDevice, st));
+    p = (const T*)buf.get();
+    return BMSP_OK;
+}
+
+// a host CSR's row_ptr starts at 0 and ends at nnz (the device input is checked by the kernels that read it)
+bool host_row_ptr_spans(const int32_t* row_ptr, int32_t rows, int64_t nnz);
+
+// Host COO -> CSR: a counting sort by row, then the columns of every row in ascending order; entries with the same (row, col) stay
+// in input order.  Entries whose row is outside [0, rows) are left out; the return value is how many.
+template <typename V>
+int64_t coo_to_csr_host(int32_t rows, int64_t nnz, const int32_t* row_idx, const int32_t* col_idx, const V* vals,
+                        std::vector<int32_t>& rp, std::vector<int32_t>& ci, std::vector<V>& v) {
+    auto inside = [&](int64_t i) { return row_idx[i] >= 0 && row_idx[i] < rows; };
+    rp.assign((size_t)rows + 1, 0);
+    int64_t outside = 0;
+    for (int64_t i = 0; i < nnz; i++) {
+        if (inside(i)) rp[(size_t)row_idx[i] + 1]++;
+        else outside++;
+    }
+    for (int32_t r = 0; r < rows; r++) rp[r + 1] += rp[r];
+    std::vector<int64_t> perm((size_t)rp[rows]);
+    {
+        std::vector<int32_t> cur(rp.begin(), rp.end() - 1);
+        for (int64_t i = 0; i < nnz; i++) if (inside(i)) perm[(size_t)cur[row_idx[i]]++] = i;
+    }
+    for (int32_t r = 0; r < rows; r++)
+        std::stable_sort(perm.begin() + rp[r], perm.begin() + rp[r + 1], [&](int64_t a, int64_t b) { return col_idx[a] < col_idx[b]; });
+    ci.resize(perm.size()); v.resize(perm.size());
+    for (size_t i = 0; i < perm.size(); i++) { ci[i] = col_idx[perm[i]]; v[i] = vals[perm[i]]; }
+    return outside;
+}
 
 // ---------------------------------------------------------------------------- device helpers
 __device__ __forceinline__ uint32_t kmask_of(uint64_t bmp) {

@@ -205,8 +205,6 @@ __global__ void __launch_bounds__(256) values_kernel(const Tin* __restrict__ val
     }
 }
 
-static size_t dsize(int dtype) { return dtype == BMSP_F16 ? 2 : 4; }
-
 // device CSR -> new matrix
 static int convert_device_csr(int32_t rows, int32_t cols, int64_t nnz, const int32_t* rp, const int32_t* ci, const void* vals,
                               int vals_dtype, int transposed, int out_dtype, cudaStream_t st, bmsp_matrix_t* out) {
@@ -255,13 +253,13 @@ static int convert_device_csr(int32_t rows, int32_t cols, int64_t nnz, const int
         BMSP_CUDA(cudaMemsetAsync(m->bmps, 0, sizeof(uint64_t) * m->nblk, st));
         emit_kernel<<<(unsigned)tiles, 1024, 0, st>>>(s_key.get(), s_p.get(), nnz, counts.get(), m->keys, m->bmps, m->offsets);
         BMSP_KERNEL_CHECK();
-        const int32_t* src = s_src.get();
-        unsigned grid = (unsigned)ceil_div(ceil_div(nnz, 8), 256);
-        if (vals_dtype == BMSP_F32 && out_dtype == BMSP_F16) values_kernel<float, __half><<<grid, 256, 0, st>>>((const float*)vals, src, nnz, (__half*)m->values);
-        else if (vals_dtype == BMSP_F16 && out_dtype == BMSP_F16) values_kernel<__half, __half><<<grid, 256, 0, st>>>((const __half*)vals, src, nnz, (__half*)m->values);
-        else if (vals_dtype == BMSP_F32 && out_dtype == BMSP_F32) values_kernel<float, float><<<grid, 256, 0, st>>>((const float*)vals, src, nnz, (float*)m->values);
-        else values_kernel<__half, float><<<grid, 256, 0, st>>>((const __half*)vals, src, nnz, (float*)m->values);
-        BMSP_KERNEL_CHECK();
+        const unsigned grid = (unsigned)ceil_div(ceil_div(nnz, 8), 256);
+        BMSP_TRY(with_value_type(vals_dtype, [&](auto in) { return with_value_type(out_dtype, [&](auto out) -> int {
+            using Tin = decltype(in); using Tout = decltype(out);
+            values_kernel<Tin, Tout><<<grid, 256, 0, st>>>((const Tin*)vals, s_src.get(), nnz, (Tout*)m->values);
+            BMSP_KERNEL_CHECK();
+            return BMSP_OK;
+        }); }));
     }
     BMSP_TRY(derive_compact(m.get(), st));
     *out = m.release();
@@ -306,42 +304,22 @@ int bmsp_create_from_csr(int32_t rows, int32_t cols, int64_t nnz, const int32_t*
         return BMSP_ERR_INVALID;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    if (mem == BMSP_DEVICE)
-        return convert_device_csr(rows, cols, nnz, row_ptr, col_idx, vals, vals_dtype, transposed, out_dtype, st, out);
-    if (row_ptr[0] != 0 || (int64_t)row_ptr[rows] != nnz) { set_error("row_ptr[0] must be 0 and row_ptr[rows] == nnz"); return BMSP_ERR_INVALID; }
-    DevBuf<int32_t> d_rp, d_ci; DevBuf<char> d_v;
-    BMSP_TRY(d_rp.alloc((size_t)rows + 1, st));
-    BMSP_TRY(d_ci.alloc((size_t)nnz, st));
-    BMSP_TRY(d_v.alloc((size_t)nnz * dsize(vals_dtype), st));
-    BMSP_CUDA(cudaMemcpyAsync(d_rp.get(), row_ptr, sizeof(int32_t) * ((size_t)rows + 1), cudaMemcpyHostToDevice, st));
-    if (nnz) {
-        BMSP_CUDA(cudaMemcpyAsync(d_ci.get(), col_idx, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, st));
-        BMSP_CUDA(cudaMemcpyAsync(d_v.get(), vals, (size_t)nnz * dsize(vals_dtype), cudaMemcpyHostToDevice, st));
-    }
-    BMSP_TRY(convert_device_csr(rows, cols, nnz, d_rp.get(), d_ci.get(), d_v.get(), vals_dtype, transposed, out_dtype, st, out));
-    BMSP_CUDA(cudaStreamSynchronize(st));      // host buffers may be freed by the caller
+    if (mem != BMSP_DEVICE && !host_row_ptr_spans(row_ptr, rows, nnz)) { set_error("row_ptr[0] must be 0 and row_ptr[rows] == nnz"); return BMSP_ERR_INVALID; }
+    DevBuf<char> d_rp, d_ci, d_v;
+    BMSP_TRY(stage(d_rp, row_ptr, sizeof(int32_t) * ((size_t)rows + 1), mem, st));
+    BMSP_TRY(stage(d_ci, col_idx, sizeof(int32_t) * (size_t)nnz, mem, st));
+    BMSP_TRY(stage(d_v, vals, (size_t)nnz * dtype_bytes(vals_dtype), mem, st));
+    BMSP_TRY(convert_device_csr(rows, cols, nnz, row_ptr, col_idx, vals, vals_dtype, transposed, out_dtype, st, out));
+    if (mem != BMSP_DEVICE) BMSP_CUDA(cudaStreamSynchronize(st));      // host buffers may be freed by the caller
     return BMSP_OK;
 }
 
-// host COO -> CSR (counting sort by row, columns sorted inside each row); duplicates summed when `merge`
+// host COO -> matrix; duplicates summed when `merge`
 static int coo_to_matrix(int32_t rows, int32_t cols, int64_t nnz, const int32_t* row_idx, const int32_t* col_idx, const double* vals,
                          int32_t transposed, int32_t out_dtype, int32_t flags, void* stream, bmsp_matrix_t* out) {
-    std::vector<int32_t> rp((size_t)rows + 1, 0);
-    for (int64_t i = 0; i < nnz; i++) {
-        if (row_idx[i] < 0 || row_idx[i] >= rows) { set_error("row index outside [0, %d)", rows); return BMSP_ERR_RANGE; }
-        rp[(size_t)row_idx[i] + 1]++;
-    }
-    for (int32_t r = 0; r < rows; r++) rp[r + 1] += rp[r];
-    std::vector<int64_t> perm((size_t)nnz);
-    {
-        std::vector<int32_t> cur(rp.begin(), rp.end() - 1);
-        for (int64_t i = 0; i < nnz; i++) perm[(size_t)cur[row_idx[i]]++] = i;
-    }
-    for (int32_t r = 0; r < rows; r++)
-        std::stable_sort(perm.begin() + rp[r], perm.begin() + rp[r + 1], [&](int64_t a, int64_t b) { return col_idx[a] < col_idx[b]; });
-    std::vector<int32_t> ci((size_t)nnz);
-    std::vector<double> dv((size_t)nnz);
-    for (int64_t i = 0; i < nnz; i++) { ci[i] = col_idx[perm[i]]; dv[i] = vals[perm[i]]; }
+    std::vector<int32_t> rp, ci;
+    std::vector<double> dv;
+    if (coo_to_csr_host(rows, nnz, row_idx, col_idx, vals, rp, ci, dv)) { set_error("row index outside [0, %d)", rows); return BMSP_ERR_RANGE; }
     int64_t n = nnz;
     if (flags & BMSP_MERGE_DUPLICATES) {
         // repeated (row, col) entries are summed in file order (what assembling a finite-element matrix means by them); the
@@ -503,12 +481,13 @@ int bmsp_block_transpose(bmsp_matrix_t A, int32_t out_dtype, void* stream, bmsp_
     if (m->nblk) {
         BMSP_CUDA(cudaMemcpyAsync(m->keys, A->keys, sizeof(uint64_t) * m->nblk, cudaMemcpyDeviceToDevice, st));
         BMSP_CUDA(cudaMemcpyAsync(m->offsets, A->offsets, sizeof(uint64_t) * m->offsets_len, cudaMemcpyDeviceToDevice, st));
-        unsigned grid = (unsigned)ceil_div(m->nblk, 128);
-        if (A->dtype == BMSP_F16 && out_dtype == BMSP_F16) block_transpose_kernel<__half, __half><<<grid, 128, 0, st>>>(A->bmps, A->offsets, (const __half*)A->values, m->bmps, (__half*)m->values, m->nblk);
-        else if (A->dtype == BMSP_F32 && out_dtype == BMSP_F16) block_transpose_kernel<float, __half><<<grid, 128, 0, st>>>(A->bmps, A->offsets, (const float*)A->values, m->bmps, (__half*)m->values, m->nblk);
-        else if (A->dtype == BMSP_F32 && out_dtype == BMSP_F32) block_transpose_kernel<float, float><<<grid, 128, 0, st>>>(A->bmps, A->offsets, (const float*)A->values, m->bmps, (float*)m->values, m->nblk);
-        else block_transpose_kernel<__half, float><<<grid, 128, 0, st>>>(A->bmps, A->offsets, (const __half*)A->values, m->bmps, (float*)m->values, m->nblk);
-        BMSP_KERNEL_CHECK();
+        const unsigned grid = (unsigned)ceil_div(m->nblk, 128);
+        BMSP_TRY(with_value_type(A->dtype, [&](auto in) { return with_value_type(out_dtype, [&](auto out) -> int {
+            using Tin = decltype(in); using Tout = decltype(out);
+            block_transpose_kernel<Tin, Tout><<<grid, 128, 0, st>>>(A->bmps, A->offsets, (const Tin*)A->values, m->bmps, (Tout*)m->values, m->nblk);
+            BMSP_KERNEL_CHECK();
+            return BMSP_OK;
+        }); }));
     }
     BMSP_TRY(derive_compact(m.get(), st));
     *At = m.release();

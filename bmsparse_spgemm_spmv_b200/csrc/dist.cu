@@ -66,7 +66,7 @@ extern "C" int bmsp_partition_block_rows(bmsp_matrix_t A, bmsp_matrix_t Bt, int3
     if (weight_spgemm) cand_weight_kernel<<<(unsigned)ceil_div(nbr, 8), 256, 0, st>>>(A->brp, A->bcol, Bt->brp, nbr, w.get());
     else {
         const bool blockpar = A->nblk > 0 && (double)A->nnz / (double)A->nblk < 2.5;      // same rule as plan_spmv
-        spmv_weight_kernel<<<(unsigned)ceil_div(nbr, 256), 256, 0, st>>>(A->brp, A->rvb, nbr, A->dtype == BMSP_F16 ? 2 : 4, blockpar ? 330 + 76 * (uint64_t)(nparts - 1) : 40, w.get());
+        spmv_weight_kernel<<<(unsigned)ceil_div(nbr, 256), 256, 0, st>>>(A->brp, A->rvb, nbr, (int)dtype_bytes(A->dtype), blockpar ? 330 + 76 * (uint64_t)(nparts - 1) : 40, w.get());
     }
     BMSP_KERNEL_CHECK();
     BMSP_TRY(exclusive_scan_u64(w.get(), w.get(), nbr, st));
@@ -93,7 +93,7 @@ extern "C" int bmsp_slice_block_rows(bmsp_matrix_t A, int32_t r0, int32_t r1, in
     BMSP_CUDA(cudaMemcpyAsync(&hv[1], A->rvb + r1, 4, cudaMemcpyDeviceToHost, st));
     BMSP_CUDA(cudaStreamSynchronize(st));
     const int64_t nblk = hb[1] - hb[0], nnz = (int64_t)hv[1] - hv[0];
-    const size_t vs = A->dtype == BMSP_F16 ? 2 : 4;
+    const size_t vs = dtype_bytes(A->dtype);
     const int64_t rows = rebase_rows ? std::min<int64_t>((int64_t)(r1 - r0) * 8, (int64_t)A->rows - (int64_t)r0 * 8) : A->rows;
     HandlePtr m;
     BMSP_TRY(new_handle((int32_t)std::max<int64_t>(rows, 0), A->cols, nblk, nnz, A->dtype, A->transposed, st, m));

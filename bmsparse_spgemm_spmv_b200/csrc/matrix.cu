@@ -187,7 +187,7 @@ int derive_compact(bmsp_matrix_s* m, cudaStream_t st) {
     return BMSP_OK;
 }
 
-static size_t dtype_size(int dtype) { return dtype == BMSP_F16 ? 2 : 4; }
+bool host_row_ptr_spans(const int32_t* row_ptr, int32_t rows, int64_t nnz) { return row_ptr[0] == 0 && (int64_t)row_ptr[rows] == nnz; }
 
 int new_handle(int32_t rows, int32_t cols, int64_t nblk, int64_t nnz, int32_t dtype, int32_t transposed, cudaStream_t st, HandlePtr& out) {
     out.reset(new bmsp_matrix_s());
@@ -198,7 +198,7 @@ int new_handle(int32_t rows, int32_t cols, int64_t nblk, int64_t nnz, int32_t dt
     BMSP_TRY(dev_alloc_t(&m->keys, (size_t)nblk + 2, st));
     BMSP_TRY(dev_alloc_t(&m->bmps, (size_t)nblk + 2, st));
     BMSP_TRY(dev_alloc_t(&m->offsets, (size_t)nblk + 2, st));
-    if (nnz >= 0) BMSP_TRY(dev_alloc(&m->values, (size_t)nnz * dtype_size(dtype) + 16, st));
+    if (nnz >= 0) BMSP_TRY(dev_alloc(&m->values, (size_t)nnz * dtype_bytes(dtype) + 16, st));
     return BMSP_OK;
 }
 
@@ -243,7 +243,7 @@ int bmsp_create_from_arrays(int32_t rows, int32_t cols, int64_t block_num, int64
         BMSP_CUDA(cudaMemcpyAsync(m->bmps, bmps, sizeof(uint64_t) * block_num, kind, st));
         BMSP_CUDA(cudaMemcpyAsync(m->offsets, offsets, sizeof(uint64_t) * offsets_len, kind, st));
     }
-    if (nnz > 0) BMSP_CUDA(cudaMemcpyAsync(m->values, values, (size_t)nnz * dtype_size(dtype), kind, st));
+    if (nnz > 0) BMSP_CUDA(cudaMemcpyAsync(m->values, values, (size_t)nnz * dtype_bytes(dtype), kind, st));
     BMSP_TRY(derive_compact(m.get(), st));
     if (mem == BMSP_HOST) BMSP_CUDA(cudaStreamSynchronize(st));   // host buffers may be freed by the caller
     *out = m.release();
@@ -281,7 +281,7 @@ int bmsp_download(bmsp_matrix_t m, uint64_t* keys, uint64_t* bmps, uint64_t* off
     if (keys && m->nblk) BMSP_CUDA(cudaMemcpy(keys, m->keys, sizeof(uint64_t) * m->nblk, cudaMemcpyDeviceToHost));
     if (bmps && m->nblk) BMSP_CUDA(cudaMemcpy(bmps, m->bmps, sizeof(uint64_t) * m->nblk, cudaMemcpyDeviceToHost));
     if (offsets && m->offsets_len) BMSP_CUDA(cudaMemcpy(offsets, m->offsets, sizeof(uint64_t) * m->offsets_len, cudaMemcpyDeviceToHost));
-    if (values && m->nnz) BMSP_CUDA(cudaMemcpy(values, m->values, (size_t)m->nnz * dtype_size(m->dtype), cudaMemcpyDeviceToHost));
+    if (values && m->nnz) BMSP_CUDA(cudaMemcpy(values, m->values, (size_t)m->nnz * dtype_bytes(m->dtype), cudaMemcpyDeviceToHost));
     return BMSP_OK;
 }
 
@@ -319,12 +319,13 @@ extern "C" int bmsp_to_coo(bmsp_matrix_t m, int32_t* rows, int32_t* cols, float*
     BMSP_TRY(dr.alloc((size_t)m->nnz, st));
     BMSP_TRY(dc.alloc((size_t)m->nnz, st));
     BMSP_TRY(dv.alloc((size_t)m->nnz, st));
-    unsigned grid = (unsigned)ceil_div(m->nblk, 128);
-    if (m->dtype == BMSP_F16)
-        to_coo_kernel<__half><<<grid, 128, 0, st>>>(m->keys, m->bmps, m->offsets, (const __half*)m->values, m->transposed, dr.get(), dc.get(), dv.get(), m->nblk);
-    else
-        to_coo_kernel<float><<<grid, 128, 0, st>>>(m->keys, m->bmps, m->offsets, (const float*)m->values, m->transposed, dr.get(), dc.get(), dv.get(), m->nblk);
-    BMSP_KERNEL_CHECK();
+    const unsigned grid = (unsigned)ceil_div(m->nblk, 128);
+    BMSP_TRY(with_value_type(m->dtype, [&](auto t) -> int {
+        using T = decltype(t);
+        to_coo_kernel<T><<<grid, 128, 0, st>>>(m->keys, m->bmps, m->offsets, (const T*)m->values, m->transposed, dr.get(), dc.get(), dv.get(), m->nblk);
+        BMSP_KERNEL_CHECK();
+        return BMSP_OK;
+    }));
     BMSP_CUDA(cudaMemcpyAsync(rows, dr.get(), sizeof(int32_t) * m->nnz, cudaMemcpyDeviceToHost, st));
     BMSP_CUDA(cudaMemcpyAsync(cols, dc.get(), sizeof(int32_t) * m->nnz, cudaMemcpyDeviceToHost, st));
     BMSP_CUDA(cudaMemcpyAsync(vals, dv.get(), sizeof(float) * m->nnz, cudaMemcpyDeviceToHost, st));
@@ -469,12 +470,12 @@ static int to_csr_device(bmsp_matrix_s* m, int32_t* d_rp, int32_t* d_ci, float* 
     BMSP_KERNEL_CHECK();
     BMSP_TRY(exclusive_scan_u32((const uint32_t*)d_rp, (uint32_t*)d_rp, m->rows, st));
     const unsigned grid = (unsigned)ceil_div(m->nbr, 8);
-    if (m->dtype == BMSP_F16)
-        csr_fill_kernel<__half><<<grid, 256, 0, st>>>(m->brp, m->bcol, m->bmps, m->offsets, (const __half*)m->values, m->nbr, m->rows, (const uint32_t*)d_rp, d_ci, d_v);
-    else
-        csr_fill_kernel<float><<<grid, 256, 0, st>>>(m->brp, m->bcol, m->bmps, m->offsets, (const float*)m->values, m->nbr, m->rows, (const uint32_t*)d_rp, d_ci, d_v);
-    BMSP_KERNEL_CHECK();
-    return BMSP_OK;
+    return with_value_type(m->dtype, [&](auto t) -> int {
+        using T = decltype(t);
+        csr_fill_kernel<T><<<grid, 256, 0, st>>>(m->brp, m->bcol, m->bmps, m->offsets, (const T*)m->values, m->nbr, m->rows, (const uint32_t*)d_rp, d_ci, d_v);
+        BMSP_KERNEL_CHECK();
+        return BMSP_OK;
+    });
 }
 
 extern "C" int bmsp_to_csr(bmsp_matrix_t m, int32_t* row_ptr, int32_t* col_idx, float* vals, int32_t mem, void* stream) {
@@ -506,16 +507,17 @@ __global__ void convert_values_kernel(const Tin* __restrict__ in, Tout* __restri
 
 // device values in m's compact order -> m->values, converted to m's dtype
 static int values_from_device(bmsp_matrix_s* m, const void* v, int32_t dtype, cudaStream_t st) {
-    if (m->nnz == 0) return BMSP_OK;
-    if (dtype == m->dtype) {
-        BMSP_CUDA(cudaMemcpyAsync(m->values, v, (size_t)m->nnz * dtype_size(dtype), cudaMemcpyDeviceToDevice, st));
-        return BMSP_OK;
-    }
     const unsigned grid = (unsigned)ceil_div(m->nnz, 256);
-    if (dtype == BMSP_F32) convert_values_kernel<float, __half><<<grid, 256, 0, st>>>((const float*)v, (__half*)m->values, m->nnz);
-    else convert_values_kernel<__half, float><<<grid, 256, 0, st>>>((const __half*)v, (float*)m->values, m->nnz);
-    BMSP_KERNEL_CHECK();
-    return BMSP_OK;
+    return with_value_type(dtype, [&](auto in) { return with_value_type(m->dtype, [&](auto out) -> int {
+        using Tin = decltype(in); using Tout = decltype(out);
+        if constexpr (std::is_same<Tin, Tout>::value) {
+            BMSP_CUDA(cudaMemcpyAsync(m->values, v, (size_t)m->nnz * sizeof(Tin), cudaMemcpyDeviceToDevice, st));
+        } else {
+            convert_values_kernel<Tin, Tout><<<grid, 256, 0, st>>>((const Tin*)v, (Tout*)m->values, m->nnz);
+            BMSP_KERNEL_CHECK();
+        }
+        return BMSP_OK;
+    }); });
 }
 
 template <bool TRANSPOSED, bool CHECK, typename Tin, typename Tout>
@@ -527,10 +529,9 @@ static int launch_scatter(bmsp_matrix_s* m, const int32_t* rp, const int32_t* ci
 }
 template <bool TRANSPOSED>
 static int scatter_values(bmsp_matrix_s* m, const int32_t* rp, const void* vals, int32_t vals_dtype, cudaStream_t st) {
-    if (vals_dtype == BMSP_F32 && m->dtype == BMSP_F16) return launch_scatter<TRANSPOSED, false, float, __half>(m, rp, nullptr, vals, nullptr, st);
-    if (vals_dtype == BMSP_F16 && m->dtype == BMSP_F16) return launch_scatter<TRANSPOSED, false, __half, __half>(m, rp, nullptr, vals, nullptr, st);
-    if (vals_dtype == BMSP_F32) return launch_scatter<TRANSPOSED, false, float, float>(m, rp, nullptr, vals, nullptr, st);
-    return launch_scatter<TRANSPOSED, false, __half, float>(m, rp, nullptr, vals, nullptr, st);
+    return with_value_type(vals_dtype, [&](auto in) { return with_value_type(m->dtype, [&](auto out) {
+        return launch_scatter<TRANSPOSED, false, decltype(in), decltype(out)>(m, rp, nullptr, vals, nullptr, st);
+    }); });
 }
 
 // device CSR with m's pattern -> m->values: the check pass, one read-back of its flag, then the scatter
@@ -552,15 +553,14 @@ extern "C" int bmsp_set_values(bmsp_matrix_t m, const void* values, int32_t dtyp
     if (!m || (values && dtype != BMSP_F16 && dtype != BMSP_F32)) { set_error("bmsp_set_values: invalid argument"); return BMSP_ERR_INVALID; }
     cudaStream_t st = (cudaStream_t)stream;
     touch(m, st);
-    if (values && mem == BMSP_DEVICE) BMSP_TRY(values_from_device(m, values, dtype, st));
-    else if (values && m->nnz > 0) {
-        if (dtype == m->dtype) {
-            BMSP_CUDA(cudaMemcpyAsync(m->values, values, (size_t)m->nnz * dtype_size(dtype), cudaMemcpyHostToDevice, st));
+    if (values && m->nnz > 0) {
+        const size_t bytes = (size_t)m->nnz * dtype_bytes(dtype);
+        DevBuf<char> d;
+        if (mem != BMSP_DEVICE && dtype == m->dtype) {
+            BMSP_CUDA(cudaMemcpyAsync(m->values, values, bytes, cudaMemcpyHostToDevice, st));      // m's type already: no staging
         } else {
-            DevBuf<char> d;
-            BMSP_TRY(d.alloc((size_t)m->nnz * dtype_size(dtype), st));
-            BMSP_CUDA(cudaMemcpyAsync(d.get(), values, (size_t)m->nnz * dtype_size(dtype), cudaMemcpyHostToDevice, st));
-            BMSP_TRY(values_from_device(m, d.get(), dtype, st));
+            BMSP_TRY(stage(d, values, bytes, mem, st));
+            BMSP_TRY(values_from_device(m, values, dtype, st));
         }
     }
     BMSP_TRY(refresh_value_copies(m, st));
@@ -576,27 +576,17 @@ extern "C" int bmsp_set_values_csr(bmsp_matrix_t m, const int32_t* row_ptr, cons
     }
     cudaStream_t st = (cudaStream_t)stream;
     touch(m, st);
-    if (mem == BMSP_DEVICE) {
-        BMSP_TRY(set_values_csr_device(m, row_ptr, col_idx, vals, vals_dtype, st));
-        return refresh_value_copies(m, st);
-    }
-    if (row_ptr[0] != 0 || (int64_t)row_ptr[m->rows] != m->nnz) {
+    if (mem != BMSP_DEVICE && !host_row_ptr_spans(row_ptr, m->rows, m->nnz)) {
         set_error("bmsp_set_values_csr: row_ptr spans %lld entries, the matrix has %lld values", (long long)row_ptr[m->rows] - row_ptr[0], (long long)m->nnz);
         return BMSP_ERR_INVALID;
     }
-    const size_t vs = vals_dtype == BMSP_F16 ? 2 : 4;
-    DevBuf<int32_t> d_rp, d_ci; DevBuf<char> d_v;
-    BMSP_TRY(d_rp.alloc((size_t)m->rows + 1, st));
-    BMSP_TRY(d_ci.alloc((size_t)m->nnz, st));
-    BMSP_TRY(d_v.alloc((size_t)m->nnz * vs, st));
-    BMSP_CUDA(cudaMemcpyAsync(d_rp.get(), row_ptr, sizeof(int32_t) * ((size_t)m->rows + 1), cudaMemcpyHostToDevice, st));
-    if (m->nnz) {
-        BMSP_CUDA(cudaMemcpyAsync(d_ci.get(), col_idx, sizeof(int32_t) * (size_t)m->nnz, cudaMemcpyHostToDevice, st));
-        BMSP_CUDA(cudaMemcpyAsync(d_v.get(), vals, (size_t)m->nnz * vs, cudaMemcpyHostToDevice, st));
-    }
-    BMSP_TRY(set_values_csr_device(m, d_rp.get(), d_ci.get(), d_v.get(), vals_dtype, st));
+    DevBuf<char> d_rp, d_ci, d_v;
+    BMSP_TRY(stage(d_rp, row_ptr, sizeof(int32_t) * ((size_t)m->rows + 1), mem, st));
+    BMSP_TRY(stage(d_ci, col_idx, sizeof(int32_t) * (size_t)m->nnz, mem, st));
+    BMSP_TRY(stage(d_v, vals, (size_t)m->nnz * dtype_bytes(vals_dtype), mem, st));
+    BMSP_TRY(set_values_csr_device(m, row_ptr, col_idx, vals, vals_dtype, st));
     BMSP_TRY(refresh_value_copies(m, st));
-    BMSP_CUDA(cudaStreamSynchronize(st));
+    if (mem != BMSP_DEVICE) BMSP_CUDA(cudaStreamSynchronize(st));      // host buffers may be freed by the caller
     return BMSP_OK;
 }
 
@@ -654,28 +644,19 @@ extern "C" int bmsp_compare_csr(bmsp_matrix_t m, const int32_t* row_ptr, const i
     if (!m || !row_ptr) { set_error("bmsp_compare_csr: null argument"); return BMSP_ERR_INVALID; }
     cudaStream_t st = (cudaStream_t)stream;
     touch(m, st);
-    DevBuf<int32_t> a_rp, a_ci, b_rp_d, b_ci_d; DevBuf<float> a_v, b_v_d; DevBuf<unsigned long long> acc;
+    DevBuf<int32_t> a_rp, a_ci; DevBuf<float> a_v; DevBuf<unsigned long long> acc; DevBuf<char> b_rp, b_ci, b_v;
     BMSP_TRY(a_rp.alloc((size_t)m->rows + 2, st));
     BMSP_TRY(a_ci.alloc((size_t)m->nnz + 1, st));
     BMSP_TRY(a_v.alloc((size_t)m->nnz + 1, st));
     BMSP_TRY(acc.alloc(8, st));
     BMSP_CUDA(cudaMemsetAsync(acc.get(), 0, 8 * sizeof(unsigned long long), st));
     BMSP_TRY(to_csr_device(m, a_rp.get(), a_ci.get(), a_v.get(), st));
-    const int32_t *b_rp = row_ptr, *b_ci = col_idx; const float* b_v = vals;
-    if (mem != BMSP_DEVICE) {
-        const int64_t n = row_ptr[m->rows];
-        BMSP_TRY(b_rp_d.alloc((size_t)m->rows + 2, st));
-        BMSP_TRY(b_ci_d.alloc((size_t)n + 1, st));
-        BMSP_TRY(b_v_d.alloc((size_t)n + 1, st));
-        BMSP_CUDA(cudaMemcpyAsync(b_rp_d.get(), row_ptr, sizeof(int32_t) * ((size_t)m->rows + 1), cudaMemcpyHostToDevice, st));
-        if (n) {
-            BMSP_CUDA(cudaMemcpyAsync(b_ci_d.get(), col_idx, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
-            BMSP_CUDA(cudaMemcpyAsync(b_v_d.get(), vals, sizeof(float) * (size_t)n, cudaMemcpyHostToDevice, st));
-        }
-        b_rp = b_rp_d.get(); b_ci = b_ci_d.get(); b_v = b_v_d.get();
-    }
+    const int64_t n = mem == BMSP_DEVICE ? 0 : row_ptr[m->rows];     // the host CSR's entry count
+    BMSP_TRY(stage(b_rp, row_ptr, sizeof(int32_t) * ((size_t)m->rows + 1), mem, st));
+    BMSP_TRY(stage(b_ci, col_idx, sizeof(int32_t) * (size_t)n, mem, st));
+    BMSP_TRY(stage(b_v, vals, sizeof(float) * (size_t)n, mem, st));
     if (m->rows > 0) {
-        compare_rows_kernel<<<(unsigned)ceil_div(m->rows, 256), 256, 0, st>>>(m->rows, a_rp.get(), a_ci.get(), a_v.get(), b_rp, b_ci, b_v, acc.get(),
+        compare_rows_kernel<<<(unsigned)ceil_div(m->rows, 256), 256, 0, st>>>(m->rows, a_rp.get(), a_ci.get(), a_v.get(), row_ptr, col_idx, vals, acc.get(),
                                                                               reinterpret_cast<double*>(acc.get() + 4));
         BMSP_KERNEL_CHECK();
     }
@@ -694,25 +675,12 @@ extern "C" int bmsp_compare_csr(bmsp_matrix_t m, const int32_t* row_ptr, const i
 extern "C" int bmsp_compare(bmsp_matrix_t m, int64_t nnz, const int32_t* rows, const int32_t* cols, const float* vals,
                             int64_t* only_in_m, int64_t* only_in_coo, double* mean_rel_err, double* max_rel_err) {
     if (!m || (nnz > 0 && (!rows || !cols || !vals))) { set_error("bmsp_compare: null argument"); return BMSP_ERR_INVALID; }
-    // the COO (any order) becomes CSR on the host -- counting sort by row, columns sorted inside each row -- and the comparison
-    // itself runs on the device (bmsp_compare_csr); entries outside the matrix count as "only in the COO"
-    std::vector<int32_t> rp((size_t)m->rows + 1, 0);
-    int64_t outside = 0;
-    for (int64_t i = 0; i < nnz; i++) {
-        if (rows[i] < 0 || rows[i] >= m->rows) { outside++; continue; }
-        rp[(size_t)rows[i] + 1]++;
-    }
-    for (int32_t r = 0; r < m->rows; r++) rp[r + 1] += rp[r];
-    const int64_t n_in = rp[m->rows];
-    std::vector<int64_t> perm((size_t)n_in);
-    {
-        std::vector<int32_t> cur(rp.begin(), rp.end() - 1);
-        for (int64_t i = 0; i < nnz; i++) if (rows[i] >= 0 && rows[i] < m->rows) perm[(size_t)cur[rows[i]]++] = i;
-    }
-    for (int32_t r = 0; r < m->rows; r++)
-        std::sort(perm.begin() + rp[r], perm.begin() + rp[r + 1], [&](int64_t a, int64_t b) { return cols[a] < cols[b]; });
-    std::vector<int32_t> ci((size_t)n_in); std::vector<float> v((size_t)n_in);
-    for (int64_t i = 0; i < n_in; i++) { ci[i] = cols[perm[i]]; v[i] = vals[perm[i]]; }
+    // the COO (any order) becomes CSR on the host and the comparison itself runs on the device (bmsp_compare_csr).  Entries whose row
+    // is outside the matrix count as "only in the COO".  Of entries with the same (row, col), the first in input order is the one
+    // compared; the others count as "only in the COO" too.
+    std::vector<int32_t> rp, ci;
+    std::vector<float> v;
+    const int64_t outside = coo_to_csr_host(m->rows, nnz, rows, cols, vals, rp, ci, v);
     int64_t ob = 0;
     BMSP_TRY(bmsp_compare_csr(m, rp.data(), ci.data(), v.data(), BMSP_HOST, m->last_stream, only_in_m, &ob, mean_rel_err, max_rel_err));
     if (only_in_coo) *only_in_coo = ob + outside;

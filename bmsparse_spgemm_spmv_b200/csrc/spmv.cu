@@ -1327,7 +1327,7 @@ static int build_palette(const bmsp_matrix_s* m, int vsize, cudaStream_t st, std
 // when they fit the per-CTA budget, else from the averages (larger tiles are then read from global memory).  Built in locals and
 // published in m, then spmv_path = 0, once all of it exists.
 static int plan_tiles(bmsp_matrix_s* m, cudaStream_t st) {
-    const int vsize = m->dtype == BMSP_F16 ? 2 : 4;
+    const int vsize = (int)dtype_bytes(m->dtype);
     // tile height: 64 block rows unless an average tile (bitmaps, x offsets, values, ~x lines) would not fit ~20 KB
     int rt = 64;
     const double row_bytes = ((double)m->nblk * (8 + 2 + 16) + (double)m->nnz * vsize) / m->nbr + 8;
@@ -1635,7 +1635,7 @@ static float* mapped_host_ptr(float* y_host) {
 
 template <typename T>
 static int spmv_host_run(bmsp_matrix_s* A, HostPipe* hp, const void* x_host, int32_t x_dtype, float* y_host, cudaStream_t st) {
-    const size_t xs = x_dtype == BMSP_F16 ? 2 : 4;
+    const size_t xs = dtype_bytes(x_dtype);
     float* y_map = A->spmv_path == 0 ? mapped_host_ptr(y_host) : nullptr;     // row-tiled kernel only: it stores 512 contiguous bytes per warp
     float* y_out = y_map ? y_map : hp->y_dev.get();
     BMSP_CUDA(cudaEventRecord(hp->ev_start, st));         // earlier work on st (and the previous call) is done with x_dev / y_dev
@@ -1654,15 +1654,16 @@ static int spmv_host_run(bmsp_matrix_s* A, HostPipe* hp, const void* x_host, int
             sent = need; last_x = hp->ev_x[c];
         }
         int64_t row0 = 0, row1 = A->rows;
+        int t0 = 0, nt = -1;                               // path 1: the whole matrix
         if (A->spmv_path == 0) {
-            const int t0 = hp->tile_lo[c], t1 = hp->tile_lo[c + 1];
+            const int t1 = hp->tile_lo[c + 1];
+            t0 = hp->tile_lo[c]; nt = t1 - t0;
             row0 = std::min<int64_t>(A->rows, t0 * rows_per_tile); row1 = std::min<int64_t>(A->rows, t1 * rows_per_tile);
-            if (x_dtype == BMSP_F32) BMSP_TRY((launch_spmv<T, float>(A, (const float*)hp->x_dev.get(), y_out, st, t0, t1 - t0)));
-            else BMSP_TRY((launch_spmv<T, __half>(A, (const __half*)hp->x_dev.get(), y_out, st, t0, t1 - t0)));
-        } else {
-            if (x_dtype == BMSP_F32) BMSP_TRY((launch_spmv<T, float>(A, (const float*)hp->x_dev.get(), y_out, st)));
-            else BMSP_TRY((launch_spmv<T, __half>(A, (const __half*)hp->x_dev.get(), y_out, st)));
         }
+        BMSP_TRY(with_value_type(x_dtype, [&](auto x) {
+            using X = decltype(x);
+            return launch_spmv<T, X>(A, (const X*)hp->x_dev.get(), y_out, st, t0, nt);
+        }));
         if (row1 > row0 && !y_map) {
             BMSP_CUDA(cudaEventRecord(hp->ev_k[c], st));
             BMSP_CUDA(cudaStreamWaitEvent(hp->s_out, hp->ev_k[c], 0));
@@ -1719,11 +1720,12 @@ extern "C" int bmsp_spmv_host(bmsp_matrix_t A, const void* x_host, int32_t x_dty
     if (A->spmv_path < 0) BMSP_TRY(plan_spmv(A, st));
     HostPipe* hp = nullptr;
     BMSP_TRY(host_pipe_get(A, st, &hp));
-    bool replayed = false;
-    if (A->dtype == BMSP_F16) BMSP_TRY(spmv_host_graph<__half>(A, hp, x_host, x_dtype, y_host, st, &replayed));
-    else BMSP_TRY(spmv_host_graph<float>(A, hp, x_host, x_dtype, y_host, st, &replayed));
-    if (replayed) return BMSP_OK;
-    return A->dtype == BMSP_F16 ? spmv_host_run<__half>(A, hp, x_host, x_dtype, y_host, st) : spmv_host_run<float>(A, hp, x_host, x_dtype, y_host, st);
+    return with_value_type(A->dtype, [&](auto t) -> int {
+        using T = decltype(t);
+        bool replayed = false;
+        BMSP_TRY(spmv_host_graph<T>(A, hp, x_host, x_dtype, y_host, st, &replayed));
+        return replayed ? BMSP_OK : spmv_host_run<T>(A, hp, x_host, x_dtype, y_host, st);
+    });
 }
 
 namespace bmsp {
@@ -1809,8 +1811,7 @@ extern "C" int bmsp_spmv_halo(bmsp_matrix_t A, const float* x_ext, float* y_own,
         if (n == 0) { h.solo_tile = 0; n = 1; }
         h.n_sig = (uint32_t)n;
         h.rot = (int)(ceil_div(A->nbr, A->tile_rows) / 2);
-        return A->dtype == BMSP_F16 ? launch_spmv<__half, float, HaloDev>(A, x_ext, y_own, st, 0, -1, h)
-                                    : launch_spmv<float, float, HaloDev>(A, x_ext, y_own, st, 0, -1, h);
+        return with_value_type(A->dtype, [&](auto t) { return launch_spmv<decltype(t), float, HaloDev>(A, x_ext, y_own, st, 0, -1, h); });
     }
     // block-parallel path: wait kernel, product, push kernel
     halo_wait_kernel<<<1, 32, 0, st>>>(h);
@@ -1850,15 +1851,16 @@ extern "C" int bmsp_spmv(bmsp_matrix_t A, const void* x, int32_t x_dtype, float*
     cudaStream_t st = (cudaStream_t)stream;
     touch(A, st);
     if (A->spmv_path < 0) BMSP_TRY(plan_spmv(A, st));
-    if (A->dtype == BMSP_F16)
-        return x_dtype == BMSP_F32 ? launch_spmv<__half, float>(A, (const float*)x, y, st) : launch_spmv<__half, __half>(A, (const __half*)x, y, st);
-    return x_dtype == BMSP_F32 ? launch_spmv<float, float>(A, (const float*)x, y, st) : launch_spmv<float, __half>(A, (const __half*)x, y, st);
+    return with_value_type(A->dtype, [&](auto t) { return with_value_type(x_dtype, [&](auto xt) {
+        using X = decltype(xt);
+        return launch_spmv<decltype(t), X>(A, (const X*)x, y, st);
+    }); });
 }
 
 // SURVEY.md section 8(d): nblk*(4+8) + nbr*(4+4) + nnz*sizeof(value) + ncols*sizeof(x) + nrows*4
 extern "C" int bmsp_spmv_bytes(bmsp_matrix_t A, int32_t x_dtype, int64_t* bytes) {
     if (!A || !bytes) { set_error("bmsp_spmv_bytes: null argument"); return BMSP_ERR_INVALID; }
-    *bytes = A->nblk * 12 + (int64_t)A->nbr * 8 + A->nnz * (A->dtype == BMSP_F16 ? 2 : 4) +
-             (int64_t)A->cols * (x_dtype == BMSP_F16 ? 2 : 4) + (int64_t)A->rows * 4;
+    *bytes = A->nblk * 12 + (int64_t)A->nbr * 8 + A->nnz * (int64_t)dtype_bytes(A->dtype) + (int64_t)A->cols * (int64_t)dtype_bytes(x_dtype) +
+             (int64_t)A->rows * 4;
     return BMSP_OK;
 }

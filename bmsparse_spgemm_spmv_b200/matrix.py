@@ -8,6 +8,7 @@ the handle's device memory (zero copy) and are only valid while the matrix is al
 from __future__ import annotations
 
 import ctypes as C
+from collections import namedtuple
 
 import numpy as np
 import torch
@@ -47,24 +48,13 @@ class bmSpMatrix:
     def from_csr(cls, num_rows, num_cols, row_ptr, col_idx, vals, transpose=False, dtype=torch.float16, stream=None):
         """CSR (torch CUDA tensors, numpy arrays or anything array-like on the host) -> bmSparse."""
         m = cls()
-        if isinstance(row_ptr, torch.Tensor) and row_ptr.is_cuda:
-            rp = row_ptr.to(torch.int32).contiguous(); ci = col_idx.to(torch.int32).contiguous()
-            v = vals.contiguous()
-            if v.dtype not in (torch.float16, torch.float32):
-                v = v.to(torch.float32)
-            L.check(L.lib().bmsp_create_from_csr(int(num_rows), int(num_cols), C.c_int64(ci.numel()), C.c_void_p(rp.data_ptr()),
-                                                 C.c_void_p(ci.data_ptr()), C.c_void_p(v.data_ptr()), _dt(v.dtype), L.DEVICE,
-                                                 int(transpose), _dt(dtype), _stream_ptr(stream), C.byref(m._h)))
+        rp = _array(row_ptr, np.int32)
+        ci = _array(col_idx, np.int32, mem=rp.mem)
+        v = _array(vals, values=True, mem=rp.mem)
+        L.check(L.lib().bmsp_create_from_csr(int(num_rows), int(num_cols), C.c_int64(ci.n), rp.ptr, ci.ptr, v.ptr, v.dt, rp.mem,
+                                             int(transpose), _dt(dtype), _stream_ptr(stream), C.byref(m._h)))
+        if rp.mem == L.DEVICE:
             (stream if stream is not None else torch.cuda.current_stream()).synchronize()      # rp / ci / v temporaries die here
-        else:
-            rp = np.ascontiguousarray(row_ptr, np.int32); ci = np.ascontiguousarray(col_idx, np.int32)
-            v = np.ascontiguousarray(vals)
-            if v.dtype not in (np.float16, np.float32):
-                v = v.astype(np.float32)
-            L.check(L.lib().bmsp_create_from_csr(int(num_rows), int(num_cols), C.c_int64(ci.size), rp.ctypes.data_as(C.c_void_p),
-                                                 ci.ctypes.data_as(C.c_void_p), v.ctypes.data_as(C.c_void_p),
-                                                 L.F16 if v.dtype == np.float16 else L.F32, L.HOST, int(transpose), _dt(dtype),
-                                                 _stream_ptr(stream), C.byref(m._h)))
         return m
 
     @classmethod
@@ -81,22 +71,12 @@ class bmSpMatrix:
     def from_arrays(cls, num_rows, num_cols, block_num, keys, bmps, offsets, values, transpose=False):
         """bmSpMatrix(num_rows, num_cols, block_num, keys, bmps, offsets, values) -- src/bmSpMatrix.cu:30-43."""
         m = cls()
-        if isinstance(keys, torch.Tensor):
-            assert keys.is_cuda
-            ptr = lambda t: C.c_void_p(t.contiguous().data_ptr())
-            keys, bmps, offsets, values = (t.contiguous() for t in (keys, bmps, offsets, values))
-            mem, n_off, n_val, dt = L.DEVICE, offsets.numel(), values.numel(), _dt(values.dtype)
-        else:
-            keys = np.ascontiguousarray(keys, np.uint64); bmps = np.ascontiguousarray(bmps, np.uint64)
-            offsets = np.ascontiguousarray(offsets, np.uint64); values = np.ascontiguousarray(values)
-            ptr = lambda a: a.ctypes.data_as(C.c_void_p)
-            mem, n_off, n_val = L.HOST, offsets.size, values.size
-            dt = L.F16 if values.dtype == np.float16 else L.F32
-            if values.dtype not in (np.float16, np.float32):
-                values = values.astype(np.float32)
-        L.check(L.lib().bmsp_create_from_arrays(int(num_rows), int(num_cols), C.c_int64(block_num), C.c_int64(n_val), ptr(keys),
-                                                ptr(bmps), ptr(offsets), C.c_int64(n_off), ptr(values), dt, mem, int(transpose),
-                                                _stream_ptr(), C.byref(m._h)))
+        assert not isinstance(keys, torch.Tensor) or keys.is_cuda, "from_arrays: tensors must be CUDA tensors"
+        k = _array(keys, np.uint64)
+        b, o = (_array(a, np.uint64, mem=k.mem) for a in (bmps, offsets))
+        v = _array(values, values=k.mem == L.HOST, mem=k.mem)        # device values are adopted as they are: fp16 or fp32 only
+        L.check(L.lib().bmsp_create_from_arrays(int(num_rows), int(num_cols), C.c_int64(block_num), C.c_int64(v.n), k.ptr, b.ptr,
+                                                o.ptr, C.c_int64(o.n), v.ptr, v.dt, k.mem, int(transpose), _stream_ptr(), C.byref(m._h)))
         torch.cuda.current_stream().synchronize()
         return m
 
@@ -146,50 +126,27 @@ class bmSpMatrix:
         if values is None:
             L.check(lib.bmsp_set_values(self._h, None, L.F32, L.DEVICE, _stream_ptr(stream)))
             return
-        if isinstance(values, torch.Tensor) and values.is_cuda:
-            v = values.contiguous()
-            if v.dtype not in (torch.float16, torch.float32):
-                v = v.to(torch.float32)
-            if v.numel() != self.nnz:
-                raise ValueError(f"set_values: {v.numel()} values for a matrix with {self.nnz}")
-            L.check(lib.bmsp_set_values(self._h, C.c_void_p(v.data_ptr()), _dt(v.dtype), L.DEVICE, _stream_ptr(stream)))
-            if v is not values and stream is not None:
-                v.record_stream(stream)        # the temporary outlives this call on `stream`
-            return
-        v = values.numpy() if isinstance(values, torch.Tensor) else np.asarray(values)
-        v = np.ascontiguousarray(v.reshape(-1))
-        if v.dtype not in (np.float16, np.float32):
-            v = v.astype(np.float32)
-        if v.size != self.nnz:
-            raise ValueError(f"set_values: {v.size} values for a matrix with {self.nnz}")
-        L.check(lib.bmsp_set_values(self._h, v.ctypes.data_as(C.c_void_p), L.F16 if v.dtype == np.float16 else L.F32, L.HOST,
-                                    _stream_ptr(stream)))
+        v = _array(values, values=True)
+        if v.n != self.nnz:
+            raise ValueError(f"set_values: {v.n} values for a matrix with {self.nnz}")
+        L.check(lib.bmsp_set_values(self._h, v.ptr, v.dt, v.mem, _stream_ptr(stream)))
+        if v.mem == L.DEVICE and v.keep is not values and stream is not None:
+            v.keep.record_stream(stream)        # the temporary outlives this call on `stream`
 
     def set_values_csr(self, row_ptr, col_idx, vals, stream=None):
         """New values as a CSR with exactly this matrix's pattern (the arrays from_csr took, for either orientation): CUDA tensors
         or host arrays, as from_csr takes them.  A different pattern raises BmspError (INVALID) and leaves the values unchanged."""
         lib = L.lib()
         v = self._view()
-        if isinstance(row_ptr, torch.Tensor) and row_ptr.is_cuda:
-            rp = row_ptr.to(torch.int32).contiguous(); ci = col_idx.to(torch.int32).contiguous(); x = vals.contiguous()
-            if x.dtype not in (torch.float16, torch.float32):
-                x = x.to(torch.float32)
-            n_rp, n_ci, n_v = rp.numel(), ci.numel(), x.numel()
-            ptrs = (C.c_void_p(rp.data_ptr()), C.c_void_p(ci.data_ptr()), C.c_void_p(x.data_ptr()))
-            dt, mem = _dt(x.dtype), L.DEVICE
-        else:
-            rp = np.ascontiguousarray(row_ptr, np.int32); ci = np.ascontiguousarray(col_idx, np.int32); x = np.ascontiguousarray(vals)
-            if x.dtype not in (np.float16, np.float32):
-                x = x.astype(np.float32)
-            n_rp, n_ci, n_v = rp.size, ci.size, x.size
-            ptrs = tuple(a.ctypes.data_as(C.c_void_p) for a in (rp, ci, x))
-            dt, mem = (L.F16 if x.dtype == np.float16 else L.F32), L.HOST
-        if n_rp != v.num_rows + 1 or n_ci != n_v:
+        rp = _array(row_ptr, np.int32)
+        ci = _array(col_idx, np.int32, mem=rp.mem)
+        x = _array(vals, values=True, mem=rp.mem)
+        if rp.n != v.num_rows + 1 or ci.n != x.n:
             raise ValueError("set_values_csr: row_ptr needs num_rows + 1 entries, col_idx and vals one per value")
-        if n_ci != v.nnz:      # the library reads nnz entries of col_idx and vals
-            raise L.BmspError(1, f"set_values_csr: the CSR has {n_ci} entries, the matrix {v.nnz} values")
-        L.check(lib.bmsp_set_values_csr(self._h, *ptrs, dt, mem, _stream_ptr(stream)))
-        if mem == L.DEVICE:
+        if ci.n != v.nnz:      # the library reads nnz entries of col_idx and vals
+            raise L.BmspError(1, f"set_values_csr: the CSR has {ci.n} entries, the matrix {v.nnz} values")
+        L.check(lib.bmsp_set_values_csr(self._h, rp.ptr, ci.ptr, x.ptr, x.dt, rp.mem, _stream_ptr(stream)))
+        if rp.mem == L.DEVICE:
             (stream if stream is not None else torch.cuda.current_stream()).synchronize()      # rp / ci / x temporaries die here
 
     @property
@@ -270,6 +227,30 @@ class bmSpMatrix:
                 self._h = C.c_void_p()
         except Exception:
             pass
+
+
+_Array = namedtuple("_Array", "ptr n dt mem keep")
+
+
+def _array(a, dtype=None, values=False, mem=None) -> _Array:
+    """One array argument of a C call: its pointer, element count, dtype code (_dt; None for index arrays), mem, and the object
+    that must stay alive while the call's work runs.  A CUDA tensor is passed where it is (L.DEVICE); a CPU tensor, a numpy array or
+    anything array-like becomes a contiguous host array (L.HOST).  dtype: the element type of an index array (host arrays are
+    converted to it; CUDA tensors to int32 only -- torch has no uint64 arithmetic, so 64-bit words are taken as they are).
+    values: fp16 and fp32 are kept, anything else becomes fp32.  mem: the mem of the call's other arrays, which this one must share."""
+    if isinstance(a, torch.Tensor) and a.is_cuda:
+        x = (a.to(torch.int32) if dtype == np.int32 else a).contiguous()
+        if values and x.dtype not in (torch.float16, torch.float32):
+            x = x.to(torch.float32)
+        ptr, n, where = C.c_void_p(x.data_ptr()), x.numel(), L.DEVICE
+    else:
+        x = np.ascontiguousarray(np.asarray(a, dtype).reshape(-1))
+        if values and x.dtype not in (np.float16, np.float32):
+            x = x.astype(np.float32)
+        ptr, n, where = x.ctypes.data_as(C.c_void_p), x.size, L.HOST
+    if mem is not None and where != mem:
+        raise ValueError("the arrays of one call must all be CUDA tensors or all be host arrays")
+    return _Array(ptr, n, _dt(x.dtype) if dtype is None else None, where, x)
 
 
 def _dt(dtype) -> int:

@@ -62,6 +62,18 @@ def test_fp32_values_and_dense_blocks(B, oracle):
     _check(B, oracle, 200, 200, rp, ci, v, True, dtype=torch.float16)
 
 
+@pytest.mark.parametrize("vals_dtype", [np.float16, np.float32])
+@pytest.mark.parametrize("dtype", [torch.float16, torch.float32])
+@pytest.mark.parametrize("transposed", [False, True])
+def test_value_dtype_pairs(B, oracle, vals_dtype, dtype, transposed):
+    """every (input values, stored values) dtype pair, host and device input; fp32 values that fp16 cannot hold exactly, so the
+    rounding on ingest is compared too"""
+    rp, ci, v = random_csr(203, 171, 0.1, seed=31, empty_block_rows=(2,), fp16=False)
+    v = v.astype(vals_dtype)
+    _check(B, oracle, 203, 171, rp, ci, v, transposed, dtype=dtype)
+    _check(B, oracle, 203, 171, rp, ci, v, transposed, dtype=dtype, device_input=True)
+
+
 def test_poisson_and_long_rows(B, oracle):
     nr, nc, rp, ci, v = B.generators.poisson5pt(64, 48)
     _check(B, oracle, nr, nc, rp, ci, v, False)
@@ -134,6 +146,22 @@ def test_from_arrays_and_block_transpose(B, oracle):
     sel = (A.keys >> np.uint64(32) >= 3) & (A.keys >> np.uint64(32) < 11)
     assert np.array_equal(ks, A.keys[sel]) and np.array_equal(bs, A.bmps[sel])
     assert np.array_equal(os_, A.offsets[sel] - A.offsets[sel][0])
+
+
+@pytest.mark.parametrize("in_dtype", [torch.float16, torch.float32])
+@pytest.mark.parametrize("out_dtype", [torch.float16, torch.float32])
+@pytest.mark.parametrize("src_transposed", [False, True])
+def test_block_transpose_dtype_pairs(B, oracle, in_dtype, out_dtype, src_transposed):
+    """block_transpose from and to either dtype equals the oracle's other form of the source's stored values"""
+    rp, ci, v = random_csr(150, 90, 0.15, seed=9, fp16=False)
+    M = B.bmSpMatrix.from_csr(150, 90, rp, ci, v, transpose=src_transposed, dtype=in_dtype)
+    stored = oracle.f16_round(v) if in_dtype == torch.float16 else v
+    exp = oracle.csr_to_bmsp(150, 90, rp, ci, stored, transposed=not src_transposed, f16=(out_dtype == torch.float16))
+    T = M.block_transpose(dtype=out_dtype)
+    assert T.transposed != src_transposed and T.dtype == out_dtype
+    k, b, o, vals = T.download()
+    assert_structure_equal((k, b, o), exp)
+    assert np.array_equal(vals.astype(np.float32), exp.values)
 
 
 def test_device_csr_row_ptr_is_validated(B):

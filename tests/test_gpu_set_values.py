@@ -52,6 +52,19 @@ def test_set_values_compact_fp32_to_fp16(B, device):
     assert torch.equal(M.values.cpu(), torch.from_numpy(new).half())
 
 
+@pytest.mark.parametrize("src", [np.float16, np.float32])
+@pytest.mark.parametrize("dtype", [torch.float16, torch.float32])
+@pytest.mark.parametrize("device", [False, True])
+def test_set_values_compact_dtype_pairs(B, src, dtype, device):
+    """compact values of either dtype into a matrix of either dtype: copied when the dtypes agree, converted when they differ"""
+    rp, ci, v = random_csr(150, 130, 0.1, seed=22)
+    M = B.bmSpMatrix.from_csr(150, 130, rp, ci, v, dtype=dtype)
+    new = _fp32_values(M.nnz, 3).astype(src)
+    M.set_values(torch.from_numpy(new).cuda() if device else new)
+    torch.cuda.synchronize()
+    assert torch.equal(M.values.cpu(), torch.from_numpy(new).to(dtype))
+
+
 def test_set_values_none_after_in_place_write(B, oracle):
     """a B operand used once (packed records built), its values rewritten through .values, set_values(None), multiplied again"""
     nr, nc, rp, ci, v = B.generators.poisson5pt(40, 36)

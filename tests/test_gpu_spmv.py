@@ -152,8 +152,10 @@ def test_host_buffer_pipeline(B):
     o = np.lexsort((cols, rows)); rows, cols = rows[o], cols[o]
     rp = np.zeros(nr + 1, np.int64); np.cumsum(np.bincount(rows, minlength=nr), out=rp[1:])
     cases.append((nr, nc, rp.astype(np.int32), cols.astype(np.int32), rng.uniform(-1, 1, rows.size).astype(np.float16).astype(np.float32)))
-    for nr, nc, rp, ci, v in cases:
-        M = B.bmSpMatrix.from_csr(nr, nc, rp, ci, v)
+    # fp32 matrices too, on both paths (chunked row-tiled, block-parallel)
+    runs = [(c, torch.float16) for c in cases] + [(cases[0], torch.float32), (cases[2], torch.float32)]
+    for (nr, nc, rp, ci, v), dtype in runs:
+        M = B.bmSpMatrix.from_csr(nr, nc, rp, ci, v, dtype=dtype)
         for xdt in (torch.float32, torch.float16):
             xh = torch.from_numpy(G.x_vector(nc)).to(xdt).pin_memory()
             yh = torch.full((nr,), 7.0).pin_memory()
@@ -162,14 +164,14 @@ def test_host_buffer_pipeline(B):
                 yh.fill_(7.0)
                 B.bmSparse_SpMV_host(M, xh, yh)
                 torch.cuda.synchronize()
-                assert torch.equal(yh, ref.cpu()), (nr, xdt, it)
+                assert torch.equal(yh, ref.cpu()), (nr, dtype, xdt, it)
             # other buffers after a capture: eager again, then re-captured
             xh2 = (xh.float() * 0.5).to(xdt).pin_memory(); yh2 = torch.empty(nr).pin_memory()
             ref2 = B.bmSparse_SpMV(M, xh2.cuda()).cpu()
             for it in range(3):
                 B.bmSparse_SpMV_host(M, xh2, yh2)
                 torch.cuda.synchronize()
-                assert torch.equal(yh2, ref2), (nr, xdt, it)
+                assert torch.equal(yh2, ref2), (nr, dtype, xdt, it)
     # pageable host memory works too (slower)
     nr, nc, rp, ci, v = cases[0]
     M = B.bmSpMatrix.from_csr(nr, nc, rp, ci, v)
