@@ -14,8 +14,10 @@
 
 #define BMSP_PAD_BYTES 256   // every array is over-allocated so 16-byte bulk copies may overrun the tail
 
-// Device-resident matrix.  keys/bmps/offsets/values are the interchange surface of the reference
-// (include/bmSpMatrix.h:28-31), bit-identical; brp/bcol/rvb/kmask are derived once.
+namespace bmsp { struct SpmvPlan; struct BIndex; }   // spmv.cu, spgemm.cu
+
+// Device-resident matrix.  keys/bmps/offsets/values are the interchange surface of the reference (include/bmSpMatrix.h:28-31),
+// bit-identical; brp/bcol/rvb/kmask are derived once; spmv / bidx are built by the first operation that needs them.
 struct bmsp_matrix_s {
     int32_t rows = 0, cols = 0;
     int64_t nnz = 0, nblk = 0, offsets_len = 0;
@@ -30,41 +32,8 @@ struct bmsp_matrix_s {
     int32_t* bcol = nullptr;    // [nblk]  block column of each block
     uint32_t* rvb = nullptr;    // [nbr+1] first value index of each block row
     uint8_t* kmask = nullptr;   // [nblk]  OR of the 8 bitmap bytes: inner-dimension (k) occupancy
-    void* pmeta = nullptr;      // [nblk]  uint4 {bitmap lo, hi, block column, value offset}; built by the first SpGEMM that uses this matrix as B
-    // SpGEMM, sparse-block operands: B's blocks bucketed by inner index (block row k, bit t of kmask) -- spgemm.cu, "fine index"
-    int32_t fine_state = 0;     // 0 not examined yet, 1 built, -1 not worth it (dense blocks: the buckets would replicate every block ~8 times)
-    uint32_t* fine_ptr = nullptr;   // [nbr * 8 + 1] bucket offsets
-    uint32_t* fine_bcol = nullptr;  // [fine_n] block column of the bucket entry
-    uint8_t* fine_kmask = nullptr;  // [fine_n] kmask of the bucket entry's block (de-duplicates blocks that sit in several buckets)
-    void* fine_rec = nullptr;       // [fine_n] 32-byte records {bitmap lo, hi, block column, value offset}, {first 8 values}
-    int64_t fine_n = 0;
-    // SpMV plan (spmv.cu)
-    int32_t spmv_path = -2;     // -2 not planned yet, 0 row-tiled (dense-ish blocks), 1 block-parallel (sparse blocks)
-    int32_t cap_blk = 0, cap_val = 0;   // per-tile smem capacities of the row-tiled kernels
-    int32_t cap_lines = 0;      // staged x lines per tile (tile plan)
-    int32_t tile_rows = 64;     // block rows per tile (64, 32 or 16)
-    int32_t spmv_kernel = 0;    // row-tiled path: 0 = streaming kernel (persistent CTAs, staged tiles in a shared-memory ring; 64-row tiles only), 1 = one CTA per tile
-    int32_t xl_pitch = 32;      // elements between staged x lines (32 for the streaming kernel's bulk copies, 33 for the per-tile kernel)
-    int32_t* spmv_sched = nullptr;  // streaming kernel: SCHED_SLOTS x {next tile to claim, CTAs done}; a launch takes the next slot
-    uint32_t spmv_sched_next = 0;
-    void* tile_rowpair = nullptr;   // [nbr+1] int2 (block_row_ptr, first value) zipped for one bulk copy per tile
-    void* tile_desc = nullptr;  // [ntiles] TileDesc (spmv.cu): block / value / x-line ranges of every tile of 64 block rows
-    uint32_t* tile_lines = nullptr;   // [nblk] distinct x lines (32 columns) of every tile, stored from the tile's first block index
-    uint16_t* tile_xoff = nullptr;    // [nblk] per block: element offset of its 8-column x segment inside the tile's staged lines
-    // streaming kernel, matrices with at most PALETTE_MAX distinct bitmaps (stencils, bands): the bitmaps are replaced by a palette
-    // and tile_xoff / tile_rowpair by the two arrays below (spmv.cu, "bitmap palette").  spmv_npal == 0: today's arrays are used.
-    int32_t spmv_npal = 0;            // palette entries (distinct bitmaps), 0 = no palette
-    void* tile_palette = nullptr;     // [spmv_npal] 16-byte entries, sorted by bitmap
-    uint32_t* tile_word = nullptr;    // [nblk] per block: x offset (bits 0-15) | palette entry byte offset (bits 16-31)
-    uint32_t* tile_rowrel = nullptr;  // [nbr] per block row: (first block - tile's first block) | (first value - tile's first value) << 16
-    int32_t* work = nullptr;    // block-parallel work items (int4 per item)
-    int32_t n_work = 0, n_split = 0;
-    float* split_partial = nullptr;
-    int32_t* split_rows = nullptr;
-    int32_t* split_list = nullptr;   // the block rows that are sliced (fix-up kernel runs over these only)
-    int32_t n_split_rows = 0;
-    int32_t max_row_blocks = 0;
-    void* host_pipe = nullptr;  // HostPipe (spmv.cu): streams, events and staging buffers of bmsp_spmv_host
+    bmsp::SpmvPlan* spmv = nullptr;   // the SpMV plan, built by the first product (with bmsp_spmv_host's pipeline); freed by spmv_release
+    bmsp::BIndex* bidx = nullptr;     // SpGEMM's index of the matrix as a B operand, built by the first such product; freed by bindex_release
     // Stream ordering of the handle's memory: every entry point that enqueues work on the arrays records its stream here
     // (bmsp::touch).  bmsp_destroy frees on that stream, so the frees are ordered behind the kernels that still read or write the
     // arrays; a handle that was used on more than one stream is drained with a device synchronisation first.  Streams passed to
@@ -105,8 +74,7 @@ void dev_free(void* p, cudaStream_t st);
 template <typename T>
 inline int dev_alloc_t(T** p, size_t n, cudaStream_t st) { return dev_alloc((void**)p, n * sizeof(T), st); }
 
-// One device allocation of n T, freed on the stream it was allocated on when the buffer goes out of scope, unless release() handed
-// it to an owner.
+// One device allocation of n T, freed on the stream it was allocated on when the buffer goes out of scope.
 template <typename T>
 class DevBuf {
 public:
@@ -117,7 +85,6 @@ public:
     int alloc(size_t n, cudaStream_t st) { reset(); st_ = st; return dev_alloc_t(&p_, n, st); }
     T* get() const { return p_; }
     void reset() { dev_free(p_, st_); p_ = nullptr; }
-    T* release() { T* p = p_; p_ = nullptr; return p; }
 private:
     T* p_ = nullptr;
     cudaStream_t st_ = nullptr;
@@ -137,11 +104,15 @@ int exclusive_scan_u64(const uint64_t* in, uint64_t* out, int64_t n, cudaStream_
 
 // derive brp/bcol/rvb/kmask from keys/bmps/offsets (matrix.cu)
 int derive_compact(bmsp_matrix_s* m, cudaStream_t st);
-int plan_spmv(bmsp_matrix_s* m, cudaStream_t st);
-void spmv_host_release(bmsp_matrix_s* m);
+// free m->spmv (spmv.cu) and m->bidx (spgemm.cu); bmsp_destroy calls them once m's streams are done with the memory
+void spmv_release(bmsp_matrix_s* m);
+void bindex_release(bmsp_matrix_s* m);
 // rebuild every copy of m's values that the library derived from them (SpGEMM's packed B records and fine index; spgemm.cu), on
 // st: after m's values changed.  The SpMV plan holds no values and is kept.
 int refresh_value_copies(bmsp_matrix_s* m, cudaStream_t st);
+
+// SpMV's path rule (spmv.cu; dist.cu weighs block rows by it): under 2.5 values per block, or no blocks, runs block-parallel
+inline bool spmv_block_parallel(const bmsp_matrix_s* m) { return m->nblk == 0 || (double)m->nnz / (double)m->nblk < 2.5; }
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 

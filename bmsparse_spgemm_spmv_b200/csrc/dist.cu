@@ -65,8 +65,8 @@ extern "C" int bmsp_partition_block_rows(bmsp_matrix_t A, bmsp_matrix_t Bt, int3
     BMSP_TRY(w.alloc((size_t)nbr + 2, st));
     if (weight_spgemm) cand_weight_kernel<<<(unsigned)ceil_div(nbr, 8), 256, 0, st>>>(A->brp, A->bcol, Bt->brp, nbr, w.get());
     else {
-        const bool blockpar = A->nblk > 0 && (double)A->nnz / (double)A->nblk < 2.5;      // same rule as plan_spmv
-        spmv_weight_kernel<<<(unsigned)ceil_div(nbr, 256), 256, 0, st>>>(A->brp, A->rvb, nbr, (int)dtype_bytes(A->dtype), blockpar ? 330 + 76 * (uint64_t)(nparts - 1) : 40, w.get());
+        const uint64_t row_cost = spmv_block_parallel(A) ? 330 + 76 * (uint64_t)(nparts - 1) : 40;
+        spmv_weight_kernel<<<(unsigned)ceil_div(nbr, 256), 256, 0, st>>>(A->brp, A->rvb, nbr, (int)dtype_bytes(A->dtype), row_cost, w.get());
     }
     BMSP_KERNEL_CHECK();
     BMSP_TRY(exclusive_scan_u64(w.get(), w.get(), nbr, st));

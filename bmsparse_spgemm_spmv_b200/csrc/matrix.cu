@@ -183,7 +183,6 @@ int derive_compact(bmsp_matrix_s* m, cudaStream_t st) {
     derive_rows_kernel<<<(unsigned)ceil_div(m->nbr + 1, 256), 256, 0, st>>>(m->keys, m->offsets, m->brp, m->rvb, m->nblk,
                                                                           m->nbr, (uint64_t)m->nnz);
     BMSP_KERNEL_CHECK();
-    m->spmv_path = -2;      // SpMV plan is built lazily by the first bmsp_spmv
     return BMSP_OK;
 }
 
@@ -255,13 +254,9 @@ int bmsp_destroy(bmsp_matrix_t m) {
     // frees are ordered behind the last work enqueued on the arrays (ADVICE r1: stream 0 does not order after non-blocking streams)
     if (m->multi_stream) cudaDeviceSynchronize();
     cudaStream_t st = m->last_stream;
-    spmv_host_release(m);
+    spmv_release(m); bindex_release(m);
     dev_free(m->keys, st); dev_free(m->bmps, st); dev_free(m->offsets, st); dev_free(m->values, st);
     dev_free(m->brp, st); dev_free(m->bcol, st); dev_free(m->rvb, st); dev_free(m->kmask, st);
-    dev_free(m->work, st); dev_free(m->split_partial, st); dev_free(m->split_rows, st); dev_free(m->split_list, st); dev_free(m->pmeta, st);
-    dev_free(m->fine_ptr, st); dev_free(m->fine_bcol, st); dev_free(m->fine_kmask, st); dev_free(m->fine_rec, st);
-    dev_free(m->tile_desc, st); dev_free(m->spmv_sched, st); dev_free(m->tile_rowpair, st); dev_free(m->tile_lines, st); dev_free(m->tile_xoff, st);
-    dev_free(m->tile_palette, st); dev_free(m->tile_word, st); dev_free(m->tile_rowrel, st);
     delete m;
     return BMSP_OK;
 }

@@ -1204,41 +1204,59 @@ static int plan_rows(const bmsp_matrix_s* A, const bmsp_matrix_s* Bt, int rb, in
     return BMSP_OK;
 }
 
+// What products build for a matrix used as their B operand, once, and reuse (bmsp_matrix_s::bidx; created by ensure_pmeta)
+struct bmsp::BIndex {
+    DevBuf<uint4> pmeta;         // [nblk] 32-byte records {bitmap lo, hi, block column, value offset}, {first 8 values} (none if nblk == 0)
+    // sparse-block operands: B's blocks bucketed by inner index (block row k, bit t of kmask), the "fine index"
+    enum { UNEXAMINED, BUILT, NOT_WORTH_IT } fine_state = UNEXAMINED;   // not worth it: dense blocks, the buckets would replicate every block ~8 times
+    DevBuf<uint32_t> fine_ptr;   // [nbr * 8 + 1] bucket offsets
+    DevBuf<uint32_t> fine_bcol;  // [entries] block column of the bucket entry
+    DevBuf<uint8_t> fine_kmask;  // [entries] kmask of the bucket entry's block (de-duplicates blocks that sit in several buckets)
+    DevBuf<uint4> fine_rec;      // [entries] 32-byte records as in pmeta
+};
+
+// the index's buffers free on the stream they were built on, in the same order as bmsp_destroy's frees (as for spmv_release)
+void bmsp::bindex_release(bmsp_matrix_s* m) { delete m->bidx; m->bidx = nullptr; }
+
 // the two copies of a B operand's values that products keep, (re)written in place: the packed block records and the fine index's
 // (the destinations are arguments: a first build writes them before they are published in Bt)
-static int pack_meta(const bmsp_matrix_s* Bt, void* pmeta, cudaStream_t st) {
+static int pack_meta(const bmsp_matrix_s* Bt, uint4* pmeta, cudaStream_t st) {
     pack_meta_kernel<<<(unsigned)ceil_div(Bt->nblk, 256), 256, 0, st>>>(Bt->bmps, Bt->bcol, Bt->offsets, (const __half*)Bt->values, Bt->nnz,
-                                                                      (uint4*)pmeta, Bt->nblk);
+                                                                      pmeta, Bt->nblk);
     BMSP_KERNEL_CHECK();
     return BMSP_OK;
 }
-static int fine_fill(const bmsp_matrix_s* Bt, const uint32_t* fptr, uint32_t* fbcol, uint8_t* fkmask, void* frec, cudaStream_t st) {
-    fine_fill_kernel<<<(unsigned)ceil_div((int64_t)Bt->nbr * 8, 128), 128, 0, st>>>(Bt->brp, Bt->kmask, (const uint4*)Bt->pmeta, Bt->nbr, fptr,
-                                                                                   fbcol, fkmask, (uint4*)frec);
+static int fine_fill(const bmsp_matrix_s* Bt, const uint32_t* fptr, uint32_t* fbcol, uint8_t* fkmask, uint4* frec, cudaStream_t st) {
+    fine_fill_kernel<<<(unsigned)ceil_div((int64_t)Bt->nbr * 8, 128), 128, 0, st>>>(Bt->brp, Bt->kmask, Bt->bidx->pmeta.get(), Bt->nbr, fptr,
+                                                                                   fbcol, fkmask, frec);
     BMSP_KERNEL_CHECK();
     return BMSP_OK;
 }
 
 int bmsp::refresh_value_copies(bmsp_matrix_s* m, cudaStream_t st) {
-    if (m->pmeta && m->nblk > 0) BMSP_TRY(pack_meta(m, m->pmeta, st));
-    if (m->fine_state == 1) BMSP_TRY(fine_fill(m, m->fine_ptr, m->fine_bcol, m->fine_kmask, m->fine_rec, st));
+    const BIndex* bi = m->bidx;
+    if (bi && bi->pmeta.get()) BMSP_TRY(pack_meta(m, bi->pmeta.get(), st));
+    if (bi && bi->fine_state == BIndex::BUILT) BMSP_TRY(fine_fill(m, bi->fine_ptr.get(), bi->fine_bcol.get(), bi->fine_kmask.get(), bi->fine_rec.get(), st));
     return BMSP_OK;
 }
 
 // B's packed block records: built once per B operand, reused by later products
 static int ensure_pmeta(bmsp_matrix_s* Bt, cudaStream_t st) {
-    if (Bt->pmeta || Bt->nblk == 0) return BMSP_OK;
-    DevBuf<uint4> pm;
-    BMSP_TRY(pm.alloc(2 * (size_t)Bt->nblk, st));
-    BMSP_TRY(pack_meta(Bt, pm.get(), st));
-    Bt->pmeta = pm.release();
+    if (Bt->bidx) return BMSP_OK;
+    std::unique_ptr<BIndex> bi(new BIndex());
+    if (Bt->nblk > 0) {
+        BMSP_TRY(bi->pmeta.alloc(2 * (size_t)Bt->nblk, st));
+        BMSP_TRY(pack_meta(Bt, bi->pmeta.get(), st));
+    }
+    Bt->bidx = bi.release();
     return BMSP_OK;
 }
 
 // Fine index of B for sparse-block operands (about one value per block: uniform random, R-MAT): examined once per B operand, by
 // the rule below only (U1M A*A: 30.8 ms by the candidate scan, 18.9 ms through the buckets).
 static int ensure_fine_index(bmsp_matrix_s* Bt, const bmsp_matrix_s* A, cudaStream_t st) {
-    if (Bt->fine_state != 0 || Bt->nblk == 0 || (int64_t)Bt->nbr * 8 + 1 >= 0x7FFFFFFFll) return BMSP_OK;
+    BIndex& bi = *Bt->bidx;
+    if (bi.fine_state != BIndex::UNEXAMINED || Bt->nblk == 0 || (int64_t)Bt->nbr * 8 + 1 >= 0x7FFFFFFFll) return BMSP_OK;
     if (!(block_density(Bt) <= 2.0 && block_density(A) <= 4.0)) return BMSP_OK;
     const size_t nb = (size_t)Bt->nbr * 8;
     DevBuf<uint32_t> fp;
@@ -1259,15 +1277,14 @@ static int ensure_fine_index(bmsp_matrix_s* Bt, const bmsp_matrix_s* A, cudaStre
     // row over up to 32 lanes, handles those better (R-MAT-18 A*A: 164 ms by scan, 181 ms through the buckets)
     const double mean_bucket = (double)total / std::max<double>(1.0, (double)nb);
     const bool even = (double)longest <= 32.0 * std::max(mean_bucket, 1.0) || longest <= 512;
-    if (!((double)total <= 1.5 * (double)Bt->nblk && even)) { Bt->fine_state = -1; return BMSP_OK; }
+    if (!((double)total <= 1.5 * (double)Bt->nblk && even)) { bi.fine_state = BIndex::NOT_WORTH_IT; return BMSP_OK; }
     DevBuf<uint32_t> fbcol; DevBuf<uint8_t> fkmask; DevBuf<uint4> frec;
     BMSP_TRY(fbcol.alloc((size_t)total + 4, st));
     BMSP_TRY(fkmask.alloc((size_t)total + 16, st));
     BMSP_TRY(frec.alloc(2 * ((size_t)total + 1), st));
     BMSP_TRY(fine_fill(Bt, fp.get(), fbcol.get(), fkmask.get(), frec.get(), st));
-    Bt->fine_ptr = fp.release(); Bt->fine_bcol = fbcol.release(); Bt->fine_kmask = fkmask.release(); Bt->fine_rec = frec.release();
-    Bt->fine_n = total;
-    Bt->fine_state = 1;
+    bi.fine_ptr = std::move(fp); bi.fine_bcol = std::move(fbcol); bi.fine_kmask = std::move(fkmask); bi.fine_rec = std::move(frec);
+    bi.fine_state = BIndex::BUILT;
     return BMSP_OK;
 }
 
@@ -1421,13 +1438,14 @@ static int spgemm_run(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts*
     BMSP_TRY(plan_rows(A, Bt, rb, re, sms, s.rowinfo.get(), s.cand.get(), ctr, h, sp, st));
     BMSP_TRY(ensure_pmeta(Bt, st));
     BMSP_TRY(ensure_fine_index(Bt, A, st));
-    const bool use_fine = s.use_fine = Bt->fine_state == 1;
+    const BIndex& bi = *Bt->bidx;
+    const bool use_fine = s.use_fine = bi.fine_state == BIndex::BUILT;
     const int path = s.path = numeric_path(A, Bt, opts);
 
     GemmArgs& g = s.g;
     memset(&g, 0, sizeof(g));
-    if (use_fine) { g.f_ptr = Bt->fine_ptr; g.f_bcol = Bt->fine_bcol; g.f_kmask = Bt->fine_kmask; g.f_rec = (const uint4*)Bt->fine_rec; }
-    g.b_pm = (const uint4*)Bt->pmeta;
+    if (use_fine) { g.f_ptr = bi.fine_ptr.get(); g.f_bcol = bi.fine_bcol.get(); g.f_kmask = bi.fine_kmask.get(); g.f_rec = bi.fine_rec.get(); }
+    g.b_pm = bi.pmeta.get();
     g.a_brp = A->brp; g.a_bcol = A->bcol; g.a_bmps = A->bmps; g.a_kmask = A->kmask; g.a_off = A->offsets; g.a_val = (const __half*)A->values;
     g.b_brp = Bt->brp; g.b_bcol = Bt->bcol; g.b_bmps = Bt->bmps; g.b_kmask = Bt->kmask; g.b_off = Bt->offsets; g.b_val = (const __half*)Bt->values;
     g.rowinfo = s.rowinfo.get(); g.row_begin = rb; g.row_end = re;

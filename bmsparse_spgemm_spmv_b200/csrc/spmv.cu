@@ -1283,6 +1283,68 @@ __global__ void work_fill_kernel(const int32_t* __restrict__ brp, int nbr, const
 
 static int env_int(const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; }
 
+// ------------------------------------------------------------------------------------ host-buffer pipeline
+// y_host = A x_host with both vectors in (pinned) host memory: the block rows are cut into chunks of whole tiles;
+// chunk c needs the columns [0, x_need[c]) of x (running maximum of the tile plan's line ranges -- for a banded matrix
+// the frontier advances with the rows, for a scattered one the first chunk needs everything and only the y copies
+// overlap).  Three streams: s_in feeds x slices (H2D), the caller's stream runs the row-range launches, s_out drains
+// y slices (D2H); PCIe is full duplex, so the step costs max(x, y) bytes over the link instead of their sum.
+struct HostPipe {
+    cudaStream_t s_in = nullptr, s_out = nullptr;
+    cudaEvent_t ev_start = nullptr, ev_done = nullptr;
+    std::vector<cudaEvent_t> ev_x, ev_k;
+    DevBuf<char> x_dev;
+    DevBuf<float> y_dev;
+    // the whole pipeline of one (x_host, y_host) pair captured as a CUDA graph: one launch instead of ~7 API calls per chunk
+    cudaStream_t s_cap = nullptr;
+    cudaGraphExec_t gexec = nullptr;
+    const void* g_x = nullptr; const void* g_y = nullptr; int32_t g_xdt = -1;      // what gexec was captured for
+    const void* seen_x = nullptr; const void* seen_y = nullptr; int32_t seen_xdt = -1;   // the previous call's buffers
+    std::vector<int> tile_lo;        // [nchunks+1] first tile of every chunk (row-tiled path); {0, 0} for the block-parallel path
+    std::vector<int64_t> x_need;     // [nchunks]  columns that must be resident before the chunk runs
+    ~HostPipe() {                    // the body runs before x_dev / y_dev are freed
+        if (s_in) { cudaStreamSynchronize(s_in); cudaStreamDestroy(s_in); }
+        if (s_out) { cudaStreamSynchronize(s_out); cudaStreamDestroy(s_out); }
+        if (s_cap) { cudaStreamSynchronize(s_cap); cudaStreamDestroy(s_cap); }
+        if (gexec) cudaGraphExecDestroy(gexec);
+        if (ev_start) cudaEventDestroy(ev_start);
+        if (ev_done) cudaEventDestroy(ev_done);
+        for (auto e : ev_x) if (e) cudaEventDestroy(e);
+        for (auto e : ev_k) if (e) cudaEventDestroy(e);
+    }
+};
+
+// Everything the first product on a matrix builds (plan_spmv), owned by the handle (bmsp_matrix_s::spmv).  Which members mean
+// anything depends on the path, and on the row-tiled path on the kernel and on whether there is a palette.
+struct SpmvPlan {
+    enum Path { ROW_TILED, BLOCK_PARALLEL } path = ROW_TILED;   // row-tiled: dense-ish blocks; block-parallel: sparse blocks
+    // row-tiled path (plan_tiles).  kernel 0 = streaming kernel (persistent CTAs, staged tiles in a shared-memory ring; 64-row tiles
+    // only), 1 = one CTA per tile; tiles of 64, 32 or 16 block rows; per-tile shared-memory capacities in blocks, values, x lines
+    int32_t kernel = 0, tile_rows = 64, cap_blk = 0, cap_val = 0, cap_lines = 0;
+    int32_t npal = 0;            // palette entries (distinct bitmaps), 0 = no palette
+    uint32_t sched_next = 0;     // the scheduler slot the streaming kernel's next launch over all tiles takes
+    DevBuf<TileDesc> desc;       // [ntiles] block / value / x-line ranges of every tile
+    DevBuf<uint32_t> lines;      // [nblk] distinct x lines (32 columns) of every tile, stored from the tile's first block index
+    DevBuf<int32_t> sched;       // streaming kernel: SCHED_SLOTS x {next tile to claim, CTAs done}; a launch takes the next slot
+    DevBuf<uint16_t> xoff;       // no palette: [nblk] per block, offset of its 8-column x segment inside the tile's staged lines
+    DevBuf<int2> rowpair;        // no palette: [nbr+1] (block_row_ptr, first value) zipped for one bulk copy per tile
+    // streaming kernel, matrices with at most PALETTE_MAX distinct bitmaps (stencils, bands): the bitmaps are replaced by a palette
+    // and xoff / rowpair by word / rowrel ("bitmap palette")
+    DevBuf<uint4> palette;       // [npal] 16-byte entries, sorted by bitmap
+    DevBuf<uint32_t> word;       // [nblk] per block: x offset (bits 0-15) | palette entry byte offset (bits 16-31)
+    DevBuf<uint32_t> rowrel;     // [nbr] per block row: (first block - tile's first block) | (first value - tile's first value) << 16
+    // block-parallel path (plan_block_parallel): n_work int4 work items; the block rows sliced into several items are listed for
+    // the fix-up kernel, which sums their items' row sums (split_partial, allocated only when there are such rows)
+    int32_t n_work = 0, n_split_rows = 0;
+    DevBuf<int4> work;
+    DevBuf<uint32_t> item_ofs;   // [nbr+1] first work item of every block row
+    DevBuf<int32_t> split_list;
+    DevBuf<float> split_partial;
+    // bmsp_spmv_host's pipeline, built by its first call.  Declared last so that it is destroyed first: its destructor drains the
+    // pipeline's streams before any of the plan's memory is freed.
+    std::unique_ptr<HostPipe> host;
+};
+
 // The streaming kernel's bitmap palette: collect the distinct bitmaps (palette_scan_kernel), sort them here and upload one 16-byte
 // entry per bitmap (layout at PalScan) into `palette`.  Leaves pal empty when the matrix has more than PALETTE_MAX distinct bitmaps.
 static int build_palette(const bmsp_matrix_s* m, int vsize, cudaStream_t st, std::vector<uint4>& pal, DevBuf<uint4>& palette) {
@@ -1324,9 +1386,8 @@ static int build_palette(const bmsp_matrix_s* m, int vsize, cudaStream_t st, std
 }
 
 // path 0 plan: tile descriptors, x lines and per-block x offsets; shared-memory capacities from the tile maxima
-// when they fit the per-CTA budget, else from the averages (larger tiles are then read from global memory).  Built in locals and
-// published in m, then spmv_path = 0, once all of it exists.
-static int plan_tiles(bmsp_matrix_s* m, cudaStream_t st) {
+// when they fit the per-CTA budget, else from the averages (larger tiles are then read from global memory).
+static int plan_tiles(const bmsp_matrix_s* m, SpmvPlan& p, cudaStream_t st) {
     const int vsize = (int)dtype_bytes(m->dtype);
     // tile height: 64 block rows unless an average tile (bitmaps, x offsets, values, ~x lines) would not fit ~20 KB
     int rt = 64;
@@ -1341,33 +1402,31 @@ static int plan_tiles(bmsp_matrix_s* m, cudaStream_t st) {
     const int xl_pitch = kernel == 1 ? XL_STRIDE : 32;
     const int ntiles = (int)ceil_div(m->nbr, rt);
     std::vector<uint4> pal;                    // kept until the synchronisation below (pageable source of the palette upload)
-    DevBuf<uint4> palette;
-    if (kernel == 0) BMSP_TRY(build_palette(m, vsize, st, pal, palette));
-    const int npal = (int)pal.size();
+    if (kernel == 0) BMSP_TRY(build_palette(m, vsize, st, pal, p.palette));
+    const int npal = p.npal = (int)pal.size();
     const bool use_pal = npal > 0;
-    DevBuf<TileDesc> desc; DevBuf<uint32_t> lines, word, rowrel; DevBuf<uint16_t> xoff; DevBuf<int2> rowpair;
-    DevBuf<unsigned long long> stats; DevBuf<int32_t> sched;
-    BMSP_TRY(desc.alloc((size_t)ntiles, st));
-    BMSP_TRY(lines.alloc((size_t)m->nblk + 8, st));
+    DevBuf<unsigned long long> stats;
+    BMSP_TRY(p.desc.alloc((size_t)ntiles, st));
+    BMSP_TRY(p.lines.alloc((size_t)m->nblk + 8, st));
     if (use_pal) {
-        BMSP_TRY(word.alloc((size_t)m->nblk + 8, st));
-        BMSP_TRY(rowrel.alloc((size_t)m->nbr + 8, st));
+        BMSP_TRY(p.word.alloc((size_t)m->nblk + 8, st));
+        BMSP_TRY(p.rowrel.alloc((size_t)m->nbr + 8, st));
     } else {
-        BMSP_TRY(xoff.alloc((size_t)m->nblk + 16, st));
-        BMSP_TRY(rowpair.alloc((size_t)m->nbr + 1 + 8, st));
-        zip_rows_kernel<<<(unsigned)ceil_div(m->nbr + 1, 256), 256, 0, st>>>(m->brp, m->rvb, m->nbr + 1, rowpair.get());
+        BMSP_TRY(p.xoff.alloc((size_t)m->nblk + 16, st));
+        BMSP_TRY(p.rowpair.alloc((size_t)m->nbr + 1 + 8, st));
+        zip_rows_kernel<<<(unsigned)ceil_div(m->nbr + 1, 256), 256, 0, st>>>(m->brp, m->rvb, m->nbr + 1, p.rowpair.get());
         BMSP_KERNEL_CHECK();
     }
     BMSP_TRY(stats.alloc(8, st));
     BMSP_CUDA(cudaMemsetAsync(stats.get(), 0, 8 * sizeof(unsigned long long), st));
-    if (kernel == 0 && !m->spmv_sched) {
+    if (kernel == 0) {
         // tile-claim counters of the streaming kernel (zero before the plan's synchronisation below, so that no later launch -- on
         // whatever stream, captured in a graph or not -- has to wait for them)
-        BMSP_TRY(sched.alloc((size_t)SCHED_SLOTS * 2, st));
-        BMSP_CUDA(cudaMemsetAsync(sched.get(), 0, sizeof(int32_t) * SCHED_SLOTS * 2, st));
+        BMSP_TRY(p.sched.alloc((size_t)SCHED_SLOTS * 2, st));
+        BMSP_CUDA(cudaMemsetAsync(p.sched.get(), 0, sizeof(int32_t) * SCHED_SLOTS * 2, st));
     }
-    tile_plan_kernel<<<ntiles, 256, 0, st>>>(m->brp, m->bcol, m->rvb, m->nbr, m->cols, rt, xl_pitch, desc.get(), lines.get(), xoff.get(),
-                                             stats.get(), m->bmps, palette.get(), npal, word.get(), rowrel.get());
+    tile_plan_kernel<<<ntiles, 256, 0, st>>>(m->brp, m->bcol, m->rvb, m->nbr, m->cols, rt, xl_pitch, p.desc.get(), p.lines.get(),
+                                             p.xoff.get(), stats.get(), m->bmps, p.palette.get(), npal, p.word.get(), p.rowrel.get());
     BMSP_KERNEL_CHECK();
     unsigned long long h[8];
     BMSP_CUDA(cudaMemcpyAsync(h, stats.get(), sizeof(h), cudaMemcpyDeviceToHost, st));
@@ -1390,51 +1449,51 @@ static int plan_tiles(bmsp_matrix_s* m, cudaStream_t st) {
     // the palette variant's relative row pairs are 16-bit: a staged tile has fewer than 65536 blocks and values (the 40 KB budget
     // above keeps both far below that already)
     if (use_pal) { cb = std::min(cb, 65528); cv = std::min(cv, 65528); }
-    m->cap_blk = cb; m->cap_val = cv; m->cap_lines = std::max(cl, 1);
-    m->tile_rows = rt; m->spmv_kernel = kernel; m->xl_pitch = xl_pitch; m->spmv_npal = npal;
-    m->tile_palette = palette.release(); m->tile_desc = desc.release(); m->tile_lines = lines.release(); m->tile_word = word.release();
-    m->tile_rowrel = rowrel.release(); m->tile_xoff = xoff.release(); m->tile_rowpair = rowpair.release();
-    if (sched.get()) m->spmv_sched = sched.release();
-    m->spmv_path = 0;
+    p.cap_blk = cb; p.cap_val = cv; p.cap_lines = std::max(cl, 1); p.tile_rows = rt; p.kernel = kernel;
     return BMSP_OK;
 }
 
-// The plan of the first product on m; path 1 is built in locals like path 0 and published, then spmv_path = 1.
-int plan_spmv(bmsp_matrix_s* m, cudaStream_t st) {
-    if (m->transposed || m->nbr == 0) { m->spmv_path = -1; return BMSP_OK; }
-    const double per_blk = m->nblk ? (double)m->nnz / (double)m->nblk : 0.0;
-    if (per_blk >= 2.5) return plan_tiles(m, st);
-    DevBuf<uint32_t> cnt;                    // item offsets per block row, kept for the fix-up
-    BMSP_TRY(cnt.alloc((size_t)m->nbr + 1, st));
-    work_count_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, cnt.get());
+// block-parallel plan: work items of at most SLICE blocks (or bundles of four short block rows), and the list of sliced block rows
+static int plan_block_parallel(const bmsp_matrix_s* m, SpmvPlan& p, cudaStream_t st) {
+    p.path = SpmvPlan::BLOCK_PARALLEL;
+    BMSP_TRY(p.item_ofs.alloc((size_t)m->nbr + 1, st));
+    work_count_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, p.item_ofs.get());
     BMSP_KERNEL_CHECK();
-    BMSP_TRY(exclusive_scan_u32(cnt.get(), cnt.get(), m->nbr, st));
+    BMSP_TRY(exclusive_scan_u32(p.item_ofs.get(), p.item_ofs.get(), m->nbr, st));
     uint32_t total = 0;
-    BMSP_CUDA(cudaMemcpyAsync(&total, cnt.get() + m->nbr, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(&total, p.item_ofs.get() + m->nbr, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     BMSP_CUDA(cudaStreamSynchronize(st));
-    DevBuf<int4> work;
-    BMSP_TRY(work.alloc((size_t)total, st));
-    work_fill_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, cnt.get(), work.get());
+    BMSP_TRY(p.work.alloc((size_t)total, st));
+    work_fill_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>(m->brp, m->nbr, p.item_ofs.get(), p.work.get());
     BMSP_KERNEL_CHECK();
     // sliced block rows (more than one item): listed on the device.  (Items minus block rows no longer says whether there are any:
     // a bundle is one item for four block rows.)  A sliced row has at least two items, so there are at most total / 2 of them.
     const size_t cap = (size_t)total / 2 + 1;
-    DevBuf<int32_t> list; DevBuf<float> partial;
-    BMSP_TRY(list.alloc(cap + 1, st));
-    int32_t* cntr = list.get() + cap;
+    BMSP_TRY(p.split_list.alloc(cap + 1, st));
+    int32_t* cntr = p.split_list.get() + cap;
     BMSP_CUDA(cudaMemsetAsync(cntr, 0, sizeof(int32_t), st));
-    split_list_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>((const int32_t*)cnt.get(), m->nbr, list.get(), cntr);
+    split_list_kernel<<<(unsigned)ceil_div(m->nbr, 256), 256, 0, st>>>((const int32_t*)p.item_ofs.get(), m->nbr, p.split_list.get(), cntr);
     BMSP_KERNEL_CHECK();
-    int32_t n_split_rows = 0;
-    BMSP_CUDA(cudaMemcpyAsync(&n_split_rows, cntr, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(&p.n_split_rows, cntr, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     BMSP_CUDA(cudaStreamSynchronize(st));
-    if (n_split_rows > 0) BMSP_TRY(partial.alloc((size_t)total * 8, st));
-    m->n_work = (int32_t)total; m->work = (int32_t*)work.release();
-    m->split_rows = (int32_t*)cnt.release(); m->split_list = list.release(); m->split_partial = partial.release();
-    m->n_split_rows = m->n_split = n_split_rows;       // > 0 iff some block row is sliced
-    m->spmv_path = 1;
+    if (p.n_split_rows > 0) BMSP_TRY(p.split_partial.alloc((size_t)total * 8, st));
+    p.n_work = (int32_t)total;
     return BMSP_OK;
 }
+
+// m->spmv, built on st by the first product and published only when complete.  m is neither transposed nor empty: the entry
+// points reject those before they plan.
+static int plan_spmv(bmsp_matrix_s* m, cudaStream_t st) {
+    if (m->spmv) return BMSP_OK;
+    std::unique_ptr<SpmvPlan> p(new SpmvPlan());
+    BMSP_TRY(spmv_block_parallel(m) ? plan_block_parallel(m, *p, st) : plan_tiles(m, *p, st));
+    m->spmv = p.release();
+    return BMSP_OK;
+}
+
+// The plan's buffers free on the stream it was built on (DevBuf), not on the handle's last stream.  That is the same order:
+// either the handle was used on that stream only, or bmsp_destroy synchronised the device before it calls this.
+void spmv_release(bmsp_matrix_s* m) { delete m->spmv; m->spmv = nullptr; }
 
 template <typename T, typename X, int RTT, int MINB, typename H>
 static int launch_tile_kernel(const TileArgs<T>& a, const X* x, float* y, const H& hd, int grid, size_t smem, cudaStream_t st) {
@@ -1500,82 +1559,54 @@ static int launch_stream_kernel(const TileArgs<T>& a, const X* x, float* y, cons
     return BMSP_OK;
 }
 
-// tile0 / ntiles: path 0 only -- launch the tiles [tile0, tile0 + ntiles) (ntiles < 0: all of them).
-// hd: NoHalo, or HaloDev for the fused multi-GPU product (path 0, fp32 x, all tiles).
+// tile0 / ntiles: row-tiled path only -- launch the tiles [tile0, tile0 + ntiles) (ntiles < 0: all of them).
+// hd: NoHalo, or HaloDev for the fused multi-GPU product (row-tiled path, fp32 x, all tiles).
 template <typename T, typename X, typename H = NoHalo>
-static int launch_spmv(bmsp_matrix_s* A, const X* x, float* y, cudaStream_t st, int tile0 = 0, int ntiles = -1, const H& hd = H()) {
-    if (A->spmv_path == 0) {
+static int launch_spmv(const bmsp_matrix_s* A, SpmvPlan& p, const X* x, float* y, cudaStream_t st, int tile0 = 0, int ntiles = -1, const H& hd = H()) {
+    if (p.path == SpmvPlan::ROW_TILED) {
         TileArgs<T> a;
         a.tile0 = tile0;
-        a.bmps = A->bmps; a.bcol = A->bcol; a.values = (const T*)A->values; a.rowpair = (const int2*)A->tile_rowpair;
-        a.desc = (const TileDesc*)A->tile_desc; a.lines = A->tile_lines; a.xoff = A->tile_xoff;
-        a.word = A->tile_word; a.rowrel = A->tile_rowrel; a.palette = (const uint4*)A->tile_palette; a.npal = A->spmv_npal;
+        a.bmps = A->bmps; a.bcol = A->bcol; a.values = (const T*)A->values; a.rowpair = p.rowpair.get();
+        a.desc = p.desc.get(); a.lines = p.lines.get(); a.xoff = p.xoff.get();
+        a.word = p.word.get(); a.rowrel = p.rowrel.get(); a.palette = p.palette.get(); a.npal = p.npal;
         a.brp = A->brp; a.rvb = A->rvb;
-        a.rows = A->rows; a.nbr = A->nbr; a.cols = A->cols; a.cap_blk = A->cap_blk; a.cap_val = A->cap_val; a.cap_lines = A->cap_lines;
-        const int rt = A->tile_rows;
+        a.rows = A->rows; a.nbr = A->nbr; a.cols = A->cols; a.cap_blk = p.cap_blk; a.cap_val = p.cap_val; a.cap_lines = p.cap_lines;
+        const int rt = p.tile_rows;
         a.so = tile_smem(rt, a.cap_blk, a.cap_val, a.cap_lines, sizeof(T), sizeof(X));
         const size_t smem = a.so.total;
         const int grid = ntiles < 0 ? (int)ceil_div(A->nbr, rt) : ntiles;
         if (grid <= 0) return BMSP_OK;
-        if (A->spmv_kernel == 0) {
+        if (p.kernel == 0) {
             // streaming kernel (tile_rows == STREAM_RT, plan_tiles).  A launch over all tiles takes one of the matrix's scheduler
             // slots in turn (launches on different streams may overlap: they must not share a counter); launches over a tile range
             // (the host-buffer pipeline's chunks) keep static shares.
-            int32_t* sched = nullptr;
-            if (ntiles < 0 && A->spmv_sched) sched = A->spmv_sched + 2 * (A->spmv_sched_next++ % SCHED_SLOTS);      // allocated and zeroed by the plan
-            if (A->spmv_npal > 0) return launch_stream_kernel<T, X, H, true>(a, x, y, hd, grid, st, sched);
+            int32_t* sched = ntiles < 0 ? p.sched.get() + 2 * (p.sched_next++ % SCHED_SLOTS) : nullptr;
+            if (p.npal > 0) return launch_stream_kernel<T, X, H, true>(a, x, y, hd, grid, st, sched);
             return launch_stream_kernel<T, X, H, false>(a, x, y, hd, grid, st, sched);
         }
         if (rt == 32) return launch_tile_kernel<T, X, 32, 24, H>(a, x, y, hd, grid, smem, st);
         if (rt == 16) return launch_tile_kernel<T, X, 16, 32, H>(a, x, y, hd, grid, smem, st);
         return launch_tile_kernel<T, X, 64, 12, H>(a, x, y, hd, grid, smem, st);
     }
-    const unsigned grid1 = (unsigned)ceil_div(A->n_work, 8), grid2 = (unsigned)ceil_div((int64_t)A->n_split_rows * 32, 256);
-    spmv_blockpar_kernel<T, X><<<grid1, 256, 0, st>>>(A->bmps, A->bcol, A->offsets, (const T*)A->values, (const int4*)A->work, A->n_work,
-                                                    A->rows, x, y, A->split_partial, A->brp);
+    const unsigned grid1 = (unsigned)ceil_div(p.n_work, 8), grid2 = (unsigned)ceil_div((int64_t)p.n_split_rows * 32, 256);
+    spmv_blockpar_kernel<T, X><<<grid1, 256, 0, st>>>(A->bmps, A->bcol, A->offsets, (const T*)A->values, p.work.get(), p.n_work,
+                                                    A->rows, x, y, p.split_partial.get(), A->brp);
     BMSP_KERNEL_CHECK();
-    if (A->n_split > 0) {
-        spmv_fixup_kernel<<<grid2, 256, 0, st>>>(A->split_rows, A->split_partial, A->split_list, A->n_split_rows, A->rows, y);
+    if (p.n_split_rows > 0) {
+        spmv_fixup_kernel<<<grid2, 256, 0, st>>>((const int32_t*)p.item_ofs.get(), p.split_partial.get(), p.split_list.get(),
+                                                 p.n_split_rows, A->rows, y);
         BMSP_KERNEL_CHECK();
     }
     return BMSP_OK;
 }
 
-// ------------------------------------------------------------------------------------ host-buffer pipeline
-// y_host = A x_host with both vectors in (pinned) host memory: the block rows are cut into chunks of whole tiles;
-// chunk c needs the columns [0, x_need[c]) of x (running maximum of the tile plan's line ranges -- for a banded matrix
-// the frontier advances with the rows, for a scattered one the first chunk needs everything and only the y copies
-// overlap).  Three streams: s_in feeds x slices (H2D), the caller's stream runs the row-range launches, s_out drains
-// y slices (D2H); PCIe is full duplex, so the step costs max(x, y) bytes over the link instead of their sum.
-struct HostPipe {
-    cudaStream_t s_in = nullptr, s_out = nullptr;
-    cudaEvent_t ev_start = nullptr, ev_done = nullptr;
-    std::vector<cudaEvent_t> ev_x, ev_k;
-    DevBuf<char> x_dev;
-    DevBuf<float> y_dev;
-    // the whole pipeline of one (x_host, y_host) pair captured as a CUDA graph: one launch instead of ~7 API calls per chunk
-    cudaStream_t s_cap = nullptr;
-    cudaGraphExec_t gexec = nullptr;
-    const void* g_x = nullptr; const void* g_y = nullptr; int32_t g_xdt = -1;      // what gexec was captured for
-    const void* seen_x = nullptr; const void* seen_y = nullptr; int32_t seen_xdt = -1;   // the previous call's buffers
-    int nchunks = 0;
-    std::vector<int> tile_lo;        // [nchunks+1] first tile of every chunk (path 0); {0, 0} for path 1
-    std::vector<int64_t> x_need;     // [nchunks]  columns that must be resident before the chunk runs
-    ~HostPipe() {                    // the body runs before x_dev / y_dev are freed
-        if (s_in) { cudaStreamSynchronize(s_in); cudaStreamDestroy(s_in); }
-        if (s_out) { cudaStreamSynchronize(s_out); cudaStreamDestroy(s_out); }
-        if (s_cap) { cudaStreamSynchronize(s_cap); cudaStreamDestroy(s_cap); }
-        if (gexec) cudaGraphExecDestroy(gexec);
-        if (ev_start) cudaEventDestroy(ev_start);
-        if (ev_done) cudaEventDestroy(ev_done);
-        for (auto e : ev_x) if (e) cudaEventDestroy(e);
-        for (auto e : ev_k) if (e) cudaEventDestroy(e);
-    }
-};
+// chunks of the host-buffer pipeline.  P4096 on PCIe 5 x16: 8 chunks 1.67 ms, 16: 1.68, 32: 1.84 (per-chunk dependencies cost
+// more than the shorter fill saves)
+constexpr int HOST_CHUNKS = 8;
 
-// A's pipeline, built on the first call and published in A only when complete
-static int host_pipe_get(bmsp_matrix_s* A, cudaStream_t st, HostPipe** out) {
-    if (A->host_pipe) { *out = (HostPipe*)A->host_pipe; return BMSP_OK; }
+// A's pipeline, built on the first call and published in the plan only when complete
+static int host_pipe_get(const bmsp_matrix_s* A, SpmvPlan& p, cudaStream_t st) {
+    if (p.host) return BMSP_OK;
     std::unique_ptr<HostPipe> hp(new HostPipe());
     BMSP_CUDA(cudaStreamCreateWithFlags(&hp->s_in, cudaStreamNonBlocking));
     BMSP_CUDA(cudaStreamCreateWithFlags(&hp->s_out, cudaStreamNonBlocking));
@@ -1584,14 +1615,12 @@ static int host_pipe_get(bmsp_matrix_s* A, cudaStream_t st, HostPipe** out) {
     BMSP_TRY(hp->x_dev.alloc((size_t)A->cols * 4 + 256, st));
     BMSP_TRY(hp->y_dev.alloc((size_t)A->rows + 64, st));
     BMSP_CUDA(cudaStreamCreateWithFlags(&hp->s_cap, cudaStreamNonBlocking));
-    int want = 8;      // P4096 on PCIe 5 x16: 8 chunks 1.67 ms, 16: 1.68, 32: 1.84 (per-chunk dependencies cost more than the shorter fill saves)
-    if (const char* e = getenv("BMSP_HOST_CHUNKS")) want = std::max(1, atoi(e));
-    if (A->spmv_path == 0 && (int64_t)A->rows * 4 >= (1 << 20)) {
-        const int rt = A->tile_rows, ntiles = (int)ceil_div(A->nbr, rt);
+    if (p.path == SpmvPlan::ROW_TILED && (int64_t)A->rows * 4 >= (1 << 20)) {
+        const int rt = p.tile_rows, ntiles = (int)ceil_div(A->nbr, rt);
         std::vector<TileDesc> desc((size_t)ntiles);
-        BMSP_CUDA(cudaMemcpyAsync(desc.data(), A->tile_desc, sizeof(TileDesc) * (size_t)ntiles, cudaMemcpyDeviceToHost, st));
+        BMSP_CUDA(cudaMemcpyAsync(desc.data(), p.desc.get(), sizeof(TileDesc) * (size_t)ntiles, cudaMemcpyDeviceToHost, st));
         BMSP_CUDA(cudaStreamSynchronize(st));
-        const int nch = std::min(want, ntiles), per = (int)ceil_div(ntiles, nch);
+        const int nch = std::min(HOST_CHUNKS, ntiles), per = (int)ceil_div(ntiles, nch);
         int64_t need = 0;
         for (int t0 = 0; t0 < ntiles; t0 += per) {
             const int t1 = std::min(ntiles, t0 + per);
@@ -1604,29 +1633,20 @@ static int host_pipe_get(bmsp_matrix_s* A, cudaStream_t st, HostPipe** out) {
     } else {
         // one chunk: all tiles of a row-tiled matrix (ADVICE r1: {0, 0} launched nothing and left y_host untouched); the
         // block-parallel path ignores tile_lo
-        hp->tile_lo = {0, A->spmv_path == 0 ? (int)ceil_div(A->nbr, A->tile_rows) : 0};
+        hp->tile_lo = {0, p.path == SpmvPlan::ROW_TILED ? (int)ceil_div(A->nbr, p.tile_rows) : 0};
         hp->x_need = {(int64_t)A->cols};
     }
-    hp->nchunks = (int)hp->x_need.size();
-    hp->ev_x.resize(hp->nchunks); hp->ev_k.resize(hp->nchunks);
+    hp->ev_x.resize(hp->x_need.size()); hp->ev_k.resize(hp->x_need.size());
     for (auto& e : hp->ev_x) BMSP_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     for (auto& e : hp->ev_k) BMSP_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    A->host_pipe = *out = hp.release();
+    p.host = std::move(hp);
     return BMSP_OK;
-}
-
-void spmv_host_release(bmsp_matrix_s* m) {
-    delete (HostPipe*)m->host_pipe;
-    m->host_pipe = nullptr;
 }
 
 // y can leave without a copy engine: when y_host is pinned (and therefore mapped into the device's address space) the
 // row-range launches store their float4 results straight into it over PCIe (posted writes), so the pipeline is
 // H2D slices of x on s_in against kernels that write host memory -- no D2H copies, no events per chunk on the way out.
 static float* mapped_host_ptr(float* y_host) {
-    static int enabled = -1;
-    if (enabled < 0) { const char* e = getenv("BMSP_HOST_ZEROCOPY"); enabled = e ? atoi(e) : 1; }
-    if (!enabled) return nullptr;
     cudaPointerAttributes at;
     if (cudaPointerGetAttributes(&at, y_host) != cudaSuccess) { cudaGetLastError(); return nullptr; }
     if (at.type != cudaMemoryTypeHost || !at.devicePointer || ((uintptr_t)at.devicePointer & 15)) return nullptr;
@@ -1634,35 +1654,35 @@ static float* mapped_host_ptr(float* y_host) {
 }
 
 template <typename T>
-static int spmv_host_run(bmsp_matrix_s* A, HostPipe* hp, const void* x_host, int32_t x_dtype, float* y_host, cudaStream_t st) {
+static int spmv_host_run(const bmsp_matrix_s* A, SpmvPlan& p, const void* x_host, int32_t x_dtype, float* y_host, cudaStream_t st) {
+    HostPipe* hp = p.host.get();
     const size_t xs = dtype_bytes(x_dtype);
-    float* y_map = A->spmv_path == 0 ? mapped_host_ptr(y_host) : nullptr;     // row-tiled kernel only: it stores 512 contiguous bytes per warp
+    float* y_map = p.path == SpmvPlan::ROW_TILED ? mapped_host_ptr(y_host) : nullptr;     // row-tiled kernel only: it stores 512 contiguous bytes per warp
     float* y_out = y_map ? y_map : hp->y_dev.get();
     BMSP_CUDA(cudaEventRecord(hp->ev_start, st));         // earlier work on st (and the previous call) is done with x_dev / y_dev
     BMSP_CUDA(cudaStreamWaitEvent(hp->s_in, hp->ev_start, 0));
     BMSP_CUDA(cudaStreamWaitEvent(hp->s_out, hp->ev_start, 0));
     int64_t sent = 0;
-    const int64_t rows_per_tile = (int64_t)A->tile_rows * 8;
-    cudaEvent_t last_x = nullptr;
-    for (int c = 0; c < hp->nchunks; c++) {
+    const int64_t rows_per_tile = (int64_t)p.tile_rows * 8;
+    for (int c = 0; c < (int)hp->x_need.size(); c++) {
         const int64_t need = hp->x_need[c];
         if (need > sent) {
             BMSP_CUDA(cudaMemcpyAsync(hp->x_dev.get() + sent * xs, (const char*)x_host + sent * xs, (size_t)(need - sent) * xs,
                                       cudaMemcpyHostToDevice, hp->s_in));
             BMSP_CUDA(cudaEventRecord(hp->ev_x[c], hp->s_in));
             BMSP_CUDA(cudaStreamWaitEvent(st, hp->ev_x[c], 0));
-            sent = need; last_x = hp->ev_x[c];
+            sent = need;
         }
         int64_t row0 = 0, row1 = A->rows;
-        int t0 = 0, nt = -1;                               // path 1: the whole matrix
-        if (A->spmv_path == 0) {
+        int t0 = 0, nt = -1;                               // block-parallel path: the whole matrix
+        if (p.path == SpmvPlan::ROW_TILED) {
             const int t1 = hp->tile_lo[c + 1];
             t0 = hp->tile_lo[c]; nt = t1 - t0;
             row0 = std::min<int64_t>(A->rows, t0 * rows_per_tile); row1 = std::min<int64_t>(A->rows, t1 * rows_per_tile);
         }
         BMSP_TRY(with_value_type(x_dtype, [&](auto x) {
             using X = decltype(x);
-            return launch_spmv<T, X>(A, (const X*)hp->x_dev.get(), y_out, st, t0, nt);
+            return launch_spmv<T, X>(A, p, (const X*)hp->x_dev.get(), y_out, st, t0, nt);
         }));
         if (row1 > row0 && !y_map) {
             BMSP_CUDA(cudaEventRecord(hp->ev_k[c], st));
@@ -1672,18 +1692,15 @@ static int spmv_host_run(bmsp_matrix_s* A, HostPipe* hp, const void* x_host, int
     }
     BMSP_CUDA(cudaEventRecord(hp->ev_done, hp->s_out));
     BMSP_CUDA(cudaStreamWaitEvent(st, hp->ev_done, 0));   // the caller synchronises `st` as for bmsp_spmv
-    (void)last_x;                                          // s_in is already joined: st waited on its last event above
     return BMSP_OK;
 }
 
 // Second call with the same pinned buffers: capture the pipeline once (origin stream s_cap, forks into s_in / s_out, all
 // joined before the capture ends) and replay it with one cudaGraphLaunch on the caller's stream from then on.
 template <typename T>
-static int spmv_host_graph(bmsp_matrix_s* A, HostPipe* hp, const void* x_host, int32_t x_dtype, float* y_host, cudaStream_t st, bool* used) {
+static int spmv_host_graph(const bmsp_matrix_s* A, SpmvPlan& p, const void* x_host, int32_t x_dtype, float* y_host, cudaStream_t st, bool* used) {
+    HostPipe* hp = p.host.get();
     *used = false;
-    static int enabled = -1;
-    if (enabled < 0) { const char* e = getenv("BMSP_HOST_GRAPH"); enabled = e ? atoi(e) : 1; }
-    if (!enabled) return BMSP_OK;
     if (!(hp->gexec && hp->g_x == x_host && hp->g_y == y_host && hp->g_xdt == x_dtype)) {
         const bool again = hp->seen_x == x_host && hp->seen_y == y_host && hp->seen_xdt == x_dtype;
         hp->seen_x = x_host; hp->seen_y = y_host; hp->seen_xdt = x_dtype;
@@ -1694,7 +1711,7 @@ static int spmv_host_graph(bmsp_matrix_s* A, HostPipe* hp, const void* x_host, i
         if (hp->gexec) { cudaGraphExecDestroy(hp->gexec); hp->gexec = nullptr; }
         cudaGraph_t graph = nullptr;
         BMSP_CUDA(cudaStreamBeginCapture(hp->s_cap, cudaStreamCaptureModeThreadLocal));
-        const int rc = spmv_host_run<T>(A, hp, x_host, x_dtype, y_host, hp->s_cap);
+        const int rc = spmv_host_run<T>(A, p, x_host, x_dtype, y_host, hp->s_cap);
         const cudaError_t ce = cudaStreamEndCapture(hp->s_cap, &graph);
         if (rc != BMSP_OK || ce != cudaSuccess || !graph) { cudaGetLastError(); if (graph) cudaGraphDestroy(graph); return BMSP_OK; }
         const cudaError_t ie = cudaGraphInstantiate(&hp->gexec, graph, 0);
@@ -1717,14 +1734,14 @@ extern "C" int bmsp_spmv_host(bmsp_matrix_t A, const void* x_host, int32_t x_dty
     if (A->rows == 0) return BMSP_OK;
     cudaStream_t st = (cudaStream_t)stream;
     touch(A, st);
-    if (A->spmv_path < 0) BMSP_TRY(plan_spmv(A, st));
-    HostPipe* hp = nullptr;
-    BMSP_TRY(host_pipe_get(A, st, &hp));
+    BMSP_TRY(plan_spmv(A, st));
+    SpmvPlan& p = *A->spmv;
+    BMSP_TRY(host_pipe_get(A, p, st));
     return with_value_type(A->dtype, [&](auto t) -> int {
         using T = decltype(t);
         bool replayed = false;
-        BMSP_TRY(spmv_host_graph<T>(A, hp, x_host, x_dtype, y_host, st, &replayed));
-        return replayed ? BMSP_OK : spmv_host_run<T>(A, hp, x_host, x_dtype, y_host, st);
+        BMSP_TRY(spmv_host_graph<T>(A, p, x_host, x_dtype, y_host, st, &replayed));
+        return replayed ? BMSP_OK : spmv_host_run<T>(A, p, x_host, x_dtype, y_host, st);
     });
 }
 
@@ -1758,11 +1775,8 @@ extern "C" int bmsp_halo_push(const float* y_own, int32_t rows, const bmsp_halo_
     HaloDev h;
     BMSP_TRY(halo_to_dev(halo, rows, &h));
     if (h.n_peer == 0) return BMSP_OK;
-    int64_t total = 0;
-    for (int i = 0; i < h.n_push; i++) total += h.hi[i] - h.lo[i];
     int lo_all = 0x7FFFFFFF, hi_all = 0;
     for (int i = 0; i < h.n_push; i++) { lo_all = std::min(lo_all, h.lo[i]); hi_all = std::max(hi_all, h.hi[i]); }
-    (void)total;
     const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div((int64_t)std::max(0, hi_all - lo_all), 1024), 592));
     h.signal_epoch = signal_epoch; h.n_sig = (uint32_t)grid;
     halo_push_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(y_own, rows, h);
@@ -1792,13 +1806,14 @@ extern "C" int bmsp_spmv_halo(bmsp_matrix_t A, const float* x_ext, float* y_own,
     BMSP_TRY(halo_to_dev(halo, A->rows, &h));
     h.wait_epoch = wait_epoch; h.signal_epoch = signal_epoch;
     if (A->rows == 0 || h.n_peer == 0) return A->rows == 0 ? BMSP_OK : bmsp_spmv(A, x_ext, BMSP_F32, y_own, stream);
-    if (A->spmv_path < 0) BMSP_TRY(plan_spmv(A, st));
-    if (A->spmv_path == 0) {
+    BMSP_TRY(plan_spmv(A, st));
+    SpmvPlan& p = *A->spmv;
+    if (p.path == SpmvPlan::ROW_TILED) {
         // One launch of the halo variant over all tiles.  Running the tiles that wait or push in a launch of their own ahead of the
         // plain kernel over the rest was slower on P4096 (one GPU as its own peer): 85.7 us on the same stream (the small launch is
         // all latency) and 79.5 us on a side stream, against 69.7 us.
         // tiles that own pushed rows (union of the ranges' tile intervals); they count down to the signal
-        const int64_t rpt = (int64_t)A->tile_rows * 8;
+        const int64_t rpt = (int64_t)p.tile_rows * 8;
         std::vector<std::pair<int64_t, int64_t>> iv;
         for (int i = 0; i < h.n_push; i++) if (h.hi[i] > h.lo[i]) iv.push_back({h.lo[i] / rpt, (h.hi[i] - 1) / rpt});
         std::sort(iv.begin(), iv.end());
@@ -1810,8 +1825,8 @@ extern "C" int bmsp_spmv_halo(bmsp_matrix_t A, const float* x_ext, float* y_own,
         }
         if (n == 0) { h.solo_tile = 0; n = 1; }
         h.n_sig = (uint32_t)n;
-        h.rot = (int)(ceil_div(A->nbr, A->tile_rows) / 2);
-        return with_value_type(A->dtype, [&](auto t) { return launch_spmv<decltype(t), float, HaloDev>(A, x_ext, y_own, st, 0, -1, h); });
+        h.rot = (int)(ceil_div(A->nbr, p.tile_rows) / 2);
+        return with_value_type(A->dtype, [&](auto t) { return launch_spmv<decltype(t), float, HaloDev>(A, p, x_ext, y_own, st, 0, -1, h); });
     }
     // block-parallel path: wait kernel, product, push kernel
     halo_wait_kernel<<<1, 32, 0, st>>>(h);
@@ -1850,10 +1865,10 @@ extern "C" int bmsp_spmv(bmsp_matrix_t A, const void* x, int32_t x_dtype, float*
     if (((uintptr_t)x & 15) || ((uintptr_t)y & 15)) { set_error("bmsp_spmv: x and y must be 16-byte aligned"); return BMSP_ERR_INVALID; }
     cudaStream_t st = (cudaStream_t)stream;
     touch(A, st);
-    if (A->spmv_path < 0) BMSP_TRY(plan_spmv(A, st));
+    BMSP_TRY(plan_spmv(A, st));
     return with_value_type(A->dtype, [&](auto t) { return with_value_type(x_dtype, [&](auto xt) {
         using X = decltype(xt);
-        return launch_spmv<decltype(t), X>(A, (const X*)x, y, st);
+        return launch_spmv<decltype(t), X>(A, *A->spmv, (const X*)x, y, st);
     }); });
 }
 

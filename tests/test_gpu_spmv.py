@@ -99,6 +99,23 @@ def test_block_parallel_bundles_of_short_block_rows(B, oracle, nbr):
     assert M.nnz / max(M.block_num, 1) < 2.5
 
 
+@pytest.mark.parametrize("nparts", [3, 64])
+def test_partition_of_a_matrix_without_blocks(B, nparts):
+    """an all-zero matrix has no blocks, runs on the block-parallel path, and is partitioned by that path's cost of a block row
+    (330 byte units + 76 per peer, dist.cu).  All block rows weigh the same: the bounds are the scan-and-search over equal weights."""
+    nr = 1000
+    M = B.bmSpMatrix.from_csr(nr, nr, np.zeros(nr + 1, np.int32), np.zeros(0, np.int32), np.zeros(0, np.float32))
+    assert M.block_num == 0
+    assert torch.equal(B.bmSparse_SpMV(M, torch.ones(nr, device="cuda")), torch.zeros(nr, device="cuda"))
+    nbr = (nr + 7) // 8
+    h = np.arange(nbr + 1, dtype=np.int64) * (330 + 76 * (nparts - 1))
+    exp = [0]
+    for p in range(1, nparts):
+        exp.append(min(max(int(np.searchsorted(h, h[-1] * p // nparts, side="left")), exp[-1]), nbr))
+    exp.append(nbr)
+    assert M.partition_block_rows(nparts).tolist() == exp
+
+
 def test_tile_overflow_falls_back_to_global(B, oracle):
     """dense-ish blocks but one tile far above the average: the row-tiled kernel must read it from global"""
     rng = np.random.default_rng(5)

@@ -1,6 +1,6 @@
-"""End-to-end SpMV through bmsp_spmv_host (x and y in pinned host memory) on P4096: wall time per step for the chunk
-count in BMSP_HOST_CHUNKS, next to the unpipelined copy / launch / copy sequence.
-usage: BMSP_HOST_CHUNKS=24 python tools/e2e_bench.py [grid] [reps]"""
+"""End-to-end SpMV through bmsp_spmv_host (x and y in pinned host memory) on P4096: wall time per step of the chunked
+pipeline, next to the unpipelined copy / launch / copy sequence.
+usage: python tools/e2e_bench.py [grid] [reps]"""
 import os
 import sys
 import time
@@ -41,5 +41,5 @@ for name, fn in (("pipelined", piped), ("plain", plain)):
     for _ in range(reps):
         fn()
     ms = (time.perf_counter() - t0) / reps * 1e3
-    print(f"E2E {name} chunks={os.environ.get('BMSP_HOST_CHUNKS', 'default')} grid={m} ms={ms:.3f} GBps={A.spmv_bytes() / ms / 1e6:.1f} "
+    print(f"E2E {name} grid={m} ms={ms:.3f} GBps={A.spmv_bytes() / ms / 1e6:.1f} "
           f"link_GBps_each_way={nr * 4 / ms / 1e6:.1f}")
