@@ -268,7 +268,23 @@ static int convert_device_csr(int32_t rows, int32_t cols, int64_t nnz, const int
 
 // ---------------------------------------------------------------------------- block transpose
 // (transpose8x8: common.cuh)
-// One thread per block: new bitmap = transpose; value of cell p=(hi,lo) moves to the rank of cell (lo,hi).
+// The values of one block in the other cell order: the value of cell p=(hi,lo) of bmp moves to the rank of cell (lo,hi) in
+// t = transpose8x8(bmp).  vin / vout point at the block's first value.
+template <typename Tin, typename Tout>
+__device__ __forceinline__ void permute_block_values(uint64_t bmp, uint64_t t, const Tin* __restrict__ vin, Tout* __restrict__ vout) {
+    uint64_t rem = bmp;
+    int k = 0;
+    while (rem) {
+        int p = __clzll((long long)rem);
+        rem &= ~(0x8000000000000000ull >> p);
+        int q = ((p & 7) << 3) | (p >> 3);
+        int rank = q == 0 ? 0 : __popcll(t >> (64 - q));
+        vout[rank] = conv<Tin, Tout>(vin[k]);
+        k++;
+    }
+}
+
+// One thread per block: new bitmap = transpose, values permuted inside the block.
 template <typename Tin, typename Tout>
 __global__ void block_transpose_kernel(const uint64_t* __restrict__ bmps, const uint64_t* __restrict__ offsets,
                                        const Tin* __restrict__ vin, uint64_t* __restrict__ bmps_out,
@@ -277,16 +293,136 @@ __global__ void block_transpose_kernel(const uint64_t* __restrict__ bmps, const 
     if (b >= nblk) return;
     uint64_t bmp = bmps[b], t = transpose8x8(bmp), off = offsets[b];
     bmps_out[b] = t;
-    uint64_t rem = bmp;
-    int k = 0;
-    while (rem) {
-        int p = __clzll((long long)rem);
-        rem &= ~(0x8000000000000000ull >> p);
-        int q = ((p & 7) << 3) | (p >> 3);
-        int rank = q == 0 ? 0 : __popcll(t >> (64 - q));
-        vout[off + rank] = conv<Tin, Tout>(vin[off + k]);
-        k++;
+    permute_block_values(bmp, t, vin + off, vout + off);
+}
+
+// ---------------------------------------------------------------------------- matrix transpose
+// A^T's block (bc, br) is A's block (br, bc), so A^T's blocks in key order are A's blocks stably sorted by block column: A is
+// sorted by (br, bc), and a stable sort keeps the blocks of one column in block-row order.  The sort is an LSD radix sort of
+// (block column, block index) with 8-bit digits; each pass is a per-tile digit histogram, one scan over the [digit][tile] table
+// and a scatter that ranks equal digits inside the tile in input order (match_any per warp, per-warp running counts).  No atomic
+// decides a position, so the result is the same on every run.
+constexpr int RADIX_T = 256, RADIX_ITEMS = 8, RADIX_TILE = RADIX_T * RADIX_ITEMS, RADIX_WARPS = RADIX_T / 32;
+
+__global__ void __launch_bounds__(RADIX_T) radix_hist_kernel(const uint32_t* __restrict__ keys, int64_t n, int shift, uint32_t* __restrict__ hist,
+                                                             int64_t ntiles) {
+    __shared__ uint32_t h[256];
+    h[threadIdx.x] = 0;
+    __syncthreads();
+    const int64_t base = (int64_t)blockIdx.x * RADIX_TILE;
+#pragma unroll
+    for (int i = 0; i < RADIX_ITEMS; i++) {
+        const int64_t e = base + i * RADIX_T + threadIdx.x;
+        if (e < n) atomicAdd(&h[(keys[e] >> shift) & 0xFFu], 1u);
     }
+    __syncthreads();
+    hist[(int64_t)threadIdx.x * ntiles + blockIdx.x] = h[threadIdx.x];
+}
+
+// pos: the exclusive scan of radix_hist_kernel's table.  vals_in nullptr: the value of an element is its index (the first pass);
+// keys_out nullptr: the keys are not needed after this pass (the last one).
+__global__ void __launch_bounds__(RADIX_T) radix_scatter_kernel(const uint32_t* __restrict__ keys_in, const uint32_t* __restrict__ vals_in, int64_t n,
+                                                                int shift, const uint32_t* __restrict__ pos, int64_t ntiles,
+                                                                uint32_t* __restrict__ keys_out, uint32_t* __restrict__ vals_out) {
+    __shared__ uint32_t cnt[RADIX_WARPS][256];      // per warp and digit: elements seen so far, then the warp's first output slot
+    for (int i = threadIdx.x; i < RADIX_WARPS * 256; i += RADIX_T) (&cnt[0][0])[i] = 0;
+    __syncthreads();
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int64_t wbase = (int64_t)blockIdx.x * RADIX_TILE + (int64_t)w * 32 * RADIX_ITEMS;   // each warp owns a contiguous run
+    uint32_t key[RADIX_ITEMS], rank[RADIX_ITEMS];
+#pragma unroll
+    for (int i = 0; i < RADIX_ITEMS; i++) {
+        const int64_t e = wbase + i * 32 + lane;
+        const bool valid = e < n;                   // the invalid elements are the tile's last ones: they rank after every valid one
+        key[i] = valid ? keys_in[e] : 0u;
+        const uint32_t d = (key[i] >> shift) & 0xFFu;
+        const uint32_t peers = __match_any_sync(0xffffffffu, valid ? d : 256u);
+        rank[i] = cnt[w][d] + __popc(peers & ((1u << lane) - 1u));
+        __syncwarp();
+        if (valid && lane == __ffs(peers) - 1) cnt[w][d] += __popc(peers);
+        __syncwarp();
+    }
+    __syncthreads();
+    {
+        uint32_t run = pos[(int64_t)threadIdx.x * ntiles + blockIdx.x];      // RADIX_T == 256: one thread per digit
+#pragma unroll
+        for (int q = 0; q < RADIX_WARPS; q++) { const uint32_t c = cnt[q][threadIdx.x]; cnt[q][threadIdx.x] = run; run += c; }
+    }
+    __syncthreads();
+#pragma unroll
+    for (int i = 0; i < RADIX_ITEMS; i++) {
+        const int64_t e = wbase + i * 32 + lane;
+        if (e >= n) continue;
+        const uint32_t slot = cnt[w][(key[i] >> shift) & 0xFFu] + rank[i];
+        if (keys_out) keys_out[slot] = key[i];
+        vals_out[slot] = vals_in ? vals_in[e] : (uint32_t)e;
+    }
+}
+
+// One thread per block of A^T: src[j] is its block in A (src nullptr: the same index).  Key (br, bc) -> (bc, br) is a rotation
+// by 32 bits; the bitmap is transposed when A's form and A^T's are the same (flip); the block's value count goes to cnt for the
+// scan that makes the offsets.
+__global__ void transpose_blocks_kernel(const uint64_t* __restrict__ keys, const uint64_t* __restrict__ bmps, const uint32_t* __restrict__ src,
+                                        int64_t nblk, int flip, uint64_t* __restrict__ keys_out, uint64_t* __restrict__ bmps_out,
+                                        uint64_t* __restrict__ cnt) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= nblk) return;
+    const int64_t s = src ? (int64_t)src[j] : j;
+    const uint64_t key = keys[s], bmp = bmps[s];
+    keys_out[j] = (key << 32) | (key >> 32);
+    bmps_out[j] = flip ? transpose8x8(bmp) : bmp;
+    cnt[j] = (uint64_t)__popcll(bmp);
+}
+
+// One thread per block of A^T: its values from A's block src[j], copied in order or permuted (flip), converted to Tout.
+template <typename Tin, typename Tout>
+__global__ void transpose_values_kernel(const uint64_t* __restrict__ bmps, const uint64_t* __restrict__ offsets, const Tin* __restrict__ vin,
+                                        const uint32_t* __restrict__ src, int64_t nblk, int flip, const uint64_t* __restrict__ offsets_out,
+                                        Tout* __restrict__ vout) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= nblk) return;
+    const int64_t s = src ? (int64_t)src[j] : j;
+    const uint64_t bmp = bmps[s];
+    const Tin* in = vin + offsets[s];
+    Tout* out = vout + offsets_out[j];
+    if (flip) {
+        permute_block_values(bmp, transpose8x8(bmp), in, out);
+    } else {
+        const int n = __popcll(bmp);
+        for (int k = 0; k < n; k++) out[k] = conv<Tin, Tout>(in[k]);
+    }
+}
+
+// src[j] = A's block that becomes A^T's block j; *src nullptr when A has at most one block column (the order is A's)
+static int transpose_block_order(const bmsp_matrix_s* A, cudaStream_t st, DevBuf<uint32_t> (&kbuf)[2], DevBuf<uint32_t> (&vbuf)[2],
+                                 const uint32_t** src) {
+    *src = nullptr;
+    const int64_t n = A->nblk, nbc = ceil_div(A->cols, 8);
+    int bits = 0;
+    while (bits < 32 && ((uint64_t)(nbc - 1) >> bits)) bits++;
+    const int passes = (bits + 7) / 8;
+    if (n == 0 || passes == 0) return BMSP_OK;
+    const int64_t ntiles = ceil_div(n, RADIX_TILE);
+    DevBuf<uint32_t> pos;
+    BMSP_TRY(pos.alloc((size_t)ntiles * 256 + 1, st));
+    for (int b = 0; b < 2; b++) {
+        if (passes > 1 + b) BMSP_TRY(kbuf[b].alloc((size_t)n, st));
+        if (passes > b) BMSP_TRY(vbuf[b].alloc((size_t)n, st));
+    }
+    const uint32_t* keys = (const uint32_t*)A->bcol;
+    const uint32_t* vals = nullptr;
+    for (int p = 0; p < passes; p++) {
+        const int shift = 8 * p;
+        radix_hist_kernel<<<(unsigned)ntiles, RADIX_T, 0, st>>>(keys, n, shift, pos.get(), ntiles);
+        BMSP_KERNEL_CHECK();
+        BMSP_TRY(exclusive_scan_u32(pos.get(), pos.get(), ntiles * 256, st));
+        uint32_t* kout = p + 1 < passes ? kbuf[p & 1].get() : nullptr;
+        radix_scatter_kernel<<<(unsigned)ntiles, RADIX_T, 0, st>>>(keys, vals, n, shift, pos.get(), ntiles, kout, vbuf[p & 1].get());
+        BMSP_KERNEL_CHECK();
+        keys = kout; vals = vbuf[p & 1].get();
+    }
+    *src = vals;
+    return BMSP_OK;
 }
 
 }  // namespace bmsp
@@ -488,6 +624,41 @@ int bmsp_block_transpose(bmsp_matrix_t A, int32_t out_dtype, void* stream, bmsp_
             BMSP_KERNEL_CHECK();
             return BMSP_OK;
         }); }));
+    }
+    BMSP_TRY(derive_compact(m.get(), st));
+    *At = m.release();
+    return BMSP_OK;
+}
+
+// A^T: the block order (transpose_block_order), then keys / bitmaps / value counts per block, the offsets by a scan, the values,
+// the derived arrays.  Every step is enqueued on st; nothing is read back.
+int bmsp_matrix_transpose(bmsp_matrix_t A, int32_t out_dtype, int32_t out_transposed, void* stream, bmsp_matrix_t* At) {
+    if (!A || !At || (out_dtype != BMSP_F16 && out_dtype != BMSP_F32)) { set_error("bmsp_matrix_transpose: invalid argument"); return BMSP_ERR_INVALID; }
+    cudaStream_t st = (cudaStream_t)stream;
+    touch(A, st);
+    HandlePtr m;
+    BMSP_TRY(new_handle(A->cols, A->rows, A->nblk, A->nnz, out_dtype, out_transposed ? 1 : 0, st, m));
+    m->offsets_len = A->offsets_len;
+    const int flip = (A->transposed != 0) == (out_transposed != 0);     // same form: the cells of a block move, so the bitmap does
+    {
+        DevBuf<uint32_t> kbuf[2], vbuf[2];
+        const uint32_t* src = nullptr;
+        BMSP_TRY(transpose_block_order(A, st, kbuf, vbuf, &src));
+        const unsigned grid = (unsigned)ceil_div(m->nblk, 256);
+        if (m->nblk) {
+            transpose_blocks_kernel<<<grid, 256, 0, st>>>(A->keys, A->bmps, src, m->nblk, flip, m->keys, m->bmps, m->offsets);
+            BMSP_KERNEL_CHECK();
+        }
+        BMSP_TRY(exclusive_scan_u64(m->offsets, m->offsets, m->nblk, st));       // offsets[nblk] = nnz, kept when offsets_len says so
+        if (m->nblk) {
+            BMSP_TRY(with_value_type(A->dtype, [&](auto in) { return with_value_type(out_dtype, [&](auto out) -> int {
+                using Tin = decltype(in); using Tout = decltype(out);
+                transpose_values_kernel<Tin, Tout><<<grid, 256, 0, st>>>(A->bmps, A->offsets, (const Tin*)A->values, src, m->nblk, flip,
+                                                                         m->offsets, (Tout*)m->values);
+                BMSP_KERNEL_CHECK();
+                return BMSP_OK;
+            }); }));
+        }
     }
     BMSP_TRY(derive_compact(m.get(), st));
     *At = m.release();

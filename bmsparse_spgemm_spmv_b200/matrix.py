@@ -204,6 +204,16 @@ class bmSpMatrix:
         L.check(L.lib().bmsp_block_transpose(self._h, _dt(dtype or self.dtype), _stream_ptr(), C.byref(out._h)))
         return out
 
+    def matrix_transpose(self, dtype=None, transpose=False, stream=None) -> "bmSpMatrix":
+        """The transpose A^T as a new matrix (num_rows and num_cols swapped).  Unlike block_transpose, which stores the same matrix A
+        in the other form, this returns a different matrix.  transpose: as in from_csr, store A^T in transposed-operand form, ready
+        to be the B of a product (A.matrix_transpose(transpose=True) is the B of A * A^T).  dtype None keeps this matrix's dtype.
+        This matrix may be in either form.  Enqueued on the stream (default: the current one) without a host synchronisation; the
+        result does not depend on this matrix afterwards."""
+        out = bmSpMatrix()
+        L.check(L.lib().bmsp_matrix_transpose(self._h, _dt(dtype or self.dtype), int(bool(transpose)), _stream_ptr(stream), C.byref(out._h)))
+        return out
+
     def slice_block_rows(self, r0, r1, rebase=False):
         out = bmSpMatrix()
         L.check(L.lib().bmsp_slice_block_rows(self._h, int(r0), int(r1), int(rebase), _stream_ptr(), C.byref(out._h)))

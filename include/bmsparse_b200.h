@@ -215,6 +215,12 @@ int bmsp_spgemm_plan_destroy(bmsp_spgemm_plan_t plan);
  * (SPGEMM.cu:759-781) is unused.  out_dtype lets an fp32 product feed the next multiply as fp16. */
 int bmsp_block_transpose(bmsp_matrix_t A, int32_t out_dtype, void* stream, bmsp_matrix_t* At);
 
+/* A^T as a new matrix: rows and columns swapped, stored plain (out_transposed = 0: SpMV operand, left SpGEMM operand) or in
+ * transposed-operand form (out_transposed = 1: the B of X * A^T), values converted to out_dtype.  A may be in either form.
+ * Enqueued on `stream` only: no host synchronisation, no read-back.  Transposing twice gives A's arrays bit for bit.
+ * No counterpart in the reference. */
+int bmsp_matrix_transpose(bmsp_matrix_t A, int32_t out_dtype, int32_t out_transposed, void* stream, bmsp_matrix_t* At);
+
 /* ---- multi-GPU helpers (block-row sharding, SURVEY.md section 8e) --------------------------- */
 /* Split block rows into nparts contiguous ranges balanced by SpMV bytes (weight_spgemm = 0) or by
  * candidate SpGEMM pairs against Bt (weight_spgemm = 1, Bt required).  bounds: int32[nparts+1]. */
