@@ -6,5 +6,5 @@ oracle/: the CPU oracle is test infrastructure.
 """
 from ._lib import BmspError, LIB_PATH, SYMBOLS, lib  # noqa: F401
 from .matrix import bmSpMatrix  # noqa: F401
-from .ops import SpGEMMPlan, bmSparse_SpMV, bmSparse_SpMV_host, bmSparse_mult, bmSparse_mult_plan  # noqa: F401
+from .ops import SpGEMMPlan, bmSparse_SpMV, bmSparse_SpMV_host, bmSparse_add, bmSparse_mult, bmSparse_mult_plan  # noqa: F401
 from . import generators  # noqa: F401

@@ -4,7 +4,7 @@
   bmSparse_mult(A, B, C, mode, VERBOSE, tc_version)  src/bmSparse_SPGEMM.cu:827-1223
 
 and bmSparse_mult_plan, which the reference does not have: the same product, kept so that C's values can be recomputed after the
-operands' values change.
+operands' values change; and bmSparse_add, C = alpha*A + beta*B, which the reference does not have either.
 """
 from __future__ import annotations
 
@@ -109,3 +109,16 @@ def bmSparse_mult_plan(A: bmSpMatrix, B: bmSpMatrix, VERBOSE: bool = False, nume
     h = C.c_void_p()
     L.check(L.lib().bmsp_spgemm_plan_create(A._h, B._h, C.byref(opts), _stream_ptr(stream), C.byref(h), C.byref(out._h), C.byref(info)))
     return SpGEMMPlan(h, A, B, out, info)
+
+
+def bmSparse_add(A: bmSpMatrix, B: bmSpMatrix, alpha: float = 1.0, beta: float = 1.0, dtype=None, stream=None) -> bmSpMatrix:
+    """C = alpha*A + beta*B as a new matrix (bmsp_add).  A and B have the same shape and storage form (block_transpose converts
+    one); C is stored in that form.  C's pattern is the union of A's and B's: entries that cancel are kept.  Each value is
+    fl(fl(alpha*a) + fl(beta*b)) in fp32, a missing entry counting as 0, rounded once to dtype.  dtype None: fp32 if either
+    operand holds fp32 values, else fp16.  Synchronises the stream (default: the current one) once; C does not depend on A or B
+    afterwards.  Shape and form errors raise BmspError with the library's code."""
+    if dtype is None:
+        dtype = torch.float32 if torch.float32 in (A.dtype, B.dtype) else torch.float16
+    out = bmSpMatrix()
+    L.check(L.lib().bmsp_add(C.c_float(alpha), A._h, C.c_float(beta), B._h, _dt(dtype), _stream_ptr(stream), C.byref(out._h)))
+    return out

@@ -221,6 +221,13 @@ int bmsp_block_transpose(bmsp_matrix_t A, int32_t out_dtype, void* stream, bmsp_
  * No counterpart in the reference. */
 int bmsp_matrix_transpose(bmsp_matrix_t A, int32_t out_dtype, int32_t out_transposed, void* stream, bmsp_matrix_t* At);
 
+/* C = alpha*A + beta*B as a new matrix.  A and B: same shape, same storage form (both plain or both transposed-operand), any
+ * dtype each.  C's pattern is the UNION of A's and B's patterns: entries whose sum is zero are kept (the pattern depends on
+ * the operands' patterns only).  Each value is fl(fl(alpha*a) + fl(beta*b)) in fp32, where a missing entry counts as 0. It is
+ * rounded once to out_dtype.  C is stored in A's form with offsets_len = block_num.  Synchronises `stream` once, because C's
+ * block and value counts must reach the host.  No counterpart in the reference. */
+int bmsp_add(float alpha, bmsp_matrix_t A, float beta, bmsp_matrix_t B, int32_t out_dtype, void* stream, bmsp_matrix_t* C);
+
 /* ---- multi-GPU helpers (block-row sharding, SURVEY.md section 8e) --------------------------- */
 /* Split block rows into nparts contiguous ranges balanced by SpMV bytes (weight_spgemm = 0) or by
  * candidate SpGEMM pairs against Bt (weight_spgemm = 1, Bt required).  bounds: int32[nparts+1]. */
