@@ -31,30 +31,7 @@ __global__ void add_partition_kernel(const uint64_t* __restrict__ ka, int64_t na
                                      int64_t ntiles, int64_t* __restrict__ split) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t > ntiles) return;
-    const int64_t d = min(t * MERGE_TILE, na + nb);
-    int64_t lo = max((int64_t)0, d - nb), hi = min(d, na);
-    while (lo < hi) {
-        const int64_t mid = (lo + hi) >> 1;
-        if (ka[mid] <= kb[d - 1 - mid]) lo = mid + 1; else hi = mid;
-    }
-    split[t] = lo;
-}
-
-// exclusive scan over the CTA (MERGE_T threads) of one value per thread; *total: the sum
-__device__ __forceinline__ uint32_t cta_exclusive_scan(uint32_t v, uint32_t* total) {
-    __shared__ uint32_t warp_sum[MERGE_T / 32];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    uint32_t incl = v;
-    for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t u = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += u;
-    }
-    if (lane == 31) warp_sum[w] = incl;
-    __syncthreads();
-    uint32_t base = 0, sum = 0;
-    for (int q = 0; q < MERGE_T / 32; q++) { const uint32_t s = warp_sum[q]; base += q < w ? s : 0; sum += s; }
-    *total = sum;
-    return base + incl - v;
+    split[t] = merge_path(ka, na, kb, nb, min(t * MERGE_TILE, na + nb));
 }
 
 // One CTA per tile of the merge.  An item is a head (the first of C's block) when it comes from A, or when it comes from B and A's
@@ -72,7 +49,6 @@ __global__ void __launch_bounds__(MERGE_T) add_merge_kernel(const uint64_t* __re
                                                             uint32_t* __restrict__ src_a, uint32_t* __restrict__ src_b) {
     __shared__ uint64_t s[MERGE_TILE];        // A's keys of the tile, then B's
     __shared__ uint64_t s_prev_a, s_next_b;   // A's key before the tile, B's key after it (NO_KEY: none)
-    __shared__ uint64_t warp_pc[MERGE_T / 32];
     const int64_t t = blockIdx.x;
     const int64_t d0 = t * MERGE_TILE, d1 = min(d0 + MERGE_TILE, na + nb);
     const int64_t i0 = split[t], i1 = split[t + 1], j0 = d0 - i0, j1 = d1 - i1;
@@ -85,12 +61,7 @@ __global__ void __launch_bounds__(MERGE_T) add_merge_kernel(const uint64_t* __re
     __syncthreads();
     // this thread's items: [diag, diag + MERGE_ITEMS) of the tile, starting at A's ia-th and B's jb-th block of the tile
     const int diag = min((int)threadIdx.x * MERGE_ITEMS, len);
-    int lo = max(0, diag - lb), hi = min(diag, la);
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (s[mid] <= s[la + diag - 1 - mid]) lo = mid + 1; else hi = mid;
-    }
-    int ia = lo, jb = diag - lo;
+    int ia = merge_path(s, la, s + la, lb, diag), jb = diag - ia;
     const int n_items = min(MERGE_ITEMS, len - diag);
     uint32_t sa[MERGE_ITEMS], sb[MERGE_ITEMS];
     uint32_t heads = 0;
@@ -117,15 +88,8 @@ __global__ void __launch_bounds__(MERGE_T) add_merge_kernel(const uint64_t* __re
     uint32_t total;
     uint32_t slot = cta_exclusive_scan(heads, &total);
     if (!FILL) {
-        for (int o = 16; o; o >>= 1) pc += __shfl_down_sync(0xffffffffu, pc, o);
-        if ((threadIdx.x & 31) == 0) warp_pc[threadIdx.x >> 5] = pc;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            uint64_t sum = 0;
-            for (int q = 0; q < MERGE_T / 32; q++) sum += warp_pc[q];
-            tile_heads[t] = total;
-            tile_nnz[t] = sum;
-        }
+        pc = cta_sum(pc);
+        if (threadIdx.x == 0) { tile_heads[t] = total; tile_nnz[t] = pc; }
         return;
     }
     slot += tile_heads[t];
@@ -187,11 +151,8 @@ __global__ void __launch_bounds__(VAL_T) add_values_kernel(const uint64_t* __res
     __syncthreads();
     const uint64_t v1 = s_off[nb];
     for (uint64_t v = s_off[0] + tid; v < v1; v += VAL_T) {
-        int lo = 0, hi = nb - 1;                       // the last block whose first value is at or before v
-        while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if (s_off[mid] <= v) lo = mid; else hi = mid - 1;
-        }
+        // the last block whose first value is at or before v; s_off[0] <= v < s_off[nb], so the search starts past block 0
+        const int lo = upper_bound(s_off, 1, nb, v) - 1;
         const int p = nth_cell(s_bmp[lo], (int)(v - s_off[lo]));
         const float a = cell_value(s_bmp_a[lo], va, s_off_a[lo], p);
         const float b = cell_value(s_bmp_b[lo], vb, s_off_b[lo], p);

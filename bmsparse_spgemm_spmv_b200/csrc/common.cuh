@@ -192,6 +192,113 @@ __device__ __forceinline__ uint64_t transpose8x8(uint64_t x) {
     return x;
 }
 
+// ---- scans, reductions and searches of the set-up kernels (count per item, scan the counts, size the output, fill it).
+// The warp functions need the full warp active.  The reductions use the xor butterfly: every lane gets the result.
+template <typename T>
+__device__ __forceinline__ T warp_inclusive_scan(T v) {
+    const int lane = threadIdx.x & 31;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const T t = __shfl_up_sync(0xffffffffu, v, o);
+        if (lane >= o) v += t;
+    }
+    return v;
+}
+template <typename T>
+__device__ __forceinline__ T warp_sum(T v) {
+#pragma unroll
+    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+// a flag counts 1: its warp sum and warp scan are a ballot and a popcount (uint32_t)
+__device__ __forceinline__ uint32_t warp_inclusive_scan(bool p) {
+    return __popc(__ballot_sync(0xffffffffu, p) & (0xffffffffu >> (31 - (threadIdx.x & 31))));
+}
+__device__ __forceinline__ uint32_t warp_sum(bool p) { return __popc(__ballot_sync(0xffffffffu, p)); }
+template <typename T>
+__device__ __forceinline__ T warp_min(T v) {
+#pragma unroll
+    for (int o = 16; o; o >>= 1) v = min(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+}
+template <typename T>
+__device__ __forceinline__ T warp_max(T v) {
+#pragma unroll
+    for (int o = 16; o; o >>= 1) v = max(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+}
+
+// The CTA functions take one value per thread from every thread of the CTA; blockDim.x is a multiple of 32, at most 1024.  Both
+// end with a barrier, so a kernel may call them more than once.
+// Exclusive scan in thread order; *total = the sum over the CTA.  Warp scans, then warp 0 scans the warp totals.  V is T, or bool
+// with T uint32_t (flags).
+template <typename V, typename T>
+__device__ __forceinline__ T cta_exclusive_scan(V v, T* total) {
+    __shared__ T s_warp[33];              // per warp: its total, then the sum of the earlier warps; [32]: the CTA's total
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const T incl = warp_inclusive_scan(v);
+    if (lane == 31) s_warp[w] = incl;
+    __syncthreads();
+    if (w == 0) {
+        const T x = lane < (int)(blockDim.x >> 5) ? s_warp[lane] : T(0);
+        const T xi = warp_inclusive_scan(x);
+        s_warp[lane] = xi - x;
+        if (lane == 31) s_warp[32] = xi;
+    }
+    __syncthreads();
+    const T ex = s_warp[w] + incl - v;
+    *total = s_warp[32];
+    __syncthreads();
+    return ex;
+}
+// The sum over the CTA, returned to every thread (uint32_t for flags).  Warp sums, then warp 0 sums the warp totals.  The total
+// is read after the last barrier: a next call writes it only after its first barrier, which every thread reaches after reading.
+template <typename V>
+__device__ __forceinline__ auto cta_sum(V v) {
+    using T = decltype(warp_sum(v));
+    __shared__ T s_warp[33];              // per warp: its sum; [32]: the CTA's
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const T ws = warp_sum(v);
+    if (lane == 0) s_warp[w] = ws;
+    __syncthreads();
+    if (w == 0) {
+        const T s = warp_sum(lane < (int)(blockDim.x >> 5) ? s_warp[lane] : T(0));
+        if (lane == 0) s_warp[32] = s;
+    }
+    __syncthreads();
+    return s_warp[32];
+}
+
+// Searches in a[lo, hi), ascending, in global or shared memory.  lower_bound: the first i with a[i] >= v; upper_bound: the first
+// i with a[i] > v (hi when there is none).  The last i with a[i] <= v is upper_bound(...) - 1.
+template <typename T, typename V, typename I>
+__device__ __forceinline__ I lower_bound(const T* a, I lo, I hi, V v) {
+    while (lo < hi) {
+        const I mid = (lo + hi) >> 1;
+        if (a[mid] < v) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+template <typename T, typename V, typename I>
+__device__ __forceinline__ I upper_bound(const T* a, I lo, I hi, V v) {
+    while (lo < hi) {
+        const I mid = (lo + hi) >> 1;
+        if (a[mid] <= v) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+// Merge path: how many of a's items are among the first diag items of the stable merge of the ascending a[0, na) and b[0, nb),
+// ties to a (a's item of an equal pair comes first).
+template <typename T, typename I>
+__device__ __forceinline__ I merge_path(const T* a, I na, const T* b, I nb, I diag) {
+    I lo = max((I)0, diag - nb), hi = min(diag, na);
+    while (lo < hi) {
+        const I mid = (lo + hi) >> 1;
+        if (a[mid] <= b[diag - 1 - mid]) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
 // streaming (read-once) loads: keep them out of L1 and mark evict-first in L2 so that x stays resident
 __device__ __forceinline__ uint64_t ld_stream_u64(const uint64_t* p) {
     return (uint64_t)__ldcs(reinterpret_cast<const unsigned long long*>(p));   // ld.global.cs: evict-first

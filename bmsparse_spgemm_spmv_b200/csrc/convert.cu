@@ -4,8 +4,8 @@
 // 4-level comparator -> 2 reduce_by_key + scan + 2 transforms) and src/reader.cu:49-110.
 // Same mapping (Appendix A of SURVEY.md), different algorithm: CSR rows are already sorted, so the
 // block-row order of an entry is a sum of eight binary searches (an 8-way merge rank) -- no global
-// sort.  Bitmaps are then built warp-cooperatively (head flags by ballot, segmented OR by shuffle,
-// ranks by popc) and values are compacted with 16-byte stores.
+// sort.  Block ids are a CTA scan of the head flags, bitmaps a warp-segmented OR by shuffle, and values
+// are compacted with 16-byte stores.
 #include "common.cuh"
 #include <vector>
 #include <algorithm>
@@ -34,14 +34,6 @@ __global__ void check_rowptr_kernel(const int32_t* __restrict__ rp, int32_t rows
     if (bad) atomicOr(flags, FLAG_ROWPTR);
 }
 
-__device__ __forceinline__ int lower_bound_i32(const int32_t* __restrict__ a, int lo, int hi, int target) {
-    while (lo < hi) {
-        int mid = (lo + hi) >> 1;
-        if (__ldg(a + mid) < target) lo = mid + 1; else hi = mid;
-    }
-    return lo;
-}
-
 // K0: the row of the first entry of every chunk of RANK_T entries (last r with rp[r] <= e), one thread per chunk.  The only
 // place that searches all of row_ptr: a search per ENTRY was 24 dependent L2 round trips on a 16 M-row matrix and two thirds of the
 // whole conversion (ncu launch list, profiles/r2_bench_launches_summary.txt).
@@ -51,12 +43,7 @@ __global__ void chunk_row_kernel(const int32_t* __restrict__ rp, int32_t rows, i
     if (b > nchunks) return;
     if (b == nchunks) { chunk_row[b] = rows - 1; return; }
     const int64_t e = b * RANK_T;
-    int lo = 0, hi = rows;   // invariant: rp[lo] <= e < rp[hi]
-    while (hi - lo > 1) {
-        int mid = (lo + hi) >> 1;
-        if ((int64_t)__ldg(rp + mid) <= e) lo = mid; else hi = mid;
-    }
-    chunk_row[b] = lo;
+    chunk_row[b] = upper_bound(rp, 1, rows, e) - 1;   // rp[0] = 0 <= e < nnz = rp[rows]: the search starts past row 0
 }
 
 // K1: one thread per CSR entry, a CTA per chunk of RANK_T entries.  The chunk's rows lie between the rows of its first entry and
@@ -77,23 +64,8 @@ __global__ void __launch_bounds__(RANK_T) rank_kernel(const int32_t* __restrict_
     __syncthreads();
     int64_t e = (int64_t)blockIdx.x * RANK_T + threadIdx.x;
     if (e >= nnz) return;
-    // row = last r with rp[r] <= e
-    int lo, hi;              // invariant: rp[lo] <= e < rp[hi]
-    if (in_smem) {
-        lo = 0; hi = span;
-        while (hi - lo > 1) {
-            int mid = (lo + hi) >> 1;
-            if ((int64_t)srp[mid] <= e) lo = mid; else hi = mid;
-        }
-        lo += r_lo;
-    } else {
-        lo = r_lo; hi = r_hi + 1;
-        while (hi - lo > 1) {
-            int mid = (lo + hi) >> 1;
-            if ((int64_t)__ldg(rp + mid) <= e) lo = mid; else hi = mid;
-        }
-    }
-    const int r = lo;
+    // row = last r with rp[r] <= e; rp[r_lo] <= e < rp[r_hi + 1], so the search starts past r_lo
+    const int r = in_smem ? r_lo + upper_bound(srp, 1, span, e) - 1 : upper_bound(rp, r_lo + 1, r_hi + 1, e) - 1;
     const int c = ci[e];
     if (c < 0 || c >= cols) { atomicOr(flags, FLAG_RANGE); return; }
     const int rs = __ldg(rp + r);
@@ -113,7 +85,7 @@ __global__ void __launch_bounds__(RANK_T) rank_kernel(const int32_t* __restrict_
         int target;
         if (TRANSPOSED) target = q < ri ? c + 1 : c;                   // (bc, ci, ri) order
         else            target = q < ri ? (bc + 1) << 3 : bc << 3;      // (bc, ri, ci) order
-        pos += lower_bound_i32(ci, s, t, target) - s;
+        pos += lower_bound(ci, s, t, target) - s;
     }
     int64_t g = (int64_t)__ldg(rp + r0) + pos;
     s_key[g] = ((uint64_t)(uint32_t)br << 32) | (uint32_t)bc;
@@ -121,21 +93,14 @@ __global__ void __launch_bounds__(RANK_T) rank_kernel(const int32_t* __restrict_
     s_src[g] = (int32_t)e;
 }
 
-// K2: heads per tile of 1024 sorted entries (ballot + popc).
+// K2: heads per tile of 1024 sorted entries.
 __global__ void __launch_bounds__(1024) head_count_kernel(const uint64_t* __restrict__ s_key, int64_t nnz,
                                                           uint32_t* __restrict__ counts) {
     int64_t i = (int64_t)blockIdx.x * 1024 + threadIdx.x;
     bool head = false;
     if (i < nnz) head = (i == 0) || (s_key[i] != s_key[i - 1]);
-    __shared__ uint32_t wc[32];
-    uint32_t b = __ballot_sync(0xffffffffu, head);
-    if ((threadIdx.x & 31) == 0) wc[threadIdx.x >> 5] = __popc(b);
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        uint32_t v = wc[threadIdx.x];
-        for (int o = 16; o; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-        if (threadIdx.x == 0) counts[blockIdx.x] = v;
-    }
+    const uint32_t n = cta_sum(head);
+    if (threadIdx.x == 0) counts[blockIdx.x] = n;
 }
 
 // K3: block ids from the scanned head counts; keys/offsets/block columns by the head lanes; bitmaps by
@@ -145,25 +110,13 @@ __global__ void __launch_bounds__(1024) emit_kernel(const uint64_t* __restrict__
                                                     uint64_t* __restrict__ keys, uint64_t* __restrict__ bmps,
                                                     uint64_t* __restrict__ offsets) {
     int64_t i = (int64_t)blockIdx.x * 1024 + threadIdx.x;
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int lane = threadIdx.x & 31;
     uint64_t key = 0;
     bool head = false;
     if (i < nnz) { key = s_key[i]; head = (i == 0) || (key != s_key[i - 1]); }
-    uint32_t b = __ballot_sync(0xffffffffu, head);
-    __shared__ uint32_t wc[32];
-    if (lane == 0) wc[wid] = __popc(b);
-    __syncthreads();
-    if (wid == 0) {
-        uint32_t v = wc[lane], inc = v;
-        for (int o = 1; o < 32; o <<= 1) {
-            uint32_t t = __shfl_up_sync(0xffffffffu, inc, o);
-            if (lane >= o) inc += t;
-        }
-        wc[lane] = inc - v;
-    }
-    __syncthreads();
-    // inclusive head count up to this lane, minus one = block id
-    int32_t blk = (int32_t)(tile_base[blockIdx.x] + wc[wid] + __popc(b & (0xffffffffu >> (31 - lane)))) - 1;
+    uint32_t tile_heads;
+    // inclusive head count up to this entry, minus one = block id
+    int32_t blk = (int32_t)(tile_base[blockIdx.x] + cta_exclusive_scan(head, &tile_heads) + head) - 1;
     if (i >= nnz) blk = -1;
     uint32_t hi = 0, lo = 0;
     if (i < nnz) {

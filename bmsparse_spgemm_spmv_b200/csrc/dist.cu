@@ -36,7 +36,7 @@ __global__ void __launch_bounds__(256) cand_weight_kernel(const int32_t* __restr
         const int k = a_bcol[a];
         c += (unsigned long long)(b_brp[k + 1] - b_brp[k]);
     }
-    for (int o = 16; o; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+    c = warp_sum(c);
     if (lane == 0) w[row] = c + 4;   // + a little per-row overhead so empty rows still spread
 }
 

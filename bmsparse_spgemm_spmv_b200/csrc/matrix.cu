@@ -56,15 +56,8 @@ __global__ void scan_tile_sums(const T* __restrict__ in, T* __restrict__ sums, i
         int64_t idx = base + (int64_t)i * blockDim.x + threadIdx.x;
         if (idx < n) s += in[idx];
     }
-    __shared__ T warp_s[32];
-    for (int o = 16; o; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
-    if ((threadIdx.x & 31) == 0) warp_s[threadIdx.x >> 5] = s;
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        T v = threadIdx.x < (blockDim.x >> 5) ? warp_s[threadIdx.x] : 0;
-        for (int o = 16; o; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-        if (threadIdx.x == 0) sums[blockIdx.x] = v;
-    }
+    s = cta_sum(s);
+    if (threadIdx.x == 0) sums[blockIdx.x] = s;
 }
 
 template <typename T>
@@ -81,27 +74,8 @@ __global__ void scan_tiles(const T* in, T* out, const T* __restrict__ tile_base,
         v[i] = idx < n ? in[idx] : 0;
         s += v[i];
     }
-    // exclusive scan of s across the block
-    T incl = s;
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    for (int o = 1; o < 32; o <<= 1) {
-        T t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += t;
-    }
-    __shared__ T warp_s[32];
-    if (lane == 31) warp_s[wid] = incl;
-    __syncthreads();
-    if (wid == 0) {
-        T w = lane < (blockDim.x >> 5) ? warp_s[lane] : 0;
-        T wi = w;
-        for (int o = 1; o < 32; o <<= 1) {
-            T t = __shfl_up_sync(0xffffffffu, wi, o);
-            if (lane >= o) wi += t;
-        }
-        warp_s[lane] = wi - w;
-    }
-    __syncthreads();
-    T run = (tile_base ? tile_base[blockIdx.x] : 0) + warp_s[wid] + (incl - s);
+    T total;
+    T run = (tile_base ? tile_base[blockIdx.x] : 0) + cta_exclusive_scan(s, &total);
 #pragma unroll
     for (int i = 0; i < ITEMS; i++) {
         int64_t idx = base + i;
@@ -156,12 +130,7 @@ __global__ void derive_rows_kernel(const uint64_t* __restrict__ keys, const uint
                                    uint64_t nnz) {
     int32_t br = blockIdx.x * blockDim.x + threadIdx.x;
     if (br > nbr) return;
-    uint64_t target = (uint64_t)br << 32;
-    int64_t lo = 0, hi = nblk;
-    while (lo < hi) {
-        int64_t mid = (lo + hi) >> 1;
-        if (keys[mid] < target) lo = mid + 1; else hi = mid;
-    }
+    const int64_t lo = lower_bound(keys, (int64_t)0, nblk, (uint64_t)br << 32);
     brp[br] = (int32_t)lo;
     rvb[br] = (uint32_t)(lo < nblk ? offsets[lo] : nnz);
 }
@@ -367,12 +336,7 @@ __device__ __forceinline__ void csr_walk_block_row(const int32_t* __restrict__ b
             lo |= (uint64_t)__popc((uint32_t)(bmp >> (56 - 8 * r)) & 0xFFu) << (16 * r);
             hi |= (uint64_t)__popc((uint32_t)(bmp >> (24 - 8 * r)) & 0xFFu) << (16 * r);
         }
-        uint64_t ilo = lo, ihi = hi;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint64_t tl = __shfl_up_sync(0xffffffffu, ilo, o), th = __shfl_up_sync(0xffffffffu, ihi, o);
-            if (lane >= o) { ilo += tl; ihi += th; }
-        }
+        const uint64_t ilo = warp_inclusive_scan(lo), ihi = warp_inclusive_scan(hi);
         const uint64_t elo = ilo - lo, ehi = ihi - hi;             // exclusive: cells of each row in the earlier blocks of this chunk
         if (valid) {
             uint64_t k = offsets[b];
@@ -615,11 +579,7 @@ __global__ void __launch_bounds__(256) compare_rows_kernel(int32_t rows, const i
     __shared__ unsigned long long s_mx;
     if (threadIdx.x == 0) { s_c[0] = s_c[1] = s_c[2] = 0; s_sum = 0.0; s_mx = 0ull; }
     __syncthreads();
-    for (int o = 16; o; o >>= 1) {
-        only_a += __shfl_xor_sync(0xffffffffu, only_a, o); only_b += __shfl_xor_sync(0xffffffffu, only_b, o);
-        common += __shfl_xor_sync(0xffffffffu, common, o); sum += __shfl_xor_sync(0xffffffffu, sum, o);
-        mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-    }
+    only_a = warp_sum(only_a); only_b = warp_sum(only_b); common = warp_sum(common); sum = warp_sum(sum); mx = warp_max(mx);
     if ((threadIdx.x & 31) == 0) {
         atomicAdd(&s_c[0], only_a); atomicAdd(&s_c[1], only_b); atomicAdd(&s_c[2], common); atomicAdd(&s_sum, sum);
         atomicMax(&s_mx, (unsigned long long)__double_as_longlong(mx));       // non-negative doubles order like their bit patterns

@@ -161,11 +161,7 @@ __global__ void __launch_bounds__(256) rowinfo_kernel(const int32_t* __restrict_
                 jmax = max(jmax, b_bcol[b1 - 1]);
             }
         }
-        for (int o = 16; o; o >>= 1) {
-            c += __shfl_xor_sync(0xffffffffu, c, o);
-            jmin = min(jmin, __shfl_xor_sync(0xffffffffu, jmin, o));
-            jmax = max(jmax, __shfl_xor_sync(0xffffffffu, jmax, o));
-        }
+        c = warp_sum(c); jmin = warp_min(jmin); jmax = warp_max(jmax);
         if (lane == 0) {
             int jbase = 0, words = 0;
             if (jmax >= 0) { jbase = jmin & ~31; words = ((jmax - jbase) >> 5) + 1; }
@@ -483,8 +479,7 @@ __device__ __forceinline__ void enumerate_vec(const GemmArgs& g, const RowCtx& r
 // B's blocks bucketed by inner index the survivors of an A block are the contiguous bucket(s) of its own inner index(es).
 __global__ void fine_max_kernel(const uint32_t* __restrict__ cnt, int64_t n, uint32_t* __restrict__ mx) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    uint32_t v = i < n ? cnt[i] : 0u;
-    for (int o = 16; o; o >>= 1) v = max(v, __shfl_xor_sync(0xffffffffu, v, o));
+    const uint32_t v = warp_max(i < n ? cnt[i] : 0u);
     if ((threadIdx.x & 31) == 0 && v) atomicMax(mx, v);
 }
 __global__ void fine_count_kernel(const uint64_t* __restrict__ keys, const uint8_t* __restrict__ kmask, int64_t nblk, uint32_t* __restrict__ cnt) {

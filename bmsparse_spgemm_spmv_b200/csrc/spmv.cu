@@ -186,9 +186,8 @@ __global__ void __launch_bounds__(256) tile_plan_kernel(const int32_t* __restric
                                                         uint32_t* __restrict__ rowrel) {
     __shared__ uint32_t s_key[PLAN_MAXB];
     __shared__ uint32_t s_uniq[PLAN_MAXB];
-    __shared__ uint32_t s_w[9];
     __shared__ uint64_t s_pal[PALETTE_MAX];
-    const int t = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const int t = blockIdx.x, tid = threadIdx.x;
     const int r0 = t * rt, r1 = min(r0 + rt, nbr);
     const int p0 = brp[r0], nb = brp[r1] - p0;
     const uint32_t v0 = rvb[r0], v1 = rvb[r1];
@@ -225,43 +224,21 @@ __global__ void __launch_bounds__(256) tile_plan_kernel(const int32_t* __restric
     const int i0 = tid * per, i1 = min(i0 + per, nb);
     uint32_t cnt = 0;
     for (int i = i0; i < i1; i++) cnt += (i == 0 || s_key[i] != s_key[i - 1]) ? 1u : 0u;
-    uint32_t inc = cnt;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t u = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += u;
-    }
-    if (lane == 31) s_w[wid] = inc;
-    __syncthreads();
-    if (tid == 0) {
-        uint32_t run = 0;
-        for (int w = 0; w < 8; w++) { const uint32_t c = s_w[w]; s_w[w] = run; run += c; }
-        s_w[8] = run;
-    }
-    __syncthreads();
-    uint32_t run = s_w[wid] + inc - cnt;
+    uint32_t total;
+    uint32_t run = cta_exclusive_scan(cnt, &total);
     for (int i = i0; i < i1; i++)
         if (i == 0 || s_key[i] != s_key[i - 1]) s_uniq[run++] = s_key[i];
-    const int nl = (int)s_w[8];
+    const int nl = (int)total;
     __syncthreads();
     for (int j = tid; j < nl; j += 256) lines[p0 + j] = s_uniq[j];
     const bool ok = nl <= XL_MAX;
     if (ok)
         for (int i = tid; i < nb; i += 256) {
-            const uint32_t c = (uint32_t)bcol[p0 + i], line = c >> 2;
-            int lo = 0, hi = nl;
-            while (lo < hi) {
-                const int mid = (lo + hi) >> 1;
-                if (s_uniq[mid] < line) lo = mid + 1; else hi = mid;
-            }
+            const uint32_t c = (uint32_t)bcol[p0 + i];
+            const int lo = lower_bound(s_uniq, 0, nl, c >> 2);
             const uint32_t xo = (uint32_t)(lo * pitch + (int)(c & 3u) * 8);
             if (word) {
-                const uint64_t b = bmps[p0 + i];
-                int pl = 0, ph = npal;
-                while (pl < ph) {
-                    const int mid = (pl + ph) >> 1;
-                    if (s_pal[mid] < b) pl = mid + 1; else ph = mid;
-                }
+                const int pl = lower_bound(s_pal, 0, npal, bmps[p0 + i]);
                 word[p0 + i] = xo | (uint32_t)pl << 20;              // entry byte offset (16 * code) in bits 16-31
             } else {
                 xoff[p0 + i] = (uint16_t)xo;
