@@ -90,6 +90,41 @@ private:
     cudaStream_t st_ = nullptr;
 };
 
+// Owners of a stream, an event and a graph executable, next to DevBuf's ownership of memory.  A Stream synchronises before it is
+// destroyed, so a struct that holds one declares it after the buffers its work uses: members are destroyed in reverse order, and
+// the stream drains before they are freed.
+struct StreamDrain { void operator()(cudaStream_t s) const { cudaStreamSynchronize(s); cudaStreamDestroy(s); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+struct GraphExecDestroy { void operator()(cudaGraphExec_t g) const { cudaGraphExecDestroy(g); } };
+using Stream = std::unique_ptr<CUstream_st, StreamDrain>;
+using Event = std::unique_ptr<CUevent_st, EventDestroy>;
+using GraphExec = std::unique_ptr<CUgraphExec_st, GraphExecDestroy>;
+inline int new_stream(Stream& s) {       // non-blocking: no implicit synchronisation with the legacy default stream
+    cudaStream_t h = nullptr;
+    BMSP_CUDA(cudaStreamCreateWithFlags(&h, cudaStreamNonBlocking));
+    s.reset(h);
+    return BMSP_OK;
+}
+inline int new_event(Event& e, bool timing = false) {
+    cudaEvent_t h = nullptr;
+    BMSP_CUDA(cudaEventCreateWithFlags(&h, timing ? cudaEventDefault : cudaEventDisableTiming));
+    e.reset(h);
+    return BMSP_OK;
+}
+
+// Facts about the current device, looked up once per device (thread-safe; matrix.cu).  The first lookup on a device also makes its
+// default memory pool keep freed blocks, so that repeated products reuse them without cudaMallocAsync going back to the driver.
+struct DeviceInfo {
+    int32_t sms = 0, cc_major = 0, cc_minor = 0;
+    size_t smem_per_sm = 0;
+    int64_t l2_bytes = 0, hbm_bytes = 0;
+};
+int current_device(const DeviceInfo** out);
+// Lets kern launch with smem bytes of dynamic shared memory on the current device: raises its limit to max(smem, 48 KB), and with
+// max_carveout prefers the largest shared-memory carveout, when the kernel is first configured on the device and whenever smem is
+// above the limit it already has there.
+int kernel_smem(const void* kern, size_t smem, bool max_carveout);
+
 // A handle under construction: bmsp_destroy frees whatever it holds unless release() handed it to the caller.
 struct HandleDeleter { void operator()(bmsp_matrix_s* m) const { bmsp_destroy(m); } };
 using HandlePtr = std::unique_ptr<bmsp_matrix_s, HandleDeleter>;

@@ -6,6 +6,8 @@
 #include <algorithm>
 #include <cmath>
 #include <cstring>
+#include <mutex>
+#include <unordered_map>
 
 namespace bmsp {
 
@@ -25,17 +27,68 @@ int cuda_fail(cudaError_t e, const char* what, const char* file, int line) {
     return BMSP_ERR_CUDA;
 }
 
-static bool g_pool_ready = false;
+// ------------------------------------------------------------------------------------ per-device state
+// One entry per device index, filled by the first lookup on that device.  The limits of kernel_smem are attributes of the
+// function in that device's context, so they are kept per device too.
+namespace {
+constexpr int MAX_DEVICES = 64;
+struct DeviceEntry {
+    std::once_flag once;
+    cudaError_t err = cudaSuccess;             // of the first lookup: an invalid device or a dead context stays so
+    DeviceInfo info;
+    std::mutex mu;                             // guards smem_limit
+    std::unordered_map<const void*, size_t> smem_limit;   // per configured kernel: its dynamic shared-memory limit
+};
+DeviceEntry g_devices[MAX_DEVICES];
+
+cudaError_t init_device(int dev, DeviceInfo& d) {
+    cudaDeviceProp p;
+    cudaError_t e = cudaGetDeviceProperties(&p, dev);
+    if (e != cudaSuccess) return e;
+    d.sms = p.multiProcessorCount; d.cc_major = p.major; d.cc_minor = p.minor;
+    d.smem_per_sm = p.sharedMemPerMultiprocessor;
+    d.l2_bytes = p.l2CacheSize; d.hbm_bytes = (int64_t)p.totalGlobalMem;
+    cudaMemPool_t pool;
+    if ((e = cudaDeviceGetDefaultMemPool(&pool, dev)) != cudaSuccess) return e;
+    uint64_t thr = UINT64_MAX;
+    return cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr);
+}
+
+int device_entry(DeviceEntry** out) {
+    int dev = 0;
+    BMSP_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= MAX_DEVICES) { set_error("device %d: at most %d devices are supported", dev, MAX_DEVICES); return BMSP_ERR_UNSUPPORTED; }
+    DeviceEntry& e = g_devices[dev];
+    std::call_once(e.once, [&] { e.err = init_device(dev, e.info); });
+    BMSP_CUDA(e.err);
+    *out = &e;
+    return BMSP_OK;
+}
+}  // namespace
+
+int current_device(const DeviceInfo** out) {
+    DeviceEntry* e = nullptr;
+    BMSP_TRY(device_entry(&e));
+    *out = &e->info;
+    return BMSP_OK;
+}
+
+int kernel_smem(const void* kern, size_t smem, bool max_carveout) {
+    DeviceEntry* e = nullptr;
+    BMSP_TRY(device_entry(&e));
+    std::lock_guard<std::mutex> lock(e->mu);
+    const auto it = e->smem_limit.find(kern);
+    if (it != e->smem_limit.end() && it->second >= smem) return BMSP_OK;
+    const size_t limit = std::max<size_t>(smem, 48 * 1024);
+    BMSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit));
+    if (max_carveout) BMSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    e->smem_limit[kern] = limit;
+    return BMSP_OK;
+}
+
 int dev_alloc(void** p, size_t bytes, cudaStream_t st) {
-    if (!g_pool_ready) {
-        int dev = 0;
-        BMSP_CUDA(cudaGetDevice(&dev));
-        cudaMemPool_t pool;
-        BMSP_CUDA(cudaDeviceGetDefaultMemPool(&pool, dev));
-        uint64_t thr = UINT64_MAX;   // keep freed blocks cached: repeated products reuse them without cudaMalloc
-        BMSP_CUDA(cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr));
-        g_pool_ready = true;
-    }
+    const DeviceInfo* d = nullptr;
+    BMSP_TRY(current_device(&d));              // sets up the device's memory pool
     *p = nullptr;
     BMSP_CUDA(cudaMallocAsync(p, bytes + BMSP_PAD_BYTES, st));
     return BMSP_OK;
@@ -180,15 +233,13 @@ int bmsp_abi_version(void) { return BMSP_ABI_VERSION; }
 const char* bmsp_last_error(void) { return g_err.c_str(); }
 
 int bmsp_device_info(int32_t* sm_count, int64_t* l2_bytes, int64_t* hbm_bytes, int32_t* cc_major, int32_t* cc_minor) {
-    int dev = 0;
-    BMSP_CUDA(cudaGetDevice(&dev));
-    cudaDeviceProp p;
-    BMSP_CUDA(cudaGetDeviceProperties(&p, dev));
-    if (sm_count) *sm_count = p.multiProcessorCount;
-    if (l2_bytes) *l2_bytes = p.l2CacheSize;
-    if (hbm_bytes) *hbm_bytes = (int64_t)p.totalGlobalMem;
-    if (cc_major) *cc_major = p.major;
-    if (cc_minor) *cc_minor = p.minor;
+    const DeviceInfo* d = nullptr;
+    BMSP_TRY(current_device(&d));
+    if (sm_count) *sm_count = d->sms;
+    if (l2_bytes) *l2_bytes = d->l2_bytes;
+    if (hbm_bytes) *hbm_bytes = d->hbm_bytes;
+    if (cc_major) *cc_major = d->cc_major;
+    if (cc_minor) *cc_minor = d->cc_minor;
     return BMSP_OK;
 }
 

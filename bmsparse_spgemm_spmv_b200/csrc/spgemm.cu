@@ -1110,7 +1110,7 @@ template <int PASS, int MAXT, bool REUSE = false>
 static int launch_pass_t(const GemmArgs& g, int T, int sms, int nrows, cudaStream_t st) {
     const size_t smem = pass_smem_bytes(PASS, T, g.cap_words, g.cap_c, g.cap_nnz, g.row_list ? 1 : g.group);
     auto kern = spgemm_pass_kernel<PASS, MAXT, REUSE>;
-    BMSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
+    BMSP_TRY(kernel_smem((const void*)kern, smem, false));
     int occ = 0;
     BMSP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, T, smem));
     if (occ < 1) { set_error("spgemm pass %d does not fit: smem %zu", PASS, smem); return BMSP_ERR_CUDA; }
@@ -1130,14 +1130,9 @@ struct RowSplit {
     bool active = false;
     DevBuf<int32_t> list;          // heavy rows (descending weight) then light rows (ascending index)
     int n_heavy = 0, n_light = 0;
-    cudaStream_t side = nullptr;
-    cudaEvent_t fork = nullptr, join = nullptr;
+    Stream side;
+    Event fork, join;
     size_t heavy_scratch_off = 0;  // words: the heavy launch's slice of g_bitset / g_wrank
-    ~RowSplit() {                  // the body runs before `list` is freed
-        if (side) { cudaStreamSynchronize(side); cudaStreamDestroy(side); }
-        if (fork) cudaEventDestroy(fork);
-        if (join) cudaEventDestroy(join);
-    }
 };
 
 template <int PASS, bool REUSE = false>
@@ -1151,12 +1146,12 @@ static int launch_pass(GemmArgs& g, int T, int sms, cudaStream_t st, const RowSp
     gh.row_list = sp.list.get(); gh.n_list = sp.n_heavy; gh.work_counter = g.work_counter + 1; gh.G = 32; gh.batch = 1;
     if (g.g_bitset) { gh.g_bitset = g.g_bitset + sp.heavy_scratch_off; gh.g_wrank = g.g_wrank + sp.heavy_scratch_off; }
     gl.row_list = sp.list.get() + sp.n_heavy; gl.n_list = sp.n_light;
-    BMSP_CUDA(cudaEventRecord(sp.fork, st));
-    BMSP_CUDA(cudaStreamWaitEvent(sp.side, sp.fork, 0));
-    BMSP_TRY((launch_pass_t<PASS, 1024, REUSE>(gh, 1024, sms, sp.n_heavy, sp.side)));
+    BMSP_CUDA(cudaEventRecord(sp.fork.get(), st));
+    BMSP_CUDA(cudaStreamWaitEvent(sp.side.get(), sp.fork.get(), 0));
+    BMSP_TRY((launch_pass_t<PASS, 1024, REUSE>(gh, 1024, sms, sp.n_heavy, sp.side.get())));
     if (sp.n_light > 0) BMSP_TRY((launch_pass_t<PASS, 256, REUSE>(gl, T, sms, sp.n_light, st)));
-    BMSP_CUDA(cudaEventRecord(sp.join, sp.side));
-    BMSP_CUDA(cudaStreamWaitEvent(st, sp.join, 0));
+    BMSP_CUDA(cudaEventRecord(sp.join.get(), sp.side.get()));
+    BMSP_CUDA(cudaStreamWaitEvent(st, sp.join.get(), 0));
     return BMSP_OK;
 }
 
@@ -1192,9 +1187,9 @@ static int plan_rows(const bmsp_matrix_s* A, const bmsp_matrix_s* Bt, int rb, in
     BMSP_TRY(sp.list.alloc((size_t)nrows + 1, st));
     BMSP_CUDA(cudaMemcpyAsync(sp.list.get(), order.data(), sizeof(int32_t) * (size_t)nrows, cudaMemcpyHostToDevice, st));
     BMSP_CUDA(cudaStreamSynchronize(st));       // `order` dies with this scope
-    BMSP_CUDA(cudaStreamCreateWithFlags(&sp.side, cudaStreamNonBlocking));
-    BMSP_CUDA(cudaEventCreateWithFlags(&sp.fork, cudaEventDisableTiming));
-    BMSP_CUDA(cudaEventCreateWithFlags(&sp.join, cudaEventDisableTiming));
+    BMSP_TRY(new_stream(sp.side));
+    BMSP_TRY(new_event(sp.fork));
+    BMSP_TRY(new_event(sp.join));
     sp.active = sp.n_heavy > 0;
     return BMSP_OK;
 }
@@ -1402,18 +1397,13 @@ static int spgemm_run(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts*
     const int nrows = re - rb;
     const bool verbose = opts && opts->verbose;
 
-    int dev = 0;
-    int& sms = s.sms;
-    BMSP_CUDA(cudaGetDevice(&dev));
-    BMSP_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const DeviceInfo* dev = nullptr;
+    BMSP_TRY(current_device(&dev));
+    const int sms = s.sms = dev->sms;
 
-    struct Timing {
-        cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};   // start, after FILL, end, after COUNT
-        ~Timing() { for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e); }
-    } t;
-    cudaEvent_t* ev = t.ev;
-    if (verbose) for (int i = 0; i < 4; i++) BMSP_CUDA(cudaEventCreate(&ev[i]));
-    if (verbose) BMSP_CUDA(cudaEventRecord(ev[0], st));
+    Event ev[4];                 // start, after FILL, end, after COUNT
+    if (verbose) for (Event& e : ev) BMSP_TRY(new_event(e, true));
+    if (verbose) BMSP_CUDA(cudaEventRecord(ev[0].get(), st));
 
     // ---- scratch
     s.nrows = nrows;
@@ -1469,7 +1459,7 @@ static int spgemm_run(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts*
         BMSP_CUDA(cudaStreamSynchronize(st));
         c_size = tot[0]; n_surv = tot[1];
     }
-    if (verbose) BMSP_CUDA(cudaEventRecord(ev[3], st));
+    if (verbose) BMSP_CUDA(cudaEventRecord(ev[3].get(), st));
     if (c_size > 0x7FFFFFFFll || h.surviving > 0xFFFFFFFFull) {
         set_error("product too large for one call: %lld C blocks, %llu surviving pairs (shard A's block rows with brow_begin/brow_end)",
                   (long long)c_size, h.surviving);
@@ -1507,24 +1497,24 @@ static int spgemm_run(bmsp_matrix_t A, bmsp_matrix_t Bt, const bmsp_spgemm_opts*
     if (c_nnz > 0xFFFFFFFFull) { set_error("C has %llu values (> 2^32-1)", (unsigned long long)c_nnz); return BMSP_ERR_TOO_LARGE; }
     C->nnz = (int64_t)c_nnz;
     BMSP_TRY(dev_alloc(&C->values, (size_t)c_nnz * 4 + 16, st));
-    if (verbose) BMSP_CUDA(cudaEventRecord(ev[1], st));
+    if (verbose) BMSP_CUDA(cudaEventRecord(ev[1].get(), st));
 
     g.c_val = (float*)C->values;
     if (c_nnz > 0) BMSP_TRY(run_numeric(g, C, h, plan, path, sp, nrows, sms, st));
     finish_rows_kernel<<<(unsigned)ceil_div(C->nbr + 1, 256), 256, 0, st>>>(row_count, row_nnz, rb, re, C->nbr, C->brp, C->rvb, C->offsets, c_size, c_nnz);
     BMSP_KERNEL_CHECK();
-    if (verbose) BMSP_CUDA(cudaEventRecord(ev[2], st));
+    if (verbose) BMSP_CUDA(cudaEventRecord(ev[2].get(), st));
 
     if (info) {
         memset(info, 0, sizeof(*info));
         info->candidate_pairs = (int64_t)h.sum_cand; info->surviving_pairs = (int64_t)h.surviving;
         info->c_blocks = c_size; info->c_nnz = (int64_t)c_nnz; info->numeric_path = path;
         if (verbose) {
-            BMSP_CUDA(cudaEventSynchronize(ev[2]));
-            cudaEventElapsedTime(&info->symbolic_ms, ev[0], ev[1]);
-            cudaEventElapsedTime(&info->numeric_ms, ev[1], ev[2]);
-            cudaEventElapsedTime(&info->count_ms, ev[0], ev[3]);
-            cudaEventElapsedTime(&info->fill_ms, ev[3], ev[1]);
+            BMSP_CUDA(cudaEventSynchronize(ev[2].get()));
+            cudaEventElapsedTime(&info->symbolic_ms, ev[0].get(), ev[1].get());
+            cudaEventElapsedTime(&info->numeric_ms, ev[1].get(), ev[2].get());
+            cudaEventElapsedTime(&info->count_ms, ev[0].get(), ev[3].get());
+            cudaEventElapsedTime(&info->fill_ms, ev[3].get(), ev[1].get());
             info->total_ms = info->symbolic_ms + info->numeric_ms;
         }
     }

@@ -1094,7 +1094,6 @@ __global__ void __launch_bounds__(256) spmv_blockpar_kernel(const uint64_t* __re
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int item = blockIdx.x * 8 + wid;
     if (item >= n_work) return;
-    const bool active = true;
     const int4 w = work[item];
     float (*acc)[32] = s_acc[wid];
 #pragma unroll
@@ -1182,7 +1181,7 @@ __global__ void __launch_bounds__(256) spmv_blockpar_kernel(const uint64_t* __re
         for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
         if (lane == r) res = v;
     }
-    if (lane < 8 && active) {
+    if (lane < 8) {
         if (w.w) partial[(int64_t)item * 8 + lane] = res;
         else {
             const int64_t row = (int64_t)w.x * 8 + lane;
@@ -1267,28 +1266,18 @@ static int env_int(const char* name, int dflt) { const char* e = getenv(name); r
 // overlap).  Three streams: s_in feeds x slices (H2D), the caller's stream runs the row-range launches, s_out drains
 // y slices (D2H); PCIe is full duplex, so the step costs max(x, y) bytes over the link instead of their sum.
 struct HostPipe {
-    cudaStream_t s_in = nullptr, s_out = nullptr;
-    cudaEvent_t ev_start = nullptr, ev_done = nullptr;
-    std::vector<cudaEvent_t> ev_x, ev_k;
     DevBuf<char> x_dev;
     DevBuf<float> y_dev;
+    Stream s_in, s_out;
+    Event ev_start, ev_done;
+    std::vector<Event> ev_x, ev_k;
     // the whole pipeline of one (x_host, y_host) pair captured as a CUDA graph: one launch instead of ~7 API calls per chunk
-    cudaStream_t s_cap = nullptr;
-    cudaGraphExec_t gexec = nullptr;
+    Stream s_cap;
+    GraphExec gexec;
     const void* g_x = nullptr; const void* g_y = nullptr; int32_t g_xdt = -1;      // what gexec was captured for
     const void* seen_x = nullptr; const void* seen_y = nullptr; int32_t seen_xdt = -1;   // the previous call's buffers
     std::vector<int> tile_lo;        // [nchunks+1] first tile of every chunk (row-tiled path); {0, 0} for the block-parallel path
     std::vector<int64_t> x_need;     // [nchunks]  columns that must be resident before the chunk runs
-    ~HostPipe() {                    // the body runs before x_dev / y_dev are freed
-        if (s_in) { cudaStreamSynchronize(s_in); cudaStreamDestroy(s_in); }
-        if (s_out) { cudaStreamSynchronize(s_out); cudaStreamDestroy(s_out); }
-        if (s_cap) { cudaStreamSynchronize(s_cap); cudaStreamDestroy(s_cap); }
-        if (gexec) cudaGraphExecDestroy(gexec);
-        if (ev_start) cudaEventDestroy(ev_start);
-        if (ev_done) cudaEventDestroy(ev_done);
-        for (auto e : ev_x) if (e) cudaEventDestroy(e);
-        for (auto e : ev_k) if (e) cudaEventDestroy(e);
-    }
 };
 
 // Everything the first product on a matrix builds (plan_spmv), owned by the handle (bmsp_matrix_s::spmv).  Which members mean
@@ -1317,8 +1306,8 @@ struct SpmvPlan {
     DevBuf<uint32_t> item_ofs;   // [nbr+1] first work item of every block row
     DevBuf<int32_t> split_list;
     DevBuf<float> split_partial;
-    // bmsp_spmv_host's pipeline, built by its first call.  Declared last so that it is destroyed first: its destructor drains the
-    // pipeline's streams before any of the plan's memory is freed.
+    // bmsp_spmv_host's pipeline, built by its first call.  Declared last so that it is destroyed first: the pipeline's streams
+    // drain before any of the plan's memory is freed.
     std::unique_ptr<HostPipe> host;
 };
 
@@ -1475,12 +1464,7 @@ void spmv_release(bmsp_matrix_s* m) { delete m->spmv; m->spmv = nullptr; }
 template <typename T, typename X, int RTT, int MINB, typename H>
 static int launch_tile_kernel(const TileArgs<T>& a, const X* x, float* y, const H& hd, int grid, size_t smem, cudaStream_t st) {
     auto kern = spmv_tile_kernel<T, X, RTT, MINB, H>;
-    static size_t configured = 0;            // per instantiation
-    if (configured < smem || configured == 0) {
-        BMSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
-        BMSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        configured = std::max<size_t>(smem, 1);
-    }
+    BMSP_TRY(kernel_smem((const void*)kern, smem, true));
     kern<<<(unsigned)grid, RTT * 2, smem, st>>>(a, x, y, hd);
     BMSP_KERNEL_CHECK();
     return BMSP_OK;
@@ -1495,16 +1479,8 @@ constexpr int STREAM_DYN_PCT = 25;
 template <typename T, typename X, typename H, bool PAL>
 static int launch_stream_kernel(const TileArgs<T>& a, const X* x, float* y, const H& hd, int ntiles, cudaStream_t st, int32_t* sched) {
     auto kern = spmv_stream_kernel<T, X, H, PAL>;
-    static int sms = 0;
-    static size_t smem_max = 0;
-    if (!sms) {
-        int dev = 0;
-        BMSP_CUDA(cudaGetDevice(&dev));
-        int v = 0;
-        BMSP_CUDA(cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev));
-        smem_max = (size_t)v;
-        BMSP_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    }
+    const DeviceInfo* dev = nullptr;
+    BMSP_TRY(current_device(&dev));
     StreamArgs<T> sa;
     sa.t = a;
     sa.so = stage_layout(a.cap_blk, a.cap_val, a.cap_lines, sizeof(T), sizeof(X), PAL);
@@ -1514,20 +1490,15 @@ static int launch_stream_kernel(const TileArgs<T>& a, const X* x, float* y, cons
     int ctas = 0, spg = 0;
     size_t per_cta = 0;
     for (int c = STREAM_CTAS; c >= 1; c--) {
-        per_cta = std::min<size_t>(smem_max / c - 1024 - 256, 227 * 1024);               // 1 KB per resident CTA is the system's; 256 B allocation granule
+        per_cta = std::min<size_t>(dev->smem_per_sm / c - 1024 - 256, 227 * 1024);   // 1 KB per resident CTA is the system's; 256 B allocation granule
         const int fit = per_cta > fixed ? (int)((per_cta - fixed) / per_stage) : 0;
         if (fit >= 2 || (c == 1 && fit >= 1)) { ctas = c; spg = std::min(fit, 8); break; }
     }
     if (ctas < 1 || spg < 1) { set_error("spmv: a tile stage of %u bytes does not fit shared memory", sa.so.stride); return BMSP_ERR_CUDA; }
     sa.spg = spg;
     const size_t smem = (size_t)spg * per_stage + fixed;
-    static size_t configured = 0;            // per instantiation
-    if (configured < smem || configured == 0) {
-        BMSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
-        BMSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        configured = std::max<size_t>(smem, 1);
-    }
-    const int grid = std::max(1, std::min(ntiles, sms * ctas));
+    BMSP_TRY(kernel_smem((const void*)kern, smem, true));
+    const int grid = std::max(1, std::min(ntiles, dev->sms * ctas));
     const int share = ntiles / grid;
     sa.sched = (sched && share >= 2) ? sched : nullptr;
     sa.n_static = sa.sched ? (int)((int64_t)share * (100 - STREAM_DYN_PCT) / 100) : 0;
@@ -1585,13 +1556,13 @@ constexpr int HOST_CHUNKS = 8;
 static int host_pipe_get(const bmsp_matrix_s* A, SpmvPlan& p, cudaStream_t st) {
     if (p.host) return BMSP_OK;
     std::unique_ptr<HostPipe> hp(new HostPipe());
-    BMSP_CUDA(cudaStreamCreateWithFlags(&hp->s_in, cudaStreamNonBlocking));
-    BMSP_CUDA(cudaStreamCreateWithFlags(&hp->s_out, cudaStreamNonBlocking));
-    BMSP_CUDA(cudaEventCreateWithFlags(&hp->ev_start, cudaEventDisableTiming));
-    BMSP_CUDA(cudaEventCreateWithFlags(&hp->ev_done, cudaEventDisableTiming));
+    BMSP_TRY(new_stream(hp->s_in));
+    BMSP_TRY(new_stream(hp->s_out));
+    BMSP_TRY(new_event(hp->ev_start));
+    BMSP_TRY(new_event(hp->ev_done));
     BMSP_TRY(hp->x_dev.alloc((size_t)A->cols * 4 + 256, st));
     BMSP_TRY(hp->y_dev.alloc((size_t)A->rows + 64, st));
-    BMSP_CUDA(cudaStreamCreateWithFlags(&hp->s_cap, cudaStreamNonBlocking));
+    BMSP_TRY(new_stream(hp->s_cap));
     if (p.path == SpmvPlan::ROW_TILED && (int64_t)A->rows * 4 >= (1 << 20)) {
         const int rt = p.tile_rows, ntiles = (int)ceil_div(A->nbr, rt);
         std::vector<TileDesc> desc((size_t)ntiles);
@@ -1614,8 +1585,8 @@ static int host_pipe_get(const bmsp_matrix_s* A, SpmvPlan& p, cudaStream_t st) {
         hp->x_need = {(int64_t)A->cols};
     }
     hp->ev_x.resize(hp->x_need.size()); hp->ev_k.resize(hp->x_need.size());
-    for (auto& e : hp->ev_x) BMSP_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    for (auto& e : hp->ev_k) BMSP_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    for (auto& e : hp->ev_x) BMSP_TRY(new_event(e));
+    for (auto& e : hp->ev_k) BMSP_TRY(new_event(e));
     p.host = std::move(hp);
     return BMSP_OK;
 }
@@ -1636,18 +1607,18 @@ static int spmv_host_run(const bmsp_matrix_s* A, SpmvPlan& p, const void* x_host
     const size_t xs = dtype_bytes(x_dtype);
     float* y_map = p.path == SpmvPlan::ROW_TILED ? mapped_host_ptr(y_host) : nullptr;     // row-tiled kernel only: it stores 512 contiguous bytes per warp
     float* y_out = y_map ? y_map : hp->y_dev.get();
-    BMSP_CUDA(cudaEventRecord(hp->ev_start, st));         // earlier work on st (and the previous call) is done with x_dev / y_dev
-    BMSP_CUDA(cudaStreamWaitEvent(hp->s_in, hp->ev_start, 0));
-    BMSP_CUDA(cudaStreamWaitEvent(hp->s_out, hp->ev_start, 0));
+    BMSP_CUDA(cudaEventRecord(hp->ev_start.get(), st));         // earlier work on st (and the previous call) is done with x_dev / y_dev
+    BMSP_CUDA(cudaStreamWaitEvent(hp->s_in.get(), hp->ev_start.get(), 0));
+    BMSP_CUDA(cudaStreamWaitEvent(hp->s_out.get(), hp->ev_start.get(), 0));
     int64_t sent = 0;
     const int64_t rows_per_tile = (int64_t)p.tile_rows * 8;
     for (int c = 0; c < (int)hp->x_need.size(); c++) {
         const int64_t need = hp->x_need[c];
         if (need > sent) {
             BMSP_CUDA(cudaMemcpyAsync(hp->x_dev.get() + sent * xs, (const char*)x_host + sent * xs, (size_t)(need - sent) * xs,
-                                      cudaMemcpyHostToDevice, hp->s_in));
-            BMSP_CUDA(cudaEventRecord(hp->ev_x[c], hp->s_in));
-            BMSP_CUDA(cudaStreamWaitEvent(st, hp->ev_x[c], 0));
+                                      cudaMemcpyHostToDevice, hp->s_in.get()));
+            BMSP_CUDA(cudaEventRecord(hp->ev_x[c].get(), hp->s_in.get()));
+            BMSP_CUDA(cudaStreamWaitEvent(st, hp->ev_x[c].get(), 0));
             sent = need;
         }
         int64_t row0 = 0, row1 = A->rows;
@@ -1662,13 +1633,13 @@ static int spmv_host_run(const bmsp_matrix_s* A, SpmvPlan& p, const void* x_host
             return launch_spmv<T, X>(A, p, (const X*)hp->x_dev.get(), y_out, st, t0, nt);
         }));
         if (row1 > row0 && !y_map) {
-            BMSP_CUDA(cudaEventRecord(hp->ev_k[c], st));
-            BMSP_CUDA(cudaStreamWaitEvent(hp->s_out, hp->ev_k[c], 0));
-            BMSP_CUDA(cudaMemcpyAsync(y_host + row0, hp->y_dev.get() + row0, (size_t)(row1 - row0) * 4, cudaMemcpyDeviceToHost, hp->s_out));
+            BMSP_CUDA(cudaEventRecord(hp->ev_k[c].get(), st));
+            BMSP_CUDA(cudaStreamWaitEvent(hp->s_out.get(), hp->ev_k[c].get(), 0));
+            BMSP_CUDA(cudaMemcpyAsync(y_host + row0, hp->y_dev.get() + row0, (size_t)(row1 - row0) * 4, cudaMemcpyDeviceToHost, hp->s_out.get()));
         }
     }
-    BMSP_CUDA(cudaEventRecord(hp->ev_done, hp->s_out));
-    BMSP_CUDA(cudaStreamWaitEvent(st, hp->ev_done, 0));   // the caller synchronises `st` as for bmsp_spmv
+    BMSP_CUDA(cudaEventRecord(hp->ev_done.get(), hp->s_out.get()));
+    BMSP_CUDA(cudaStreamWaitEvent(st, hp->ev_done.get(), 0));   // the caller synchronises `st` as for bmsp_spmv
     return BMSP_OK;
 }
 
@@ -1685,18 +1656,20 @@ static int spmv_host_graph(const bmsp_matrix_s* A, SpmvPlan& p, const void* x_ho
         cudaPointerAttributes ax, ay;
         if (cudaPointerGetAttributes(&ax, x_host) != cudaSuccess || cudaPointerGetAttributes(&ay, y_host) != cudaSuccess ||
             ax.type != cudaMemoryTypeHost || ay.type != cudaMemoryTypeHost) { cudaGetLastError(); return BMSP_OK; }   // pageable: eager only
-        if (hp->gexec) { cudaGraphExecDestroy(hp->gexec); hp->gexec = nullptr; }
+        hp->gexec.reset();
         cudaGraph_t graph = nullptr;
-        BMSP_CUDA(cudaStreamBeginCapture(hp->s_cap, cudaStreamCaptureModeThreadLocal));
-        const int rc = spmv_host_run<T>(A, p, x_host, x_dtype, y_host, hp->s_cap);
-        const cudaError_t ce = cudaStreamEndCapture(hp->s_cap, &graph);
+        BMSP_CUDA(cudaStreamBeginCapture(hp->s_cap.get(), cudaStreamCaptureModeThreadLocal));
+        const int rc = spmv_host_run<T>(A, p, x_host, x_dtype, y_host, hp->s_cap.get());
+        const cudaError_t ce = cudaStreamEndCapture(hp->s_cap.get(), &graph);
         if (rc != BMSP_OK || ce != cudaSuccess || !graph) { cudaGetLastError(); if (graph) cudaGraphDestroy(graph); return BMSP_OK; }
-        const cudaError_t ie = cudaGraphInstantiate(&hp->gexec, graph, 0);
+        cudaGraphExec_t ge = nullptr;
+        const cudaError_t ie = cudaGraphInstantiate(&ge, graph, 0);
         cudaGraphDestroy(graph);
-        if (ie != cudaSuccess) { cudaGetLastError(); hp->gexec = nullptr; return BMSP_OK; }
+        if (ie != cudaSuccess) { cudaGetLastError(); return BMSP_OK; }
+        hp->gexec.reset(ge);
         hp->g_x = x_host; hp->g_y = y_host; hp->g_xdt = x_dtype;
     }
-    BMSP_CUDA(cudaGraphLaunch(hp->gexec, st));
+    BMSP_CUDA(cudaGraphLaunch(hp->gexec.get(), st));
     *used = true;
     return BMSP_OK;
 }

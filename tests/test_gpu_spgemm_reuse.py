@@ -183,6 +183,7 @@ def test_cuda_graph_replay(B, oracle, monkeypatch, case):
     A = B.bmSpMatrix.from_csr(*sh, *a); Bt = B.bmSpMatrix.from_csr(*sh, *a, transpose=True)
     plan = B.bmSparse_mult_plan(A, Bt)
     s = torch.cuda.Stream()
+    s.wait_stream(torch.cuda.current_stream())      # the plan's first NUMERIC pass, enqueued by its creation, makes C's offsets absolute
     with torch.cuda.stream(s):
         plan.numeric()
     s.synchronize()
