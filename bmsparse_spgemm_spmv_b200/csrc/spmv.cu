@@ -1829,3 +1829,41 @@ extern "C" int bmsp_spmv_bytes(bmsp_matrix_t A, int32_t x_dtype, int64_t* bytes)
              (int64_t)A->rows * 4;
     return BMSP_OK;
 }
+
+extern "C" int bmsp_debug_spmv_plan(bmsp_matrix_t A, bmsp_spmv_plan_info* out, void* stream) {
+    if (!A || !out) { set_error("bmsp_debug_spmv_plan: null argument"); return BMSP_ERR_INVALID; }
+    if (A->transposed || A->rows == 0) { set_error("bmsp_debug_spmv_plan: the matrix is transposed or empty"); return BMSP_ERR_UNSUPPORTED; }
+    cudaStream_t st = (cudaStream_t)stream;
+    touch(A, st);
+    BMSP_TRY(plan_spmv(A, st));
+    const SpmvPlan& p = *A->spmv;
+    memset(out, 0, sizeof(*out));
+    if (p.path == SpmvPlan::BLOCK_PARALLEL) {
+        out->path = 1;
+        out->n_work = p.n_work; out->n_split_rows = p.n_split_rows;
+        std::vector<int4> work((size_t)p.n_work);
+        if (p.n_work > 0) BMSP_CUDA(cudaMemcpyAsync(work.data(), p.work.get(), sizeof(int4) * work.size(), cudaMemcpyDeviceToHost, st));
+        BMSP_CUDA(cudaStreamSynchronize(st));
+        for (const int4& w : work) out->n_bundles += w.w == 2;
+        return BMSP_OK;
+    }
+    out->kernel = p.kernel; out->tile_rows = p.tile_rows; out->npal = p.npal;
+    out->cap_blk = p.cap_blk; out->cap_val = p.cap_val; out->cap_lines = p.cap_lines;
+    const int ntiles = out->ntiles = (int)ceil_div(A->nbr, p.tile_rows);
+    std::vector<TileDesc> desc((size_t)ntiles);
+    BMSP_CUDA(cudaMemcpyAsync(desc.data(), p.desc.get(), sizeof(TileDesc) * desc.size(), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));
+    for (const TileDesc& d : desc) {
+        out->empty_tiles += d.nb == 0;
+        out->tail_line_tiles += (d.flags & 2) != 0;
+        if (!(d.flags & 1)) {
+            out->unplanned_tiles++;
+            if (d.nb > PLAN_MAXB) out->unplanned_blocks++;
+            else if (d.nl > XL_MAX) out->unplanned_lines++;
+            continue;
+        }
+        out->over_cap_tiles += d.nb > p.cap_blk || d.nv > p.cap_val || d.nl > p.cap_lines;
+        if (d.nb > 0) out->runs[d.nruns]++;
+    }
+    return BMSP_OK;
+}

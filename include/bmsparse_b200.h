@@ -275,6 +275,27 @@ int bmsp_peer_free(void* ptr);
  * SPGEMM.cu:787-810) on n host pairs; used by the parity tests only. */
 int bmsp_debug_pair_bitmap(int64_t n, const uint64_t* a, const uint64_t* bt, uint64_t* out);
 
+/* What the SpMV plan of A chose, and how its tiles and work items fall into the kernels' branches: lets a test assert that its
+ * input reaches the branch it is written for.  Builds the plan (on `stream`) if A has none, then reads it back (synchronises
+ * `stream`).  A must be plain and non-empty.  Used by the tests only. */
+typedef struct {
+    int32_t path;              /* 0 row-tiled, 1 block-parallel                                                  */
+    int32_t kernel;            /* row-tiled: 0 streaming kernel, 1 one CTA per tile                              */
+    int32_t tile_rows, npal;   /* block rows per tile; palette entries (0: no palette)                           */
+    int32_t cap_blk, cap_val, cap_lines;   /* a tile's shared-memory capacities: blocks, values, x lines         */
+    int32_t ntiles;
+    int32_t empty_tiles;       /* tiles without blocks                                                           */
+    int32_t unplanned_tiles;   /* tiles the planner left to global memory: ...                                   */
+    int32_t unplanned_blocks;  /*   ... because they have more blocks than it sorts (2048)                       */
+    int32_t unplanned_lines;   /*   ... because they touch more x lines than it offsets (1900)                   */
+    int32_t over_cap_tiles;    /* planned tiles above a capacity: read from global memory too                    */
+    int32_t tail_line_tiles;   /* tiles whose last x line reaches past the last column (guarded load)            */
+    int32_t runs[4];           /* non-empty planned tiles by runs of consecutive x lines (runs[0]: more than 3)  */
+    int32_t n_work, n_bundles, n_split_rows;   /* block-parallel: work items, bundles of four short block rows,
+                                                  block rows sliced into several items                          */
+} bmsp_spmv_plan_info;
+int bmsp_debug_spmv_plan(bmsp_matrix_t A, bmsp_spmv_plan_info* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
