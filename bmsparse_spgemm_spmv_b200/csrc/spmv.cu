@@ -728,7 +728,8 @@ __global__ void __launch_bounds__(RTT * 2, MINB) spmv_tile_kernel(const TileArgs
             half_block_row<T, X>(a.bmps, a.bcol, a.values, (int)pb, (int)pe, kv, h, x, acc);
         }
         float* yr = y + row;
-        if (row + 4 <= a.rows) *reinterpret_cast<float4*>(yr) = make_float4(acc[0], acc[1], acc[2], acc[3]);
+        // row <= rows - 4, not row + 4 <= rows: row + 4 overflows int for the last four rows of a matrix of 2^31 - 1 rows
+        if (row <= a.rows - 4) *reinterpret_cast<float4*>(yr) = make_float4(acc[0], acc[1], acc[2], acc[3]);
         else {
 #pragma unroll
             for (int q = 0; q < 4; q++) if (row + q < a.rows) yr[q] = acc[q];
@@ -1054,7 +1055,7 @@ __global__ void __launch_bounds__(32 + STREAM_RT * 2, STREAM_CTAS) spmv_stream_k
                     }
                 }
                 float* yr = y + row;
-                if (row + 4 <= a.rows) *reinterpret_cast<float4*>(yr) = make_float4(acc[0], acc[1], acc[2], acc[3]);
+                if (row <= a.rows - 4) *reinterpret_cast<float4*>(yr) = make_float4(acc[0], acc[1], acc[2], acc[3]);
                 else {
 #pragma unroll
                     for (int q = 0; q < 4; q++) if (row + q < a.rows) yr[q] = acc[q];
