@@ -575,13 +575,14 @@ __device__ __forceinline__ void halo_signal(const HaloDev& h) {
         for (int p = 0; p < h.n_peer; p++) st_release_sys(h.peer_flag[p], h.signal_epoch);
     }
 }
-// rows [row, row + 4) of y (row a multiple of 4; the ragged tail stops at `rows`) to every peer range that contains them
+// rows [row, row + 4) of y (row a multiple of 4; the ragged tail stops at `rows`) to every peer range that contains them.
+// Compared as row <= hi - 4, not row + 4 <= hi: row + 4 overflows int for the last quad of a matrix of 2^31 - 1 rows.
 __device__ __forceinline__ void halo_store(const HaloDev& h, int row, int rows, const float (&acc)[4]) {
     for (int i = 0; i < h.n_push; i++) {
         const int lo = h.lo[i], hi = h.hi[i];
-        if (row >= hi || row + 4 <= lo) continue;
+        if (row >= hi || row <= lo - 4) continue;
         float* d = h.dst[i] + (row - lo);
-        if (row >= lo && row + 4 <= hi && row + 4 <= rows) {
+        if (row >= lo && row <= hi - 4 && row <= rows - 4) {
             *reinterpret_cast<float4*>(d) = make_float4(acc[0], acc[1], acc[2], acc[3]);
         } else {
 #pragma unroll
@@ -596,18 +597,23 @@ __global__ void halo_wait_kernel(const HaloDev h) {
 // stand-alone push (first exchange after set_x, and products that run the block-parallel kernel): every thread reads four rows of y
 // once and stores them to every peer range that contains them -- 16-byte stores, 512 contiguous bytes per warp and peer, all
 // peers' links busy at the same time (for a scattered matrix every peer needs the whole slice: an all-gather written by the owner)
+// The loop counter is 64-bit: a range that ends at 2^31 - 1 would step an int counter past INT_MAX, and with no range at all
+// (lo_all = INT_MAX) the first row would already overflow.  Inside the loop r < hi_all <= rows fits in int; the quad tests
+// compare against hi - 4 and rows - 4 for the same reason as halo_store.
 __global__ void __launch_bounds__(256) halo_push_kernel(const float* __restrict__ y, int rows, const HaloDev h) {
     int lo_all = 0x7FFFFFFF, hi_all = 0;
     for (int i = 0; i < h.n_push; i++) { lo_all = min(lo_all, h.lo[i]); hi_all = max(hi_all, h.hi[i]); }
-    for (int r = lo_all + 4 * (int)(blockIdx.x * blockDim.x + threadIdx.x); r < hi_all; r += 4 * (int)(gridDim.x * blockDim.x)) {
+    const int64_t step = 4 * (int64_t)(gridDim.x * blockDim.x);
+    for (int64_t r64 = lo_all + 4 * (int64_t)(blockIdx.x * blockDim.x + threadIdx.x); r64 < hi_all; r64 += step) {
+        const int r = (int)r64;
         float v[4];
-        if (r + 4 <= rows) { const float4 t = *reinterpret_cast<const float4*>(y + r); v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w; }
+        if (r <= rows - 4) { const float4 t = *reinterpret_cast<const float4*>(y + r); v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w; }
         else { for (int q = 0; q < 4; q++) v[q] = r + q < rows ? y[r + q] : 0.f; }
         for (int i = 0; i < h.n_push; i++) {
             const int lo = h.lo[i], hi = h.hi[i];
-            if (r >= hi || r + 4 <= lo) continue;
+            if (r >= hi || r <= lo - 4) continue;
             float* d = h.dst[i] + (r - lo);
-            if (r >= lo && r + 4 <= hi) *reinterpret_cast<float4*>(d) = make_float4(v[0], v[1], v[2], v[3]);
+            if (r >= lo && r <= hi - 4) *reinterpret_cast<float4*>(d) = make_float4(v[0], v[1], v[2], v[3]);
             else { for (int q = 0; q < 4; q++) if (r + q >= lo && r + q < hi) d[q] = v[q]; }
         }
     }
@@ -663,7 +669,9 @@ __global__ void __launch_bounds__(RTT * 2, MINB) spmv_tile_kernel(const TileArgs
     }
     bool part = false;               // DIST: this tile owns rows a peer needs (CTA-uniform)
     if constexpr (DIST) {
-        const int trow0 = r0 * 8, trow1 = min(a.rows, (r0 + nrow) * 8);
+        // trow1 in 64 bits: (r0 + nrow) * 8 is 2^31 for the last tile of a matrix of 2^31 - 1 rows
+        const int trow0 = r0 * 8;
+        const int64_t trow1 = min((int64_t)a.rows, (int64_t)(r0 + nrow) * 8);
         part = t == hd.solo_tile;
         for (int i = 0; i < hd.n_push; i++) part |= hd.lo[i] < trow1 && hd.hi[i] > trow0;
         // A tile depends on the peers when its x lines leave this rank's own columns (it reads rows they pushed) or when it
@@ -1703,6 +1711,9 @@ static int halo_to_dev(const bmsp_halo_desc* d, int rows, HaloDev* h) {
     if (!d || d->n_push < 0 || d->n_push > HALO_MAX || d->n_peer < 0 || d->n_peer > HALO_MAX || (d->n_peer > 0 && !d->scratch)) {
         set_error("halo descriptor: bad counts or missing scratch"); return BMSP_ERR_INVALID;
     }
+    // n_peer is the union of both directions: a rank that pushes rows has at least the peers it pushes to.  Without this check
+    // such a descriptor would silently push nothing (bmsp_spmv_halo takes the plain product, bmsp_halo_push returns at once).
+    if (d->n_push > 0 && d->n_peer == 0) { set_error("halo descriptor: push ranges without peers"); return BMSP_ERR_INVALID; }
     memset(h, 0, sizeof(*h));
     h->n_push = 0; h->n_peer = d->n_peer; h->scratch = (uint32_t*)d->scratch; h->solo_tile = -1;
     h->own_c0 = d->own_col_lo; h->own_c1 = d->own_col_hi;
@@ -1722,7 +1733,7 @@ static int halo_to_dev(const bmsp_halo_desc* d, int rows, HaloDev* h) {
 using namespace bmsp;
 
 extern "C" int bmsp_halo_push(const float* y_own, int32_t rows, const bmsp_halo_desc* halo, uint32_t signal_epoch, void* stream) {
-    if (!y_own) { set_error("bmsp_halo_push: null vector"); return BMSP_ERR_INVALID; }
+    if (!y_own && rows > 0) { set_error("bmsp_halo_push: null vector"); return BMSP_ERR_INVALID; }
     HaloDev h;
     BMSP_TRY(halo_to_dev(halo, rows, &h));
     if (h.n_peer == 0) return BMSP_OK;
@@ -1748,7 +1759,8 @@ extern "C" int bmsp_halo_status(const bmsp_halo_desc* halo, void* stream, int32_
 
 extern "C" int bmsp_spmv_halo(bmsp_matrix_t A, const float* x_ext, float* y_own, const bmsp_halo_desc* halo, uint32_t wait_epoch,
                               uint32_t signal_epoch, void* stream) {
-    if (!A || !x_ext || !y_own) { set_error("bmsp_spmv_halo: null argument"); return BMSP_ERR_INVALID; }
+    // a rank that owns no rows (an empty shard) reads and writes no vector: its x and y may be empty tensors (null pointers)
+    if (!A || (A->rows > 0 && (!x_ext || !y_own))) { set_error("bmsp_spmv_halo: null argument"); return BMSP_ERR_INVALID; }
     if (A->transposed) { set_error("bmsp_spmv_halo: matrix is in transposed-operand form"); return BMSP_ERR_UNSUPPORTED; }
     if (((uintptr_t)x_ext & 15) || ((uintptr_t)y_own & 15)) { set_error("bmsp_spmv_halo: x and y must be 16-byte aligned"); return BMSP_ERR_INVALID; }
     cudaStream_t st = (cudaStream_t)stream;
@@ -1756,7 +1768,9 @@ extern "C" int bmsp_spmv_halo(bmsp_matrix_t A, const float* x_ext, float* y_own,
     HaloDev h;
     BMSP_TRY(halo_to_dev(halo, A->rows, &h));
     h.wait_epoch = wait_epoch; h.signal_epoch = signal_epoch;
-    if (A->rows == 0 || h.n_peer == 0) return A->rows == 0 ? BMSP_OK : bmsp_spmv(A, x_ext, BMSP_F32, y_own, stream);
+    // no rows: nothing to wait for or push, but the peers wait for this rank's epoch
+    if (A->rows == 0) return h.n_peer == 0 ? BMSP_OK : bmsp_halo_push(y_own, 0, halo, signal_epoch, stream);
+    if (h.n_peer == 0) return bmsp_spmv(A, x_ext, BMSP_F32, y_own, stream);
     BMSP_TRY(plan_spmv(A, st));
     SpmvPlan& p = *A->spmv;
     if (p.path == SpmvPlan::ROW_TILED) {

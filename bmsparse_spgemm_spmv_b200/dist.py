@@ -50,6 +50,26 @@ def csr_row_slice(rp, ci, v, r0, r1):
     return (np.asarray(rp[r0:r1 + 1]) - s).astype(np.int32), ci[s:e], v[s:e]
 
 
+def halo_ranges(rank, bounds, ranges):
+    """The range halo of one rank: (recv, send), lists of (peer, a, b) global rows [a, b).  What I receive from peer p: the
+    overlap of my extended range with p's owned rows; what I send to p: the overlap of p's extended range with my owned rows.
+    bounds: the global row split (len world + 1); ranges[p] = (ext_lo, ext_hi) of every rank, mine included."""
+    own_lo, own_hi = int(bounds[rank]), int(bounds[rank + 1])
+    ext_lo, ext_hi = ranges[rank]
+    recv, send = [], []
+    for p in range(len(ranges)):
+        if p == rank:
+            continue
+        plo, phi = int(bounds[p]), int(bounds[p + 1])
+        a, b = max(ext_lo, plo), min(ext_hi, phi)
+        if a < b:
+            recv.append((p, a, b))
+        a, b = max(ranges[p][0], own_lo), min(ranges[p][1], own_hi)
+        if a < b:
+            send.append((p, a, b))
+    return recv, send
+
+
 class ShardedSpMV:
     """y = A x with A sharded by rows and x sharded the same way (square matrices).
 
@@ -78,18 +98,7 @@ class ShardedSpMV:
         allr = [torch.zeros_like(mine) for _ in range(self.world)]
         dist.all_gather(allr, mine, group=group)
         ranges = [tuple(int(t) for t in a.cpu()) for a in allr]
-        # what I receive from peer p: overlap(my ext range, p's owned range); what I send: the mirror image
-        self.recv, self.send = [], []
-        for p in range(self.world):
-            if p == self.rank:
-                continue
-            plo, phi = int(self.bounds[p]), int(self.bounds[p + 1])
-            a, b = max(self.ext_lo, plo), min(self.ext_hi, phi)
-            if a < b:
-                self.recv.append((p, a, b))
-            a, b = max(ranges[p][0], self.own_lo), min(ranges[p][1], self.own_hi)
-            if a < b:
-                self.send.append((p, a, b))
+        self.recv, self.send = halo_ranges(self.rank, self.bounds, ranges)
         n_ext = self.ext_hi - self.ext_lo
         self.cur = 0
         self.x = None
@@ -230,8 +239,17 @@ def halo_descriptor(buf, rank, send, peers, own_lo, own_hi, ext_lo, my_base, pee
     return d
 
 
+def halo_peers(recv, send, world, inbox=1024):
+    """the ranks one rank exchanges epochs with (both directions, sorted); RuntimeError when one halo descriptor cannot hold them"""
+    from . import _lib as L
+    peers = sorted({p for p, _, _ in send} | {p for p, _, _ in recv})
+    if len(peers) > L.HALO_MAX or len(send) > L.HALO_MAX or world > inbox // 4:
+        raise RuntimeError("too many peers for one halo descriptor")
+    return peers
+
+
 class PeerHalo:
-    """Peer-mapped ping-pong x buffers + epoch inbox of one rank, and the bmsp_halo_desc of each buffer.
+    """Three rotating peer-mapped x buffers + epoch inbox of one rank, and the bmsp_halo_desc of each buffer.
 
     Region layout (one cudaMalloc per rank, exported as a CUDA IPC handle and opened by the ranks that talk to it):
         [0, 1024)            inbox: uint32 epoch slot per source rank
@@ -257,9 +275,7 @@ class PeerHalo:
         self.base = None
         ok = True
         try:
-            peers = sorted({p for p, _, _ in sh.send} | {p for p, _, _ in sh.recv})
-            if len(peers) > L.HALO_MAX or len(sh.send) > L.HALO_MAX or sh.world > cls.INBOX // 4:
-                raise RuntimeError("too many peers for one halo descriptor")
+            peers = halo_peers(sh.recv, sh.send, sh.world, cls.INBOX)
             stride = (n_ext * 4 + 255) // 256 * 256
             base = C.c_void_p(); handle = (C.c_ubyte * 64)()
             L.check(L.lib().bmsp_peer_alloc(C.c_int64(cls.INBOX + cls.NBUF * stride), C.byref(base), handle))

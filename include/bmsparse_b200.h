@@ -239,12 +239,17 @@ int bmsp_slice_block_rows(bmsp_matrix_t A, int32_t brow_begin, int32_t brow_end,
                           void* stream, bmsp_matrix_t* out);
 
 /* Multi-GPU SpMV with the halo exchange over peer memory (NVLink P2P stores), fused into the product.
- * Every rank owns a contiguous row range, keeps x for the columns it touches ("extended range") in two
- * peer-mapped ping-pong buffers and an inbox of epoch flags (bmsp_peer_alloc / bmsp_peer_open).  One step:
+ * Every rank owns a contiguous row range, keeps x for the columns it touches ("extended range") in three
+ * rotating peer-mapped buffers and an inbox of epoch flags (bmsp_peer_alloc / bmsp_peer_open).  One step:
  *   bmsp_spmv_halo(A_local, x_ext[cur], own slice of x_ext[nxt], desc[nxt], e, e + 1, stream)
  * waits (in the kernel) until every peer published epoch e, computes y, stores the rows each peer needs straight
  * into that peer's x_ext[nxt] and publishes epoch e + 1.  No NCCL call, no extra launch (row-tiled kernel; the
- * block-parallel kernel uses a wait and a push kernel around the product). */
+ * block-parallel kernel uses a wait and a push kernel around the product).  Three buffers, not two: a peer may
+ * write the next-but-one buffer while this rank's kernel still reads the current one.
+ * Descriptor rules (BMSP_ERR_INVALID otherwise): n_push and n_peer in [0, BMSP_HALO_MAX]; every push range
+ * 0 <= lo <= hi <= rows with lo a multiple of 4 and a 16-byte aligned push_dst; scratch set when n_peer > 0;
+ * n_push > 0 only with n_peer > 0 (n_peer counts every peer of both directions, so it includes each peer
+ * pushed to).  An empty range (lo == hi) pushes nothing.  With n_peer == 0 the call is the plain product. */
 #define BMSP_HALO_MAX 8
 typedef struct {
     int32_t n_push;                      /* row ranges of my y that some peer needs                          */

@@ -32,6 +32,7 @@ import torch
 
 from tests.test_gpu_device_memory import USED_MEM_CURRENT, USED_MEM_HIGH, _Pool, pool  # noqa: F401
 from tests.test_gpu_spmv_exact import PAD, SENTINEL, plan_info
+from tests.test_gpu_spmv_halo import Halo, _halo_push, _spmv_halo
 
 pytestmark = pytest.mark.gpu
 
@@ -616,8 +617,9 @@ def _few_blocks(rows, cols, br, bc, bmps, value=_val16):
     return Spec(rows, cols, keys[o], bm, offsets, value, F16)
 
 
-def _sparse_check(B, M, spec, x, n_out, transpose=False):
-    """y = M x over n_out rows (up to 2^31 - 1): the rows the reference touches equal it, every other row is 0"""
+def _sparse_check(B, M, spec, x, n_out, transpose=False, run=None):
+    """y = M x over n_out rows (up to 2^31 - 1): the rows the reference touches equal it, every other row is 0.  run(M, x, y) computes
+    the product (default bmSparse_SpMV).  Returns the touched rows and their float64 values."""
     rows, vals = [], []
     for r, v, va in _ref_parts(spec, x, transpose):
         keep = (r >= 0) & (r < n_out)
@@ -627,12 +629,13 @@ def _sparse_check(B, M, spec, x, n_out, transpose=False):
     ref = torch.zeros(rows.numel(), dtype=torch.float64, device="cuda").index_add_(0, inv, torch.cat(vals))
     ybuf = _y_buffer(n_out)
     y = ybuf[PAD:PAD + n_out]
-    B.bmSparse_SpMV(M, x, y)
+    (run or B.bmSparse_SpMV)(M, x, y)
     got = y[rows].double()
     assert torch.equal(got, ref), f"touched rows differ: {got[got != ref][:4].tolist()} vs {ref[got != ref][:4].tolist()}"
     nz = int(torch.count_nonzero(y))          # NaN counts as nonzero: a row left unwritten shows up here
     assert nz == int(torch.count_nonzero(ref)), f"{nz} nonzero rows, expected {int(torch.count_nonzero(ref))}"
     assert bool((ybuf[:PAD] == SENTINEL).all()) and bool((ybuf[PAD + n_out:] == SENTINEL).all())
+    return rows, ref
 
 
 ROWS7 = 0xFFFFFFFFFFFFFF00          # rows 0 .. 6 of a block
@@ -699,3 +702,70 @@ def test_block_parallel_past_2_31(B):
     assert plan_info(M).path == 1
     x = _small_x(64, F16, seed=11)
     _spmv_exact(B, M, x, _ref_spmv(spec, x, spec.rows), "block-parallel")
+
+
+# ---------------------------------------------------------------------------------------------------------------- 8: halo paths at 2^31 - 1 rows
+class _Rows:
+    """y over [0, n) given by its nonzero rows: a slice [lo:hi] is the dense float64 rows lo .. hi - 1"""
+
+    def __init__(self, rows, vals):
+        self.rows, self.vals = rows.cpu().numpy(), vals.cpu().numpy()
+
+    def __getitem__(self, s):
+        out = np.zeros(s.stop - s.start)
+        m = (self.rows >= s.start) & (self.rows < s.stop)
+        out[self.rows[m] - s.start] = self.vals[m]
+        return out
+
+
+def _tall_ranges(last):
+    """rows [0, 8), a range around the middle block row, and the last 1001 rows up to 2^31 - 1"""
+    mid = (last // 2) * 8
+    return [(0, 8), ((mid - 12) & ~3, mid + 21), ((INT32_MAX - 1001) & ~3, INT32_MAX)]
+
+
+@pytest.mark.parametrize("kernel", ["streaming", "per_tile", "block_parallel"])
+def test_halo_product_at_int32_rows(B, monkeypatch, kernel):
+    """bmsp_spmv_halo on a matrix of 2^31 - 1 rows with blocks in block row 0, in the middle block row and in the last, partial
+    block row; push ranges [0, 8), one around the middle block row and one ending at 2^31 - 1, each into a guarded sink.  y is
+    checked as _sparse_check does; the sinks, their guards, the peer slots and scratch as test_gpu_spmv_halo does.  The streaming
+    kernel, the per-tile kernel (BMSP_SPMV_KERNEL=1) and the block-parallel path (one or two cells per block: wait kernel, product,
+    push kernel)"""
+    last = (INT32_MAX + 7) // 8 - 1
+    _need(INT32_MAX * 6 + (last + 1) * 32 + 2 * GB, "vectors of 2^31 - 1 elements")
+    if kernel == "block_parallel":
+        bmps = [(1 << 63) | (1 << 54), 1 << 43, (1 << 15) | (1 << 8), 1 << 13]
+    else:
+        bmps = [FULL, 0x8000000000000001, ROWS7, ROWS7 & 0x5A5A5A5A5A5A5A5A]
+    spec = _few_blocks(INT32_MAX, 16, [0, last // 2, last, last], [1, 0, 0, 1], bmps)
+    M = _build(B, spec)
+    if kernel == "per_tile":
+        monkeypatch.setenv("BMSP_SPMV_KERNEL", "1")
+    info = plan_info(M)
+    monkeypatch.delenv("BMSP_SPMV_KERNEL", raising=False)
+    assert (info.path, info.kernel if info.path == 0 else -1) == {"streaming": (0, 0), "per_tile": (0, 1), "block_parallel": (1, -1)}[kernel]
+    x = _small_x(16, F32, seed=12)
+    h = Halo(_tall_ranges(last), (0, 16))
+    from bmsparse_spgemm_spmv_b200 import _lib as L
+    run = lambda M, x, y: L.check(_spmv_halo(M, x.data_ptr(), y.data_ptr(), h.desc, 1, 2))
+    rows, ref = _sparse_check(B, M, spec, x, INT32_MAX, run=run)
+    torch.cuda.synchronize()
+    h.check(_Rows(rows, ref), 2, kernel)
+
+
+def test_halo_push_at_int32_rows(B):
+    """bmsp_halo_push with rows = 2^31 - 1: a range ending at 2^31 - 1 (the push loop's last rows) next to [0, 8), and no range at
+    all with peers (the loop must skip its body and still signal)"""
+    _need(INT32_MAX * 4 + 2 * GB, "y of 2^31 - 1 elements")
+    y = torch.empty(INT32_MAX, device="cuda")            # only the pushed rows are read
+    lo = (INT32_MAX - 1001) & ~3
+    vals = {0: torch.arange(1, 9, dtype=torch.float64), lo: -torch.arange(1, INT32_MAX - lo + 1, dtype=torch.float64)}
+    for a, v in vals.items():
+        y[a:a + v.numel()] = v.float().cuda()
+    yref = _Rows(torch.cat([torch.arange(a, a + v.numel()) for a, v in vals.items()]), torch.cat(list(vals.values())))
+    for ranges, epoch in (([(lo, INT32_MAX), (0, 8)], 3), ([], 4)):
+        h = Halo(ranges, (0, 16))
+        from bmsparse_spgemm_spmv_b200 import _lib as L
+        L.check(_halo_push(y.data_ptr(), INT32_MAX, h.desc, epoch))
+        torch.cuda.synchronize()
+        h.check(yref, epoch, f"{len(ranges)} ranges")
