@@ -60,7 +60,7 @@ SYMBOLS = ["bmsp_abi_version", "bmsp_last_error", "bmsp_device_info", "bmsp_crea
            "bmsp_partition_block_rows", "bmsp_slice_block_rows", "bmsp_debug_pair_bitmap", "bmsp_spmv_halo", "bmsp_halo_push",
            "bmsp_halo_status", "bmsp_peer_alloc", "bmsp_peer_open", "bmsp_peer_close", "bmsp_peer_free", "bmsp_set_values",
            "bmsp_set_values_csr", "bmsp_spgemm_plan_create", "bmsp_spgemm_numeric", "bmsp_spgemm_plan_bytes", "bmsp_spgemm_plan_destroy",
-           "bmsp_matrix_transpose", "bmsp_add", "bmsp_debug_spmv_plan"]
+           "bmsp_matrix_transpose", "bmsp_add", "bmsp_debug_spmv_plan", "bmsp_debug_spmv_shapes"]
 
 _lib = None
 

@@ -129,12 +129,13 @@ enum : uint32_t { PAL_DIAG = 1u << 8, PAL_TRI = 1u << 9, PAL_SINGLE = 1u << 10, 
 struct PalScan { unsigned long long key[PAL_GSLOTS]; uint32_t count, has_zero, overflow, pad; };
 
 __device__ __forceinline__ uint32_t pal_hash(uint64_t b, int bits) { return (uint32_t)((b * 0x9E3779B97F4A7C15ull) >> (64 - bits)); }
-// insert the non-zero bitmap b: 1 = inserted, 0 = already present, -1 = table full
-__device__ __forceinline__ int pal_insert(unsigned long long* tab, int bits, uint64_t b) {
+// insert the non-zero key b: 1 = inserted, 0 = already present, -1 = table full; *at = its slot
+__device__ __forceinline__ int pal_insert(unsigned long long* tab, int bits, uint64_t b, uint32_t* at = nullptr) {
     const uint32_t mask = (1u << bits) - 1u;
     uint32_t i = pal_hash(b, bits);
     for (uint32_t n = 0; n <= mask; n++, i = (i + 1u) & mask) {
         unsigned long long cur = *reinterpret_cast<volatile unsigned long long*>(tab + i);
+        if (at) *at = i;
         if (cur == b) return 0;
         if (cur == 0ull) {
             cur = atomicCAS(tab + i, 0ull, (unsigned long long)b);
@@ -264,6 +265,119 @@ __global__ void __launch_bounds__(256) tile_plan_kernel(const int32_t* __restric
     }
 }
 
+// ---- row shapes (streaming kernel with a palette) ----
+// On a stencil or band matrix the block words of a block row repeat from row to row once the x offset is taken relative to the row:
+// a block column c of block row lbr in a tile whose lines are consecutive sits at x offset 8 c - 32 (first line), so xo - 8 lbr is
+// the same for every interior row (P4096: 14 distinct rows in all 32 768 tiles).  When the staged rows of a matrix have at most
+// SHAPE_MAX distinct such sequences ("shapes"), the streaming kernel keeps them in one table in shared memory next to the palette
+// and streams no block words: a row's 4-byte word names its shape instead of its first block.
+//   shape word  = x offset - 8 lbr + SHAPE_BIAS (bits 0-15) | palette entry byte offset (bits 16-31), as in `word`.  The bias keeps
+//                 the field positive: a row can touch a line that lies before the lines of the tile's earlier rows (xo < 8 lbr), and
+//                 xo + SHAPE_BIAS - 8 lbr lies in [8, 61304] for every planned tile (xo < XL_MAX * 32, lbr < 64).
+//   row word    = shape's first word in the table (bits 0-10) | its block count (bits 11-15) | first value relative to the tile
+//                 (bits 16-31, as in `rowrel`).  An empty row is {0, 0}.
+// The consumer moves its staged-x base by (8 lbr - SHAPE_BIAS) elements and walks the shape with tile_half_row_pal unchanged.
+constexpr int SHAPE_MAX = 128;         // distinct shapes per matrix
+constexpr int SHAPE_NB = 31;           // blocks per shape (5-bit count)
+constexpr int SHAPE_WORDS = 1024;      // words in the table (4 KB of shared memory per CTA at most)
+constexpr uint32_t SHAPE_BIAS = 512;   // > 8 * (STREAM_RT - 1)
+constexpr int SHP_SLOTS = 512, SHP_GSLOTS = 1024;   // open-addressing tables of row hashes: per CTA (shared) and per matrix (global)
+struct ShapeScan { unsigned long long key[SHP_GSLOTS]; uint32_t rep[SHP_GSLOTS]; uint32_t count, overflow, nout, pad; };
+
+__device__ __forceinline__ uint32_t shape_word(uint32_t w, int lbr) { return (w & 0xFFFF0000u) | ((w & 0xFFFFu) + SHAPE_BIAS - 8u * (uint32_t)lbr); }
+__device__ __forceinline__ unsigned long long shape_hash(const uint32_t* __restrict__ w, int nb, int lbr) {
+    unsigned long long h = 0x243F6A8885A308D3ull ^ (uint32_t)nb;
+    for (int i = 0; i < nb; i++) { h = (h ^ shape_word(__ldg(w + i), lbr)) * 0x9E3779B97F4A7C15ull; h ^= h >> 29; }
+    return h | 1ull;
+}
+// the rows of a tile the streaming kernel stages (the test of its producer); the others read brp / bcol / bmps from global memory
+__device__ __forceinline__ bool shape_row_staged(const TileDesc* __restrict__ desc, int r, int cb, int cv, int cl) {
+    const int4 d0 = __ldg(reinterpret_cast<const int4*>(desc + r / 64)), d1 = __ldg(reinterpret_cast<const int4*>(desc + r / 64) + 1);
+    return (d1.y & 1) && d0.y <= cb && d0.w <= cv && d1.x <= cl;
+}
+
+// One pass over the staged block rows: every CTA collects the hashes of its distinct non-empty shapes (and one row of each) in
+// shared memory, then merges them into the global table; gives up (overflow) as soon as a table holds more than SHAPE_MAX or a row
+// has more than SHAPE_NB blocks.  Two shapes with one hash become one entry here: shape_assign_kernel compares every row's words.
+__global__ void __launch_bounds__(256) shape_scan_kernel(const int32_t* __restrict__ brp, const uint32_t* __restrict__ word,
+                                                         const TileDesc* __restrict__ desc, int nbr, int cb, int cv, int cl,
+                                                         ShapeScan* __restrict__ ss) {
+    __shared__ unsigned long long s_tab[SHP_SLOTS];
+    __shared__ uint32_t s_rep[SHP_SLOTS];
+    __shared__ uint32_t s_cnt, s_over;
+    const int tid = threadIdx.x;
+    for (int i = tid; i < SHP_SLOTS; i += 256) s_tab[i] = 0ull;
+    if (tid == 0) { s_cnt = 0; s_over = 0; }
+    __syncthreads();
+    // as palette_scan_kernel: the table never holds more than SHAPE_MAX + 256 < SHP_SLOTS keys
+    uint32_t it = 0;
+    for (int r = blockIdx.x * 256 + tid; r < nbr; r += gridDim.x * 256, it++) {
+        if (*reinterpret_cast<volatile uint32_t*>(&s_cnt) > (uint32_t)SHAPE_MAX) break;
+        if ((it & 15u) == 0 && *reinterpret_cast<volatile uint32_t*>(&ss->overflow)) break;
+        if (!shape_row_staged(desc, r, cb, cv, cl)) continue;
+        const int p = __ldg(brp + r), nb = __ldg(brp + r + 1) - p;
+        if (nb == 0) continue;
+        if (nb > SHAPE_NB) { s_over = 1; break; }
+        uint32_t at = 0;
+        const int res = pal_insert(s_tab, 9, shape_hash(word + p, nb, r & 63), &at);
+        if (res > 0) { s_rep[at] = (uint32_t)r; atomicAdd(&s_cnt, 1u); }
+        else if (res < 0) { s_over = 1; break; }
+    }
+    __syncthreads();
+    if (s_over || s_cnt > (uint32_t)SHAPE_MAX) { if (tid == 0) atomicExch(&ss->overflow, 1u); return; }
+    for (int j = tid; j < SHP_SLOTS; j += 256) {
+        const uint64_t k = s_tab[j];
+        if (k == 0ull) continue;
+        if (*reinterpret_cast<volatile uint32_t*>(&ss->overflow)) break;
+        uint32_t at = 0;
+        const int res = pal_insert(ss->key, 10, k, &at);
+        if (res > 0) ss->rep[at] = s_rep[j];
+        if (res < 0 || (res > 0 && atomicAdd(&ss->count, 1u) >= (uint32_t)SHAPE_MAX)) { atomicExch(&ss->overflow, 1u); break; }
+    }
+}
+
+// the words of every shape, from the row the scan kept for it: out[k] = {global slot | block count << 16, words ...}
+__global__ void shape_gather_kernel(const int32_t* __restrict__ brp, const uint32_t* __restrict__ word, ShapeScan* __restrict__ ss,
+                                    uint32_t* __restrict__ out) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= SHP_GSLOTS || ss->overflow || ss->key[j] == 0ull) return;
+    const uint32_t k = atomicAdd(&ss->nout, 1u);
+    if (k >= (uint32_t)SHAPE_MAX) return;
+    const int r = (int)ss->rep[j], p = brp[r], nb = brp[r + 1] - p;
+    uint32_t* o = out + (size_t)k * (SHAPE_NB + 1);
+    o[0] = (uint32_t)j | (uint32_t)nb << 16;
+    for (int i = 0; i < nb; i++) o[1 + i] = shape_word(word[p + i], r & 63);
+}
+
+// Row words of the shape layout (into srow; rowrel stays as it is).  Exactness does not rest on the hash: every staged row's words
+// are compared with the words of the shape its hash names, and any difference -- or a hash the table does not hold -- sets *bad,
+// which keeps the matrix in the word layout.
+__global__ void __launch_bounds__(256) shape_assign_kernel(const int32_t* __restrict__ brp, const uint32_t* __restrict__ word,
+                                                           const uint32_t* __restrict__ rowrel, const TileDesc* __restrict__ desc,
+                                                           int nbr, int cb, int cv, int cl, const unsigned long long* __restrict__ gkey,
+                                                           const uint32_t* __restrict__ gval, const uint32_t* __restrict__ table,
+                                                           uint32_t* __restrict__ srow, uint32_t* __restrict__ bad) {
+    const int r = blockIdx.x * 256 + threadIdx.x;
+    if (r >= nbr) return;
+    uint32_t f = 0;
+    if (shape_row_staged(desc, r, cb, cv, cl)) {
+        const int p = __ldg(brp + r), nb = __ldg(brp + r + 1) - p;
+        if (nb > SHAPE_NB) { atomicExch(bad, 1u); return; }
+        if (nb > 0) {
+            const unsigned long long k = shape_hash(word + p, nb, r & 63);
+            uint32_t i = pal_hash(k, 10), n = 0;
+            while (n < SHP_GSLOTS && gkey[i] != k && gkey[i] != 0ull) { i = (i + 1u) & (SHP_GSLOTS - 1); n++; }
+            if (n == SHP_GSLOTS || gkey[i] != k) { atomicExch(bad, 1u); return; }
+            f = gval[i];
+            const uint32_t* s = table + (f & 0x7FFu);
+            bool same = (int)(f >> 11) == nb;
+            for (int b = 0; b < nb && same; b++) same = __ldg(s + b) == shape_word(__ldg(word + p + b), r & 63);
+            if (!same) { atomicExch(bad, 1u); return; }
+        }
+    }
+    srow[r] = f | (rowrel[r] & 0xFFFF0000u);
+}
+
 // shared-memory carve-up of spmv_tile_kernel (cap_blk and cap_val are multiples of 8); computed on the host
 struct TileSmem { uint32_t xo, val, row, xs, bar, total; };
 inline TileSmem tile_smem(int rt, int cap_blk, int cap_val, int cap_lines, int vsize, int xsize) {
@@ -282,6 +396,7 @@ struct TileArgs {
     const uint64_t* bmps; const int32_t* bcol; const T* values; const int2* rowpair;   // rowpair[r] = (block_row_ptr[r], first value of row r)
     const TileDesc* desc; const uint32_t* lines; const uint16_t* xoff;
     const uint32_t* word; const uint32_t* rowrel; const uint4* palette; int32_t npal;   // streaming kernel with a palette (tile_plan_kernel)
+    int32_t shape_words;                                                                 // ... and row shapes: table words behind the palette
     const int32_t* brp; const uint32_t* rvb;                                             // ... whose unstaged tiles read their row pointers here
     int32_t rows, nbr, cols, cap_blk, cap_val, cap_lines;
     int32_t tile0;       // first tile of this launch (row-range launches of the host-buffer pipeline)
@@ -772,16 +887,18 @@ __global__ void __launch_bounds__(RTT * 2, MINB) spmv_tile_kernel(const TileArgs
 // Several groups with a producer each per CTA were slower than one group per CTA (P4096: 6 groups x 1 CTA 69.7 us, 1 x 7 67.8 us).
 constexpr int STREAM_RT = 64;      // block rows per tile
 constexpr int STREAM_CTAS = 7;     // CTAs per SM the kernel's registers must allow (P4096: 7 x 2 stages, the measured optimum)
+static_assert(STREAM_RT == 64 && SHAPE_BIAS > 8u * (STREAM_RT - 1), "row shapes: 64-row tiles (r & 63), positive biased x offsets");
 // pal: the palette variant -- a 32-byte header (the second 16 bytes: the tile's block and value counts as the last row's end), one
-// 32-bit word per block in place of bitmaps and x offsets (`bm`; `xo` unused), 4-byte relative row pairs
+// 32-bit word per block in place of bitmaps and x offsets (`bm`; `xo` unused), 4-byte relative row pairs; shp: the palette variant
+// with row shapes -- no block words at all
 struct StageLayout { uint32_t bm, xo, val, row, xs, stride; };
-inline StageLayout stage_layout(int cap_blk, int cap_val, int cap_lines, int vsize, int xsize, bool pal) {
+inline StageLayout stage_layout(int cap_blk, int cap_val, int cap_lines, int vsize, int xsize, bool pal, bool shp) {
     constexpr uint32_t rt = STREAM_RT;
     auto up16 = [](uint32_t v) { return (v + 15u) & ~15u; };
     StageLayout s;
     if (pal) {
         s.bm = 32;
-        s.xo = s.val = up16(s.bm + (uint32_t)(cap_blk + 4) * 4);
+        s.xo = s.val = shp ? s.bm : up16(s.bm + (uint32_t)(cap_blk + 4) * 4);
         s.row = up16(s.val + (uint32_t)(cap_val + 16) * vsize);
         s.xs = up16(s.row + (rt + 4) * 4);
     } else {
@@ -834,9 +951,11 @@ __device__ __noinline__ void halo_push_tile(const HaloDev* hd, int row, int rows
 }
 
 // PAL: the matrix has a bitmap palette (see palette_scan_kernel); it is loaded once per CTA, behind the descriptor ring.
-template <typename T, typename X, typename H = NoHalo, bool PAL = false>
+// SHP (with PAL): row shapes (see shape_scan_kernel); their table follows the palette in the same buffer and the same bulk copy.
+template <typename T, typename X, typename H = NoHalo, bool PAL = false, bool SHP = false>
 __global__ void __launch_bounds__(32 + STREAM_RT * 2, STREAM_CTAS) spmv_stream_kernel(const __grid_constant__ StreamArgs<T> sa, const X* __restrict__ x,
                                                                                     float* __restrict__ y, const __grid_constant__ H hd) {
+    static_assert(PAL || !SHP, "row shapes come with a palette");
     constexpr bool DIST = !std::is_same<H, NoHalo>::value;
     constexpr int GT = STREAM_RT * 2;      // consumer threads: two per block row
     constexpr int VA = 16 / sizeof(T);
@@ -860,8 +979,9 @@ __global__ void __launch_bounds__(32 + STREAM_RT * 2, STREAM_CTAS) spmv_stream_k
     __syncthreads();
     if constexpr (PAL) {
         if (tid == 0) {
-            mbar_arrive_expect_tx(pal_bar, (uint32_t)a.npal * 16u);
-            bulk_g2s(smem + pal_off + 16, a.palette, (uint32_t)a.npal * 16u, pal_bar);
+            const uint32_t nbytes = (uint32_t)a.npal * 16u + (SHP ? (uint32_t)a.shape_words * 4u : 0u);    // shape_words: a multiple of 4
+            mbar_arrive_expect_tx(pal_bar, nbytes);
+            bulk_g2s(smem + pal_off + 16, a.palette, nbytes, pal_bar);
         }
     }
     const int grid = (int)gridDim.x;
@@ -942,7 +1062,8 @@ __global__ void __launch_bounds__(32 + STREAM_RT * 2, STREAM_CTAS) spmv_stream_k
             uint32_t n8 = 0, n2 = 0, nvb = 0;
             int nlc = 0;                                                  // x lines that arrive by bulk copy
             if (staged && nb > 0) {
-                if constexpr (PAL) n8 = (uint32_t)((p0 + nb - p0a + 3) & ~3) * 4;
+                if constexpr (SHP) {}                                     // no block words: the shapes are in shared memory
+                else if constexpr (PAL) n8 = (uint32_t)((p0 + nb - p0a + 3) & ~3) * 4;
                 else {
                     n8 = (uint32_t)((p0 + nb - p0a + 1) & ~1) * 8;
                     n2 = (uint32_t)((p0 + nb - p0x + 7) & ~7) * 2;
@@ -1021,6 +1142,7 @@ __global__ void __launch_bounds__(32 + STREAM_RT * 2, STREAM_CTAS) spmv_stream_k
         const int gt = tid - 32;
         const int lbr = gt >> 1, h = gt & 1;
         const uint32_t pal_h = sbase + pal_off + 16u + 8u * (uint32_t)h;    // PAL: this half's 8 bytes of entry 0
+        const uint32_t shp_t = sbase + pal_off + 16u + (uint32_t)a.npal * 16u;   // SHP: the shape table
         if constexpr (PAL) mbar_wait(pal_bar, 0);
         int s = 0; uint32_t par = 0;
         for (;;) {
@@ -1036,7 +1158,18 @@ __global__ void __launch_bounds__(32 + STREAM_RT * 2, STREAM_CTAS) spmv_stream_k
             const bool active = lbr < nrow && row < a.rows;
             float acc[4] = {0.f, 0.f, 0.f, 0.f};
             if (active) {
-                if constexpr (PAL) {
+                if constexpr (SHP) {
+                    if (staged) {
+                        // {shape, block count, first value relative to the tile}; the shape's x offsets are relative to this row (biased)
+                        const uint32_t rp = lds_u32(sb + so.row + 4u * lbr);
+                        const uint32_t a_v = sb + so.val + ((uint32_t)hdr.y - v0a + (rp >> 16)) * (uint32_t)sizeof(T);
+                        const uint32_t xs31 = sb + so.xs + (31u + 8u * (uint32_t)lbr - SHAPE_BIAS) * SX;
+                        tile_half_row_pal<T, X>(shp_t + (rp & 0x7FFu) * 4u, pal_h, a_v, (int)((rp >> 11) & 31u), h, xs31, acc);
+                    } else {
+                        const int br = r0 + lbr;
+                        half_block_row<T, X>(a.bmps, a.bcol, a.values, __ldg(a.brp + br), __ldg(a.brp + br + 1), __ldg(a.rvb + br), h, x, acc);
+                    }
+                } else if constexpr (PAL) {
                     if (staged) {
                         // (first block, first value) of this block row and of the next one, relative to the tile; the tile's counts end the last row
                         const uint32_t rp = lds_u32(sb + so.row + 4u * lbr);
@@ -1305,9 +1438,12 @@ struct SpmvPlan {
     DevBuf<int2> rowpair;        // no palette: [nbr+1] (block_row_ptr, first value) zipped for one bulk copy per tile
     // streaming kernel, matrices with at most PALETTE_MAX distinct bitmaps (stencils, bands): the bitmaps are replaced by a palette
     // and xoff / rowpair by word / rowrel ("bitmap palette")
-    DevBuf<uint4> palette;       // [npal] 16-byte entries, sorted by bitmap
-    DevBuf<uint32_t> word;       // [nblk] per block: x offset (bits 0-15) | palette entry byte offset (bits 16-31)
+    DevBuf<uint4> palette;       // [npal] 16-byte entries, sorted by bitmap (row shapes: then the shape table, shape_words words)
+    DevBuf<uint32_t> word;       // [nblk] per block: x offset (bits 0-15) | palette entry byte offset (bits 16-31); freed with shapes
     DevBuf<uint32_t> rowrel;     // [nbr] per block row: (first block - tile's first block) | (first value - tile's first value) << 16
+                                 // (row shapes: {shape, block count} in bits 0-15, see shape_scan_kernel)
+    bool shapes = false;         // palette matrices whose staged rows have at most SHAPE_MAX distinct shapes ("row shapes")
+    int32_t nshapes = 0, shape_words = 0;   // shapes; table words, padded to a multiple of 4 (one bulk copy with the palette)
     // block-parallel path (plan_block_parallel): n_work int4 work items; the block rows sliced into several items are listed for
     // the fix-up kernel, which sums their items' row sums (split_partial, allocated only when there are such rows)
     int32_t n_work = 0, n_split_rows = 0;
@@ -1357,6 +1493,70 @@ static int build_palette(const bmsp_matrix_s* m, int vsize, cudaStream_t st, std
     }
     BMSP_TRY(palette.alloc(pal.size(), st));
     BMSP_CUDA(cudaMemcpyAsync(palette.get(), pal.data(), sizeof(uint4) * pal.size(), cudaMemcpyHostToDevice, st));
+    return BMSP_OK;
+}
+
+// Row shapes of a palette matrix (layout at shape_scan_kernel): collect them on the device, sort them here and lay them out behind
+// the palette, then rewrite the row words and compare every staged row with its shape.  The word layout stays when the matrix has
+// more than SHAPE_MAX shapes or SHAPE_WORDS words in all, a staged row has more than SHAPE_NB blocks, or a row differs from the
+// shape of its hash.  Otherwise the per-block words are freed.
+static int build_shapes(const bmsp_matrix_s* m, SpmvPlan& p, cudaStream_t st) {
+    const int nbr = m->nbr, cb = p.cap_blk, cv = p.cap_val, cl = p.cap_lines, npal = p.npal;
+    constexpr int OUTW = SHAPE_NB + 1;
+    DevBuf<ShapeScan> ss;
+    DevBuf<uint32_t> out;
+    BMSP_TRY(ss.alloc(1, st));
+    BMSP_TRY(out.alloc((size_t)SHAPE_MAX * OUTW, st));
+    BMSP_CUDA(cudaMemsetAsync(ss.get(), 0, sizeof(ShapeScan), st));
+    const int grid = (int)std::min<int64_t>(1024, std::max<int64_t>(1, ceil_div(nbr, 256 * 8)));
+    shape_scan_kernel<<<grid, 256, 0, st>>>(m->brp, p.word.get(), p.desc.get(), nbr, cb, cv, cl, ss.get());
+    BMSP_KERNEL_CHECK();
+    shape_gather_kernel<<<SHP_GSLOTS / 256, 256, 0, st>>>(m->brp, p.word.get(), ss.get(), out.get());
+    BMSP_KERNEL_CHECK();
+    uint32_t cnt[3];                                     // count, overflow, nout
+    std::vector<uint32_t> h((size_t)SHAPE_MAX * OUTW);
+    BMSP_CUDA(cudaMemcpyAsync(cnt, &ss.get()->count, sizeof(cnt), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaMemcpyAsync(h.data(), out.get(), sizeof(uint32_t) * h.size(), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));
+    out.reset();
+    if (cnt[1] || cnt[2] > (uint32_t)SHAPE_MAX) return BMSP_OK;
+    const int ns = (int)cnt[2];
+    std::vector<std::vector<uint32_t>> shp((size_t)ns);
+    std::vector<int> order((size_t)ns);
+    for (int k = 0; k < ns; k++) {
+        const uint32_t* o = h.data() + (size_t)k * OUTW;
+        shp[k].assign(o + 1, o + 1 + (o[0] >> 16));
+        order[k] = k;
+    }
+    std::sort(order.begin(), order.end(), [&](int i, int j) { return shp[i] < shp[j]; });
+    std::vector<uint32_t> gval(SHP_GSLOTS, 0u), words;
+    for (const int k : order) {
+        gval[h[(size_t)k * OUTW] & 0xFFFFu] = (uint32_t)words.size() | (uint32_t)shp[k].size() << 11;
+        words.insert(words.end(), shp[k].begin(), shp[k].end());
+    }
+    if (words.size() > (size_t)SHAPE_WORDS) return BMSP_OK;
+    words.resize((words.size() + 3) & ~(size_t)3, 0u);
+    DevBuf<uint4> comb;                                  // palette, then the table: one bulk copy per CTA
+    DevBuf<uint32_t> gv, srow, bad;
+    BMSP_TRY(comb.alloc((size_t)npal + words.size() / 4 + 1, st));
+    BMSP_TRY(gv.alloc(SHP_GSLOTS, st));
+    BMSP_TRY(srow.alloc((size_t)nbr + 8, st));
+    BMSP_TRY(bad.alloc(1, st));
+    BMSP_CUDA(cudaMemcpyAsync(comb.get(), p.palette.get(), sizeof(uint4) * npal, cudaMemcpyDeviceToDevice, st));
+    if (!words.empty())
+        BMSP_CUDA(cudaMemcpyAsync(comb.get() + npal, words.data(), sizeof(uint32_t) * words.size(), cudaMemcpyHostToDevice, st));
+    BMSP_CUDA(cudaMemcpyAsync(gv.get(), gval.data(), sizeof(uint32_t) * SHP_GSLOTS, cudaMemcpyHostToDevice, st));
+    BMSP_CUDA(cudaMemsetAsync(bad.get(), 0, sizeof(uint32_t), st));
+    shape_assign_kernel<<<(unsigned)ceil_div(nbr, 256), 256, 0, st>>>(m->brp, p.word.get(), p.rowrel.get(), p.desc.get(), nbr, cb, cv, cl,
+                                                                      ss.get()->key, gv.get(), reinterpret_cast<const uint32_t*>(comb.get() + npal),
+                                                                      srow.get(), bad.get());
+    BMSP_KERNEL_CHECK();
+    uint32_t hbad = 1;
+    BMSP_CUDA(cudaMemcpyAsync(&hbad, bad.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    BMSP_CUDA(cudaStreamSynchronize(st));                // also the end of the pageable uploads above
+    if (hbad) return BMSP_OK;
+    p.palette = std::move(comb); p.rowrel = std::move(srow); p.word.reset();
+    p.shapes = true; p.nshapes = ns; p.shape_words = (int32_t)words.size();
     return BMSP_OK;
 }
 
@@ -1425,6 +1625,7 @@ static int plan_tiles(const bmsp_matrix_s* m, SpmvPlan& p, cudaStream_t st) {
     // above keeps both far below that already)
     if (use_pal) { cb = std::min(cb, 65528); cv = std::min(cv, 65528); }
     p.cap_blk = cb; p.cap_val = cv; p.cap_lines = std::max(cl, 1); p.tile_rows = rt; p.kernel = kernel;
+    if (use_pal) BMSP_TRY(build_shapes(m, p, st));      // which tiles are staged is known from here on
     return BMSP_OK;
 }
 
@@ -1485,16 +1686,17 @@ static int launch_tile_kernel(const TileArgs<T>& a, const X* x, float* y, const 
 // The last STREAM_DYN_PCT per cent of every CTA's share are claimed at run time (P4096: 0 % 68.6 us, 12-25 % 66.5 us, 50 % 67.6 us,
 // 100 % 75.6 us -- 32 768 atomics on one address are too many).
 constexpr int STREAM_DYN_PCT = 25;
-template <typename T, typename X, typename H, bool PAL>
+template <typename T, typename X, typename H, bool PAL, bool SHP>
 static int launch_stream_kernel(const TileArgs<T>& a, const X* x, float* y, const H& hd, int ntiles, cudaStream_t st, int32_t* sched) {
-    auto kern = spmv_stream_kernel<T, X, H, PAL>;
+    auto kern = spmv_stream_kernel<T, X, H, PAL, SHP>;
     const DeviceInfo* dev = nullptr;
     BMSP_TRY(current_device(&dev));
     StreamArgs<T> sa;
     sa.t = a;
-    sa.so = stage_layout(a.cap_blk, a.cap_val, a.cap_lines, sizeof(T), sizeof(X), PAL);
+    sa.so = stage_layout(a.cap_blk, a.cap_val, a.cap_lines, sizeof(T), sizeof(X), PAL, SHP);
     sa.ntiles = ntiles;
-    const size_t fixed = (size_t)STREAM_DR * 64 + 64 + (PAL ? 16 + (size_t)a.npal * 16 : 0);   // descriptor ring (+ palette)
+    // descriptor ring (+ palette, + shape table)
+    const size_t fixed = (size_t)STREAM_DR * 64 + 64 + (PAL ? 16 + (size_t)a.npal * 16 : 0) + (SHP ? (size_t)a.shape_words * 4 : 0);
     const size_t per_stage = (size_t)sa.so.stride + 16;
     int ctas = 0, spg = 0;
     size_t per_cta = 0;
@@ -1525,7 +1727,7 @@ static int launch_spmv(const bmsp_matrix_s* A, SpmvPlan& p, const X* x, float* y
         a.tile0 = tile0;
         a.bmps = A->bmps; a.bcol = A->bcol; a.values = (const T*)A->values; a.rowpair = p.rowpair.get();
         a.desc = p.desc.get(); a.lines = p.lines.get(); a.xoff = p.xoff.get();
-        a.word = p.word.get(); a.rowrel = p.rowrel.get(); a.palette = p.palette.get(); a.npal = p.npal;
+        a.word = p.word.get(); a.rowrel = p.rowrel.get(); a.palette = p.palette.get(); a.npal = p.npal; a.shape_words = p.shape_words;
         a.brp = A->brp; a.rvb = A->rvb;
         a.rows = A->rows; a.nbr = A->nbr; a.cols = A->cols; a.cap_blk = p.cap_blk; a.cap_val = p.cap_val; a.cap_lines = p.cap_lines;
         const int rt = p.tile_rows;
@@ -1538,8 +1740,9 @@ static int launch_spmv(const bmsp_matrix_s* A, SpmvPlan& p, const X* x, float* y
             // slots in turn (launches on different streams may overlap: they must not share a counter); launches over a tile range
             // (the host-buffer pipeline's chunks) keep static shares.
             int32_t* sched = ntiles < 0 ? p.sched.get() + 2 * (p.sched_next++ % SCHED_SLOTS) : nullptr;
-            if (p.npal > 0) return launch_stream_kernel<T, X, H, true>(a, x, y, hd, grid, st, sched);
-            return launch_stream_kernel<T, X, H, false>(a, x, y, hd, grid, st, sched);
+            if (p.shapes) return launch_stream_kernel<T, X, H, true, true>(a, x, y, hd, grid, st, sched);
+            if (p.npal > 0) return launch_stream_kernel<T, X, H, true, false>(a, x, y, hd, grid, st, sched);
+            return launch_stream_kernel<T, X, H, false, false>(a, x, y, hd, grid, st, sched);
         }
         if (rt == 32) return launch_tile_kernel<T, X, 32, 24, H>(a, x, y, hd, grid, smem, st);
         if (rt == 16) return launch_tile_kernel<T, X, 16, 32, H>(a, x, y, hd, grid, smem, st);
@@ -1880,5 +2083,17 @@ extern "C" int bmsp_debug_spmv_plan(bmsp_matrix_t A, bmsp_spmv_plan_info* out, v
         out->over_cap_tiles += d.nb > p.cap_blk || d.nv > p.cap_val || d.nl > p.cap_lines;
         if (d.nb > 0) out->runs[d.nruns]++;
     }
+    return BMSP_OK;
+}
+
+extern "C" int bmsp_debug_spmv_shapes(bmsp_matrix_t A, int32_t* nshapes, int32_t* nwords, void* stream) {
+    if (!A || !nshapes || !nwords) { set_error("bmsp_debug_spmv_shapes: null argument"); return BMSP_ERR_INVALID; }
+    if (A->transposed || A->rows == 0) { set_error("bmsp_debug_spmv_shapes: the matrix is transposed or empty"); return BMSP_ERR_UNSUPPORTED; }
+    cudaStream_t st = (cudaStream_t)stream;
+    touch(A, st);
+    BMSP_TRY(plan_spmv(A, st));
+    const SpmvPlan& p = *A->spmv;
+    *nshapes = p.shapes ? p.nshapes : -1;
+    *nwords = p.shapes ? p.shape_words : -1;
     return BMSP_OK;
 }

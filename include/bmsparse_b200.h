@@ -301,6 +301,12 @@ typedef struct {
 } bmsp_spmv_plan_info;
 int bmsp_debug_spmv_plan(bmsp_matrix_t A, bmsp_spmv_plan_info* out, void* stream);
 
+/* Whether the SpMV plan of A streams row shapes: the streaming kernel's palette layout in which every block row names one of a
+ * per-matrix table of block-word sequences instead of streaming a word per block.  *nshapes = distinct shapes, *nwords = words of
+ * the table (padded to a multiple of 4); both -1 when the plan uses another layout.  Builds the plan as bmsp_debug_spmv_plan does.
+ * Used by the tests only. */
+int bmsp_debug_spmv_shapes(bmsp_matrix_t A, int32_t* nshapes, int32_t* nwords, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
